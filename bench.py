@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py - throughput of the generation hot path on N B200s of one node, BASELINE.json metric and configs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload W]      # this framework (N > 1: launched by torchrun)
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload W] [--dump-outputs DIR]   # this framework (N > 1: torchrun)
     python bench.py --impl reference [--workload W] [...]                   # the reference's algorithm on the host CPU cores
 
 Workloads (BASELINE.json `configs`; the default is configs[1], the configuration the metric is quoted on):
@@ -65,7 +65,11 @@ def parse():
                          "0 = the workload's default (gen_teacher 2, gen_qa_ppl 3, the tensor-bound ones 1)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-budget-s", type=float, default=150.0, help="wall-clock cap of the reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the results of the last timed step (rank 0) as DIR/<name>.npy, float32 / float64, for comparing two builds")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.batch <= 0:
         a.batch = {"gen_teacher": 64, "gen_qa_ppl": 32, "select_data": 256, "nsp_rank": 40}[a.workload]
     if a.streams <= 0:
@@ -388,6 +392,31 @@ def run_step(a, sl, dev, from_host, to_host):
         return outs
 
 
+# names of the tensors run_step returns, per workload
+OUTPUT_NAMES = {"gen_teacher": ("answers", "abnormal"), "gen_qa_ppl": ("answers", "abnormal", "questions", "answer_ppl"),
+                "select_data": ("answer_ppl",), "nsp_rank": ("nsp_scores",)}
+DUMP_MAX_BYTES = 64 * 10**6
+
+
+def dump_outputs(a, outs, out_dir):
+    """Writes one step's results as <out_dir>/<name>.npy: floating-point results as float32, integer ones (token ids, flags) as
+    float64, which holds them exactly.  Above DUMP_MAX_BYTES in all, a fixed seeded sample of rows (leading dimension, the same
+    rows for every array) is written instead, with their indices as sample_rows.npy."""
+    import numpy as np
+    arrs = {n: o.detach().cpu().numpy().astype(np.float32 if o.is_floating_point() else np.float64)
+            for n, o in zip(OUTPUT_NAMES[a.workload], outs)}
+    total = sum(x.nbytes for x in arrs.values())
+    rows = next(iter(arrs.values())).shape[0]
+    if total > DUMP_MAX_BYTES:
+        keep = max(1, rows * (DUMP_MAX_BYTES - 8 * rows) // total)         # 8 * rows: room for sample_rows
+        idx = np.sort(np.random.default_rng(0).choice(rows, size=keep, replace=False))
+        arrs = {n: x[idx] for n, x in arrs.items()}
+        arrs["sample_rows"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for n, x in arrs.items():
+        np.save(os.path.join(out_dir, f"{n}.npy"), x)
+
+
 def h2d_bytes(a, sl):
     skip = ("image_id", "dec_att_mask", "hist_len_bound")
     return sum(v.numel() * v.element_size() for k, v in sl["host"].items() if k not in skip)
@@ -563,6 +592,8 @@ def main():
     ms, launches, prof, outs, first, _ = timed(False, False, a.steps, False)
     host_issue_ms, host_cpu_ms = host_ms[0], host_ms[1]
     clocks = sampler.stop() if sampler else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a, outs[(a.steps - 1) % S_], a.dump_outputs)      # step i ran on slot i % S_
     # ---- self-check of the timed outputs (a silent garbage path must not print a number) ----
     out0 = outs[0]
     check = {"ids_checksum": _checksum(out0[0]), "finite": True, "in_range": True, "deterministic": None, "varied": True}

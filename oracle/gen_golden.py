@@ -28,6 +28,24 @@ from oracle import ref_shim  # noqa: E402
 from oracle import restatement as R  # noqa: E402
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+PART_BYTES = 960_000        # uncompressed bytes per golden file: keeps every committed file under 1 MB
+
+
+def save_golden(tag: str, out: dict) -> list:
+    """Writes ``out`` as tests/golden/<tag>.npz and, for the arrays that do not fit, <tag>.part2.npz, <tag>.part3.npz, ...
+    (tests/helpers.py:load_golden merges them).  Returns the paths written."""
+    parts, size = [{}], 0
+    for k, v in out.items():
+        if parts[-1] and size + v.nbytes > PART_BYTES:
+            parts.append({})
+            size = 0
+        parts[-1][k] = v
+        size += v.nbytes
+    os.makedirs(GOLDEN, exist_ok=True)
+    paths = [os.path.join(GOLDEN, f"{tag}.npz" if i == 0 else f"{tag}.part{i + 1}.npz") for i in range(len(parts))]
+    for path, part in zip(paths, parts):
+        np.savez_compressed(path, **part)
+    return paths
 
 
 def history_batch(enc_cfg, start, count, rounds=2):
@@ -140,10 +158,8 @@ def run_case(tag, enc_path, dec_path, batch_size, full_dump):
         top = ref_logits.topk(8, dim=-1)
         out["greedy_logits_top_val"] = top.values.numpy(); out["greedy_logits_top_idx"] = top.indices.numpy().astype(np.int32)
         out["greedy_logits_lse"] = torch.logsumexp(ref_logits, -1).numpy()
-    os.makedirs(GOLDEN, exist_ok=True)
-    path = os.path.join(GOLDEN, f"{tag}.npz")
-    np.savez_compressed(path, **out)
-    print(f"[{tag}] wrote {path} ({os.path.getsize(path) / 1e6:.2f} MB)")
+    for path in save_golden(tag, out):
+        print(f"[{tag}] wrote {path} ({os.path.getsize(path) / 1e6:.2f} MB)")
 
 
 def main():

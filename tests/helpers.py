@@ -30,7 +30,13 @@ def history_batch(enc_cfg, start, count, rounds=2):
 
 
 def load_golden(golden_dir, tag):
-    return dict(np.load(os.path.join(golden_dir, f"{tag}.npz")))
+    """Arrays of <tag>.npz and of its continuation files <tag>.part2.npz, ... (oracle/gen_golden.py:save_golden)."""
+    g = dict(np.load(os.path.join(golden_dir, f"{tag}.npz")))
+    i = 2
+    while os.path.exists(os.path.join(golden_dir, f"{tag}.part{i}.npz")):
+        g.update(np.load(os.path.join(golden_dir, f"{tag}.part{i}.npz")))
+        i += 1
+    return g
 
 
 def rel_rms(a: torch.Tensor, ref: torch.Tensor) -> float:

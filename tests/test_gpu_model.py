@@ -663,6 +663,24 @@ def test_evaluate_gen_cli_synthetic(tmp_path):
     assert 0.0 <= m["mrr"] <= 1.0 and 1.0 <= m["mean"] <= 7.0
 
 
+def test_bench_dump_outputs(tmp_path):
+    """bench.py --dump-outputs writes the last timed step's results as .npy files (select_data: the fp32 perplexities); the JSON line
+    reports the requested number of timed steps."""
+    import json
+    import subprocess
+    import sys
+    from helpers import ROOT
+    cmd = [sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "select_data", "--batch", "8", "--steps", "3", "--warmup", "1",
+           "--no-cpu-baseline", "--dump-outputs", str(tmp_path / "out")]
+    r = subprocess.run(cmd, capture_output=True, text=True, timeout=900)
+    assert r.returncode == 0, r.stdout + r.stderr
+    line = json.loads(r.stdout.strip().splitlines()[-1])
+    assert line["steps"] == 3 and line["config"]["output_check"]["deterministic"] is True
+    assert sorted(os.listdir(tmp_path / "out")) == ["answer_ppl.npy"]
+    ppl = np.load(tmp_path / "out" / "answer_ppl.npy")
+    assert ppl.dtype == np.float32 and ppl.shape == (8,) and np.isfinite(ppl).all() and (ppl > 1).all()
+
+
 def test_pair_gemm_encoder_prefill_match_single(full_cfgs, full_sd):
     """Whole encoder, cross-K/V prefill (head-major TMA-store epilogue) and the decode that reads the cache with the CTA-pair GEMM
     forced on every eligible problem against the single-CTA kernel: outputs within bf16 noise, token ids identical."""
