@@ -4,6 +4,7 @@ generate.py: same single-dash flags, same output JSON layout), running on the B2
 
     python generate.py -mode cc12m_gen -start_path_q ckpt_q -start_path_a ckpt_a -cc12m_image_feats ... -save_name out.json
     python generate.py -synthetic 128 -batch_size 64 -num_beams 5          # seeded synthetic images + random weights
+    python generate.py -synthetic 128 -batch_size 64 -num_beams 5 -q_num_beams 5   # beam-searched questions too (4-gram blocked)
 
 Multi-GPU: launch with torchrun (one process per GPU); images are sharded by rank and gathered once at the end.
 The dataset readers (LMDB / tokenizer) of the reference are host I/O outside the hot path: without them (-synthetic)
@@ -79,6 +80,8 @@ def main(argv=None):
     if params['num_beams'] > 1:
         a_kwargs.update(num_beams=params['num_beams'])
     q_kwargs = dict(temperature=0.7, top_k=7, top_p=0.0, ngram_blocking_size=4)
+    if params['q_num_beams'] > 1:
+        q_kwargs.update(num_beams=params['q_num_beams'])
     decode = None
     if params['vocab_file']:
         from transformers import BertTokenizer

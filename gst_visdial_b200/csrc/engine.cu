@@ -331,7 +331,7 @@ void alloc_workspace(gstvd_ctx* c) {
     c->labels.alloc(B * (size_t)c->Ldec_max * 8);
     c->cross_len.alloc(B * 4);
     c->sel_val.alloc(R * kSelMax * 4); c->sel_idx.alloc(R * kSelMax * 4); c->logz.alloc(R * 4);
-    c->ban_tokens.alloc(B * Lt * 4); c->ban_count.alloc(B * 4);
+    c->ban_tokens.alloc(B * K * Lt * 4); c->ban_count.alloc(B * K * 4);   // one ban list per decode row (beam rows included)
     c->hist_ids_own.alloc(B * Lt * 8); c->hist_seg_own.alloc(B * Lt * 8);
     c->r_ids.alloc(B * Lt * 8); c->r_seg.alloc(B * Lt * 8); c->r_att.alloc(B * Lt * 4);
     c->r_feat.alloc(B * Lv * (size_t)c->cfg.v_feature_size * 4); c->r_loc.alloc(B * Lv * 5 * 4); c->r_imask.alloc(B * Lv * 4);
@@ -667,9 +667,16 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     const int nsel = 2 * g.K;
     // bf16: log-sum-exp terms in fp32 (mode 2); the fp32 parity path keeps the fp64 terms of the bit-exact contract (mode 0)
     static const bool exact_lse = getenv("GSTVD_EXACT_LSE") != nullptr;
-    c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, (c->dtype == kBF16 && !exact_lse) ? 2 : 0,
-                                     (const float*)c->beam_scores.p, 1.f, nullptr, nullptr, 0, nsel, sv, si, nullptr, s);
     BeamBuffers bb = beam_buffers(c);
+    const int32_t* bt = nullptr; const int32_t* bc = nullptr;
+    // n-gram blocking: before step n-1 every key still holds the [CLS], which no banned n-gram contains - nothing to launch
+    if (gp.ngram_blocking_size > 0 && step_host >= gp.ngram_blocking_size - 1) {
+      c->launches += launch_beam_ngram_ban(g.B, g.K, g.T, Lh, hist_ids, hist_seg, bb.tokens + (int64_t)(step_host & 1) * M * g.T, step_host,
+                                           gp.ngram_blocking_size, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
+      bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
+    }
+    c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, (c->dtype == kBF16 && !exact_lse) ? 2 : 0,
+                                     (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, nullptr, s);
     c->launches += launch_beam_step(bb, g.B, g.K, g.T, c->V, nsel, sv, si, 102, nullptr, nullptr, nullptr, s);
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
@@ -707,15 +714,14 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* hist
   if (gp.mode == GSTVD_SELECT_BEAM) {
     K = gp.num_beams;
     if (K < 1 || K > c->K_max || 2 * K > kSelMax) throw InvalidArg("generate: num_beams out of range");
-    if (gp.ngram_blocking_size > 0) throw Unsupported("generate: n-gram blocking is only implemented for GSTVD_SELECT_SAMPLE");
   } else if (gp.mode == GSTVD_SELECT_SAMPLE) {
     if (gp.top_k < 0 || gp.top_k > GSTVD_MAX_TOP_K) throw Unsupported("generate: top_k must be 0 (no top-k cut) or in 1..16");
     if (gp.top_k == 0 && c->V > 32768) throw Unsupported("generate: top_k = 0 needs a vocabulary of at most 32768 entries");
     if (!(gp.temperature > 0.f)) throw InvalidArg("generate: temperature must be > 0");
-    if (gp.ngram_blocking_size > 0 && (!hist_ids || !hist_seg || Lh < 1 || Lh > c->Lt_max)) throw InvalidArg("generate: n-gram blocking needs hist_ids / hist_segments");
   } else {
     throw InvalidArg("generate: unknown mode");
   }
+  if (gp.ngram_blocking_size > 0 && (!hist_ids || !hist_seg || Lh < 1 || Lh > c->Lt_max)) throw InvalidArg("generate: n-gram blocking needs hist_ids / hist_segments");
   return K;
 }
 

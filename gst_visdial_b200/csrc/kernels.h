@@ -159,7 +159,8 @@ int launch_reorder_cache(int dtype, const DecodeGeom& g, void* self_cache, const
 constexpr int kSelMax = 16;   // per-row candidates kept (>= 2*max_beams, >= max top_k)
 // Per row: logZ (fp64 accumulate) and the top `nsel` entries of  score_j by (score desc, index asc), where
 //   mode 0 (beam):   score_j = fp32(fp32(x_j - logZ) + row_bias[row])   (mode 2: the same with the exp terms of logZ in fp32)
-//   mode 1 (sample): score_j = x_j / temperature, banned tokens = -inf
+//   mode 1 (sample): score_j = x_j / temperature
+//   banned tokens (every mode) = -inf, applied after the transform: logZ is over the full row
 // logits [rows, ldl] fp32.  ban_tokens [rows, ban_stride] / ban_count [rows] may be null.
 int launch_row_select(int rows, int V, const float* logits, int64_t ldl, int mode, const float* row_bias, float temperature,
                       const int32_t* ban_tokens, const int32_t* ban_count, int ban_stride, int nsel,
@@ -190,6 +191,10 @@ int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, in
 int launch_ngram_ban(int rows, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
                      int prefix_stride, const int* d_step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
                      cudaStream_t stream);
+// the same for the B*K beam rows: key = the last n-1 tokens of beam row b*K+k in `tokens` [B, K, T] (the beam token buffer of
+// this step's parity); history row = b.  Needs n - 1 <= step < T (earlier keys hold the start token and ban nothing).
+int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* tokens, int step,
+                          int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream);
 // sample-mode selection from row_select output; writes seq[row, step] and cur_tokens[row], prefix[row, step+1]
 // top_k == 0: multinomial over the whole (optionally nucleus-filtered) vocabulary; writes the same state as launch_sample_step
 int launch_full_vocab_sample(int rows, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,

@@ -5,7 +5,8 @@
 //   row_select     : replaces torch.topk + masked fill (utils/decoding_utils.py:17-21) and, for beams, the
 //                    log_softmax + top-2K of HF beam_search (absent from the reference; contract in oracle/beam.py)
 //   beam_step/...  : BeamSearchScorer.process / finalize + BeamHypotheses (transformers 4.16.2 semantics)
-//   ngram_ban      : batch_ngram_blocking (utils/decoding_utils.py:38-78) without host round trips
+//   ngram_ban      : batch_ngram_blocking (utils/decoding_utils.py:38-78) without host round trips; beam_ngram_ban: the
+//                    same ban lists for every beam row (contract in oracle/beam_ngram.py)
 //   sample_step    : softmax + multinomial (models/visual_dialog_model.py:106-107), counter-based RNG
 //   ce_loss        : CrossEntropyLoss(ignore_index=0, reduction='none') (models/visual_dialog_decoder.py:70-77)
 //   splice         : generate.py:145-160 and :214-228
@@ -79,15 +80,17 @@ row_select_kernel(int V, const float* __restrict__ logits, int64_t ldl, int mode
 #pragma unroll
     for (int s = 0; s < kSlots; ++s)
       if (tid + s * kSelThreads < V) v[s] = __fdiv_rn(v[s], temperature);
-    const int nb = ban_count ? ban_count[row] : 0;
-    for (int j = 0; j < nb; ++j) {
-      const int w = ban_tokens[(int64_t)row * ban_stride + j];
-      if ((w % kSelThreads) == tid) {
-        const int slot = w / kSelThreads;
+  }
+  // banned tokens -> -inf after the transform: in beam mode logZ stays over the full row (log_softmax, then the n-gram
+  // processor, then the beam score - the order of HF beam_search, oracle/beam_ngram.py)
+  const int nb = ban_count ? ban_count[row] : 0;
+  for (int j = 0; j < nb; ++j) {
+    const int w = ban_tokens[(int64_t)row * ban_stride + j];
+    if ((w % kSelThreads) == tid) {
+      const int slot = w / kSelThreads;
 #pragma unroll
-        for (int s = 0; s < kSlots; ++s)
-          if (s == slot) v[s] = -INFINITY;
-      }
+      for (int s = 0; s < kSlots; ++s)
+        if (s == slot) v[s] = -INFINITY;
     }
   }
   // iterative arg-max; ties resolved towards the lower index.  Each thread caches the best of its own slots and
@@ -293,15 +296,17 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
 #pragma unroll
     for (int s = 0; s < kRsSlots; ++s)
       if (base + tid + s * kRsThreads < V) v[s] = __fdiv_rn(v[s], temperature);
-    const int nb = ban_count ? ban_count[row] : 0;
-    for (int j = 0; j < nb; ++j) {
-      const int w = ban_tokens[(int64_t)row * ban_stride + j] - base;
-      if (w >= 0 && w < kRsSpan && (w % kRsThreads) == tid) {
-        const int slot = w / kRsThreads;
+  }
+  // banned tokens -> -inf after the transform: in the beam modes logZ stays over the full row (log_softmax, then the n-gram
+  // processor, then the beam score - the order of HF beam_search, oracle/beam_ngram.py)
+  const int nb = ban_count ? ban_count[row] : 0;
+  for (int j = 0; j < nb; ++j) {
+    const int w = ban_tokens[(int64_t)row * ban_stride + j] - base;
+    if (w >= 0 && w < kRsSpan && (w % kRsThreads) == tid) {
+      const int slot = w / kRsThreads;
 #pragma unroll
-        for (int s = 0; s < kRsSlots; ++s)
-          if (s == slot) v[s] = -INFINITY;
-      }
+      for (int s = 0; s < kRsSlots; ++s)
+        if (s == slot) v[s] = -INFINITY;
     }
   }
   // ---- this CTA's nsel best ----
@@ -587,6 +592,46 @@ ngram_ban_kernel(int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __
   }
   __syncthreads();
   if (threadIdx.x == 0) ban_count[row] = cnt < ban_stride ? cnt : ban_stride;
+}
+
+// Beam mode: one CTA per image scans its question history once and tests every n-gram against the K beam keys.  The key of beam
+// k at step t is the last n-1 tokens of [CLS] + tokens[b, k, :t]; the host launches this only for t >= n-1, where the key lies
+// inside the generated tokens (an earlier key holds the [CLS], and n-grams with a special id are never banned).  Ban lists are
+// per beam row b*K + k.
+constexpr int kBanMaxK = 8;
+__global__ void __launch_bounds__(256)
+beam_ngram_ban_kernel(int K, int T, int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __restrict__ hist_seg,
+                      const int32_t* __restrict__ tokens, int step, int n, int32_t* __restrict__ ban_tokens,
+                      int32_t* __restrict__ ban_count, int ban_stride) {
+  __shared__ int32_t s_key[kBanMaxK][kHypMaxT];
+  __shared__ int s_cnt[kBanMaxK];
+  pdl_wait();
+  pdl_launch_dependents();
+  const int b = blockIdx.x, klen = n - 1, first = step - klen;
+  for (int i = threadIdx.x; i < K * klen; i += blockDim.x) {
+    const int k = i / klen, j = i - k * klen;
+    s_key[k][j] = tokens[((int64_t)b * K + k) * T + first + j];
+  }
+  if (threadIdx.x < K) s_cnt[threadIdx.x] = 0;
+  __syncthreads();
+  const int64_t* ids = hist_ids + (int64_t)b * Lh;
+  const int64_t* seg = hist_seg + (int64_t)b * Lh;
+  for (int p = threadIdx.x; p + n <= Lh; p += blockDim.x) {
+    bool ok = true;                                      // question history = ids * (segments == 0); no special id inside
+    for (int j = 0; j < n && ok; ++j) ok = seg[p + j] == 0 && !is_special(ids[p + j]);
+    if (!ok) continue;
+    const int32_t w = (int32_t)ids[p + n - 1];
+    for (int k = 0; k < K; ++k) {
+      bool match = true;
+      for (int j = 0; j < klen && match; ++j) match = ids[p + j] == (int64_t)s_key[k][j];
+      if (match) {
+        const int slot = atomicAdd(&s_cnt[k], 1);
+        if (slot < ban_stride) ban_tokens[((int64_t)b * K + k) * ban_stride + slot] = w;
+      }
+    }
+  }
+  __syncthreads();
+  if (threadIdx.x < K) ban_count[b * K + threadIdx.x] = s_cnt[threadIdx.x] < ban_stride ? s_cnt[threadIdx.x] : ban_stride;
 }
 
 __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
@@ -919,6 +964,13 @@ int launch_ngram_ban(int rows, int Lh, const int64_t* hist_ids, const int64_t* h
                      cudaStream_t stream) {
   if (rows <= 0) return 0;
   launch_k(ngram_ban_kernel, dim3(rows), dim3(256), 0, stream, Lh, hist_ids, hist_seg, prefix, prefix_stride, d_step, n, ban_tokens, ban_count, ban_stride);
+  return 1;
+}
+int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* tokens, int step,
+                          int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream) {
+  if (B <= 0) return 0;
+  if (K > kBanMaxK || n < 1 || n - 1 > step || step >= T || T > kHypMaxT) throw std::runtime_error("beam_ngram_ban: K <= 8, 1 <= n <= step + 1, step < T <= 32");
+  launch_k(beam_ngram_ban_kernel, dim3(B), dim3(256), 0, stream, K, T, Lh, hist_ids, hist_seg, tokens, step, n, ban_tokens, ban_count, ban_stride);
   return 1;
 }
 int launch_sample_step(int rows, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,

@@ -34,6 +34,8 @@ def read_command_line(argv=None):
     # ---- additions ----
     p.add_argument('-compute_dtype', default='bf16', choices=['bf16', 'fp32'], help='arithmetic of the CUDA engine')
     p.add_argument('-num_beams', default=1, type=int, help='>1: beam search for the answers instead of top-k sampling')
+    p.add_argument('-q_num_beams', default=1, type=int,
+                   help='>1: beam search for the questions instead of top-k sampling (keeps the 4-gram blocking against the question history)')
     p.add_argument('-synthetic', default=0, type=int, help='generate dialogs for N seeded synthetic images (no dataset / checkpoint needed)')
     p.add_argument('-feature_shards', default='', help='comma-separated shard directories (gst_visdial_b200.io.features) instead of the LMDB')
     p.add_argument('-caption_ids', default='', help='json {image_id: [caption token ids]} for the images of the shards (pre-tokenized captions)')
@@ -45,7 +47,7 @@ def read_command_line(argv=None):
     params = vars(args)
     params['device'] = f"cuda:{params['gpu_ids'][0]}"
     params['engine_max_batch'] = params['batch_size']
-    params['engine_max_beams'] = max(1, params['num_beams'])
+    params['engine_max_beams'] = max(1, params['num_beams'], params['q_num_beams'])
     if params['save_name'] == '':
         params['save_name'] = 'generated_dialogs.json'
     os.makedirs(params['save_path'], exist_ok=True)

@@ -87,7 +87,8 @@ typedef struct {
                                  whole - optionally nucleus-filtered - vocabulary (utils/decoding_utils.py:17 skips the cut) */
   float temperature;          /* sample mode: logits / temperature */
   float top_p;                /* sample mode: nucleus threshold applied inside the top-k set; 0 = off */
-  int32_t ngram_blocking_size;/* 0 = off; n: ban tokens completing an n-gram of the question history */
+  int32_t ngram_blocking_size;/* sample and beam mode: 0 = off; n: ban tokens completing an n-gram of the question history (beam mode:
+                                 per beam, on the log-softmax scores before the beam score is added; contract in oracle/beam_ngram.py) */
   uint64_t seed;              /* sample mode RNG seed (counter-based; reproducible per (seed, row_offset + row, step)) */
   int64_t row_offset;         /* global index of row 0 (e.g. the image index of the first sample of this batch / shard): the
                                  draws of an image do not depend on how the images were split into batches or ranks */
@@ -140,8 +141,8 @@ int gstvd_prefill_cross(gstvd_ctx* ctx, int B, int Le, const float* enc_hidden, 
 
 /* Replaces the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:74-120) including
  * batch_ngram_blocking / batch_top_k_top_p_sampling (utils/decoding_utils.py:4-78), with a persistent KV cache.
- *   hist_ids, hist_segments : int64 [B, Lh] encoder input ids / segments (only read when ngram_blocking_size > 0;
- *                             the question history is ids * (segments == 0), visual_dialog_model.py:98-99)
+ *   hist_ids, hist_segments : int64 [B, Lh] encoder input ids / segments (only read when ngram_blocking_size > 0, in sample and
+ *                             beam mode; the question history is ids * (segments == 0), visual_dialog_model.py:98-99)
  *   out_ids    : int64 [B, max_new_tokens] - sampled / best-beam tokens, PAD(0) after the first [SEP]
  *   out_scores : fp32 [B] (may be NULL)    - beam mode: best hypothesis score (sum log-prob / length) */
 int gstvd_generate(gstvd_ctx* ctx, int B, const gstvd_gen_params* params,
