@@ -3,12 +3,14 @@
 // The reference has no KV cache: it re-runs the whole decoder over the whole prefix and re-projects the
 // cross-attention K/V on every step (use_cache=False hard-wired, models/visual_dialog_decoder.py:64; loop at
 // models/visual_dialog_model.py:86-110).  Here each step processes ONE new position per beam row:
-//   dec_self_attn  : appends the new K/V at position *d_step and attends over positions 0..*d_step
+//   dec_self_attn  : appends the new K/V at position g.P0 + *d_step and attends over positions 0..g.P0 + *d_step
+//                    (g.P0 = decoder prefix length - 1; positions below it were stored by prefix_kv_store)
 //   dec_cross_attn : every beam row of an image attends over that image's cross K/V (stored once per image)
 //   reorder_cache  : in-place beam gather, the semantic of _reorder_cache / index_select(0, beam_idx)
 //                    (models/visual_dialog_decoder.py:29-31,177-181)
 // Layouts:  self cache  [layer][k|v][image][position][beam][hidden]   (a beam gather touches contiguous rows)
 //           cross cache [layer][image][k|v, head][position][head_dim]  (one contiguous block per (image, head))
+#include <algorithm>
 #include <cstdlib>
 #include <stdexcept>
 
@@ -19,7 +21,8 @@ namespace gstvd {
 
 namespace {
 
-constexpr int kMaxSteps = 32;     // one score per lane
+constexpr int kMaxSteps = 32;     // one score per lane / one ancestry row of today's decode calls
+constexpr int kMaxPos = 64;       // cached positions of a prefixed call (prefix up to max_dec_len + new tokens): two scores per lane
 constexpr int kMaxBeams = 8;
 
 template <typename T> struct Raw16 {};
@@ -37,11 +40,11 @@ template <> struct Raw16<float> {
 };
 
 // Self-attention of one new position per (beam row, head) over the persistent cache (one warp per (row, head)).
-// Scores: lane t owns cached position t and reads its whole key row (16-byte loads, all issued back to back) against the
+// Scores: lane t owns cached positions t and, with NS = 2 (more than 32 positions), t + 32 and reads its whole key row (16-byte loads, all issued back to back) against the
 // query held in shared memory - no serial chain of load + warp-reduction per position; the new position's score is one
 // warp reduction.  P*V: lanes split the head dimension; the value rows of the first 16 positions are requested BEFORE the
 // scores are computed (they do not depend on them), so key and value loads share one memory round trip.
-template <typename T, int ND>
+template <typename T, int ND, int NS>
 __global__ void __launch_bounds__(128)
 dec_self_attn_kernel(DecodeGeom g, int layer, const T* __restrict__ qkv, T* __restrict__ cache, const int* __restrict__ d_step,
                      T* __restrict__ out) {
@@ -54,7 +57,7 @@ dec_self_attn_kernel(DecodeGeom g, int layer, const T* __restrict__ qkv, T* __re
   const int h = blockIdx.y * 4 + warp;
   if (h >= g.heads) return;
   const int b = row / g.K, kb = row - b * g.K;
-  const int step = *d_step;
+  const int step = g.P0 + *d_step;             // cache position of the new token
   const int H = g.H, D = g.D;
   constexpr int nd = ND;                       // dims per lane (2 for D=64, 4 for D=128)
   const T* qrow = qkv + (int64_t)row * 3 * H + h * D;
@@ -96,36 +99,49 @@ dec_self_attn_kernel(DecodeGeom g, int layer, const T* __restrict__ qkv, T* __re
 #pragma unroll
   for (int u = 0; u < 4; ++u) part = fmaf(q[u], kn[u], part);
   const float s_new = warp_sum(part) / scale_div;
-  // scores of the cached positions: lane t reads key row t
-  float my_score = -INFINITY;
-  if (lane < step) {
-    const T* kc = cache_ptr(0, lane);
-    float dot = 0.f;
-    for (int c = 0; c < D / EPL; ++c) {
-      float kr[EPL];
-      const uint4 raw = *reinterpret_cast<const uint4*>(kc + c * EPL);
-      Raw16<T>::unpack(raw, kr);
+  // scores of the cached positions: lane t reads key rows t (+ 32)
+  float my_score[NS];
 #pragma unroll
-      for (int e4 = 0; e4 < EPL; e4 += 4) {
-        const float4 qv = *reinterpret_cast<const float4*>(&qs[warp][c * EPL + e4]);
-        dot = fmaf(qv.x, kr[e4], dot); dot = fmaf(qv.y, kr[e4 + 1], dot);
-        dot = fmaf(qv.z, kr[e4 + 2], dot); dot = fmaf(qv.w, kr[e4 + 3], dot);
+  for (int s = 0; s < NS; ++s) {
+    const int t = lane + 32 * s;
+    my_score[s] = -INFINITY;
+    if (t < step) {
+      const T* kc = cache_ptr(0, t);
+      float dot = 0.f;
+      for (int c = 0; c < D / EPL; ++c) {
+        float kr[EPL];
+        const uint4 raw = *reinterpret_cast<const uint4*>(kc + c * EPL);
+        Raw16<T>::unpack(raw, kr);
+#pragma unroll
+        for (int e4 = 0; e4 < EPL; e4 += 4) {
+          const float4 qv = *reinterpret_cast<const float4*>(&qs[warp][c * EPL + e4]);
+          dot = fmaf(qv.x, kr[e4], dot); dot = fmaf(qv.y, kr[e4 + 1], dot);
+          dot = fmaf(qv.z, kr[e4 + 2], dot); dot = fmaf(qv.w, kr[e4 + 3], dot);
+        }
       }
+      my_score[s] = dot / scale_div;
+    } else if (t == step) {
+      my_score[s] = s_new;
     }
-    my_score = dot / scale_div;
-  } else if (lane == step) {
-    my_score = s_new;
   }
-  const float mx = warp_max(my_score);
-  const float e = (lane <= step) ? expf(my_score - mx) : 0.f;
-  const float sum = warp_sum(e);
-  const float pr = e / sum;
+  float mx = my_score[0];
+#pragma unroll
+  for (int s = 1; s < NS; ++s) mx = fmaxf(mx, my_score[s]);
+  mx = warp_max(mx);
+  float e[NS], esum = 0.f;
+#pragma unroll
+  for (int s = 0; s < NS; ++s) { e[s] = (lane + 32 * s <= step) ? expf(my_score[s] - mx) : 0.f; esum += e[s]; }
+  const float sum = warp_sum(esum);
+  float pr[NS];
+#pragma unroll
+  for (int s = 0; s < NS; ++s) pr[s] = e[s] / sum;
   float acc[4] = {0.f, 0.f, 0.f, 0.f};
   for (int t0 = 0; t0 < step; t0 += VB) {
     if (t0 > 0) load_v(t0);
+    const float prs = (NS == 1 || t0 < 32) ? pr[0] : pr[NS - 1];   // VB divides 32: one score register per batch
 #pragma unroll
     for (int i = 0; i < VB; ++i) {
-      const float pt = __shfl_sync(0xffffffffu, pr, (t0 + i) & 31);
+      const float pt = __shfl_sync(0xffffffffu, prs, (t0 + i) & 31);
       if (t0 + i < step) {
 #pragma unroll
         for (int u = 0; u < ND; ++u) acc[u] = fmaf(pt, vv[i][u], acc[u]);
@@ -133,7 +149,7 @@ dec_self_attn_kernel(DecodeGeom g, int layer, const T* __restrict__ qkv, T* __re
     }
   }
   {
-    const float pt = __shfl_sync(0xffffffffu, pr, step);
+    const float pt = __shfl_sync(0xffffffffu, (NS == 1 || step < 32) ? pr[0] : pr[NS - 1], step & 31);
     // in bf16 mode later steps read the ROUNDED new value from the cache; use the same value now
 #pragma unroll
     for (int u = 0; u < 4; ++u) acc[u] = fmaf(pt, to_f32(from_f32<T>(vn[u])), acc[u]);
@@ -154,6 +170,8 @@ dec_self_attn_kernel(DecodeGeom g, int layer, const T* __restrict__ qkv, T* __re
 //   * P * V: each lane accumulates its 8 dims over its positions, one 2-step butterfly per dim merges the four groups and lanes 0-7
 //     store the 128-byte output row.
 // The new position's k / v are taken from qkv (rounded to bf16, i.e. exactly what later steps will read back from the cache).
+// NIT = 16 covers the 64 positions of a prefixed call; its ancestry rows are 64 entries wide (kAncRow).
+template <int NIT> struct AncRow { static constexpr int value = NIT * 4 > kMaxSteps ? kMaxPos : kMaxSteps; };
 template <int NIT>
 __global__ void __launch_bounds__(128)
 dec_self_attn_v2_kernel(DecodeGeom g, int layer, const bf16* __restrict__ qkv, bf16* __restrict__ cache, const int* __restrict__ d_step,
@@ -173,20 +191,22 @@ dec_self_attn_v2_kernel(DecodeGeom g, int layer, const bf16* __restrict__ qkv, b
   const uint4 vn_raw = *reinterpret_cast<const uint4*>(qrow + 2 * H);
   // step_host >= 0: the launch knows the step (eager loops and the all-steps graph unroll them), so the loads below are bounded by
   // it - on average half of the g.T cache rows - without waiting for *d_step; otherwise every row is requested and masked afterwards
-  const int step = step_host >= 0 ? step_host : *d_step;
-  const int bound = step_host >= 0 ? step_host : g.T;          // cache positions < bound are requested
+  const int step = g.P0 + (step_host >= 0 ? step_host : *d_step);   // cache position of the new token
+  const int bound = step_host >= 0 ? step : g.T;                   // cache positions < bound are requested
   // element offset of (kv, position t) for this beam / head / chunk
   const int64_t pos_stride = (int64_t)g.K * H;
   const int64_t k_base = ((((int64_t)layer * 2 + 0) * g.B + b) * g.T) * pos_stride + h * 64 + chunk * 8;   // slot 0 of position 0
   const int64_t v_base = k_base + (int64_t)g.B * g.T * pos_stride;
   // Beam search without moving the cache (anc != null): position t of this beam's history lives in the slot of the beam that
-  // wrote it, anc[(b*K + kb)*32 + t] (anc_update_kernel permutes the 32-byte rows after every selection); the new position is
-  // always written to the beam's own slot.  Entries at or past *d_step are stale but always < 8; they are clamped and masked.
+  // wrote it, anc[(b*K + kb)*W + t] (anc_update_kernel permutes the W-byte rows after every selection); the new position is
+  // always written to the beam's own slot.  Entries at or past the new position are stale but always < 8; they are clamped and
+  // masked.  Prefix positions (below g.P0) hold the same K / V in every slot, so whatever their entries say is correct.
+  constexpr int W = AncRow<NIT>::value;
   int slot[NIT];
 #pragma unroll
   for (int it = 0; it < NIT; ++it) {
     const int t = it * 4 + grp;
-    slot[it] = (anc != nullptr && t < bound) ? min((int)anc[((int64_t)b * g.K + kb) * kMaxSteps + (t & (kMaxSteps - 1))], g.K - 1) : kb;
+    slot[it] = (anc != nullptr && t < bound) ? min((int)anc[((int64_t)b * g.K + kb) * W + (t & (W - 1))], g.K - 1) : kb;
   }
   uint4 k_raw[NIT], v_raw[NIT];
 #pragma unroll
@@ -587,21 +607,44 @@ void launch_cross_t(const DecodeGeom& g, const void* q, const void* kv_layer, co
 // Beam reorder without moving the cache: new beam k continues old beam parent = beam_idx[b][k]; its history row becomes the
 // parent's row and the position just written (t = *d_step) is found in the parent's slot.  One CTA per image; every entry is
 // read before any is written (parents may repeat).  Replaces reorder_cache_kernel (up to 2 x 100 MB of HBM traffic per step at
-// B = 64, K = 5) when the self-attention kernel reads through the table (dec_self_attn_v2_kernel).
-__global__ void __launch_bounds__(kMaxBeams * kMaxSteps)
-anc_update_kernel(int B, int K, const int32_t* __restrict__ beam_idx, const int* __restrict__ d_step, uint8_t* __restrict__ anc) {
+// B = 64, K = 5) when the self-attention kernel reads through the table (dec_self_attn_v2_kernel).  W = row width (positions);
+// the position just written is p0 + *d_step.
+template <int W>
+__global__ void __launch_bounds__(kMaxBeams * W)
+anc_update_kernel(int B, int K, int p0, const int32_t* __restrict__ beam_idx, const int* __restrict__ d_step, uint8_t* __restrict__ anc) {
   pdl_wait();
   pdl_launch_dependents();
-  const int b = blockIdx.x, k = threadIdx.x / kMaxSteps, t = threadIdx.x % kMaxSteps;
-  const int step = *d_step;
+  const int b = blockIdx.x, k = threadIdx.x / W, t = threadIdx.x % W;
+  const int step = p0 + *d_step;
   int val = 0;
   const bool live = k < K && t <= step;
   if (live) {
     const int parent = beam_idx[b * K + k];
-    val = (t == step) ? parent : anc[((int64_t)b * K + parent) * kMaxSteps + t];
+    val = (t == step) ? parent : anc[((int64_t)b * K + parent) * W + t];
   }
   __syncthreads();
-  if (live) anc[((int64_t)b * K + k) * kMaxSteps + t] = (uint8_t)val;
+  if (live) anc[((int64_t)b * K + k) * W + t] = (uint8_t)val;
+}
+
+// Decoder prefix prefill: K / V of the first P-1 prefix positions of every image, computed by a teacher-forced pass (qkv rows
+// [B * P0][3H], row = b * P0 + p), copied into EVERY beam slot of that image's cache rows 0..P0-1 - all beams share the prefix, so the
+// gather (reorder_cache) and the ancestry path both read correct data there whatever their tables say.  16-byte chunks.
+template <typename T>
+__global__ void __launch_bounds__(256)
+prefix_kv_store_kernel(DecodeGeom g, int layer, const T* __restrict__ qkv, T* __restrict__ cache) {
+  constexpr int EPL = 16 / sizeof(T);
+  const int chunks = g.H / EPL;
+  const int64_t n = (int64_t)g.B * g.P0 * 2 * chunks;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const int c = (int)(i % chunks);
+    const int64_t r2 = i / chunks;
+    const int kv = (int)(r2 & 1);
+    const int64_t row = r2 >> 1;
+    const int b = (int)(row / g.P0), p = (int)(row - (int64_t)b * g.P0);
+    const uint4 v = *reinterpret_cast<const uint4*>(qkv + row * 3 * g.H + (1 + kv) * g.H + c * EPL);
+    T* dst = cache + ((((int64_t)layer * 2 + kv) * g.B + b) * g.T + p) * g.K * g.H + c * EPL;
+    for (int k = 0; k < g.K; ++k) *reinterpret_cast<uint4*>(dst + (int64_t)k * g.H) = v;
+  }
 }
 
 // One CTA per (image, layer*2+kv).  Thread-local dependency only: every thread loads the K source values of its
@@ -614,7 +657,7 @@ reorder_cache_kernel(DecodeGeom g, T* __restrict__ cache, const int32_t* __restr
   pdl_launch_dependents();
   const int b = blockIdx.x, lk = blockIdx.y;
   if (d_skip && d_skip[b]) return;
-  const int len = d_len ? (*d_len + 1) : len_host;
+  const int len = d_len ? (*d_len + 1) : len_host;   // positions after the prefix rows (identical in every slot, never moved)
   int parent[kMaxBeams];
   bool moved = false;
 #pragma unroll
@@ -624,7 +667,7 @@ reorder_cache_kernel(DecodeGeom g, T* __restrict__ cache, const int32_t* __restr
   }
   if (!moved) return;
   const int chunks = g.H / 8;
-  T* base = cache + ((int64_t)lk * g.B + b) * g.T * g.K * g.H;
+  T* base = cache + (((int64_t)lk * g.B + b) * g.T + g.P0) * g.K * g.H;
   for (int i = threadIdx.x; i < len * chunks; i += blockDim.x) {
     const int t = i / chunks, c = (i - t * chunks) * 8;
     T* p = base + (int64_t)t * g.K * g.H + c;
@@ -640,39 +683,58 @@ reorder_cache_kernel(DecodeGeom g, T* __restrict__ cache, const int32_t* __restr
 
 }  // namespace
 
+template <int NS>
+static void launch_self_generic(int dtype, const DecodeGeom& g, dim3 grid, int layer, const void* qkv, void* self_cache, const int* d_step, void* out,
+                         cudaStream_t stream) {
+  if (g.D == 64) {
+    if (dtype == kF32) launch_k(dec_self_attn_kernel<float, 2, NS>, grid, dim3(128), 0, stream, g, layer, (const float*)qkv, (float*)self_cache, d_step, (float*)out);
+    else launch_k(dec_self_attn_kernel<bf16, 2, NS>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, (bf16*)out);
+  } else {
+    if (dtype == kF32) launch_k(dec_self_attn_kernel<float, 4, NS>, grid, dim3(128), 0, stream, g, layer, (const float*)qkv, (float*)self_cache, d_step, (float*)out);
+    else launch_k(dec_self_attn_kernel<bf16, 4, NS>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, (bf16*)out);
+  }
+}
+
 bool dec_self_attn_v2_active(int dtype, const DecodeGeom& g, const void* qkv, const void* self_cache, const void* out) {
   const char* v2_env = getenv("GSTVD_SELF_V2");            // read per call (captured graphs keep what was set at capture time)
   const bool v2 = v2_env == nullptr || atoi(v2_env) != 0;  // default on; GSTVD_SELF_V2=0 selects the first kernel
-  return v2 && dtype == kBF16 && g.D == 64 && g.H % 8 == 0 && g.T <= kMaxSteps && g.K <= kMaxBeams &&
+  return v2 && dtype == kBF16 && g.D == 64 && g.H % 8 == 0 && g.T <= kMaxPos && g.K <= kMaxBeams &&
          (reinterpret_cast<uintptr_t>(qkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(self_cache) & 15) == 0 &&
          (reinterpret_cast<uintptr_t>(out) & 15) == 0;
 }
 
 int launch_anc_update(const DecodeGeom& g, const int32_t* beam_idx, const int* d_step, uint8_t* anc, cudaStream_t stream) {
-  if (g.K > kMaxBeams || g.T > kMaxSteps) throw std::runtime_error("anc_update: at most 8 beams and 32 positions");
-  launch_k(anc_update_kernel, dim3(g.B), dim3(kMaxBeams * kMaxSteps), 0, stream, g.B, g.K, beam_idx, d_step, anc);
+  if (g.K > kMaxBeams || g.T > kMaxPos) throw std::runtime_error("anc_update: at most 8 beams and 64 positions");
+  if (g.T <= kMaxSteps) launch_k(anc_update_kernel<kMaxSteps>, dim3(g.B), dim3(kMaxBeams * kMaxSteps), 0, stream, g.B, g.K, g.P0, beam_idx, d_step, anc);
+  else launch_k(anc_update_kernel<kMaxPos>, dim3(g.B), dim3(kMaxBeams * kMaxPos), 0, stream, g.B, g.K, g.P0, beam_idx, d_step, anc);
+  return 1;
+}
+
+int launch_prefix_kv_store(int dtype, const DecodeGeom& g, int layer, const void* qkv, void* self_cache, cudaStream_t stream) {
+  if (g.P0 < 1) return 0;
+  if (g.H % 8) throw std::runtime_error("prefix_kv_store: hidden % 8 != 0");
+  const int64_t n = (int64_t)g.B * g.P0 * 2 * (g.H / (dtype == kF32 ? 4 : 8));
+  const int blocks = (int)std::min<int64_t>((n + 255) / 256, 1024);
+  if (dtype == kF32) prefix_kv_store_kernel<float><<<blocks, 256, 0, stream>>>(g, layer, (const float*)qkv, (float*)self_cache);
+  else prefix_kv_store_kernel<bf16><<<blocks, 256, 0, stream>>>(g, layer, (const bf16*)qkv, (bf16*)self_cache);
   return 1;
 }
 
 int launch_dec_self_attn(int dtype, const DecodeGeom& g, int layer, const void* qkv, void* self_cache, const int* d_step, int step_host,
                          const uint8_t* anc, void* out, cudaStream_t stream) {
   if (g.D != 64 && g.D != 128) throw std::runtime_error("dec_self_attn: head_dim must be 64 or 128");
-  if (g.T > kMaxSteps) throw std::runtime_error("dec_self_attn: at most 32 cached positions");
+  if (g.T > kMaxPos) throw std::runtime_error("dec_self_attn: at most 64 cached positions");
   dim3 grid(g.B * g.K, (g.heads + 3) / 4);
   // lean variant: bf16, 64-dim heads, 16-byte aligned rows
   if (dec_self_attn_v2_active(dtype, g, qkv, self_cache, out)) {
     if (g.T <= 20) launch_k(dec_self_attn_v2_kernel<5>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, step_host, anc, (bf16*)out);
-    else launch_k(dec_self_attn_v2_kernel<8>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, step_host, anc, (bf16*)out);
+    else if (g.T <= kMaxSteps) launch_k(dec_self_attn_v2_kernel<8>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, step_host, anc, (bf16*)out);
+    else launch_k(dec_self_attn_v2_kernel<16>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, step_host, anc, (bf16*)out);
     return 1;
   }
   if (anc != nullptr) throw std::runtime_error("dec_self_attn: the ancestry table is only read by the bf16 / 64-dim kernel");
-  if (g.D == 64) {
-    if (dtype == kF32) launch_k(dec_self_attn_kernel<float, 2>, grid, dim3(128), 0, stream, g, layer, (const float*)qkv, (float*)self_cache, d_step, (float*)out);
-    else launch_k(dec_self_attn_kernel<bf16, 2>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, (bf16*)out);
-  } else {
-    if (dtype == kF32) launch_k(dec_self_attn_kernel<float, 4>, grid, dim3(128), 0, stream, g, layer, (const float*)qkv, (float*)self_cache, d_step, (float*)out);
-    else launch_k(dec_self_attn_kernel<bf16, 4>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, (bf16*)out);
-  }
+  if (g.T <= kMaxSteps) launch_self_generic<1>(dtype, g, grid, layer, qkv, self_cache, d_step, out, stream);
+  else launch_self_generic<2>(dtype, g, grid, layer, qkv, self_cache, d_step, out, stream);
   return 1;
 }
 

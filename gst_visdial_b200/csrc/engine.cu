@@ -66,10 +66,11 @@ struct DevBuf {
   void release() { if (p) cudaFree(p); p = nullptr; bytes = 0; }
 };
 
-// Shapes and selection parameters only: the n-gram blocking history is copied into context-owned buffers before a replay, so the
-// caller's tensor addresses are not part of the key (a caching allocator hands out a new address per batch).
+// Shapes and selection parameters only: the n-gram blocking history and the decoder prefix are copied into context-owned buffers
+// before a replay, so the caller's tensor addresses are not part of the key (a caching allocator hands out a new address per batch).
+// P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start.
 struct GraphKey {
-  int B, K, mode, T, top_k, ngram, Lh, Le; float temperature, top_p;
+  int B, K, mode, T, top_k, ngram, Lh, Le, P, has_prefix; float temperature, top_p;
   bool operator<(const GraphKey& o) const { return std::memcmp(this, &o, sizeof(GraphKey)) < 0; }
 };
 constexpr size_t kMaxGraphs = 24;      // least-recently-used graphs beyond this are destroyed (an 18-step graph holds ~2k kernel nodes)
@@ -113,7 +114,8 @@ struct gstvd_ctx {
   DevBuf ban_tokens, ban_count, prefix, seq;          // sample-mode state
   DevBuf beam_scores, beam_tokens, cur_tokens, beam_idx, beam_done, hyp_score, hyp_len, hyp_tokens, hyp_count, hyp_worst;
   DevBuf d_step, d_seed;
-  DevBuf anc;                                         // uint8 [B*K][32]: beam ancestry table (launch_anc_update)
+  DevBuf anc;                                         // uint8 [B*K][64]: beam ancestry table (launch_anc_update; rows of 32 up to 32 positions)
+  DevBuf dec_prefix_own, dec_prefix_head;             // int64 [B_max, max_dec_len]: decoder prefix of a call; [B, P-1]: its prefill ids
   DevBuf fold16, foldvec;                             // deferred LayerNorm: folded bf16 weights, c / d vectors
   DevBuf st1, st2, st3;                               // float2 [rows][kLnStatStride]: partial row statistics of the raw x1 / x2 / x3
   bool fold_ready = false;
@@ -128,7 +130,7 @@ struct gstvd_ctx {
   uint64_t graph_clock = 0;
   // whole-round graphs (gstvd_round): encoder + cross-K/V prefill + every decode step of one forward call in ONE graph, keyed by shapes
   struct RoundKey {
-    int B, Lt, Lv, K, mode, T, top_k, ngram, has_seg, has_att, has_imask; float temperature, top_p;
+    int B, Lt, Lv, K, mode, T, top_k, ngram, has_seg, has_att, has_imask, P, has_prefix; float temperature, top_p;
     bool operator<(const RoundKey& o) const { return std::memcmp(this, &o, sizeof(RoundKey)) < 0; }
   };
   std::map<RoundKey, GraphEntry> round_graphs;
@@ -327,7 +329,9 @@ void alloc_workspace(gstvd_ctx* c) {
     A(c->dffn, R * c->dec_F); A(c->dqc, R * H);
     c->logits.alloc(R * (size_t)c->Vpad * 4);
     A(c->cross_cache, (size_t)c->dec_layers * B * 2 * H * Le);
-    A(c->self_cache, (size_t)c->dec_layers * 2 * B * T * K * H);
+    // max_new_tokens + max_dec_len - 1 positions per row: a decoder prefix of P tokens occupies P - 1 positions before the first
+    // generated one.  A call's cache stride is its own position count (P - 1 + its max_new_tokens).
+    A(c->self_cache, (size_t)c->dec_layers * 2 * B * (T + c->Ldec_max - 1) * K * H);
     c->labels.alloc(B * (size_t)c->Ldec_max * 8);
     c->cross_len.alloc(B * 4);
     c->sel_val.alloc(R * kSelMax * 4); c->sel_idx.alloc(R * kSelMax * 4); c->logz.alloc(R * 4);
@@ -336,13 +340,14 @@ void alloc_workspace(gstvd_ctx* c) {
     c->r_ids.alloc(B * Lt * 8); c->r_seg.alloc(B * Lt * 8); c->r_att.alloc(B * Lt * 4);
     c->r_feat.alloc(B * Lv * (size_t)c->cfg.v_feature_size * 4); c->r_loc.alloc(B * Lv * 5 * 4); c->r_imask.alloc(B * Lv * 4);
     c->r_out_ids.alloc(B * T * 8); c->r_out_scores.alloc(B * 4);
-    c->prefix.alloc(B * (T + 1) * 4); c->seq.alloc(B * T * 4);
+    c->prefix.alloc(B * (T + c->Ldec_max) * 4); c->seq.alloc(B * T * 4);
+    c->dec_prefix_own.alloc(B * c->Ldec_max * 8); c->dec_prefix_head.alloc(B * c->Ldec_max * 8);
     c->beam_scores.alloc(B * K * 4); c->beam_tokens.alloc(2 * B * K * T * 4); c->cur_tokens.alloc(R * 4);
     c->beam_idx.alloc(B * K * 4); c->beam_done.alloc(B); c->hyp_score.alloc(B * (K + 1) * 8);
     c->hyp_len.alloc(B * (K + 1) * 4); c->hyp_tokens.alloc(B * (K + 1) * T * 4); c->hyp_count.alloc(B * 4);
     c->hyp_worst.alloc(B * 8);
-    c->anc.alloc(B * K * 32);
-    CUDA_CHECK(cudaMemset(c->anc.p, 0, B * K * 32));
+    c->anc.alloc(B * K * 64);
+    CUDA_CHECK(cudaMemset(c->anc.p, 0, B * K * 64));
     c->stats_ld = (int64_t)((R + 15) & ~size_t(15));
     c->st1.alloc(c->stats_ld * kLnStatStride * 8); c->st2.alloc(c->stats_ld * kLnStatStride * 8); c->st3.alloc(c->stats_ld * kLnStatStride * 8);
   }
@@ -583,9 +588,11 @@ void do_prefill(gstvd_ctx* c, int B, int Le, const float* enc_hidden, const floa
   c->cross_B = B; c->cross_Le = Le;
 }
 
-DecodeGeom make_geom(gstvd_ctx* c, int B, int K, int T) {
+// T = new tokens; P = decoder prefix length (its first P - 1 positions are prefilled, the last one is the first step's input)
+DecodeGeom make_geom(gstvd_ctx* c, int B, int K, int T, int P = 1) {
   DecodeGeom g;
-  g.B = B; g.K = K; g.H = c->H; g.heads = c->dec_heads; g.D = c->H / c->dec_heads; g.layers = c->dec_layers; g.T = T; g.Le = c->cross_Le;
+  g.B = B; g.K = K; g.H = c->H; g.heads = c->dec_heads; g.D = c->H / c->dec_heads; g.layers = c->dec_layers; g.T = P - 1 + T; g.Le = c->cross_Le;
+  g.P0 = P - 1;
   return g;
 }
 
@@ -598,14 +605,85 @@ BeamBuffers beam_buffers(gstvd_ctx* c) {
   return bb;
 }
 
+// Teacher-forced decoder layer stack (HF BertLayer: causal self-attention, cross-attention, FFN) over B sequences of L positions whose
+// embeddings are in c->dh; `options` consecutive sequences share one image's cross K/V.  kv != null (decoder prefix prefill): after
+// each layer's q|k|v GEMM that layer's K / V rows are stored into every beam slot of the self cache, and the last layer stops there
+// (its output feeds nothing: no FFN, no LM head).
+void dec_teacher_layers(gstvd_ctx* c, Exec& X, int B, int L, const float* dec_mask, int options, const DecodeGeom* kv) {
+  const int H = c->H, M = B * L, D = H / c->dec_heads, Le = c->cross_Le;
+  const int64_t per_image = (int64_t)2 * c->dec_heads * Le * D;
+  for (int l = 0; l < c->dec_layers; ++l) {
+    const DecLayer& Ly = c->d_layers[l];
+    X.gemm(c->dh.p, H, Ly.qkv, c->dqkv.p, 3 * H, M);
+    if (kv) {
+      c->launches += launch_prefix_kv_store(c->dtype, *kv, l, c->dqkv.p, c->self_cache.p, X.s);
+      if (l == c->dec_layers - 1) return;
+    }
+    X.attention(c->dqkv.p, 3 * H, L, X.off(c->dqkv.p, H), X.off(c->dqkv.p, 2 * H), 3 * H, L, c->dctx.p, H, B, c->dec_heads, D, dec_mask,
+                -10000.0f, 1);
+    X.gemm(c->dctx.p, H, Ly.o, c->dtmp.p, H, M);
+    X.add_ln(c->dtmp.p, c->dh.p, Ly.ln_att, c->da.p, M);
+    X.gemm(c->da.p, H, Ly.cq, c->dqc.p, H, M);
+    {
+      AttnArgs a;
+      const char* kbase = (const char*)c->cross_cache.p + (size_t)l * (B / options) * per_image * c->esz;
+      a.q = c->dqc.p; a.q_bs = (int64_t)L * H; a.q_hs = D; a.q_rs = H;
+      a.k = kbase; a.k_bs = per_image; a.k_hs = (int64_t)Le * D; a.k_rs = D;
+      a.v = kbase + (size_t)c->dec_heads * Le * D * c->esz; a.v_bs = per_image; a.v_hs = a.k_hs; a.v_rs = D;
+      a.o = c->dctx.p; a.o_bs = (int64_t)L * H; a.o_hs = D; a.o_rs = H;
+      a.kmask = (const float*)c->fused_mask.p; a.kmask_bs = Le; a.neg = -1e9f; a.causal = 0;
+      a.B = B; a.H = c->dec_heads; a.Lq = L; a.Lk = Le; a.D = D; a.kv_batch_div = options;
+      X.run_attention(a);
+    }
+    X.gemm(c->dctx.p, H, Ly.co, c->dtmp.p, H, M);
+    X.add_ln(c->dtmp.p, c->da.p, Ly.ln_cross, c->db.p, M);
+    X.gemm(c->db.p, H, Ly.f1, c->dffn.p, c->dec_F, M, 1);
+    X.gemm(c->dffn.p, c->dec_F, Ly.f2, c->dtmp.p, H, M);
+    X.add_ln(c->dtmp.p, c->db.p, Ly.ln_out, c->dh.p, M);
+  }
+}
+
+// Decoder prefix prefill: a teacher-forced pass over the first P0 = P - 1 prefix positions of the g.B images (ids in
+// c->dec_prefix_head, [SEP] embedded as [PAD] like the in-place replacement of models/visual_dialog_decoder.py:57) that leaves every
+// layer's K / V of those positions in the self cache.  P = 1 launches nothing.
+void prefix_prefill(gstvd_ctx* c, const DecodeGeom& g, cudaStream_t s) {
+  if (g.P0 == 0) return;
+  PdlScope pdl_scope(!(c->cfg.flags & GSTVD_FLAG_NO_PDL));
+  Exec X{c, s};
+  c->launches += launch_embed_text(c->dtype, g.B * g.P0, g.P0, c->H, (const int64_t*)c->dec_prefix_head.p, nullptr, nullptr, 1, c->word, c->pos,
+                                   c->type, c->type_ext, c->cfg.type_vocab_size, c->emb_ln.g, c->emb_ln.b, c->dh.p, s);
+  dec_teacher_layers(c, X, g.B, g.P0, nullptr, 1, &g);
+}
+
+// Copies the caller's decoder prefix [B, P] into the context (captured graphs read it there) and its first P - 1 columns, the prefill
+// ids, into the compact [B, P - 1] buffer.  Returns the context copy, or null for the implicit [CLS] start (prefix == null).
+const int64_t* stage_prefix(gstvd_ctx* c, int B, const int64_t* prefix, int P, cudaStream_t s) {
+  if (!prefix) return nullptr;
+  CUDA_CHECK(cudaMemcpyAsync(c->dec_prefix_own.p, prefix, (size_t)B * P * 8, cudaMemcpyDeviceToDevice, s));
+  if (P > 1)
+    CUDA_CHECK(cudaMemcpy2DAsync(c->dec_prefix_head.p, (size_t)(P - 1) * 8, prefix, (size_t)P * 8, (size_t)(P - 1) * 8, B,
+                                 cudaMemcpyDeviceToDevice, s));
+  return (const int64_t*)c->dec_prefix_own.p;
+}
+
+// Selection state of a decode call: beams / sample rows start from the last token of the prefix (the [CLS] when it is null).
+void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* prefix, cudaStream_t s) {
+  const int P = g.P0 + 1, T = gp.max_new_tokens;
+  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, T, 101, prefix, P, s);
+  else c->launches += launch_sample_init(g.B, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, P + T, (int*)c->d_step.p,
+                                         prefix, P, s);
+}
+
 // One decode step for all M = B*K rows: embeddings -> 12 x [self-attn over cache, cross-attn, FFN] -> LM head -> selection.
 // step_host = index of this step when the caller knows it (it always does: eager loops and the captured graph both unroll the
 // steps), so kernels that only need it to bound their loads take it as a launch parameter instead of reading *d_step first.
-void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* hist_ids, const int64_t* hist_seg,
-                 int Lh, cudaStream_t s, int step_host) {
+// prefix: int64 [B, P] decoder prefix (P = g.P0 + 1), null for the [CLS] start.
+void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* prefix, const int64_t* hist_ids,
+                 const int64_t* hist_seg, int Lh, cudaStream_t s, int step_host) {
   Exec X{c, s};
   PdlScope pdl_scope(!(c->cfg.flags & GSTVD_FLAG_NO_PDL));
   const int H = c->H, M = g.B * g.K;
+  const int P = g.P0 + 1, Tn = g.T - g.P0;          // prefix length, new tokens (stride of the token buffers)
   const int* d_step = (const int*)c->d_step.p;
   // Beam mode with the lean self-attention kernel: the cache is never gathered, the kernel reads each history position from the
   // slot recorded in the ancestry table (token ids identical to the gather, +3 % dialogs/s; env GSTVD_SELF_ANC=0 restores the gather)
@@ -613,7 +691,7 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   const bool use_anc = gp.mode == GSTVD_SELECT_BEAM && (anc_env == nullptr || atoi(anc_env) != 0) &&
                        dec_self_attn_v2_active(c->dtype, g, c->dqkv.p, c->self_cache.p, c->dctx.p);
   const uint8_t* anc = use_anc ? (const uint8_t*)c->anc.p : nullptr;
-  c->launches += launch_embed_step(c->dtype, M, H, (const int32_t*)c->cur_tokens.p, d_step, c->word, c->pos, c->type,
+  c->launches += launch_embed_step(c->dtype, M, H, (const int32_t*)c->cur_tokens.p, g.P0, d_step, c->word, c->pos, c->type,
                                    c->emb_ln.g, c->emb_ln.b, c->dh.p, s);
   // Deferred LayerNorm (default for bf16): no LayerNorm kernel inside the layer stack - the three dense -> LN(x + input) pairs of a
   // layer store raw sums + partial row statistics, their consumers normalise on the fly (GemmArgs::fold_* / res_*), and one
@@ -669,46 +747,58 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     static const bool exact_lse = getenv("GSTVD_EXACT_LSE") != nullptr;
     BeamBuffers bb = beam_buffers(c);
     const int32_t* bt = nullptr; const int32_t* bc = nullptr;
-    // n-gram blocking: before step n-1 every key still holds the [CLS], which no banned n-gram contains - nothing to launch
-    if (gp.ngram_blocking_size > 0 && step_host >= gp.ngram_blocking_size - 1) {
-      c->launches += launch_beam_ngram_ban(g.B, g.K, g.T, Lh, hist_ids, hist_seg, bb.tokens + (int64_t)(step_host & 1) * M * g.T, step_host,
-                                           gp.ngram_blocking_size, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
+    // n-gram blocking: nothing to launch while every key is shorter than n-1 tokens (P + t < n-1) or, for the [CLS] start, still
+    // holds the [CLS], which no banned n-gram contains (t < n-1).  A caller's prefix may hold anything: no position is known special.
+    const int n = gp.ngram_blocking_size;
+    if (n > 0 && step_host >= (prefix ? n - 1 - P : n - 1)) {
+      c->launches += launch_beam_ngram_ban(g.B, g.K, Tn, Lh, hist_ids, hist_seg, prefix, P, bb.tokens + (int64_t)(step_host & 1) * M * Tn,
+                                           step_host, n, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }
     c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, (c->dtype == kBF16 && !exact_lse) ? 2 : 0,
                                      (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, nullptr, s);
-    c->launches += launch_beam_step(bb, g.B, g.K, g.T, c->V, nsel, sv, si, 102, nullptr, nullptr, nullptr, s);
+    c->launches += launch_beam_step(bb, g.B, g.K, Tn, c->V, nsel, sv, si, 102, P, nullptr, nullptr, nullptr, s);
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
   } else {
     const int nsel = kSelMax;
     const int32_t* bt = nullptr; const int32_t* bc = nullptr;
+    // key buffer c->prefix [M, P + Tn]: the decoder prefix, then the generated tokens; the samplers append token t at P + t
+    const int kst = P + Tn;
+    int32_t* key_next = (int32_t*)c->prefix.p + (P - 1);
     if (gp.ngram_blocking_size > 0) {
-      c->launches += launch_ngram_ban(M, Lh, hist_ids, hist_seg, (const int32_t*)c->prefix.p, g.T + 1, d_step, gp.ngram_blocking_size,
+      c->launches += launch_ngram_ban(M, Lh, hist_ids, hist_seg, (const int32_t*)c->prefix.p, kst, d_step, P, gp.ngram_blocking_size,
                                       (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }
     if (gp.top_k == 0) {
       // no top-k cut (utils/decoding_utils.py:17 skips it): multinomial over the whole, optionally nucleus-filtered, vocabulary
-      c->launches += launch_full_vocab_sample(M, c->V, (const float*)c->logits.p, c->Vpad, gp.temperature, gp.top_p, bt, bc, Lh, g.T, 0, 0,
+      c->launches += launch_full_vocab_sample(M, c->V, (const float*)c->logits.p, c->Vpad, gp.temperature, gp.top_p, bt, bc, Lh, Tn, 0, 0,
                                               (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p,
-                                              (int32_t*)c->prefix.p, g.T + 1, nullptr, s);
+                                              key_next, kst, nullptr, s);
     } else {
       c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, 1, nullptr, gp.temperature, bt, bc, Lh, nsel, sv, si,
                                        nullptr, s);
-      c->launches += launch_sample_step(M, g.T, nsel, sv, si, gp.top_k, gp.top_p, 0, 0, (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p,
-                                        (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, g.T + 1, nullptr, s);
+      c->launches += launch_sample_step(M, Tn, nsel, sv, si, gp.top_k, gp.top_p, 0, 0, (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p,
+                                        (int32_t*)c->cur_tokens.p, key_next, kst, nullptr, s);
     }
   }
   c->launches += launch_step_advance((int*)c->d_step.p, s);
 }
 
 // Argument checks of a generate call; returns the beams per image.
-int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* hist_ids, const int64_t* hist_seg, int Lh, const int64_t* out_ids) {
+int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_seg,
+                   int Lh, const int64_t* out_ids) {
   check_ready(c);
   if (c->dec_layers == 0) throw StateError("generate: encoder-only context");
   const int T = gp.max_new_tokens;
   if (T < 1 || T > c->T_max) throw InvalidArg("generate: max_new_tokens out of range");
+  if (P < 1 || P > c->Ldec_max) throw InvalidArg(fmt("generate: decoder prefix length %d outside 1..max_dec_len (%d)", P, c->Ldec_max));
+  if (!prefix && P > 1) throw InvalidArg("generate: the decoder prefix is NULL but its length is above 1");
+  if (P - 1 + T > 64)
+    throw InvalidArg(fmt("generate: prefix length %d + %d new tokens need %d cached positions; the decode kernels hold at most 64", P, T, P - 1 + T));
+  if (P - 1 + T > c->cfg.max_position_embeddings)
+    throw InvalidArg(fmt("generate: prefix length %d + %d new tokens exceed max_position_embeddings (%d)", P, T, c->cfg.max_position_embeddings));
   if (!out_ids) throw InvalidArg("generate: out_ids is NULL");
   int K = 1;
   if (gp.mode == GSTVD_SELECT_BEAM) {
@@ -725,30 +815,32 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* hist
   return K;
 }
 
-void generate_finalize(gstvd_ctx* c, int B, int K, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
+void generate_finalize(gstvd_ctx* c, int B, int K, int P, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
   const int T = gp.max_new_tokens;
-  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, out_ids, out_scores, s);
+  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, P, out_ids, out_scores, s);
   else c->launches += launch_sample_finalize(B, T, 102, (const int32_t*)c->seq.p, out_ids, s);
 }
 
-void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t* hist_ids, const int64_t* hist_seg, int Lh,
-                 int64_t* out_ids, float* out_scores, cudaStream_t s) {
-  const int K = check_generate(c, gp, hist_ids, hist_seg, Lh, out_ids);
+void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_seg,
+                 int Lh, int64_t* out_ids, float* out_scores, cudaStream_t s) {
+  const int K = check_generate(c, gp, prefix, P, hist_ids, hist_seg, Lh, out_ids);
   if (c->cross_B != B) throw StateError(fmt("generate: cross K/V prefilled for %d images, asked for %d", c->cross_B, B));
   const int T = gp.max_new_tokens;
-  const DecodeGeom g = make_geom(c, B, K, T);
+  const DecodeGeom g = make_geom(c, B, K, T, P);
+  const int64_t* pre = stage_prefix(c, B, prefix, P, s);
   // the sampling seed lives in device memory so that a captured graph can be replayed with a new seed
   c->launches += launch_set_u64((uint64_t*)c->d_seed.p, gp.seed, (uint64_t)gp.row_offset, s);
-  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_init(beam_buffers(c), B, K, T, 101, s);
-  else c->launches += launch_sample_init(B, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, T + 1, (int*)c->d_step.p, s);
+  decode_init(c, g, gp, pre, s);
 
   const bool use_graph = !(c->cfg.flags & GSTVD_FLAG_NO_CUDA_GRAPH);
   if (!use_graph) {
-    for (int t = 0; t < T; ++t) decode_step(c, g, gp, hist_ids, hist_seg, Lh, s, t);
+    prefix_prefill(c, g, s);
+    for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, hist_ids, hist_seg, Lh, s, t);
   } else {
     GraphKey key;
     std::memset(&key, 0, sizeof key);
     key.B = B; key.K = K; key.mode = gp.mode; key.T = T; key.top_k = gp.top_k; key.ngram = gp.ngram_blocking_size; key.Lh = Lh;
+    key.P = P; key.has_prefix = pre != nullptr;
     key.temperature = gp.temperature; key.top_p = gp.top_p;
     key.Le = c->cross_Le;                    // the cross cache geometry is part of the captured launch parameters
     const int64_t* g_ids = hist_ids; const int64_t* g_seg = hist_seg;
@@ -771,7 +863,8 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
       cudaGraph_t graph;
       CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
       try {
-        for (int t = 0; t < T; ++t) decode_step(c, g, gp, g_ids, g_seg, Lh, s, t);   // all T steps in ONE graph: no host round trip between steps
+        prefix_prefill(c, g, s);
+        for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, g_ids, g_seg, Lh, s, t);   // all T steps in ONE graph: no host round trip between steps
       } catch (...) {
         cudaGraph_t dead; cudaStreamEndCapture(s, &dead);
         throw;
@@ -787,7 +880,7 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
     CUDA_CHECK(cudaGraphLaunch(it->second.exec, s));
     c->launches += it->second.kernels;
   }
-  generate_finalize(c, B, K, gp, out_ids, out_scores, s);
+  generate_finalize(c, B, K, P, gp, out_ids, out_scores, s);
 }
 
 // One forward call of the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:24-120) - encoder, fusion,
@@ -796,8 +889,9 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
 // order, same results as gstvd_encode + gstvd_prefill_cross + gstvd_generate (asserted by the tests); eager when graphs are
 // disabled or while the GEMM profiler is on (events cannot be recorded inside a graph).
 void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int64_t* seg, const float* att, const float* feat,
-              const float* loc, const float* imask, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
-  const int K = check_generate(c, gp, ids, seg ? seg : ids, Lt, out_ids);
+              const float* loc, const float* imask, const gstvd_gen_params& gp, const int64_t* prefix, int P, int64_t* out_ids,
+              float* out_scores, cudaStream_t s) {
+  const int K = check_generate(c, gp, prefix, P, ids, seg ? seg : ids, Lt, out_ids);
   if (B < 1 || B > c->B_max || Lt < 1 || Lt > c->Lt_max || Lv < 1 || Lv > c->Lv_max) throw InvalidArg("round: shape exceeds capacity");
   if (!ids || !feat || !loc) throw InvalidArg("round: input_ids / image_feat / image_loc must not be NULL");
   if (gp.ngram_blocking_size > 0 && !seg) throw InvalidArg("round: n-gram blocking needs token_type_ids");
@@ -805,6 +899,7 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
   auto d2d = [&](void* dst, const void* src, size_t bytes) { if (src) CUDA_CHECK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s)); };
   d2d(c->r_ids.p, ids, (size_t)B * Lt * 8); d2d(c->r_seg.p, seg, (size_t)B * Lt * 8); d2d(c->r_att.p, att, (size_t)B * Lt * 4);
   d2d(c->r_feat.p, feat, (size_t)B * Lv * F * 4); d2d(c->r_loc.p, loc, (size_t)B * Lv * 5 * 4); d2d(c->r_imask.p, imask, (size_t)B * Lv * 4);
+  const int64_t* pre = stage_prefix(c, B, prefix, P, s);
   c->launches += launch_set_u64((uint64_t*)c->d_seed.p, gp.seed, (uint64_t)gp.row_offset, s);
   const int64_t* g_ids = (const int64_t*)c->r_ids.p;
   const int64_t* g_seg = seg ? (const int64_t*)c->r_seg.p : nullptr;
@@ -812,11 +907,11 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
     do_encode(c, B, Lt, Lv, g_ids, g_seg, att ? (const float*)c->r_att.p : nullptr, (const float*)c->r_feat.p, (const float*)c->r_loc.p,
               imask ? (const float*)c->r_imask.p : nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, s);
     do_prefill(c, B, Lv + Lt, nullptr, nullptr, s);
-    const DecodeGeom g = make_geom(c, B, K, T);
-    if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_init(beam_buffers(c), B, K, T, 101, s);
-    else c->launches += launch_sample_init(B, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, T + 1, (int*)c->d_step.p, s);
-    for (int t = 0; t < T; ++t) decode_step(c, g, gp, g_ids, g_seg, Lt, s, t);
-    generate_finalize(c, B, K, gp, (int64_t*)c->r_out_ids.p, out_scores ? (float*)c->r_out_scores.p : nullptr, s);
+    const DecodeGeom g = make_geom(c, B, K, T, P);
+    decode_init(c, g, gp, pre, s);
+    prefix_prefill(c, g, s);
+    for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, g_ids, g_seg, Lt, s, t);
+    generate_finalize(c, B, K, P, gp, (int64_t*)c->r_out_ids.p, out_scores ? (float*)c->r_out_scores.p : nullptr, s);
   };
   const bool use_graph = !(c->cfg.flags & GSTVD_FLAG_NO_CUDA_GRAPH) && !c->profiling;
   if (!use_graph) {
@@ -827,6 +922,7 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
     key.B = B; key.Lt = Lt; key.Lv = Lv; key.K = K; key.mode = gp.mode; key.T = T; key.top_k = gp.top_k; key.ngram = gp.ngram_blocking_size;
     key.has_seg = seg != nullptr; key.has_att = att != nullptr; key.has_imask = imask != nullptr;
     key.temperature = gp.temperature; key.top_p = gp.top_p;
+    key.P = P; key.has_prefix = pre != nullptr;
     if (out_scores) key.has_imask |= 2;
     auto it = c->round_graphs.find(key);
     if (it == c->round_graphs.end()) {
@@ -876,7 +972,7 @@ void do_score(gstvd_ctx* c, int B, int L, int64_t* dec_ids, const float* dec_mas
   if (!dec_ids) throw InvalidArg("score: dec_ids is NULL");
   PdlScope pdl_scope(!(c->cfg.flags & GSTVD_FLAG_NO_PDL));
   Exec X{c, s};
-  const int H = c->H, M = B * L, D = H / c->dec_heads, Le = c->cross_Le;
+  const int H = c->H, M = B * L;
   const int64_t* lab = labels;
   if (!labels) {
     c->launches += launch_shift_labels(B, L, dec_ids, (int64_t*)c->labels.p, 102, s);   // also [SEP] -> PAD in place (:53-57)
@@ -884,32 +980,7 @@ void do_score(gstvd_ctx* c, int B, int L, int64_t* dec_ids, const float* dec_mas
   }
   c->launches += launch_embed_text(c->dtype, M, L, H, dec_ids, nullptr, nullptr, 0, c->word, c->pos, c->type, c->type_ext,
                                    c->cfg.type_vocab_size, c->emb_ln.g, c->emb_ln.b, c->dh.p, s);
-  const int64_t per_image = (int64_t)2 * c->dec_heads * Le * D;
-  for (int l = 0; l < c->dec_layers; ++l) {
-    const DecLayer& Ly = c->d_layers[l];
-    X.gemm(c->dh.p, H, Ly.qkv, c->dqkv.p, 3 * H, M);
-    X.attention(c->dqkv.p, 3 * H, L, X.off(c->dqkv.p, H), X.off(c->dqkv.p, 2 * H), 3 * H, L, c->dctx.p, H, B, c->dec_heads, D, dec_mask,
-                -10000.0f, 1);
-    X.gemm(c->dctx.p, H, Ly.o, c->dtmp.p, H, M);
-    X.add_ln(c->dtmp.p, c->dh.p, Ly.ln_att, c->da.p, M);
-    X.gemm(c->da.p, H, Ly.cq, c->dqc.p, H, M);
-    {
-      AttnArgs a;
-      const char* kbase = (const char*)c->cross_cache.p + (size_t)l * (B / options) * per_image * c->esz;
-      a.q = c->dqc.p; a.q_bs = (int64_t)L * H; a.q_hs = D; a.q_rs = H;
-      a.k = kbase; a.k_bs = per_image; a.k_hs = (int64_t)Le * D; a.k_rs = D;
-      a.v = kbase + (size_t)c->dec_heads * Le * D * c->esz; a.v_bs = per_image; a.v_hs = a.k_hs; a.v_rs = D;
-      a.o = c->dctx.p; a.o_bs = (int64_t)L * H; a.o_hs = D; a.o_rs = H;
-      a.kmask = (const float*)c->fused_mask.p; a.kmask_bs = Le; a.neg = -1e9f; a.causal = 0;
-      a.B = B; a.H = c->dec_heads; a.Lq = L; a.Lk = Le; a.D = D; a.kv_batch_div = options;
-      X.run_attention(a);
-    }
-    X.gemm(c->dctx.p, H, Ly.co, c->dtmp.p, H, M);
-    X.add_ln(c->dtmp.p, c->da.p, Ly.ln_cross, c->db.p, M);
-    X.gemm(c->db.p, H, Ly.f1, c->dffn.p, c->dec_F, M, 1);
-    X.gemm(c->dffn.p, c->dec_F, Ly.f2, c->dtmp.p, H, M);
-    X.add_ln(c->dtmp.p, c->db.p, Ly.ln_out, c->dh.p, M);
-  }
+  dec_teacher_layers(c, X, B, L, dec_mask, options, nullptr);
   float* lg = out_logits ? out_logits : (float*)c->logits.p;
   const int64_t ldl = out_logits ? c->V : c->Vpad;
   X.gemm(c->dh.p, H, c->lm_head, lg, ldl, M, 0, true);
@@ -1022,7 +1093,7 @@ void gstvd_destroy(gstvd_ctx* c) {
                     &c->tmp_v, &c->ffn_t, &c->ffn_v, &c->feat_cast, &c->fused, &c->pool, &c->fused_mask, &c->dh, &c->da, &c->db, &c->dqkv,
                     &c->dctx, &c->dtmp, &c->dffn, &c->dqc, &c->logits, &c->cross_cache, &c->self_cache, &c->cross_len, &c->labels, &c->sel_val, &c->sel_idx,
                     &c->logz, &c->ban_tokens, &c->ban_count, &c->prefix, &c->seq, &c->beam_scores, &c->beam_tokens, &c->cur_tokens,
-                    &c->beam_idx, &c->beam_done, &c->hyp_score, &c->hyp_len, &c->hyp_tokens, &c->hyp_count, &c->hyp_worst, &c->d_step, &c->d_seed, &c->anc, &c->fold16, &c->foldvec,
+                    &c->beam_idx, &c->beam_done, &c->hyp_score, &c->hyp_len, &c->hyp_tokens, &c->hyp_count, &c->hyp_worst, &c->d_step, &c->d_seed, &c->anc, &c->dec_prefix_own, &c->dec_prefix_head, &c->fold16, &c->foldvec,
                     &c->st1, &c->st2, &c->st3, &c->hist_ids_own, &c->hist_seg_own, &c->r_ids, &c->r_seg, &c->r_att,
                     &c->r_feat, &c->r_loc, &c->r_imask, &c->r_out_ids, &c->r_out_scores};
   for (DevBuf* b : bufs) b->release();
@@ -1091,12 +1162,17 @@ int gstvd_prefill_cross(gstvd_ctx* c, int B, int Le, const float* enc_hidden, co
 
 int gstvd_generate(gstvd_ctx* c, int B, const gstvd_gen_params* params, const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
                    int64_t* out_ids, float* out_scores, void* stream) {
+  return gstvd_generate_prefixed(c, B, params, nullptr, 1, hist_ids, hist_segments, Lh, out_ids, out_scores, stream);
+}
+
+int gstvd_generate_prefixed(gstvd_ctx* c, int B, const gstvd_gen_params* params, const int64_t* prefix, int P, const int64_t* hist_ids,
+                            const int64_t* hist_segments, int Lh, int64_t* out_ids, float* out_scores, void* stream) {
   if (!c || !params) { g_last_error = "gstvd_generate: NULL argument"; return GSTVD_ERR_INVALID; }
   return guarded(c, [&] {
     cudaStream_t user = (cudaStream_t)stream;
     CUDA_CHECK(cudaEventRecord(c->ev_in, user));
     CUDA_CHECK(cudaStreamWaitEvent(c->own_stream, c->ev_in, 0));
-    do_generate(c, B, *params, hist_ids, hist_segments, Lh, out_ids, out_scores, c->own_stream);
+    do_generate(c, B, *params, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores, c->own_stream);
     CUDA_CHECK(cudaEventRecord(c->ev_out, c->own_stream));
     CUDA_CHECK(cudaStreamWaitEvent(user, c->ev_out, 0));
   });
@@ -1105,12 +1181,20 @@ int gstvd_generate(gstvd_ctx* c, int B, const gstvd_gen_params* params, const in
 int gstvd_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
                 const float* image_feat, const float* image_loc, const float* image_mask, const gstvd_gen_params* params, int64_t* out_ids,
                 float* out_scores, void* stream) {
+  return gstvd_round_prefixed(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, params, nullptr, 1,
+                              out_ids, out_scores, stream);
+}
+
+int gstvd_round_prefixed(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, const int64_t* token_type_ids,
+                         const float* attention_mask, const float* image_feat, const float* image_loc, const float* image_mask,
+                         const gstvd_gen_params* params, const int64_t* prefix, int P, int64_t* out_ids, float* out_scores, void* stream) {
   if (!c || !params) { g_last_error = "gstvd_round: NULL argument"; return GSTVD_ERR_INVALID; }
   return guarded(c, [&] {
     cudaStream_t user = (cudaStream_t)stream;
     CUDA_CHECK(cudaEventRecord(c->ev_in, user));
     CUDA_CHECK(cudaStreamWaitEvent(c->own_stream, c->ev_in, 0));
-    do_round(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, *params, out_ids, out_scores, c->own_stream);
+    do_round(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, *params, prefix, P, out_ids, out_scores,
+             c->own_stream);
     CUDA_CHECK(cudaEventRecord(c->ev_out, c->own_stream));
     CUDA_CHECK(cudaStreamWaitEvent(user, c->ev_out, 0));
   });
@@ -1361,7 +1445,7 @@ int gstvd_op_beam_begin(gstvd_ctx* c, int B, int K, int max_new, void* stream) {
     if (c->dec_layers == 0) throw StateError("beam ops need a decoder context");
     if (B < 1 || B > c->B_max || K < 1 || K > c->K_max || max_new < 1 || max_new > c->T_max) throw InvalidArg("beam_begin: shape out of range");
     c->op_B = B; c->op_K = K; c->op_T = max_new;
-    c->launches += launch_beam_init(beam_buffers(c), B, K, max_new, 101, (cudaStream_t)stream);
+    c->launches += launch_beam_init(beam_buffers(c), B, K, max_new, 101, nullptr, 1, (cudaStream_t)stream);
   });
 }
 
@@ -1375,7 +1459,7 @@ int gstvd_op_beam_step(gstvd_ctx* c, const float* logits, int64_t ldl, int32_t* 
     c->launches += launch_row_select(B * K, c->V, logits, ldl, 0, (const float*)c->beam_scores.p, 1.f, nullptr, nullptr, 0, nsel,
                                      (float*)c->sel_val.p, (int32_t*)c->sel_idx.p, nullptr, s);
     c->launches += launch_beam_step(beam_buffers(c), B, K, T, c->V, nsel, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, 102,
-                                    beam_idx, next_tokens, next_scores, s);
+                                    1, beam_idx, next_tokens, next_scores, s);
     c->launches += launch_step_advance((int*)c->d_step.p, s);
   });
 }
@@ -1384,7 +1468,7 @@ int gstvd_op_beam_end(gstvd_ctx* c, int64_t* out_ids, float* out_scores, void* s
   if (!c || !out_ids) return GSTVD_ERR_INVALID;
   return guarded(c, [&] {
     if (c->op_B == 0) throw StateError("beam_end before beam_begin");
-    c->launches += launch_beam_finalize(beam_buffers(c), c->op_B, c->op_K, c->op_T, 102, out_ids, out_scores, (cudaStream_t)stream);
+    c->launches += launch_beam_finalize(beam_buffers(c), c->op_B, c->op_K, c->op_T, 102, 1, out_ids, out_scores, (cudaStream_t)stream);
     c->op_B = 0;
   });
 }
@@ -1407,7 +1491,7 @@ int gstvd_op_sample(gstvd_ctx* c, int rows, const float* logits, int64_t ldl, co
       if (!hist_ids || !hist_segments || !prefix || prefix_len != step + 1) throw InvalidArg("op_sample: n-gram blocking needs history and a prefix of step+1 tokens");
       CUDA_CHECK(cudaMemsetAsync(c->prefix.p, 0, c->prefix.bytes, s));
       c->launches += launch_build_prefix_from_ids(rows, prefix_len, prefix, (int32_t*)c->prefix.p, T + 1, 102, s);
-      c->launches += launch_ngram_ban(rows, Lh, hist_ids, hist_segments, (const int32_t*)c->prefix.p, T + 1, (const int*)c->d_step.p,
+      c->launches += launch_ngram_ban(rows, Lh, hist_ids, hist_segments, (const int32_t*)c->prefix.p, T + 1, (const int*)c->d_step.p, 1,
                                       gp->ngram_blocking_size, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }

@@ -106,8 +106,8 @@ int launch_ln_apply_stats(int rows, int width, const void* x, const float2* stat
 int launch_embed_text(int dtype, int rows, int L, int width, const int64_t* ids, const int64_t* seg, const int* d_pos_offset,
                       int eos_to_pad, const float* word, const float* pos, const float* type, const float* type_ext,
                       int type_vocab, const float* gamma, const float* beta, void* y, cudaStream_t stream);
-// decode-step embeddings from int32 current tokens (EOS -> PAD applied), position *d_step
-int launch_embed_step(int dtype, int rows, int width, const int32_t* tokens, const int* d_step, const float* word,
+// decode-step embeddings from int32 current tokens (EOS -> PAD applied), position pos0 + *d_step
+int launch_embed_step(int dtype, int rows, int width, const int32_t* tokens, int pos0, const int* d_step, const float* word,
                       const float* pos, const float* type, const float* gamma, const float* beta, void* y, cudaStream_t stream);
 // image embeddings: y = LN(x(+bias already) + loc * Wloc^T + bloc)
 int launch_image_embed_ln(int dtype, int rows, int width, const void* x, const float* loc, const float* wloc,
@@ -127,19 +127,23 @@ int launch_gather_first_rows(int dtype, int B, int L, int width, const void* src
 
 // ---- decode-step kernels (persistent KV cache) ------------------------------------------------------------
 struct DecodeGeom {
-  int B, K, H, heads, D, layers, T;   // T = max positions in the self cache
+  int B, K, H, heads, D, layers, T;   // T = max positions in the self cache (P0 + new tokens)
   int Le;                             // encoder length (cross keys)
+  int P0 = 0;                         // decoder prefix length - 1: cache positions 0..P0-1 hold the prefix (launch_prefix_kv_store)
 };
-// self-attention for one new position per row: appends k/v at position *d_step and attends over 0..*d_step
+// self-attention for one new position per row: appends k/v at position P0 + *d_step and attends over 0..P0 + *d_step
 // qkv [M, 3H]; cache layout [layer][kv][b][t][k][H]
 // step_host >= 0: the caller knows the step index (must equal *d_step); the lean kernel then only loads positions <= step
 int launch_dec_self_attn(int dtype, const DecodeGeom& g, int layer, const void* qkv, void* self_cache, const int* d_step, int step_host,
                          const uint8_t* anc, void* out, cudaStream_t stream);
 // the lean bf16 / 64-dim kernel will run for these arguments (default on; env GSTVD_SELF_V2=0 disables it)
 bool dec_self_attn_v2_active(int dtype, const DecodeGeom& g, const void* qkv, const void* self_cache, const void* out);
-// anc: uint8 [B*K][32] ancestry table (slot that holds position t of beam k's history), permuted instead of gathering the cache;
+// anc: uint8 [B*K][32] (rows of 64 when g.T > 32) ancestry table (slot that holds position t of beam k's history), permuted instead of gathering the cache;
 // only the lean kernel reads it - pass null to the self-attention and call launch_reorder_cache otherwise
 int launch_anc_update(const DecodeGeom& g, const int32_t* beam_idx, const int* d_step, uint8_t* anc, cudaStream_t stream);
+// decoder prefix prefill: stores layer `layer`'s K / V of the qkv rows [B * P0][3H] (teacher-forced pass over the first P0 prefix
+// positions) into every beam slot of cache positions 0..P0-1; launches nothing when P0 = 0
+int launch_prefix_kv_store(int dtype, const DecodeGeom& g, int layer, const void* qkv, void* self_cache, cudaStream_t stream);
 // cross-attention of every beam row over its image's cross K/V. cross layout [layer][b][kv*heads+h][Le][D]
 int launch_dec_cross_attn(int dtype, const DecodeGeom& g, int layer, const void* q, const void* cross_cache,
                           const float* enc_mask, void* out, cudaStream_t stream);
@@ -179,22 +183,24 @@ struct BeamBuffers {
   double* hyp_worst;       // [B]
   int* d_step;             // device step counter
 };
-int launch_beam_init(const BeamBuffers& bb, int B, int K, int T, int start_token, cudaStream_t stream);
+// prefix: int64 [B, P] decoder prefix (null: start_token, P = 1); len0 = P, the prefix length counted in every hypothesis length
+int launch_beam_init(const BeamBuffers& bb, int B, int K, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream);
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int T, int V, int nsel, const float* sel_val,
-                     const int32_t* sel_idx, int eos, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
+                     const int32_t* sel_idx, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
                      cudaStream_t stream);
-int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int64_t* out_ids, float* out_scores,
+int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int64_t* out_ids, float* out_scores,
                          cudaStream_t stream);
 
 // n-gram blocking (utils/decoding_utils.py:38-78): ban list per row from the question history and the decoded prefix.
-// prefix_tokens int32 [rows, T+1] (start token at 0, EOS already replaced by PAD), prefix_len = *d_step + 1
+// prefix_tokens int32 [rows, P+T] (decoder prefix of len0 = P tokens, then the generated ones; EOS already replaced by PAD),
+// prefix_len = *d_step + len0
 int launch_ngram_ban(int rows, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
-                     int prefix_stride, const int* d_step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
+                     int prefix_stride, const int* d_step, int len0, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
                      cudaStream_t stream);
-// the same for the B*K beam rows: key = the last n-1 tokens of beam row b*K+k in `tokens` [B, K, T] (the beam token buffer of
-// this step's parity); history row = b.  Needs n - 1 <= step < T (earlier keys hold the start token and ban nothing).
-int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* tokens, int step,
-                          int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream);
+// the same for the B*K beam rows: key = the last n-1 tokens of prefix_b ([SEP] read as [PAD]; null: [CLS], P = 1) followed by beam
+// row b*K+k of `tokens` [B, K, T] (the beam token buffer of this step's parity); history row = b.  Needs n - 1 <= P + step, step < T.
+int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int64_t* prefix, int P,
+                          const int32_t* tokens, int step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream);
 // sample-mode selection from row_select output; writes seq[row, step] and cur_tokens[row], prefix[row, step+1]
 // top_k == 0: multinomial over the whole (optionally nucleus-filtered) vocabulary; writes the same state as launch_sample_step
 int launch_full_vocab_sample(int rows, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,
@@ -204,8 +210,9 @@ int launch_full_vocab_sample(int rows, int V, const float* logits, int64_t ldl, 
 int launch_sample_step(int rows, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
                        uint64_t seed, uint64_t row_offset, const uint64_t* d_seed, const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
                        int prefix_stride, int32_t* out_tokens, cudaStream_t stream);
+// dec_prefix: int64 [rows, P] decoder prefix (null: start_token, P = 1); the key buffer `prefix` [rows, prefix_stride >= P + T]
 int launch_sample_init(int rows, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                       int prefix_stride, int* d_step, cudaStream_t stream);
+                       int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, cudaStream_t stream);
 int launch_sample_finalize(int rows, int T, int eos, const int32_t* seq, int64_t* out_ids, cudaStream_t stream);
 int launch_step_advance(int* d_step, cudaStream_t stream);
 // device-side scalar set (a pageable-memory cudaMemcpyAsync would synchronise the stream with the host)

@@ -173,7 +173,7 @@ embed_text_kernel(int rows, int L, int width, const int64_t* __restrict__ ids, c
 
 template <typename T>
 __global__ void __launch_bounds__(kRowsPerBlock * 32)
-embed_step_kernel(int rows, int width, const int32_t* __restrict__ tokens, const int* __restrict__ d_step,
+embed_step_kernel(int rows, int width, const int32_t* __restrict__ tokens, int pos0, const int* __restrict__ d_step,
                   const float* __restrict__ word, const float* __restrict__ pos, const float* __restrict__ type,
                   const float* __restrict__ gamma, const float* __restrict__ beta, T* __restrict__ y) {
   pdl_wait();
@@ -183,7 +183,7 @@ embed_step_kernel(int rows, int width, const int32_t* __restrict__ tokens, const
   if (row >= rows) return;
   int id = tokens[row];
   if (id == 102) id = 0;      // the decoder never sees [SEP] as an input (models/visual_dialog_decoder.py:57)
-  const int p = *d_step;
+  const int p = pos0 + *d_step;   // pos0 = decoder prefix length - 1
   float v[kMaxChunks][8];
 #pragma unroll
   for (int c = 0; c < kMaxChunks; ++c) {
@@ -411,14 +411,14 @@ int launch_embed_text(int dtype, int rows, int L, int width, const int64_t* ids,
   return 1;
 }
 
-int launch_embed_step(int dtype, int rows, int width, const int32_t* tokens, const int* d_step, const float* word,
+int launch_embed_step(int dtype, int rows, int width, const int32_t* tokens, int pos0, const int* d_step, const float* word,
                       const float* pos, const float* type, const float* gamma, const float* beta, void* y, cudaStream_t stream) {
   if (rows <= 0) return 0;
   check_width(width);
   if (dtype == kF32)
-    launch_k(embed_step_kernel<float>, grid_rows(rows), kRowsPerBlock * 32, 0, stream, rows, width, tokens, d_step, word, pos, type, gamma, beta, (float*)y);
+    launch_k(embed_step_kernel<float>, grid_rows(rows), kRowsPerBlock * 32, 0, stream, rows, width, tokens, pos0, d_step, word, pos, type, gamma, beta, (float*)y);
   else
-    launch_k(embed_step_kernel<bf16>, grid_rows(rows), kRowsPerBlock * 32, 0, stream, rows, width, tokens, d_step, word, pos, type, gamma, beta, (bf16*)y);
+    launch_k(embed_step_kernel<bf16>, grid_rows(rows), kRowsPerBlock * 32, 0, stream, rows, width, tokens, pos0, d_step, word, pos, type, gamma, beta, (bf16*)y);
   return 1;
 }
 

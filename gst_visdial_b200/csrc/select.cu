@@ -416,13 +416,14 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
 }
 
 // ------------------------------------------------------------------------------------------------------------
-__global__ void beam_init_kernel(BeamBuffers bb, int B, int K, int T, int start_token) {
+// prefix != null: int64 [B, P] decoder prefix shared by the K beams of an image; the first step's input is its last token
+__global__ void beam_init_kernel(BeamBuffers bb, int B, int K, int T, int start_token, const int64_t* __restrict__ prefix, int P) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0) *bb.d_step = 0;
   if (i < B) { bb.done[i] = 0; bb.hyp_count[i] = 0; bb.hyp_worst[i] = 1e9; }
   if (i < B * K) {
     bb.beam_scores[i] = (i % K == 0) ? 0.f : -1e9f;
-    bb.cur_tokens[i] = start_token;
+    bb.cur_tokens[i] = prefix ? (int32_t)prefix[(int64_t)(i / K) * P + P - 1] : start_token;
     bb.beam_idx[i] = i % K;
   }
   for (int j = i; j < 2 * B * K * T; j += gridDim.x * blockDim.x) bb.tokens[j] = 0;
@@ -465,7 +466,7 @@ __device__ void hyp_add(const BeamBuffers& bb, int b, int K, int T, const int32_
 constexpr int kBeamWarps = 4;
 __global__ void __launch_bounds__(kBeamWarps * 32)
 beam_step_kernel(BeamBuffers bb, int B, int K, int T, int V, int nsel, const float* __restrict__ sel_val,
-                 const int32_t* __restrict__ sel_idx, int eos, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
+                 const int32_t* __restrict__ sel_idx, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
   __shared__ float s_val[kBeamWarps][128];
   __shared__ int s_flat[kBeamWarps][128];
   __shared__ int s_order[kBeamWarps][16];
@@ -477,7 +478,7 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int T, int V, int nsel, const flo
   const int b = blockIdx.x * kBeamWarps + warp;
   if (b >= B) return;
   const int t = *bb.d_step;
-  const int cur_len = t + 1;
+  const int cur_len = t + len0;                // HF input_ids.shape[-1]: decoder prefix (len0 tokens) + t generated
   const int32_t* src = bb.tokens + (int64_t)(t & 1) * B * K * T + (int64_t)b * K * T;
   int32_t* dst = bb.tokens + (int64_t)((t + 1) & 1) * B * K * T + (int64_t)b * K * T;
   const int n = K * nsel;                      // <= 8 * 16 = 128
@@ -539,14 +540,14 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int T, int V, int nsel, const flo
   }
 }
 
-__global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eos, int64_t* out_ids, float* out_scores) {
+__global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eos, int len0, int64_t* out_ids, float* out_scores) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const int t = *bb.d_step;                     // steps executed
   const int HK = K + 1;
   if (!bb.done[b]) {
     const int32_t* cur = bb.tokens + (int64_t)(t & 1) * B * K * T + (int64_t)b * K * T;
-    for (int k = 0; k < K; ++k) hyp_add(bb, b, K, T, cur + (int64_t)k * T, t, bb.beam_scores[b * K + k], t + 1);
+    for (int k = 0; k < K; ++k) hyp_add(bb, b, K, T, cur + (int64_t)k * T, t, bb.beam_scores[b * K + k], t + len0);
   }
   const double* hs = bb.hyp_score + (int64_t)b * HK;
   const int cnt = bb.hyp_count[b];
@@ -563,7 +564,7 @@ __device__ __forceinline__ bool is_special(int64_t t) { return t == 0 || (t >= 1
 
 __global__ void __launch_bounds__(256)
 ngram_ban_kernel(int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __restrict__ hist_seg,
-                 const int32_t* __restrict__ prefix, int prefix_stride, const int* __restrict__ d_step, int n,
+                 const int32_t* __restrict__ prefix, int prefix_stride, const int* __restrict__ d_step, int len0, int n,
                  int32_t* __restrict__ ban_tokens, int32_t* __restrict__ ban_count, int ban_stride) {
   __shared__ int cnt;
   pdl_wait();
@@ -571,7 +572,7 @@ ngram_ban_kernel(int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __
   const int row = blockIdx.x;
   if (threadIdx.x == 0) cnt = 0;
   __syncthreads();
-  const int cur_len = *d_step + 1;
+  const int cur_len = *d_step + len0;                    // decoder prefix (len0 tokens) + generated
   const int start = cur_len + 1 - n;
   if (start >= 0) {                                      // a shorter key can never equal an (n-1)-gram
     const int64_t* ids = hist_ids + (int64_t)row * Lh;
@@ -595,22 +596,28 @@ ngram_ban_kernel(int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __
 }
 
 // Beam mode: one CTA per image scans its question history once and tests every n-gram against the K beam keys.  The key of beam
-// k at step t is the last n-1 tokens of [CLS] + tokens[b, k, :t]; the host launches this only for t >= n-1, where the key lies
-// inside the generated tokens (an earlier key holds the [CLS], and n-grams with a special id are never banned).  Ban lists are
-// per beam row b*K + k.
+// k at step t is the last n-1 tokens of prefix_b + tokens[b, k, :t], with prefix_b the image's decoder prefix ([SEP] read as
+// [PAD]; [CLS] when prefix is null, P = 1).  The host launches this only when P + t >= n-1 (a shorter key bans nothing) and, for
+// the [CLS] start, only once the key has left it (n-grams with a special id are never banned).  Ban lists are per beam row b*K + k.
 constexpr int kBanMaxK = 8;
 __global__ void __launch_bounds__(256)
 beam_ngram_ban_kernel(int K, int T, int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __restrict__ hist_seg,
-                      const int32_t* __restrict__ tokens, int step, int n, int32_t* __restrict__ ban_tokens,
-                      int32_t* __restrict__ ban_count, int ban_stride) {
+                      const int64_t* __restrict__ prefix, int P, const int32_t* __restrict__ tokens, int step, int n,
+                      int32_t* __restrict__ ban_tokens, int32_t* __restrict__ ban_count, int ban_stride) {
   __shared__ int32_t s_key[kBanMaxK][kHypMaxT];
   __shared__ int s_cnt[kBanMaxK];
   pdl_wait();
   pdl_launch_dependents();
-  const int b = blockIdx.x, klen = n - 1, first = step - klen;
+  const int b = blockIdx.x, klen = n - 1, first = P + step - klen;   // first key position in prefix + generated tokens
   for (int i = threadIdx.x; i < K * klen; i += blockDim.x) {
-    const int k = i / klen, j = i - k * klen;
-    s_key[k][j] = tokens[((int64_t)b * K + k) * T + first + j];
+    const int k = i / klen, j = i - k * klen, q = first + j;
+    int32_t w;
+    if (q >= P) w = tokens[((int64_t)b * K + k) * T + q - P];
+    else {
+      w = prefix ? (int32_t)prefix[(int64_t)b * P + q] : 101;
+      if (w == 102) w = 0;                               // the decoder input holds [PAD] where the prefix has [SEP]
+    }
+    s_key[k][j] = w;
   }
   if (threadIdx.x < K) s_cnt[threadIdx.x] = 0;
   __syncthreads();
@@ -641,15 +648,19 @@ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
   return x ^ (x >> 31);
 }
 
+// dec_prefix != null: int64 [rows, P] decoder prefix; `prefix` (the n-gram key buffer) starts with it, [SEP] read as [PAD]
 __global__ void sample_init_kernel(int rows, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                                   int prefix_stride, int* d_step) {
+                                   int prefix_stride, int* d_step, const int64_t* __restrict__ dec_prefix, int P) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0) *d_step = 0;
   if (i < rows) {
-    cur_tokens[i] = start_token;
+    cur_tokens[i] = dec_prefix ? (int32_t)dec_prefix[(int64_t)i * P + P - 1] : start_token;
     for (int j = 0; j < T; ++j) seq[(int64_t)i * T + j] = 0;
     for (int j = 0; j < prefix_stride; ++j) prefix[(int64_t)i * prefix_stride + j] = 0;
-    prefix[(int64_t)i * prefix_stride] = start_token;
+    for (int j = 0; j < P; ++j) {
+      const int32_t w = dec_prefix ? (int32_t)dec_prefix[(int64_t)i * P + j] : start_token;
+      prefix[(int64_t)i * prefix_stride + j] = w == 102 ? 0 : w;
+    }
   }
 }
 
@@ -942,35 +953,36 @@ int launch_row_select(int rows, int V, const float* logits, int64_t ldl, int mod
   return 1;
 }
 
-int launch_beam_init(const BeamBuffers& bb, int B, int K, int T, int start_token, cudaStream_t stream) {
+int launch_beam_init(const BeamBuffers& bb, int B, int K, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream) {
   const int n = B * K;
-  beam_init_kernel<<<(n + 255) / 256, 256, 0, stream>>>(bb, B, K, T, start_token);
+  beam_init_kernel<<<(n + 255) / 256, 256, 0, stream>>>(bb, B, K, T, start_token, prefix, P);
   return 1;
 }
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int T, int V, int nsel, const float* sel_val,
-                     const int32_t* sel_idx, int eos, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
+                     const int32_t* sel_idx, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
                      cudaStream_t stream) {
   if (K > 8 || T > kHypMaxT) throw std::runtime_error("beam_step: K <= 8 and T <= 32");
-  launch_k(beam_step_kernel, dim3((B + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, B, K, T, V, nsel, sel_val, sel_idx, eos, out_beam_idx, out_tokens, out_scores);
+  launch_k(beam_step_kernel, dim3((B + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, B, K, T, V, nsel, sel_val, sel_idx, eos, len0, out_beam_idx, out_tokens, out_scores);
   return 1;
 }
-int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int64_t* out_ids, float* out_scores,
+int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int64_t* out_ids, float* out_scores,
                          cudaStream_t stream) {
-  beam_finalize_kernel<<<(B + 31) / 32, 32, 0, stream>>>(bb, B, K, T, eos, out_ids, out_scores);
+  beam_finalize_kernel<<<(B + 31) / 32, 32, 0, stream>>>(bb, B, K, T, eos, len0, out_ids, out_scores);
   return 1;
 }
 int launch_ngram_ban(int rows, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
-                     int prefix_stride, const int* d_step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
+                     int prefix_stride, const int* d_step, int len0, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
                      cudaStream_t stream) {
   if (rows <= 0) return 0;
-  launch_k(ngram_ban_kernel, dim3(rows), dim3(256), 0, stream, Lh, hist_ids, hist_seg, prefix, prefix_stride, d_step, n, ban_tokens, ban_count, ban_stride);
+  launch_k(ngram_ban_kernel, dim3(rows), dim3(256), 0, stream, Lh, hist_ids, hist_seg, prefix, prefix_stride, d_step, len0, n, ban_tokens, ban_count, ban_stride);
   return 1;
 }
-int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* tokens, int step,
-                          int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream) {
+int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int64_t* prefix, int P,
+                          const int32_t* tokens, int step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream) {
   if (B <= 0) return 0;
-  if (K > kBanMaxK || n < 1 || n - 1 > step || step >= T || T > kHypMaxT) throw std::runtime_error("beam_ngram_ban: K <= 8, 1 <= n <= step + 1, step < T <= 32");
-  launch_k(beam_ngram_ban_kernel, dim3(B), dim3(256), 0, stream, K, T, Lh, hist_ids, hist_seg, tokens, step, n, ban_tokens, ban_count, ban_stride);
+  if (K > kBanMaxK || n < 1 || n - 1 > P + step || n - 1 > kHypMaxT || step >= T || T > kHypMaxT || P < 1 || (P > 1 && !prefix))
+    throw std::runtime_error("beam_ngram_ban: K <= 8, 1 <= n <= min(P + step, 32) + 1, step < T <= 32, prefix given when P > 1");
+  launch_k(beam_ngram_ban_kernel, dim3(B), dim3(256), 0, stream, K, T, Lh, hist_ids, hist_seg, prefix, P, tokens, step, n, ban_tokens, ban_count, ban_stride);
   return 1;
 }
 int launch_sample_step(int rows, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
@@ -999,8 +1011,9 @@ int launch_full_vocab_sample(int rows, int V, const float* logits, int64_t ldl, 
   return 1;
 }
 int launch_sample_init(int rows, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                       int prefix_stride, int* d_step, cudaStream_t stream) {
-  sample_init_kernel<<<(rows + 63) / 64, 64, 0, stream>>>(rows, T, start_token, seq, cur_tokens, prefix, prefix_stride, d_step);
+                       int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, cudaStream_t stream) {
+  if (P < 1 || P > prefix_stride || (P > 1 && !dec_prefix)) throw std::runtime_error("sample_init: 1 <= P <= prefix_stride, prefix given when P > 1");
+  sample_init_kernel<<<(rows + 63) / 64, 64, 0, stream>>>(rows, T, start_token, seq, cur_tokens, prefix, prefix_stride, d_step, dec_prefix, P);
   return 1;
 }
 int launch_sample_finalize(int rows, int T, int eos, const int32_t* seq, int64_t* out_ids, cudaStream_t stream) {

@@ -59,7 +59,7 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
         self.config = {"encoder": encoder.config.to_dict(), "decoder": decoder.config.to_dict()}
         self._init_engine_state(params)
         self._calls = 0
-        self._start_checked = False
+        self._cls_start = None                # (tensor, version) last found to be all [CLS], see _decoder_prefix
         encoder._version = self._version      # one change counter for the whole model
         # plain attributes, not sub-modules: a registered back-reference would make the module tree cyclic
         object.__setattr__(encoder, "_owner", self)
@@ -132,7 +132,7 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
                               want_logits=decoding_kwargs.get("want_logits", True))
             return out.loss, out.logits
 
-        # decode mode (models/visual_dialog_model.py:74-120): 18 new tokens, PAD after the first [SEP]
+        # decode mode (models/visual_dialog_model.py:74-120): 18 new tokens after the caller's dec_input_ids, PAD after the first [SEP]
         self._check_decoder_start(dec_input_ids)
         self._calls += 1
         seed = decoding_kwargs.get("seed")
@@ -151,15 +151,15 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
             seed=seed,
             row_offset=int(decoding_kwargs.get("row_offset", 0)),
         )
+        gen_kw["prefix"] = self._decoder_prefix(dec_input_ids, B, gen_kw["num_beams"], gen_kw["ngram_blocking_size"])
         if whole_round:
             # the n-gram blocking history is the (trimmed) encoder input itself: positions past the bound hold no token
             return eng.round(ids_e, enc_image_features, enc_image_spatials, seg_e, att_e, enc_image_mask, **gen_kw)
         return eng.generate(B, hist_ids=enc_input_ids, hist_segments=enc_segments, **gen_kw)
 
     def _check_decoder_start(self, dec_input_ids):
-        """The reference continues from whatever prefix the caller passes (models/visual_dialog_model.py:86-110); every caller on
-        the path passes a single [CLS] (generate.py:111, dataloader_cc12m_gen.py:99).  The engine's cached decode starts from
-        bos_token_id, so anything else is refused instead of silently ignored."""
+        """The reference continues from whatever prefix the caller passes (models/visual_dialog_model.py:86-110), and so does the
+        engine (include/gstvd.h gstvd_generate_prefixed); its token bookkeeping needs the BERT bos / eos ids."""
         if dec_input_ids is None:
             return
         bos = int(getattr(self.decoder.config, "bos_token_id", 101) or 101)
@@ -168,10 +168,21 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
             # the engine's token bookkeeping (start token, [SEP] -> [PAD] in the prefix, end of hypothesis) uses the BERT ids the
             # reference's configs carry (config/bert_base_6layer_6conect_dec.json: bos 101, eos 102)
             raise NotImplementedError(f"the engine decodes with bos_token_id 101 / eos_token_id 102; the decoder config says {bos} / {eos}")
-        if dec_input_ids.dim() != 2 or dec_input_ids.shape[1] != 1:
-            raise ValueError(f"decode mode starts from one start token per row (dec_input_ids [B, 1]), got {tuple(dec_input_ids.shape)}")
-        if not self._start_checked:
-            # one host read per model instance (a device sync): later calls of the round loop pass the same tensor
-            if not bool((dec_input_ids == bos).all()):
-                raise ValueError(f"decode mode starts from bos_token_id = {bos}; other prefixes are not supported")
-            self._start_checked = True
+
+    def _decoder_prefix(self, dec_input_ids, B, num_beams, ngram_blocking_size):
+        """The decoder input the engine continues from: ``dec_input_ids`` [B, P], or None for one [CLS] per row.  None is only
+        chosen where it changes the work: beam search with n-gram blocking skips the ban kernel of steps whose keys still hold a
+        known [CLS] start, so a single-column all-[CLS] start is passed as None there (one host read per new tensor; the round loop
+        passes the same tensor again).  Elsewhere the engine reads the start token on the device."""
+        if dec_input_ids is None:
+            return None
+        if dec_input_ids.dim() != 2 or dec_input_ids.shape[0] != B:
+            raise ValueError(f"dec_input_ids must be [B={B}, P], got {tuple(dec_input_ids.shape)}")
+        if dec_input_ids.shape[1] == 1 and num_beams > 1 and ngram_blocking_size > 0:
+            seen = self._cls_start
+            if seen is not None and seen[0] is dec_input_ids and seen[1] == dec_input_ids._version:
+                return None
+            if bool((dec_input_ids == 101).all()):
+                self._cls_start = (dec_input_ids, dec_input_ids._version)
+                return None
+        return dec_input_ids

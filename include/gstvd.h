@@ -149,6 +149,18 @@ int gstvd_generate(gstvd_ctx* ctx, int B, const gstvd_gen_params* params,
                    const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
                    int64_t* out_ids, float* out_scores, void* stream);
 
+/* gstvd_generate continuing from a caller-supplied decoder prefix, the reference's dec_input_ids (models/visual_dialog_model.py:86-110
+ * continues from whatever the caller passes).  gstvd_generate is this call with prefix = NULL, P = 1.
+ *   prefix : int64 [B, P], 1 <= P <= max_dec_len, shared by the beams of an image; NULL means one [CLS] per row (P must be 1).  At every
+ *            step the decoder sees prefix + the tokens generated so far at positions 0 .. P-1+t, without a padding mask; a [SEP] in the
+ *            prefix is read as [PAD] (models/visual_dialog_decoder.py:57).  n-gram keys may reach into the prefix.  Beam hypotheses
+ *            count the prefix in their length (HF beam_search input_ids.shape[-1]).  The caller's tensor is not modified.
+ *   P - 1 + max_new_tokens must not exceed 64 (cached positions of the decode kernels) nor max_position_embeddings.
+ *   out_ids holds the new tokens only, as in gstvd_generate. */
+int gstvd_generate_prefixed(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, const int64_t* prefix, int P,
+                            const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
+                            int64_t* out_ids, float* out_scores, void* stream);
+
 /* One whole forward call of the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:24-120): the same work and
  * results as gstvd_encode (no exported outputs) + gstvd_prefill_cross(resident states) + gstvd_generate, replayed from ONE CUDA graph
  * per shape - the host enqueues a few device-to-device copies of the inputs and one graph launch.  The n-gram blocking history is the
@@ -158,6 +170,13 @@ int gstvd_round(gstvd_ctx* ctx, int B, int Lt, int Lv,
                 const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
                 const float* image_feat, const float* image_loc, const float* image_mask,
                 const gstvd_gen_params* params, int64_t* out_ids, float* out_scores, void* stream);
+
+/* gstvd_round continuing from a decoder prefix [B, P] (NULL, P = 1: the [CLS] start); the prefix contract of gstvd_generate_prefixed. */
+int gstvd_round_prefixed(gstvd_ctx* ctx, int B, int Lt, int Lv,
+                         const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
+                         const float* image_feat, const float* image_loc, const float* image_mask,
+                         const gstvd_gen_params* params, const int64_t* prefix, int P,
+                         int64_t* out_ids, float* out_scores, void* stream);
 
 /* Replaces VisualDialogDecoder.forward in loss mode (models/visual_dialog_decoder.py:33-86) as driven by
  * generate.py:183-209 and evaluate_gen.py:94-106: teacher-forced pass over dec_ids [B, L].
