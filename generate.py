@@ -5,6 +5,7 @@ generate.py: same single-dash flags, same output JSON layout), running on the B2
     python generate.py -mode cc12m_gen -start_path_q ckpt_q -start_path_a ckpt_a -cc12m_image_feats ... -save_name out.json
     python generate.py -synthetic 128 -batch_size 64 -num_beams 5          # seeded synthetic images + random weights
     python generate.py -synthetic 128 -batch_size 64 -num_beams 5 -q_num_beams 5   # beam-searched questions too (4-gram blocked)
+    python generate.py -synthetic 128 -batch_size 64 -answer_candidates 5          # 5 sampled answers per round, lowest perplexity kept
 
 Multi-GPU: launch with torchrun (one process per GPU); images are sharded by rank and gathered once at the end.
 The dataset readers (LMDB / tokenizer) of the reference are host I/O outside the hot path: without them (-synthetic)
@@ -112,7 +113,8 @@ def main(argv=None):
                 # sampling keyed by (-seed, model role, round, GLOBAL image index, step): the tokens of an image do not depend on the
                 # batch size or on how many ranks share the job
                 res = generate_dialogs(a_model, batch, q_model=q_model, num_rounds=params['num_rounds'], a_kwargs=a_kwargs, q_kwargs=q_kwargs,
-                                       with_ppl=True, device=params['device'], seed=params.get('seed', 0), row_offset=span_start)
+                                       with_ppl=True, device=params['device'], seed=params.get('seed', 0), row_offset=span_start,
+                                       answer_candidates=params['answer_candidates'])
                 meta = {int(i): {"url": "", "caption": (decode or ids_to_text)(IOO.strip_ids(row) if decode else row)}
                         for i, row in zip(batch["image_id"].tolist(), batch["enc_input_ids"].tolist())}
                 writer.write(IOO.batch_records(batch["image_id"], res.questions, res.answers, res.answer_ppl, res.abnormal,

@@ -68,9 +68,9 @@ struct DevBuf {
 
 // Shapes and selection parameters only: the n-gram blocking history and the decoder prefix are copied into context-owned buffers
 // before a replay, so the caller's tensor addresses are not part of the key (a caching allocator hands out a new address per batch).
-// P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start.
+// P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start; N = sequences returned per image.
 struct GraphKey {
-  int B, K, mode, T, top_k, ngram, Lh, Le, P, has_prefix; float temperature, top_p;
+  int B, K, mode, T, top_k, ngram, Lh, Le, P, has_prefix, N; float temperature, top_p;
   bool operator<(const GraphKey& o) const { return std::memcmp(this, &o, sizeof(GraphKey)) < 0; }
 };
 constexpr size_t kMaxGraphs = 24;      // least-recently-used graphs beyond this are destroyed (an 18-step graph holds ~2k kernel nodes)
@@ -111,7 +111,7 @@ struct gstvd_ctx {
   DevBuf cross_len;                                   // int32 [B]: keys up to the last unmasked one (launch_cross_len)
   DevBuf labels;                                      // int64 [B*Ldec]
   DevBuf sel_val, sel_idx, logz;                      // [rows, kSelMax]
-  DevBuf ban_tokens, ban_count, prefix, seq;          // sample-mode state
+  DevBuf ban_tokens, ban_count, prefix, seq;          // sample-mode state, one row per decode row (B*K: sampled candidates)
   DevBuf beam_scores, beam_tokens, cur_tokens, beam_idx, beam_done, hyp_score, hyp_len, hyp_tokens, hyp_count, hyp_worst;
   DevBuf d_step, d_seed;
   DevBuf anc;                                         // uint8 [B*K][64]: beam ancestry table (launch_anc_update; rows of 32 up to 32 positions)
@@ -130,7 +130,7 @@ struct gstvd_ctx {
   uint64_t graph_clock = 0;
   // whole-round graphs (gstvd_round): encoder + cross-K/V prefill + every decode step of one forward call in ONE graph, keyed by shapes
   struct RoundKey {
-    int B, Lt, Lv, K, mode, T, top_k, ngram, has_seg, has_att, has_imask, P, has_prefix; float temperature, top_p;
+    int B, Lt, Lv, K, mode, T, top_k, ngram, has_seg, has_att, has_imask, P, has_prefix, N; float temperature, top_p;
     bool operator<(const RoundKey& o) const { return std::memcmp(this, &o, sizeof(RoundKey)) < 0; }
   };
   std::map<RoundKey, GraphEntry> round_graphs;
@@ -339,8 +339,9 @@ void alloc_workspace(gstvd_ctx* c) {
     c->hist_ids_own.alloc(B * Lt * 8); c->hist_seg_own.alloc(B * Lt * 8);
     c->r_ids.alloc(B * Lt * 8); c->r_seg.alloc(B * Lt * 8); c->r_att.alloc(B * Lt * 4);
     c->r_feat.alloc(B * Lv * (size_t)c->cfg.v_feature_size * 4); c->r_loc.alloc(B * Lv * 5 * 4); c->r_imask.alloc(B * Lv * 4);
-    c->r_out_ids.alloc(B * T * 8); c->r_out_scores.alloc(B * 4);
-    c->prefix.alloc(B * (T + c->Ldec_max) * 4); c->seq.alloc(B * T * 4);
+    // outputs and sample-mode state hold up to K_max rows per image: N-best beams / N sampled candidates
+    c->r_out_ids.alloc(B * K * T * 8); c->r_out_scores.alloc(B * K * 4);
+    c->prefix.alloc(B * K * (T + c->Ldec_max) * 4); c->seq.alloc(B * K * T * 4);
     c->dec_prefix_own.alloc(B * c->Ldec_max * 8); c->dec_prefix_head.alloc(B * c->Ldec_max * 8);
     c->beam_scores.alloc(B * K * 4); c->beam_tokens.alloc(2 * B * K * T * 4); c->cur_tokens.alloc(R * 4);
     c->beam_idx.alloc(B * K * 4); c->beam_done.alloc(B); c->hyp_score.alloc(B * (K + 1) * 8);
@@ -670,7 +671,7 @@ const int64_t* stage_prefix(gstvd_ctx* c, int B, const int64_t* prefix, int P, c
 void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* prefix, cudaStream_t s) {
   const int P = g.P0 + 1, T = gp.max_new_tokens;
   if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, T, 101, prefix, P, s);
-  else c->launches += launch_sample_init(g.B, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, P + T, (int*)c->d_step.p,
+  else c->launches += launch_sample_init(g.B * g.K, g.K, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, P + T, (int*)c->d_step.p,
                                          prefix, P, s);
 }
 
@@ -761,33 +762,35 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
   } else {
+    // g.K rows per image: the sampled candidates of gstvd_generate_candidates, each with its own n-gram key and RNG stream
     const int nsel = kSelMax;
     const int32_t* bt = nullptr; const int32_t* bc = nullptr;
     // key buffer c->prefix [M, P + Tn]: the decoder prefix, then the generated tokens; the samplers append token t at P + t
     const int kst = P + Tn;
     int32_t* key_next = (int32_t*)c->prefix.p + (P - 1);
     if (gp.ngram_blocking_size > 0) {
-      c->launches += launch_ngram_ban(M, Lh, hist_ids, hist_seg, (const int32_t*)c->prefix.p, kst, d_step, P, gp.ngram_blocking_size,
+      c->launches += launch_ngram_ban(M, g.K, Lh, hist_ids, hist_seg, (const int32_t*)c->prefix.p, kst, d_step, P, gp.ngram_blocking_size,
                                       (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }
     if (gp.top_k == 0) {
       // no top-k cut (utils/decoding_utils.py:17 skips it): multinomial over the whole, optionally nucleus-filtered, vocabulary
-      c->launches += launch_full_vocab_sample(M, c->V, (const float*)c->logits.p, c->Vpad, gp.temperature, gp.top_p, bt, bc, Lh, Tn, 0, 0,
+      c->launches += launch_full_vocab_sample(M, g.K, c->V, (const float*)c->logits.p, c->Vpad, gp.temperature, gp.top_p, bt, bc, Lh, Tn, 0, 0,
                                               (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p,
                                               key_next, kst, nullptr, s);
     } else {
       c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, 1, nullptr, gp.temperature, bt, bc, Lh, nsel, sv, si,
                                        nullptr, s);
-      c->launches += launch_sample_step(M, Tn, nsel, sv, si, gp.top_k, gp.top_p, 0, 0, (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p,
+      c->launches += launch_sample_step(M, g.K, Tn, nsel, sv, si, gp.top_k, gp.top_p, 0, 0, (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p,
                                         (int32_t*)c->cur_tokens.p, key_next, kst, nullptr, s);
     }
   }
   c->launches += launch_step_advance((int*)c->d_step.p, s);
 }
 
-// Argument checks of a generate call; returns the beams per image.
-int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_seg,
+// Argument checks of a generate call returning N sequences per image; returns the decode rows per image (beam mode: the beams;
+// sample mode: the N candidates).
+int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, int N, const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_seg,
                    int Lh, const int64_t* out_ids) {
   check_ready(c);
   if (c->dec_layers == 0) throw StateError("generate: encoder-only context");
@@ -804,7 +807,10 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* pref
   if (gp.mode == GSTVD_SELECT_BEAM) {
     K = gp.num_beams;
     if (K < 1 || K > c->K_max || 2 * K > kSelMax) throw InvalidArg("generate: num_beams out of range");
+    if (N < 1 || N > K) throw InvalidArg(fmt("generate: %d return sequences outside 1..num_beams (%d)", N, K));
   } else if (gp.mode == GSTVD_SELECT_SAMPLE) {
+    if (N < 1 || N > c->K_max || N > 8) throw InvalidArg(fmt("generate: %d sampled candidates outside 1..min(8, max_beams = %d)", N, c->K_max));
+    K = N;
     if (gp.top_k < 0 || gp.top_k > GSTVD_MAX_TOP_K) throw Unsupported("generate: top_k must be 0 (no top-k cut) or in 1..16");
     if (gp.top_k == 0 && c->V > 32768) throw Unsupported("generate: top_k = 0 needs a vocabulary of at most 32768 entries");
     if (!(gp.temperature > 0.f)) throw InvalidArg("generate: temperature must be > 0");
@@ -815,15 +821,16 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* pref
   return K;
 }
 
-void generate_finalize(gstvd_ctx* c, int B, int K, int P, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
+// out_ids [B*N, T] image-major (sample mode: N == K, one row per candidate)
+void generate_finalize(gstvd_ctx* c, int B, int K, int P, int N, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
   const int T = gp.max_new_tokens;
-  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, P, out_ids, out_scores, s);
-  else c->launches += launch_sample_finalize(B, T, 102, (const int32_t*)c->seq.p, out_ids, s);
+  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, P, N, out_ids, out_scores, s);
+  else c->launches += launch_sample_finalize(B * K, T, 102, (const int32_t*)c->seq.p, out_ids, s);
 }
 
-void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_seg,
-                 int Lh, int64_t* out_ids, float* out_scores, cudaStream_t s) {
-  const int K = check_generate(c, gp, prefix, P, hist_ids, hist_seg, Lh, out_ids);
+void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, int N, const int64_t* prefix, int P, const int64_t* hist_ids,
+                 const int64_t* hist_seg, int Lh, int64_t* out_ids, float* out_scores, cudaStream_t s) {
+  const int K = check_generate(c, gp, N, prefix, P, hist_ids, hist_seg, Lh, out_ids);
   if (c->cross_B != B) throw StateError(fmt("generate: cross K/V prefilled for %d images, asked for %d", c->cross_B, B));
   const int T = gp.max_new_tokens;
   const DecodeGeom g = make_geom(c, B, K, T, P);
@@ -840,7 +847,7 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
     GraphKey key;
     std::memset(&key, 0, sizeof key);
     key.B = B; key.K = K; key.mode = gp.mode; key.T = T; key.top_k = gp.top_k; key.ngram = gp.ngram_blocking_size; key.Lh = Lh;
-    key.P = P; key.has_prefix = pre != nullptr;
+    key.P = P; key.has_prefix = pre != nullptr; key.N = N;
     key.temperature = gp.temperature; key.top_p = gp.top_p;
     key.Le = c->cross_Le;                    // the cross cache geometry is part of the captured launch parameters
     const int64_t* g_ids = hist_ids; const int64_t* g_seg = hist_seg;
@@ -880,7 +887,7 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
     CUDA_CHECK(cudaGraphLaunch(it->second.exec, s));
     c->launches += it->second.kernels;
   }
-  generate_finalize(c, B, K, P, gp, out_ids, out_scores, s);
+  generate_finalize(c, B, K, P, N, gp, out_ids, out_scores, s);
 }
 
 // One forward call of the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:24-120) - encoder, fusion,
@@ -889,9 +896,9 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
 // order, same results as gstvd_encode + gstvd_prefill_cross + gstvd_generate (asserted by the tests); eager when graphs are
 // disabled or while the GEMM profiler is on (events cannot be recorded inside a graph).
 void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int64_t* seg, const float* att, const float* feat,
-              const float* loc, const float* imask, const gstvd_gen_params& gp, const int64_t* prefix, int P, int64_t* out_ids,
+              const float* loc, const float* imask, const gstvd_gen_params& gp, int N, const int64_t* prefix, int P, int64_t* out_ids,
               float* out_scores, cudaStream_t s) {
-  const int K = check_generate(c, gp, prefix, P, ids, seg ? seg : ids, Lt, out_ids);
+  const int K = check_generate(c, gp, N, prefix, P, ids, seg ? seg : ids, Lt, out_ids);
   if (B < 1 || B > c->B_max || Lt < 1 || Lt > c->Lt_max || Lv < 1 || Lv > c->Lv_max) throw InvalidArg("round: shape exceeds capacity");
   if (!ids || !feat || !loc) throw InvalidArg("round: input_ids / image_feat / image_loc must not be NULL");
   if (gp.ngram_blocking_size > 0 && !seg) throw InvalidArg("round: n-gram blocking needs token_type_ids");
@@ -911,7 +918,7 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
     decode_init(c, g, gp, pre, s);
     prefix_prefill(c, g, s);
     for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, g_ids, g_seg, Lt, s, t);
-    generate_finalize(c, B, K, P, gp, (int64_t*)c->r_out_ids.p, out_scores ? (float*)c->r_out_scores.p : nullptr, s);
+    generate_finalize(c, B, K, P, N, gp, (int64_t*)c->r_out_ids.p, out_scores ? (float*)c->r_out_scores.p : nullptr, s);
   };
   const bool use_graph = !(c->cfg.flags & GSTVD_FLAG_NO_CUDA_GRAPH) && !c->profiling;
   if (!use_graph) {
@@ -922,7 +929,7 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
     key.B = B; key.Lt = Lt; key.Lv = Lv; key.K = K; key.mode = gp.mode; key.T = T; key.top_k = gp.top_k; key.ngram = gp.ngram_blocking_size;
     key.has_seg = seg != nullptr; key.has_att = att != nullptr; key.has_imask = imask != nullptr;
     key.temperature = gp.temperature; key.top_p = gp.top_p;
-    key.P = P; key.has_prefix = pre != nullptr;
+    key.P = P; key.has_prefix = pre != nullptr; key.N = N;
     if (out_scores) key.has_imask |= 2;
     auto it = c->round_graphs.find(key);
     if (it == c->round_graphs.end()) {
@@ -955,8 +962,8 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
     // host-side state the captured calls set (a replay does not run them again)
     c->enc_B = B; c->enc_Le = Lv + Lt; c->cross_B = B; c->cross_Le = Lv + Lt;
   }
-  CUDA_CHECK(cudaMemcpyAsync(out_ids, c->r_out_ids.p, (size_t)B * T * 8, cudaMemcpyDeviceToDevice, s));
-  if (out_scores) CUDA_CHECK(cudaMemcpyAsync(out_scores, c->r_out_scores.p, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
+  CUDA_CHECK(cudaMemcpyAsync(out_ids, c->r_out_ids.p, (size_t)B * N * T * 8, cudaMemcpyDeviceToDevice, s));
+  if (out_scores) CUDA_CHECK(cudaMemcpyAsync(out_scores, c->r_out_scores.p, (size_t)B * N * 4, cudaMemcpyDeviceToDevice, s));
 }
 
 // `options` decoder sequences per image share that image's cross-attention K/V (evaluate_gen.py:62-107 re-encodes the same
@@ -1167,12 +1174,18 @@ int gstvd_generate(gstvd_ctx* c, int B, const gstvd_gen_params* params, const in
 
 int gstvd_generate_prefixed(gstvd_ctx* c, int B, const gstvd_gen_params* params, const int64_t* prefix, int P, const int64_t* hist_ids,
                             const int64_t* hist_segments, int Lh, int64_t* out_ids, float* out_scores, void* stream) {
+  return gstvd_generate_candidates(c, B, params, 1, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores, stream);
+}
+
+int gstvd_generate_candidates(gstvd_ctx* c, int B, const gstvd_gen_params* params, int N, const int64_t* prefix, int P,
+                              const int64_t* hist_ids, const int64_t* hist_segments, int Lh, int64_t* out_ids, float* out_scores,
+                              void* stream) {
   if (!c || !params) { g_last_error = "gstvd_generate: NULL argument"; return GSTVD_ERR_INVALID; }
   return guarded(c, [&] {
     cudaStream_t user = (cudaStream_t)stream;
     CUDA_CHECK(cudaEventRecord(c->ev_in, user));
     CUDA_CHECK(cudaStreamWaitEvent(c->own_stream, c->ev_in, 0));
-    do_generate(c, B, *params, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores, c->own_stream);
+    do_generate(c, B, *params, N, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores, c->own_stream);
     CUDA_CHECK(cudaEventRecord(c->ev_out, c->own_stream));
     CUDA_CHECK(cudaStreamWaitEvent(user, c->ev_out, 0));
   });
@@ -1188,13 +1201,21 @@ int gstvd_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, c
 int gstvd_round_prefixed(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, const int64_t* token_type_ids,
                          const float* attention_mask, const float* image_feat, const float* image_loc, const float* image_mask,
                          const gstvd_gen_params* params, const int64_t* prefix, int P, int64_t* out_ids, float* out_scores, void* stream) {
+  return gstvd_round_candidates(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, params, 1, prefix,
+                                P, out_ids, out_scores, stream);
+}
+
+int gstvd_round_candidates(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, const int64_t* token_type_ids,
+                           const float* attention_mask, const float* image_feat, const float* image_loc, const float* image_mask,
+                           const gstvd_gen_params* params, int N, const int64_t* prefix, int P, int64_t* out_ids, float* out_scores,
+                           void* stream) {
   if (!c || !params) { g_last_error = "gstvd_round: NULL argument"; return GSTVD_ERR_INVALID; }
   return guarded(c, [&] {
     cudaStream_t user = (cudaStream_t)stream;
     CUDA_CHECK(cudaEventRecord(c->ev_in, user));
     CUDA_CHECK(cudaStreamWaitEvent(c->own_stream, c->ev_in, 0));
-    do_round(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, *params, prefix, P, out_ids, out_scores,
-             c->own_stream);
+    do_round(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, *params, N, prefix, P, out_ids,
+             out_scores, c->own_stream);
     CUDA_CHECK(cudaEventRecord(c->ev_out, c->own_stream));
     CUDA_CHECK(cudaStreamWaitEvent(user, c->ev_out, 0));
   });
@@ -1468,7 +1489,7 @@ int gstvd_op_beam_end(gstvd_ctx* c, int64_t* out_ids, float* out_scores, void* s
   if (!c || !out_ids) return GSTVD_ERR_INVALID;
   return guarded(c, [&] {
     if (c->op_B == 0) throw StateError("beam_end before beam_begin");
-    c->launches += launch_beam_finalize(beam_buffers(c), c->op_B, c->op_K, c->op_T, 102, 1, out_ids, out_scores, (cudaStream_t)stream);
+    c->launches += launch_beam_finalize(beam_buffers(c), c->op_B, c->op_K, c->op_T, 102, 1, 1, out_ids, out_scores, (cudaStream_t)stream);
     c->op_B = 0;
   });
 }
@@ -1491,19 +1512,19 @@ int gstvd_op_sample(gstvd_ctx* c, int rows, const float* logits, int64_t ldl, co
       if (!hist_ids || !hist_segments || !prefix || prefix_len != step + 1) throw InvalidArg("op_sample: n-gram blocking needs history and a prefix of step+1 tokens");
       CUDA_CHECK(cudaMemsetAsync(c->prefix.p, 0, c->prefix.bytes, s));
       c->launches += launch_build_prefix_from_ids(rows, prefix_len, prefix, (int32_t*)c->prefix.p, T + 1, 102, s);
-      c->launches += launch_ngram_ban(rows, Lh, hist_ids, hist_segments, (const int32_t*)c->prefix.p, T + 1, (const int*)c->d_step.p, 1,
+      c->launches += launch_ngram_ban(rows, 1, Lh, hist_ids, hist_segments, (const int32_t*)c->prefix.p, T + 1, (const int*)c->d_step.p, 1,
                                       gp->ngram_blocking_size, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }
     if (gp->top_k == 0) {
-      c->launches += launch_full_vocab_sample(rows, c->V, logits, ldl, gp->temperature, gp->top_p, bt, bc, Lh, T, gp->seed, (uint64_t)gp->row_offset, nullptr,
+      c->launches += launch_full_vocab_sample(rows, 1, c->V, logits, ldl, gp->temperature, gp->top_p, bt, bc, Lh, T, gp->seed, (uint64_t)gp->row_offset, nullptr,
                                               (const int*)c->d_step.p, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, T + 1,
                                               out_tokens, s);
       return;
     }
     c->launches += launch_row_select(rows, c->V, logits, ldl, 1, nullptr, gp->temperature, bt, bc, Lh, kSelMax, (float*)c->sel_val.p,
                                      (int32_t*)c->sel_idx.p, nullptr, s);
-    c->launches += launch_sample_step(rows, T, kSelMax, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, gp->top_k, gp->top_p, gp->seed, (uint64_t)gp->row_offset, nullptr,
+    c->launches += launch_sample_step(rows, 1, T, kSelMax, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, gp->top_k, gp->top_p, gp->seed, (uint64_t)gp->row_offset, nullptr,
                                       (const int*)c->d_step.p, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, T + 1,
                                       out_tokens, s);
   });

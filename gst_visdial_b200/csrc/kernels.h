@@ -188,13 +188,15 @@ int launch_beam_init(const BeamBuffers& bb, int B, int K, int T, int start_token
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int T, int V, int nsel, const float* sel_val,
                      const int32_t* sel_idx, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
                      cudaStream_t stream);
-int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int64_t* out_ids, float* out_scores,
+// out_ids [B*N, T] / out_scores [B*N]: the N <= K best finished hypotheses of every image, image-major, in the pop order of HF
+// BeamSearchScorer.finalize (score descending, the later-inserted first among equal scores); N = 1 is the single best
+int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores,
                          cudaStream_t stream);
 
 // n-gram blocking (utils/decoding_utils.py:38-78): ban list per row from the question history and the decoded prefix.
 // prefix_tokens int32 [rows, P+T] (decoder prefix of len0 = P tokens, then the generated ones; EOS already replaced by PAD),
-// prefix_len = *d_step + len0
-int launch_ngram_ban(int rows, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
+// prefix_len = *d_step + len0.  N rows per image (sampled candidates): row r reads the history of image r / N
+int launch_ngram_ban(int rows, int N, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
                      int prefix_stride, const int* d_step, int len0, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
                      cudaStream_t stream);
 // the same for the B*K beam rows: key = the last n-1 tokens of prefix_b ([SEP] read as [PAD]; null: [CLS], P = 1) followed by beam
@@ -203,15 +205,17 @@ int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, 
                           const int32_t* tokens, int step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream);
 // sample-mode selection from row_select output; writes seq[row, step] and cur_tokens[row], prefix[row, step+1]
 // top_k == 0: multinomial over the whole (optionally nucleus-filtered) vocabulary; writes the same state as launch_sample_step
-int launch_full_vocab_sample(int rows, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,
+// N rows per image (sampled candidates): row r draws as row r / N of a single-sample call seeded candidate_seed(seed, r % N)
+int launch_full_vocab_sample(int rows, int N, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,
                              const int32_t* ban_count, int ban_stride, int T, uint64_t seed, uint64_t row_offset, const uint64_t* d_seed,
                              const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens,
                              cudaStream_t stream);
-int launch_sample_step(int rows, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
+int launch_sample_step(int rows, int N, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
                        uint64_t seed, uint64_t row_offset, const uint64_t* d_seed, const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
                        int prefix_stride, int32_t* out_tokens, cudaStream_t stream);
-// dec_prefix: int64 [rows, P] decoder prefix (null: start_token, P = 1); the key buffer `prefix` [rows, prefix_stride >= P + T]
-int launch_sample_init(int rows, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
+// dec_prefix: int64 [rows / N, P] decoder prefix (null: start_token, P = 1), shared by the N rows of an image; the key buffer
+// `prefix` [rows, prefix_stride >= P + T]
+int launch_sample_init(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
                        int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, cudaStream_t stream);
 int launch_sample_finalize(int rows, int T, int eos, const int32_t* seq, int64_t* out_ids, cudaStream_t stream);
 int launch_step_advance(int* d_step, cudaStream_t stream);

@@ -540,7 +540,9 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int T, int V, int nsel, const flo
   }
 }
 
-__global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eos, int len0, int64_t* out_ids, float* out_scores) {
+// BeamSearchScorer.finalize: a stable ascending sort of the image's hypotheses (kept in insertion order by hyp_add), then N pops.
+// Output n of image b is the hypothesis of rank n by (score desc, insertion index desc); N = 1 is the last of the best scores.
+__global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const int t = *bb.d_step;                     // steps executed
@@ -551,19 +553,23 @@ __global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eo
   }
   const double* hs = bb.hyp_score + (int64_t)b * HK;
   const int cnt = bb.hyp_count[b];
-  int best = 0;
-  for (int i = 1; i < cnt; ++i) if (hs[i] >= hs[best]) best = i;   // stable ascending sort, take the last
-  const int len = bb.hyp_len[(int64_t)b * HK + best];
-  const int32_t* ht = bb.hyp_tokens + ((int64_t)b * HK + best) * T;
-  for (int j = 0; j < T; ++j) out_ids[(int64_t)b * T + j] = (j < len) ? ht[j] : (j == len ? eos : 0);
-  if (out_scores) out_scores[b] = (float)hs[best];
+  for (int i = 0; i < cnt; ++i) {
+    int rank = 0;
+    for (int j = 0; j < cnt; ++j) rank += (hs[j] > hs[i] || (hs[j] == hs[i] && j > i)) ? 1 : 0;
+    if (rank >= N) continue;
+    const int len = bb.hyp_len[(int64_t)b * HK + i];
+    const int32_t* ht = bb.hyp_tokens + ((int64_t)b * HK + i) * T;
+    const int64_t o = (int64_t)b * N + rank;
+    for (int j = 0; j < T; ++j) out_ids[o * T + j] = (j < len) ? ht[j] : (j == len ? eos : 0);
+    if (out_scores) out_scores[o] = (float)hs[i];
+  }
 }
 
 // ------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ bool is_special(int64_t t) { return t == 0 || (t >= 100 && t <= 103); }
 
 __global__ void __launch_bounds__(256)
-ngram_ban_kernel(int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __restrict__ hist_seg,
+ngram_ban_kernel(int N, int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __restrict__ hist_seg,
                  const int32_t* __restrict__ prefix, int prefix_stride, const int* __restrict__ d_step, int len0, int n,
                  int32_t* __restrict__ ban_tokens, int32_t* __restrict__ ban_count, int ban_stride) {
   __shared__ int cnt;
@@ -575,8 +581,8 @@ ngram_ban_kernel(int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __
   const int cur_len = *d_step + len0;                    // decoder prefix (len0 tokens) + generated
   const int start = cur_len + 1 - n;
   if (start >= 0) {                                      // a shorter key can never equal an (n-1)-gram
-    const int64_t* ids = hist_ids + (int64_t)row * Lh;
-    const int64_t* seg = hist_seg + (int64_t)row * Lh;
+    const int64_t* ids = hist_ids + (int64_t)(row / N) * Lh;   // the history of the row's image
+    const int64_t* seg = hist_seg + (int64_t)(row / N) * Lh;
     const int32_t* key = prefix + (int64_t)row * prefix_stride + start;
     for (int p = threadIdx.x; p + n <= Lh; p += blockDim.x) {
       bool ok = true;
@@ -648,23 +654,31 @@ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
   return x ^ (x >> 31);
 }
 
-// dec_prefix != null: int64 [rows, P] decoder prefix; `prefix` (the n-gram key buffer) starts with it, [SEP] read as [PAD]
-__global__ void sample_init_kernel(int rows, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
+// Sampling seed of candidate n of an image (gstvd_generate_candidates): candidate n draws what a single-sample call seeded
+// candidate_seed(seed, n) draws, and candidate 0 is that call itself.  Mirrored by models/visual_dialog_model.candidate_seed.
+__device__ __forceinline__ uint64_t candidate_seed(uint64_t seed, int n) {
+  return n == 0 ? seed : splitmix64(seed ^ splitmix64((uint64_t)n * 0xD1B54A32D192ED03ull));
+}
+
+// dec_prefix != null: int64 [rows / N, P] decoder prefix of the row's image; `prefix` (the n-gram key buffer) starts with it, [SEP]
+// read as [PAD]
+__global__ void sample_init_kernel(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
                                    int prefix_stride, int* d_step, const int64_t* __restrict__ dec_prefix, int P) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0) *d_step = 0;
   if (i < rows) {
-    cur_tokens[i] = dec_prefix ? (int32_t)dec_prefix[(int64_t)i * P + P - 1] : start_token;
+    const int64_t img = i / N;
+    cur_tokens[i] = dec_prefix ? (int32_t)dec_prefix[img * P + P - 1] : start_token;
     for (int j = 0; j < T; ++j) seq[(int64_t)i * T + j] = 0;
     for (int j = 0; j < prefix_stride; ++j) prefix[(int64_t)i * prefix_stride + j] = 0;
     for (int j = 0; j < P; ++j) {
-      const int32_t w = dec_prefix ? (int32_t)dec_prefix[(int64_t)i * P + j] : start_token;
+      const int32_t w = dec_prefix ? (int32_t)dec_prefix[img * P + j] : start_token;
       prefix[(int64_t)i * prefix_stride + j] = w == 102 ? 0 : w;
     }
   }
 }
 
-__global__ void sample_step_kernel(int rows, int T, int nsel, const float* __restrict__ sel_val, const int32_t* __restrict__ sel_idx,
+__global__ void sample_step_kernel(int rows, int N, int T, int nsel, const float* __restrict__ sel_val, const int32_t* __restrict__ sel_idx,
                                    int top_k, float top_p, uint64_t seed, uint64_t row_offset, const uint64_t* __restrict__ d_seed,
                                    const int* __restrict__ d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens) {
   pdl_wait();
@@ -695,9 +709,10 @@ __global__ void sample_step_kernel(int rows, int T, int nsel, const float* __res
   }
   int choice = 0;
   if (kept > 1 && top_k > 1) {     // top_k == 1 is the deterministic greedy path (lowest index among exact ties)
-    // keyed by the GLOBAL row (d_seed[1] = row offset of this batch): the draws of an image are the same whichever batch / rank holds it
-    const uint64_t sd = d_seed ? d_seed[0] : seed;
-    const uint64_t grow = (uint64_t)row + (d_seed ? d_seed[1] : row_offset);
+    // keyed by the GLOBAL image (d_seed[1] = row offset of this batch): the draws of an image are the same whichever batch / rank
+    // holds it; candidate row % N of the image draws with its own seed
+    const uint64_t sd = candidate_seed(d_seed ? d_seed[0] : seed, row % N);
+    const uint64_t grow = (uint64_t)(row / N) + (d_seed ? d_seed[1] : row_offset);
     const uint64_t h = splitmix64(sd ^ splitmix64((grow << 20) ^ (uint64_t)step));
     const float u = (float)(h >> 40) * (1.0f / 16777216.0f) * sum;
     float c = 0.f;
@@ -737,7 +752,7 @@ __device__ __forceinline__ float fv_block_sum(float v, float* s_red) {      // e
   return t;
 }
 __global__ void __launch_bounds__(kFvThreads)
-full_vocab_sample_kernel(int V, const float* __restrict__ logits, int64_t ldl, float temperature, float top_p,
+full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t ldl, float temperature, float top_p,
                          const int32_t* __restrict__ ban_tokens, const int32_t* __restrict__ ban_count, int ban_stride,
                          int T, uint64_t seed, uint64_t row_offset, const uint64_t* __restrict__ d_seed, const int* __restrict__ d_step, int eos,
                          int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens) {
@@ -805,8 +820,8 @@ full_vocab_sample_kernel(int V, const float* __restrict__ logits, int64_t ldl, f
     }
   }
   // draw: first token (in index order) whose inclusive prefix sum exceeds u * total
-  const uint64_t sd = d_seed ? d_seed[0] : seed;
-  const uint64_t grow = (uint64_t)row + (d_seed ? d_seed[1] : row_offset);
+  const uint64_t sd = candidate_seed(d_seed ? d_seed[0] : seed, row % N);
+  const uint64_t grow = (uint64_t)(row / N) + (d_seed ? d_seed[1] : row_offset);
   const uint64_t h = splitmix64(sd ^ splitmix64((grow << 20) ^ (uint64_t)step));
   const float target = (float)(h >> 40) * (1.0f / 16777216.0f) * total;
   float incl = local;
@@ -965,16 +980,18 @@ int launch_beam_step(const BeamBuffers& bb, int B, int K, int T, int V, int nsel
   launch_k(beam_step_kernel, dim3((B + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, B, K, T, V, nsel, sel_val, sel_idx, eos, len0, out_beam_idx, out_tokens, out_scores);
   return 1;
 }
-int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int64_t* out_ids, float* out_scores,
+int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores,
                          cudaStream_t stream) {
-  beam_finalize_kernel<<<(B + 31) / 32, 32, 0, stream>>>(bb, B, K, T, eos, len0, out_ids, out_scores);
+  if (N < 1 || N > K) throw std::runtime_error("beam_finalize: 1 <= N <= K");
+  beam_finalize_kernel<<<(B + 31) / 32, 32, 0, stream>>>(bb, B, K, T, eos, len0, N, out_ids, out_scores);
   return 1;
 }
-int launch_ngram_ban(int rows, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
+int launch_ngram_ban(int rows, int N, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
                      int prefix_stride, const int* d_step, int len0, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
                      cudaStream_t stream) {
   if (rows <= 0) return 0;
-  launch_k(ngram_ban_kernel, dim3(rows), dim3(256), 0, stream, Lh, hist_ids, hist_seg, prefix, prefix_stride, d_step, len0, n, ban_tokens, ban_count, ban_stride);
+  if (N < 1 || rows % N != 0) throw std::runtime_error("ngram_ban: rows must be a multiple of N >= 1");
+  launch_k(ngram_ban_kernel, dim3(rows), dim3(256), 0, stream, N, Lh, hist_ids, hist_seg, prefix, prefix_stride, d_step, len0, n, ban_tokens, ban_count, ban_stride);
   return 1;
 }
 int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int64_t* prefix, int P,
@@ -985,19 +1002,21 @@ int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, 
   launch_k(beam_ngram_ban_kernel, dim3(B), dim3(256), 0, stream, K, T, Lh, hist_ids, hist_seg, prefix, P, tokens, step, n, ban_tokens, ban_count, ban_stride);
   return 1;
 }
-int launch_sample_step(int rows, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
+int launch_sample_step(int rows, int N, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
                        uint64_t seed, uint64_t row_offset, const uint64_t* d_seed, const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
                        int prefix_stride, int32_t* out_tokens, cudaStream_t stream) {
   if (top_k < 1 || top_k > nsel) throw std::runtime_error("sample_step: top_k out of range");
-  launch_k(sample_step_kernel, dim3((rows + 63) / 64), dim3(64), 0, stream, rows, T, nsel, sel_val, sel_idx, top_k, top_p, seed, row_offset, d_seed, d_step, eos, seq,
+  if (N < 1 || rows % N != 0) throw std::runtime_error("sample_step: rows must be a multiple of N >= 1");
+  launch_k(sample_step_kernel, dim3((rows + 63) / 64), dim3(64), 0, stream, rows, N, T, nsel, sel_val, sel_idx, top_k, top_p, seed, row_offset, d_seed, d_step, eos, seq,
                                                           cur_tokens, prefix, prefix_stride, out_tokens);
   return 1;
 }
-int launch_full_vocab_sample(int rows, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,
+int launch_full_vocab_sample(int rows, int N, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,
                              const int32_t* ban_count, int ban_stride, int T, uint64_t seed, uint64_t row_offset, const uint64_t* d_seed,
                              const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens,
                              cudaStream_t stream) {
   if (rows <= 0) return 0;
+  if (N < 1 || rows % N != 0) throw std::runtime_error("full_vocab_sample: rows must be a multiple of N >= 1");
   if (V > kFvThreads * kFvPer) throw std::runtime_error("full_vocab_sample: vocab > 32768");
   constexpr size_t smem = (size_t)kFvThreads * kFvPer * sizeof(float);
   static bool attr_set = false;
@@ -1006,14 +1025,15 @@ int launch_full_vocab_sample(int rows, int V, const float* logits, int64_t ldl, 
     if (e != cudaSuccess) throw std::runtime_error(std::string("full_vocab_sample: cudaFuncSetAttribute: ") + cudaGetErrorString(e));
     attr_set = true;
   }
-  launch_k(full_vocab_sample_kernel, dim3(rows), dim3(kFvThreads), smem, stream, V, logits, ldl, temperature, top_p, ban_tokens, ban_count, ban_stride,
+  launch_k(full_vocab_sample_kernel, dim3(rows), dim3(kFvThreads), smem, stream, N, V, logits, ldl, temperature, top_p, ban_tokens, ban_count, ban_stride,
            T, seed, row_offset, d_seed, d_step, eos, seq, cur_tokens, prefix, prefix_stride, out_tokens);
   return 1;
 }
-int launch_sample_init(int rows, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
+int launch_sample_init(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
                        int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, cudaStream_t stream) {
   if (P < 1 || P > prefix_stride || (P > 1 && !dec_prefix)) throw std::runtime_error("sample_init: 1 <= P <= prefix_stride, prefix given when P > 1");
-  sample_init_kernel<<<(rows + 63) / 64, 64, 0, stream>>>(rows, T, start_token, seq, cur_tokens, prefix, prefix_stride, d_step, dec_prefix, P);
+  if (N < 1 || rows % N != 0) throw std::runtime_error("sample_init: rows must be a multiple of N >= 1");
+  sample_init_kernel<<<(rows + 63) / 64, 64, 0, stream>>>(rows, N, T, start_token, seq, cur_tokens, prefix, prefix_stride, d_step, dec_prefix, P);
   return 1;
 }
 int launch_sample_finalize(int rows, int T, int eos, const int32_t* seq, int64_t* out_ids, cudaStream_t stream) {

@@ -38,8 +38,32 @@ def _model_call(model, st, dec_input_ids, **kw):
         dec_attention_mask=(dec_input_ids != 0).float(), **kw)
 
 
+def _answer_ppl(a_model, st, ans, mode):
+    """Perplexity pass of generate.py:183-209 over ``ans`` [B, 18] against the resident cross-K/V; replaces [SEP] by [PAD] in place."""
+    am = _unwrap(a_model)
+    am.params["mode"] = "train"                              # the reference's mode-flip trick (generate.py:185,211)
+    try:
+        loss, _ = _model_call(a_model, st, ans, loss_reduction=False, reuse_encoder=True, want_logits=False)
+    finally:
+        am.params["mode"] = mode
+    ans_len = (ans != 0).sum(-1)                             # counted after the in-place [SEP] -> [PAD]
+    return torch.exp(loss.reshape(ans.shape[0], -1).sum(-1) / ans_len)
+
+
+def _best_candidate(a_model, st, cands, mode):
+    """cands [B, N, 18]: every candidate through the perplexity pass, then per image the one with the lowest perplexity (a stable
+    ascending sort puts NaN last and keeps the lowest candidate index among ties).  Returns (answers [B, 18], perplexities [B])."""
+    B, N, L = cands.shape
+    rows = [cands[:, n].contiguous() for n in range(N)]
+    ppl = torch.stack([_answer_ppl(a_model, st, r, mode) for r in rows], 1)
+    best = torch.sort(ppl, dim=1, stable=True).indices[:, :1]
+    ans = torch.stack(rows, 1).gather(1, best[:, :, None].expand(B, 1, L)).squeeze(1)
+    return ans, ppl.gather(1, best).squeeze(1)
+
+
 def generate_dialogs(a_model, batch, q_model=None, questions=None, num_rounds=10, a_kwargs=None, q_kwargs=None,
-                     with_ppl=True, device=None, trim_history=True, max_new_tokens=18, seed=None, row_offset=0) -> DialogResult:
+                     with_ppl=True, device=None, trim_history=True, max_new_tokens=18, seed=None, row_offset=0,
+                     answer_candidates=1) -> DialogResult:
     """``batch`` uses the reference dataloader's keys (generate.py:95-111).  Either ``q_model`` or ``questions``
     (int64 [B, num_rounds, 18], zero padded, each ending in [SEP]) must be given.  ``a_kwargs`` / ``q_kwargs`` are the
     decoding kwargs of EncoderDecoderModel.forward; defaults are generate.py:138-141 / :177-180.
@@ -51,7 +75,10 @@ def generate_dialogs(a_model, batch, q_model=None, questions=None, num_rounds=10
     ``trim_history``: the encoder runs on ceil32(longest history) text positions instead of all ``max_seq_len`` (see
     ``enc_valid_len`` in EncoderDecoderModel.forward).  The bound is kept on the HOST - caption lengths are read once at the
     start, every round adds the question length (or ``max_new_tokens`` for a generated question) and ``max_new_tokens`` for
-    the answer - so no round waits for the device.  Token ids, perplexities and flags are identical with or without it."""
+    the answer - so no round waits for the device.  Token ids, perplexities and flags are identical with or without it.
+
+    ``answer_candidates`` > 1 (needs ``with_ppl``): per round the teacher draws that many answers in one call (samples, or the best of
+    its ``num_beams`` beams), and the one with the lowest perplexity is spliced and reported."""
     a_kwargs = dict(a_kwargs or dict(temperature=0.7, top_k=7, top_p=0.0, ngram_blocking_size=0))
     q_kwargs = dict(q_kwargs or dict(temperature=0.7, top_k=7, top_p=0.0, ngram_blocking_size=4))
     am = _unwrap(a_model)
@@ -79,6 +106,9 @@ def generate_dialogs(a_model, batch, q_model=None, questions=None, num_rounds=10
         questions = questions.to(dtype=torch.int64, **nb)
     elif q_model is None:
         raise ValueError("generate_dialogs needs q_model or questions")
+    n_cand = int(answer_candidates)
+    if n_cand < 1 or (n_cand > 1 and not with_ppl):
+        raise ValueError("answer_candidates must be >= 1, and more than one candidate is ranked by perplexity (with_ppl=True)")
     ques_all, ans_all, ppl_all = [], [], []
     mode = am.params["mode"]
     Lmax = st["ids"].shape[1]
@@ -105,17 +135,17 @@ def generate_dialogs(a_model, batch, q_model=None, questions=None, num_rounds=10
         eng.splice(st["ids"], st["seg"], st["mask"], enc_len, ques, segment_value=-1, strip_sep=False, abnormal=abnormal)
         if ub is not None:
             ub = ub + (q_host[:, rnd] if q_host is not None else max_new_tokens)
-        ans = _model_call(a_model, st, dec_start, enc_valid_len=bound(), **a_kwargs)
+        if n_cand > 1:
+            cands = _model_call(a_model, st, dec_start, enc_valid_len=bound(), num_return_sequences=n_cand, **a_kwargs)
+        else:
+            ans = _model_call(a_model, st, dec_start, enc_valid_len=bound(), **a_kwargs)
         if ub is not None:
             ub = ub + max_new_tokens
-        if with_ppl:
-            am.params["mode"] = "train"                      # the reference's mode-flip trick (generate.py:185,211)
-            try:
-                loss, _ = _model_call(a_model, st, ans, loss_reduction=False, reuse_encoder=True, want_logits=False)
-            finally:
-                am.params["mode"] = mode
-            ans_len = (ans != 0).sum(-1)                     # counted after the in-place [SEP] -> [PAD]
-            ppl_all.append(torch.exp(loss.reshape(B, -1).sum(-1) / ans_len))
+        if n_cand > 1:
+            ans, ppl = _best_candidate(a_model, st, cands.reshape(B, n_cand, -1), mode)
+            ppl_all.append(ppl)
+        elif with_ppl:
+            ppl_all.append(_answer_ppl(a_model, st, ans, mode))
         eng.splice(st["ids"], st["seg"], st["mask"], enc_len, ans, segment_value=1, strip_sep=True, abnormal=abnormal)
         ques_all.append(ques)
         ans_all.append(ans)

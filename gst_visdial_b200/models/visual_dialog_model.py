@@ -25,6 +25,15 @@ def derive_seed(base, role, index) -> int:
     return _splitmix64(_splitmix64(int(base) & 0xFFFFFFFFFFFFFFFF) ^ _splitmix64(tag) ^ ((int(index) + 1) * 0x632BE59BD9B4E019 & 0xFFFFFFFFFFFFFFFF))
 
 
+def candidate_seed(seed, n) -> int:
+    """Sampling seed of candidate ``n`` of an image in a ``num_return_sequences`` call: candidate n draws what a single-sample call
+    with this seed draws (mirror of candidate_seed in csrc/select.cu).  Candidate 0 keeps ``seed``."""
+    seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+    if int(n) == 0:
+        return seed
+    return _splitmix64(seed ^ _splitmix64((int(n) * 0xD1B54A32D192ED03) & 0xFFFFFFFFFFFFFFFF))
+
+
 class VLFusion(nn.Module):
     """Parameters of models/visual_dialog_model.py:123-129; the projection itself runs inside the engine."""
 
@@ -41,6 +50,8 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
 
     Extra keyword arguments (all default to the reference behaviour):
       num_beams=1        >1 switches the token selection to beam search (contract: oracle/beam.py)
+      num_return_sequences=1  N sequences per image, image-major [B*N, 18]: the N best beams (oracle/beam_nbest.py), or N sampled
+                         candidates, candidate n drawing like a single-sample call with seed candidate_seed(seed, n)
       seed=None          sampling seed (a per-call counter when None)
       enc_valid_len=None   upper bound (python int) on the number of leading history positions that hold a token in ANY row.
                          The encoder, the cross-K/V prefill and the cross-attention then run on ceil32(bound) text positions
@@ -151,6 +162,9 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
             seed=seed,
             row_offset=int(decoding_kwargs.get("row_offset", 0)),
         )
+        n_ret = int(decoding_kwargs.get("num_return_sequences", 1))
+        if n_ret != 1:
+            gen_kw["num_return_sequences"] = n_ret
         gen_kw["prefix"] = self._decoder_prefix(dec_input_ids, B, gen_kw["num_beams"], gen_kw["ngram_blocking_size"])
         if whole_round:
             # the n-gram blocking history is the (trimmed) encoder input itself: positions past the bound hold no token

@@ -36,6 +36,9 @@ def read_command_line(argv=None):
     p.add_argument('-num_beams', default=1, type=int, help='>1: beam search for the answers instead of top-k sampling')
     p.add_argument('-q_num_beams', default=1, type=int,
                    help='>1: beam search for the questions instead of top-k sampling (keeps the 4-gram blocking against the question history)')
+    p.add_argument('-answer_candidates', default=1, type=int,
+                   help='>1: the teacher draws this many answers per round (samples, or the best of its -num_beams beams) and the one with '
+                        'the lowest perplexity goes into the dialog')
     p.add_argument('-synthetic', default=0, type=int, help='generate dialogs for N seeded synthetic images (no dataset / checkpoint needed)')
     p.add_argument('-feature_shards', default='', help='comma-separated shard directories (gst_visdial_b200.io.features) instead of the LMDB')
     p.add_argument('-caption_ids', default='', help='json {image_id: [caption token ids]} for the images of the shards (pre-tokenized captions)')
@@ -47,7 +50,7 @@ def read_command_line(argv=None):
     params = vars(args)
     params['device'] = f"cuda:{params['gpu_ids'][0]}"
     params['engine_max_batch'] = params['batch_size']
-    params['engine_max_beams'] = max(1, params['num_beams'], params['q_num_beams'])
+    params['engine_max_beams'] = max(1, params['num_beams'], params['q_num_beams'], params['answer_candidates'])
     if params['save_name'] == '':
         params['save_name'] = 'generated_dialogs.json'
     os.makedirs(params['save_path'], exist_ok=True)

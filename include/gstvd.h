@@ -81,7 +81,7 @@ typedef struct {
 
 typedef struct {
   int32_t mode;               /* gstvd_select_mode */
-  int32_t num_beams;          /* beam mode: K (<= max_beams); sample mode: ignored (1 row per image) */
+  int32_t num_beams;          /* beam mode: K (<= max_beams); sample mode: ignored (N rows per image, gstvd_generate_candidates) */
   int32_t max_new_tokens;     /* <= config.max_new_tokens */
   int32_t top_k;              /* sample mode; 1 = greedy; 2..GSTVD_MAX_TOP_K = top-k set (ties kept); 0 = no top-k cut: multinomial over the
                                  whole - optionally nucleus-filtered - vocabulary (utils/decoding_utils.py:17 skips the cut) */
@@ -161,6 +161,21 @@ int gstvd_generate_prefixed(gstvd_ctx* ctx, int B, const gstvd_gen_params* param
                             const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
                             int64_t* out_ids, float* out_scores, void* stream);
 
+/* gstvd_generate_prefixed returning N sequences per image (HF num_return_sequences); gstvd_generate_prefixed is this call with N = 1.
+ *   out_ids    : int64 [B*N, max_new_tokens], image-major (row b*N + n), PAD(0) after the first [SEP]
+ *   out_scores : fp32 [B*N] (may be NULL; beam mode only)
+ *   beam mode, 1 <= N <= num_beams: the N best finished hypotheses of BeamSearchScorer.finalize (transformers 4.16.2) in its pop order -
+ *     score descending, the later-inserted hypothesis first among equal scores; contract in oracle/beam_nbest.py.  Decoding is the same
+ *     as with N = 1; only the finalisation differs.
+ *   sample mode, 1 <= N <= min(8, max_beams): N independent continuations per image, decoded as N rows that share the image's cross
+ *     K/V, decoder prefix and n-gram history.  Candidate n of image b draws exactly what an N = 1 call with seed
+ *     candidate_seed(seed, n) draws for image b (the RNG row stays row_offset + b); candidate_seed(seed, 0) = seed and, for n >= 1,
+ *     splitmix64(seed ^ splitmix64(n * 0xD1B54A32D192ED03)) (splitmix64 as in the sampler).  No scores are written.
+ *   Other N are rejected with GSTVD_ERR_INVALID. */
+int gstvd_generate_candidates(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, int N, const int64_t* prefix, int P,
+                              const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
+                              int64_t* out_ids, float* out_scores, void* stream);
+
 /* One whole forward call of the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:24-120): the same work and
  * results as gstvd_encode (no exported outputs) + gstvd_prefill_cross(resident states) + gstvd_generate, replayed from ONE CUDA graph
  * per shape - the host enqueues a few device-to-device copies of the inputs and one graph launch.  The n-gram blocking history is the
@@ -177,6 +192,14 @@ int gstvd_round_prefixed(gstvd_ctx* ctx, int B, int Lt, int Lv,
                          const float* image_feat, const float* image_loc, const float* image_mask,
                          const gstvd_gen_params* params, const int64_t* prefix, int P,
                          int64_t* out_ids, float* out_scores, void* stream);
+
+/* gstvd_round_prefixed returning N sequences per image: the contract of gstvd_generate_candidates (out_ids [B*N, max_new_tokens],
+ * out_scores [B*N]); gstvd_round_prefixed is this call with N = 1. */
+int gstvd_round_candidates(gstvd_ctx* ctx, int B, int Lt, int Lv,
+                           const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
+                           const float* image_feat, const float* image_loc, const float* image_mask,
+                           const gstvd_gen_params* params, int N, const int64_t* prefix, int P,
+                           int64_t* out_ids, float* out_scores, void* stream);
 
 /* Replaces VisualDialogDecoder.forward in loss mode (models/visual_dialog_decoder.py:33-86) as driven by
  * generate.py:183-209 and evaluate_gen.py:94-106: teacher-forced pass over dec_ids [B, L].

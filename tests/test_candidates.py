@@ -1,0 +1,425 @@
+"""Several sequences per image from one encoder pass (num_return_sequences; include/gstvd.h gstvd_generate_candidates).
+
+CPU: the N-best oracle (oracle/beam_nbest.py) is the plain finalize at N = 1 for all three beam states and returns equal-score
+hypotheses in HF pop order; candidate_seed; the -answer_candidates flag.
+GPU: N-best beams identical to the oracle in fp32 on every call path (with and without blocking and a decoder prefix); sampled
+candidate n identical to a single-sample call seeded candidate_seed(seed, n); the bf16 product path agrees across call paths; the
+dialog loop keeps the lowest-perplexity candidate; the CLI; every rejected N raises.
+"""
+import copy
+import os
+
+import pytest
+import torch
+
+from helpers import R, history_batch
+from oracle import beam as OB
+from oracle import beam_ngram as BN
+from oracle.beam_nbest import finalize_nbest
+from test_decoder_prefix import A4, PrefixBeamState, _prefixes, _with_bias, _with_question, contains_banned_ngram
+
+_GREEDY = dict(temperature=1.0, top_k=1, top_p=0.0)
+
+
+def _random_logits(B, K, V, T, seed):
+    g = torch.Generator().manual_seed(seed)
+    logits = [torch.randn(B * K, V, generator=g) * 3 for _ in range(T)]
+    for lg in logits[3:]:
+        lg[:, OB.EOS] += 4.0
+    return logits
+
+
+def prefix_beam_state(sd, enc_cfg, dec_cfg, batch, num_beams, max_new=18, ngram_blocking_size=0, prefix=None):
+    """The decode loop of test_decoder_prefix.prefix_beam_search, returning the state before finalisation."""
+    ids, seg, att = batch["enc_input_ids"], batch["enc_segments"], batch["enc_att_mask"]
+    B, K = ids.shape[0], num_beams
+    seq_t, seq_v = R.encoder(sd, enc_cfg, ids, batch["enc_image_feat"], batch["enc_image_loc"], seg, att, batch["enc_image_mask"])
+    enc_h, enc_m = R.vlfusion(sd, seq_t, seq_v, att, batch["enc_image_mask"])
+    enc_h, enc_m = enc_h.repeat_interleave(K, 0), enc_m.repeat_interleave(K, 0)
+    hist = BN.question_history(ids, seg)
+    st = PrefixBeamState(B, K, dec_cfg.vocab_size, max_new, prefix)
+    start = st.prefix.repeat_interleave(K, 0)
+    for t in range(max_new):
+        h = R.decoder_hidden(sd, dec_cfg, torch.cat((start, st.tokens.reshape(B * K, -1)[:, :t]), 1), None, enc_h, enc_m)
+        st.step(R.lm_logits(sd, h[:, -1]), ngram_blocking_size, hist)
+        if bool(st.done.all()):
+            break
+    return st
+
+
+def _nbest(st, Ns):
+    return {N: finalize_nbest(copy.deepcopy(st), N) for N in Ns}
+
+
+# ---- CPU -----------------------------------------------------------------------------------------------------------
+def test_nbest_oracle_n1_is_finalize():
+    B, K, V, T = 3, 4, 160, 10
+    a, c = 120, 121
+    hist = [[R.CLS, a, c, a, a, c, R.EOS], [0, 130, a, a, c, 0], [a, c, a]]
+    prefix = torch.tensor([[R.CLS, 9, a], [7, R.EOS, a], [R.CLS, R.CLS, R.CLS]])
+    logits = _random_logits(B, K, V, T, seed=3)
+    for lg in logits:
+        lg[:, [a, c]] += 3.0
+    makers = [(lambda: OB.BeamState(B, K, V, T), lambda st, lg: st.step(lg)),
+              (lambda: BN.BlockedBeamState(B, K, V, T), lambda st, lg: st.step(lg, 3, hist)),
+              (lambda: PrefixBeamState(B, K, V, T, prefix=prefix), lambda st, lg: st.step(lg, 3, hist))]
+    for make, step in makers:
+        st = make()
+        for lg in logits:
+            step(st, lg)
+        ref = copy.deepcopy(st).finalize()
+        got = finalize_nbest(st, 1)
+        assert torch.equal(ref[0], got[0]) and torch.equal(ref[1], got[1])
+
+
+def test_nbest_oracle_orders_like_hf_pop():
+    st = OB.BeamState(1, 4, 200, 6)
+    st.done[0] = True
+    st.hyps[0] = [(-1.0, [5]), (-0.5, [6, 8]), (-1.0, [7, 9, 10, 11, 12, 13]), (-2.0, [4])]
+    seq, sc = finalize_nbest(copy.deepcopy(st), 4)
+    # stable ascending sort, then pop(): -0.5, then the later-inserted of the two -1.0, then the earlier, then -2.0
+    assert seq.tolist() == [[6, 8, OB.EOS, 0, 0, 0], [7, 9, 10, 11, 12, 13], [5, OB.EOS, 0, 0, 0, 0], [4, OB.EOS, 0, 0, 0, 0]]
+    assert sc.tolist() == [-0.5, -1.0, -1.0, -2.0]
+    seq2, sc2 = finalize_nbest(copy.deepcopy(st), 2)
+    assert torch.equal(seq2, seq[:2]) and torch.equal(sc2, sc[:2])
+    with pytest.raises(ValueError):
+        finalize_nbest(copy.deepcopy(st), 5)
+
+
+def test_nbest_oracle_rows_are_image_major_and_descending():
+    B, K, V, T = 2, 5, 150, 9
+    st = OB.BeamState(B, K, V, T)
+    for lg in _random_logits(B, K, V, T, seed=11):
+        st.step(lg)
+    best = copy.deepcopy(st).finalize()
+    seq, sc = finalize_nbest(st, K)
+    assert torch.equal(seq.view(B, K, T)[:, 0], best[0]) and torch.equal(sc.view(B, K)[:, 0], best[1])
+    assert bool((sc.view(B, K)[:, :-1] >= sc.view(B, K)[:, 1:]).all())
+
+
+def test_candidate_seed():
+    from gst_visdial_b200.models.visual_dialog_model import candidate_seed
+    for s in (0, 1, 12345, 2**64 - 1):
+        assert candidate_seed(s, 0) == s
+        seeds = [candidate_seed(s, n) for n in range(8)]
+        assert len(set(seeds)) == 8 and all(0 <= x < 2**64 for x in seeds)
+
+
+def test_answer_candidates_option(tmp_path):
+    from gst_visdial_b200 import options
+    base = ["-save_path", str(tmp_path)]
+    p = options.read_command_line(base)
+    assert p["answer_candidates"] == 1 and p["engine_max_beams"] == 1
+    p = options.read_command_line(base + ["-answer_candidates", "5"])
+    assert p["answer_candidates"] == 5 and p["engine_max_beams"] == 5
+    p = options.read_command_line(base + ["-answer_candidates", "3", "-num_beams", "4", "-q_num_beams", "2"])
+    assert p["engine_max_beams"] == 4
+    p = options.read_command_line(base + ["-answer_candidates", "6", "-num_beams", "4", "-q_num_beams", "5"])
+    assert p["engine_max_beams"] == 6
+
+
+# ---- GPU: helpers --------------------------------------------------------------------------------------------------
+def _engine(enc_cfg, dec_cfg, sd, dtype, b, B=None, **kw):
+    from gst_visdial_b200.engine import Engine
+    B = B or b["enc_input_ids"].shape[0]
+    kw.setdefault("max_beams", 5)
+    e = Engine(enc_cfg, dec_cfg, dtype=dtype, max_batch=B, **kw)
+    e.load_state_dict(sd)
+    _resident(e, b)
+    return e
+
+
+def _resident(e, b):
+    o = e.encode(b["enc_input_ids"], b["enc_image_feat"], b["enc_image_loc"], b["enc_segments"], b["enc_att_mask"], b["enc_image_mask"])
+    e.prefill_cross(b["enc_input_ids"].shape[0], o["Le"])
+
+
+def _sub(b, lo, hi):
+    return {k: (v[lo:hi] if torch.is_tensor(v) else v) for k, v in b.items()}
+
+
+def _hist(b):
+    return dict(hist_ids=b["enc_input_ids"], hist_segments=b["enc_segments"])
+
+
+def _questions(enc_cfg, B, rounds):
+    from gst_visdial_b200 import synthetic as S
+    q = torch.zeros(B, rounds, 18, dtype=torch.int64)
+    for i in range(B):
+        for r in range(rounds):
+            u = S.synthetic_utterance(i, 40 + r, enc_cfg.vocab_size)
+            u = u[u != 0][:17]
+            q[i, r, :len(u)] = u
+            if R.EOS not in u.tolist():
+                q[i, r, len(u)] = R.EOS
+    return q
+
+
+# ---- GPU: N-best beams against the oracle --------------------------------------------------------------------------
+@pytest.mark.gpu
+@pytest.mark.parametrize("path", ["separate_calls", "whole_round", "no_cuda_graph"])
+@pytest.mark.parametrize("n", [0, 4])
+@pytest.mark.parametrize("K", [3, 5])
+def test_tiny_fp32_nbest_beams_match_oracle(tiny_cfgs, tiny_sd, K, n, path):
+    from gst_visdial_b200 import _lib, weights as W
+    from test_gpu_model import _build_model, _call
+    enc_cfg, dec_cfg = tiny_cfgs
+    a, b4, c, _ = A4["tiny"]
+    sd = _with_bias(tiny_sd, {R.EOS: 3.5})                     # hypotheses end early and replace each other
+    b = _with_question(history_batch(enc_cfg, 0, 3), A4["tiny"])
+    pre5 = _prefixes(3, 5, enc_cfg.vocab_size)
+    pre5[0, -3:] = torch.tensor([a, b4, c])
+    cls = torch.full((3, 1), R.CLS, dtype=torch.int64)
+    kw = {"separate_calls": dict(engine_round_graph=False), "whole_round": {},
+          "no_cuda_graph": dict(engine_flags=_lib.GSTVD_FLAG_NO_CUDA_GRAPH)}[path]
+    model, _ = _build_model(W.TINY_ENC_CONFIG, W.TINY_DEC_CONFIG, sd, "fp32", **kw)
+    eng = model.module._engine(torch.device("cuda:0"))
+    Ns = range(1, K + 1)
+    for dec_ids, prefix in ((cls, None), (pre5, pre5)):
+        with torch.no_grad():
+            refs = _nbest(prefix_beam_state(sd, enc_cfg, dec_cfg, b, K, ngram_blocking_size=n, prefix=prefix), Ns)
+        assert (refs[K][0] == R.EOS).any()
+        single, _ = _call(model, b, dec_ids=dec_ids.clone(), ngram_blocking_size=n, num_beams=K, **_GREEDY)
+        for N in Ns:
+            ref, ref_sc = refs[N]
+            seq, _ = _call(model, b, dec_ids=dec_ids.clone(), ngram_blocking_size=n, num_beams=K, num_return_sequences=N, **_GREEDY)
+            assert seq.shape == (3 * N, 18)
+            assert torch.equal(seq.cpu(), ref), f"P={dec_ids.shape[1]} N={N}: {seq.cpu().tolist()} vs {ref.tolist()}"
+            assert torch.equal(seq.view(3, N, 18)[:, 0], single), "candidate 0 differs from the single-sequence output"
+            seq2, sc2 = eng.generate(3, num_beams=K, ngram_blocking_size=n, prefix=prefix, want_scores=True, num_return_sequences=N, **_hist(b))
+            assert torch.equal(seq2.cpu(), ref)
+            assert torch.allclose(sc2.cpu().double(), ref_sc, atol=1e-4), (sc2, ref_sc)
+
+
+@pytest.mark.gpu
+def test_full_fp32_nbest_beams_match_oracle(full_cfgs, full_sd):
+    enc_cfg, dec_cfg = full_cfgs
+    sd = _with_bias(full_sd, {R.EOS: 2.5})
+    b = _with_question(history_batch(enc_cfg, 0, 2), A4["full"])
+    K = 5
+    with torch.no_grad():
+        refs = _nbest(prefix_beam_state(sd, enc_cfg, dec_cfg, b, K, ngram_blocking_size=4), range(1, K + 1))
+    e = _engine(enc_cfg, dec_cfg, sd, "fp32", b)
+    try:
+        for N, (ref, ref_sc) in refs.items():
+            seq, sc = e.generate(2, num_beams=K, ngram_blocking_size=4, want_scores=True, num_return_sequences=N, **_hist(b))
+            assert torch.equal(seq.cpu(), ref), f"N={N}"
+            assert torch.allclose(sc.cpu().double(), ref_sc, atol=1e-4)
+    finally:
+        e.close()
+
+
+# ---- GPU: sampled candidates -----------------------------------------------------------------------------------------
+_SAMPLE_CASES = {
+    "topk7": (dict(temperature=0.7, top_k=7, top_p=0.0), 0, None),
+    "nucleus": (dict(temperature=1.0, top_k=0, top_p=0.9), 0, None),
+    "topk7_ngram4": (dict(temperature=0.7, top_k=7, top_p=0.0), 4, None),
+    "topk7_prefix5": (dict(temperature=0.7, top_k=7, top_p=0.0), 4, 5),
+}
+
+
+def _sample_kw(case, b, vocab):
+    mk, n, P = _SAMPLE_CASES[case]
+    B = b["enc_input_ids"].shape[0]
+    return dict(mk, ngram_blocking_size=n, prefix=_prefixes(B, P, vocab) if P else None, **_hist(b))
+
+
+@pytest.mark.gpu
+@pytest.mark.parametrize("size", ["tiny", "full"])
+def test_fp32_sampled_candidates_equal_single_calls(size, tiny_cfgs, tiny_sd, full_cfgs, full_sd):
+    from gst_visdial_b200.models.visual_dialog_model import candidate_seed
+    enc_cfg, dec_cfg = tiny_cfgs if size == "tiny" else full_cfgs
+    sd = tiny_sd if size == "tiny" else full_sd
+    B, N, seed = (4, 4, 77) if size == "tiny" else (3, 4, 78)
+    b = _with_question(history_batch(enc_cfg, 0, B), A4[size])
+    e = _engine(enc_cfg, dec_cfg, sd, "fp32", b)
+    try:
+        for case in _SAMPLE_CASES:
+            kw = _sample_kw(case, b, enc_cfg.vocab_size)
+            cand = e.generate(B, seed=seed, num_return_sequences=N, **kw).cpu().view(B, N, 18)
+            for n in range(N):
+                one = e.generate(B, seed=candidate_seed(seed, n), **kw).cpu()
+                assert torch.equal(cand[:, n], one), f"{case}: candidate {n} differs from the single-sample call"
+            assert all(len({tuple(r) for r in cand[i].tolist()}) > 1 for i in range(B)), f"{case}: an image's candidates are all equal"
+            if case == "topk7_ngram4":
+                hist = BN.question_history(b["enc_input_ids"], b["enc_segments"])
+                assert not any(contains_banned_ngram(hist[i], cand[i, n].tolist(), 4, [R.CLS]) for i in range(B) for n in range(N))
+            # the same images split into two calls with row offsets 0 and k
+            k = B // 2
+            parts = []
+            for lo, hi in ((0, k), (k, B)):
+                bs = _sub(b, lo, hi)
+                _resident(e, bs)
+                kws = dict(kw, prefix=kw["prefix"][lo:hi] if kw["prefix"] is not None else None, **_hist(bs))
+                parts.append(e.generate(hi - lo, seed=seed, num_return_sequences=N, row_offset=lo, **kws).cpu())
+            _resident(e, b)
+            assert torch.equal(torch.cat(parts).view(B, N, 18), cand), f"{case}: split calls differ"
+    finally:
+        e.close()
+
+
+# Sampled candidates in bf16 run with M = B*N decode rows instead of B.  Share of (image, candidate) pairs whose tokens equal the
+# single-sample call with candidate_seed(seed, n), full config, B = 64, N = 5, top-k 7 with 4-gram blocking: measured 1.000 (320 of
+# 320) on an NVIDIA B200 at its 1000 W power limit; the per-row arithmetic of the decode step does not depend on M there.
+BF16_CANDIDATE_AGREEMENT_MIN = 1.0
+
+
+@pytest.mark.gpu
+def test_full_bf16_candidates_paths_agree(full_cfgs, full_sd):
+    from gst_visdial_b200 import _lib, weights as W
+    from gst_visdial_b200.models.visual_dialog_model import candidate_seed
+    from test_gpu_model import _build_model, _call
+    enc_cfg, dec_cfg = full_cfgs
+    B, N, seed = 64, 5, 21
+    b = history_batch(enc_cfg, 0, B)
+    modes = {"sample": dict(temperature=0.7, top_k=7, top_p=0.0, ngram_blocking_size=4, seed=seed),
+             "beam": dict(num_beams=5, ngram_blocking_size=4, **_GREEDY)}
+    outs = {}
+    for name, kw in (("whole_round", {}), ("separate_calls", dict(engine_round_graph=False)),
+                     ("no_cuda_graph", dict(engine_round_graph=False, engine_flags=_lib.GSTVD_FLAG_NO_CUDA_GRAPH))):
+        model, _ = _build_model(W.DEFAULT_ENC_CONFIG, W.DEFAULT_DEC_CONFIG, full_sd, "bf16", engine_max_batch=B, **kw)
+        for m, mk in modes.items():
+            runs = [_call(model, b, num_return_sequences=N, **mk)[0].cpu() for _ in range(2)]
+            assert runs[0].shape == (B * N, 18)
+            assert torch.equal(runs[0], runs[1]), f"{name} / {m}: repeated calls differ"
+            outs[(name, m)] = runs[0]
+            one = _call(model, b, **mk)[0].cpu()
+            assert torch.equal(runs[0].view(B, N, 18)[:, 0], one), f"{name} / {m}: candidate 0 differs from the N = 1 output"
+        del model
+        torch.cuda.empty_cache()
+    for m in modes:
+        assert torch.equal(outs[("separate_calls", m)], outs[("whole_round", m)]), f"{m}: whole-round graph differs from separate calls"
+        assert torch.equal(outs[("no_cuda_graph", m)], outs[("whole_round", m)]), f"{m}: eager decode differs from the captured graph"
+    hist = BN.question_history(b["enc_input_ids"], b["enc_segments"])
+    for m in modes:
+        cand = outs[("whole_round", m)].view(B, N, 18)
+        assert not any(contains_banned_ngram(hist[i], cand[i, n].tolist(), 4, [R.CLS]) for i in range(B) for n in range(N)), m
+    e = _engine(enc_cfg, dec_cfg, full_sd, "bf16", b)
+    try:
+        kw = dict(modes["sample"], **_hist(b))
+        kw.pop("seed")
+        cand = e.generate(B, seed=seed, num_return_sequences=N, **kw).cpu().view(B, N, 18)
+        assert torch.equal(cand, outs[("separate_calls", "sample")].view(B, N, 18))
+        same = torch.stack([(cand[:, n] == e.generate(B, seed=candidate_seed(seed, n), **kw).cpu()).all(1) for n in range(N)], 1)
+        agree = same.float().mean().item()
+        print(f"bf16 sampled candidates equal to their single-sample calls: {agree:.3f} of {B * N} (image, candidate) pairs")
+        assert bool(same[:, 0].all()), "candidate 0 must be the N = 1 sample"
+        assert agree >= BF16_CANDIDATE_AGREEMENT_MIN, agree
+    finally:
+        e.close()
+
+
+# ---- GPU: dialog loop --------------------------------------------------------------------------------------------------
+def _dialog(model, b, q, **kw):
+    from gst_visdial_b200.dialog import generate_dialogs
+    eng = model.module._engine(torch.device("cuda:0"))
+    l0 = eng.launch_count
+    res = generate_dialogs(model, b, questions=q, num_rounds=q.shape[1], device="cuda:0", trim_history=False, seed=5, **kw)
+    torch.cuda.synchronize()
+    return res, eng.launch_count - l0
+
+
+@pytest.mark.gpu
+def test_dialog_answer_candidates(tiny_cfgs, tiny_sd):
+    from gst_visdial_b200 import ranking, weights as W
+    from gst_visdial_b200.models.visual_dialog_model import derive_seed
+    from test_gpu_model import _build_model, _call
+    enc_cfg, _ = tiny_cfgs
+    B, rounds, N = 3, 2, 3
+    b = history_batch(enc_cfg, 0, B)
+    q = _questions(enc_cfg, B, rounds)
+    model, _ = _build_model(W.TINY_ENC_CONFIG, W.TINY_DEC_CONFIG, tiny_sd, "fp32")
+    # answer_candidates = 1 is the plain loop
+    base, n_base = _dialog(model, b, q)
+    one, n_one = _dialog(model, b, q, answer_candidates=1)
+    assert torch.equal(base.answers, one.answers) and torch.equal(base.abnormal, one.abnormal) and n_base == n_one
+    assert torch.equal(base.answer_ppl, one.answer_ppl)
+    res, _ = _dialog(model, b, q, answer_candidates=N)
+    assert res.answers.shape == (B, rounds, 18) and res.answer_ppl.shape == (B, rounds)
+    # every round: the spliced answer is one of the candidates of a direct num_return_sequences call, with the least perplexity
+    h = {k: (v.clone() if torch.is_tensor(v) else v) for k, v in b.items()}
+    ids, seg = h["enc_input_ids"], h["enc_segments"]
+    enc_len = (ids != 0).sum(-1)
+    for r in range(rounds):
+        enc_len = enc_len + R.splice(ids, seg, enc_len, q[:, r], None, set())
+        h["enc_att_mask"] = (ids != 0).float()
+        cands, _ = _call(model, h, num_return_sequences=N, temperature=0.7, top_k=7, top_p=0.0, ngram_blocking_size=0,
+                         seed=derive_seed(5, "a", r), row_offset=0)
+        cands = cands.cpu().view(B, N, 18)
+        ppl = torch.stack([ranking.answer_perplexity(model, h, cands[:, n]).cpu() for n in range(N)], 1)
+        chosen = res.answers[:, r].cpu()
+        masked = cands.masked_fill(cands == R.EOS, R.PAD)
+        assert all(any(torch.equal(chosen[i], masked[i, n]) for n in range(N)) for i in range(B)), f"round {r}"
+        best = torch.sort(ppl, dim=1, stable=True).values[:, 0]
+        assert torch.allclose(res.answer_ppl[:, r].cpu(), best, rtol=1e-5, equal_nan=True), (res.answer_ppl[:, r], ppl)
+        enc_len = enc_len + R.splice(ids, seg, enc_len, chosen, 1, set())
+
+
+@pytest.mark.gpu
+def test_tiny_fp32_beam_dialog_candidates_match_oracle(tiny_cfgs, tiny_sd):
+    from gst_visdial_b200 import weights as W
+    from test_gpu_model import _build_model
+    enc_cfg, dec_cfg = tiny_cfgs
+    B, rounds, K = 3, 2, 3
+    sd = _with_bias(tiny_sd, {R.EOS: 2.5})
+    b = history_batch(enc_cfg, 0, B)
+    q = _questions(enc_cfg, B, rounds)
+    model, _ = _build_model(W.TINY_ENC_CONFIG, W.TINY_DEC_CONFIG, sd, "fp32")
+    res, _ = _dialog(model, b, q, a_kwargs=dict(num_beams=K, ngram_blocking_size=0, **_GREEDY), answer_candidates=K)
+    # oracle composition: N-best beams -> perplexity of each (restatement.score_answers) -> argmin -> splice
+    h = {k: (v.clone() if torch.is_tensor(v) else v) for k, v in b.items()}
+    ids, seg = h["enc_input_ids"], h["enc_segments"]
+    enc_len = (ids != 0).sum(-1)
+    with torch.no_grad():
+        for r in range(rounds):
+            enc_len = enc_len + R.splice(ids, seg, enc_len, q[:, r], None, set())
+            h["enc_att_mask"] = (ids != 0).float()
+            cands = finalize_nbest(prefix_beam_state(sd, enc_cfg, dec_cfg, h, K), K)[0].view(B, K, 18)
+            ppl = torch.stack([R.score_answers(sd, enc_cfg, dec_cfg, h, cands[:, n])[2] for n in range(K)], 1)
+            best = torch.sort(ppl, dim=1, stable=True).indices[:, 0]
+            ans = cands[torch.arange(B), best]
+            ans = ans.masked_fill(ans == R.EOS, R.PAD)
+            assert torch.equal(res.answers[:, r].cpu(), ans), f"round {r}: {res.answers[:, r].tolist()} vs {ans.tolist()}"
+            assert torch.allclose(res.answer_ppl[:, r].cpu().double(), ppl[torch.arange(B), best].double(), rtol=1e-4)
+            enc_len = enc_len + R.splice(ids, seg, enc_len, ans, 1, set())
+
+
+@pytest.mark.gpu
+def test_generate_cli_answer_candidates(tmp_path):
+    import json
+    import subprocess
+    import sys
+    from helpers import ROOT
+    cmd = [sys.executable, os.path.join(ROOT, "generate.py"), "-synthetic", "8", "-batch_size", "8", "-answer_candidates", "3",
+           "-num_rounds", "2", "-save_path", str(tmp_path), "-save_name", "o.json"]
+    r = subprocess.run(cmd, capture_output=True, text=True, timeout=1200)
+    assert r.returncode == 0, r.stdout + r.stderr
+    out = json.load(open(tmp_path / "o.json"))
+    assert len(out) == 8 and all(len(d["dialog"]) == 2 for d in out)
+
+
+# ---- GPU: argument checks ------------------------------------------------------------------------------------------
+@pytest.mark.gpu
+def test_candidate_rejections(tiny_cfgs, tiny_sd):
+    from gst_visdial_b200._lib import GstvdError
+    GSTVD_ERR_INVALID = -1
+    enc_cfg, dec_cfg = tiny_cfgs
+    B = 2
+    b = history_batch(enc_cfg, 0, B)
+    rnd = (b["enc_input_ids"], b["enc_image_feat"], b["enc_image_loc"], b["enc_segments"], b["enc_att_mask"], b["enc_image_mask"])
+    for max_beams, bad in ((5, [dict(num_return_sequences=0), dict(num_beams=3, num_return_sequences=4), dict(num_return_sequences=6),
+                                 dict(num_beams=3, num_return_sequences=0)]),
+                           (8, [dict(num_return_sequences=9)])):
+        e = _engine(enc_cfg, dec_cfg, tiny_sd, "fp32", b, max_beams=max_beams)
+        try:
+            for kw in bad:
+                with pytest.raises(GstvdError) as ei:
+                    e.generate(B, **kw)
+                assert ei.value.status == GSTVD_ERR_INVALID, kw
+                with pytest.raises(GstvdError) as ei:
+                    e.round(*rnd, **kw)
+                assert ei.value.status == GSTVD_ERR_INVALID, kw
+            assert e.generate(B, num_return_sequences=max_beams).shape == (B * max_beams, 18)
+            assert e.generate(B, num_beams=3, num_return_sequences=3).shape == (B * 3, 18)
+        finally:
+            e.close()
