@@ -6,6 +6,8 @@ generate.py: same single-dash flags, same output JSON layout), running on the B2
     python generate.py -synthetic 128 -batch_size 64 -num_beams 5          # seeded synthetic images + random weights
     python generate.py -synthetic 128 -batch_size 64 -num_beams 5 -q_num_beams 5   # beam-searched questions too (4-gram blocked)
     python generate.py -synthetic 128 -batch_size 64 -answer_candidates 5          # 5 sampled answers per round, lowest perplexity kept
+    python generate.py -synthetic 128 -batch_size 64 -num_beams 6 -num_beam_groups 3 -diversity_penalty 0.5 -answer_candidates 6
+                                                                                   # diverse beams ranked by perplexity
 
 Multi-GPU: launch with torchrun (one process per GPU); images are sharded by rank and gathered once at the end.
 The dataset readers (LMDB / tokenizer) of the reference are host I/O outside the hot path: without them (-synthetic)
@@ -79,10 +81,11 @@ def main(argv=None):
     start, end = D.shard_range(total, rank, world)
     a_kwargs = dict(temperature=0.7, top_k=7, top_p=0.0, ngram_blocking_size=0)
     if params['num_beams'] > 1:
-        a_kwargs.update(num_beams=params['num_beams'])
+        a_kwargs.update(num_beams=params['num_beams'], num_beam_groups=params['num_beam_groups'], diversity_penalty=params['diversity_penalty'])
     q_kwargs = dict(temperature=0.7, top_k=7, top_p=0.0, ngram_blocking_size=4)
     if params['q_num_beams'] > 1:
-        q_kwargs.update(num_beams=params['q_num_beams'])
+        q_kwargs.update(num_beams=params['q_num_beams'], num_beam_groups=params['q_num_beam_groups'],
+                        diversity_penalty=params['q_diversity_penalty'])
     decode = None
     if params['vocab_file']:
         from transformers import BertTokenizer

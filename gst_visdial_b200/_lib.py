@@ -70,9 +70,12 @@ SYMBOLS = [
     ("gstvd_generate", c_int, [_P, c_int, POINTER(GstvdGenParams), _P, _P, c_int, _P, _P, _P]),
     ("gstvd_generate_prefixed", c_int, [_P, c_int, POINTER(GstvdGenParams), _P, c_int, _P, _P, c_int, _P, _P, _P]),
     ("gstvd_generate_candidates", c_int, [_P, c_int, POINTER(GstvdGenParams), c_int, _P, c_int, _P, _P, c_int, _P, _P, _P]),
+    ("gstvd_generate_groups", c_int, [_P, c_int, POINTER(GstvdGenParams), c_int, c_float, c_int, _P, c_int, _P, _P, c_int, _P, _P, _P]),
     ("gstvd_round", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(GstvdGenParams), _P, _P, _P]),
     ("gstvd_round_prefixed", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(GstvdGenParams), _P, c_int, _P, _P, _P]),
     ("gstvd_round_candidates", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(GstvdGenParams), c_int, _P, c_int, _P, _P, _P]),
+    ("gstvd_round_groups", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(GstvdGenParams), c_int, c_float, c_int, _P, c_int,
+                                   _P, _P, _P]),
     ("gstvd_score", c_int, [_P, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     ("gstvd_score_options", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     ("gstvd_reorder_cache", c_int, [_P, c_int, c_int, c_int, _P, _P]),

@@ -6,6 +6,7 @@
 // (call site models/visual_dialog_decoder.py:300-311).
 #include <cuda_runtime.h>
 
+#include <cmath>
 #include <cstdarg>
 #include <cstdlib>
 #include <cstdio>
@@ -68,9 +69,10 @@ struct DevBuf {
 
 // Shapes and selection parameters only: the n-gram blocking history and the decoder prefix are copied into context-owned buffers
 // before a replay, so the caller's tensor addresses are not part of the key (a caching allocator hands out a new address per batch).
-// P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start; N = sequences returned per image.
+// P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start; N = sequences returned per image; G / penalty = beam groups
+// and diversity penalty.
 struct GraphKey {
-  int B, K, mode, T, top_k, ngram, Lh, Le, P, has_prefix, N; float temperature, top_p;
+  int B, K, mode, T, top_k, ngram, Lh, Le, P, has_prefix, N, G; float temperature, top_p, penalty;
   bool operator<(const GraphKey& o) const { return std::memcmp(this, &o, sizeof(GraphKey)) < 0; }
 };
 constexpr size_t kMaxGraphs = 24;      // least-recently-used graphs beyond this are destroyed (an 18-step graph holds ~2k kernel nodes)
@@ -130,7 +132,7 @@ struct gstvd_ctx {
   uint64_t graph_clock = 0;
   // whole-round graphs (gstvd_round): encoder + cross-K/V prefill + every decode step of one forward call in ONE graph, keyed by shapes
   struct RoundKey {
-    int B, Lt, Lv, K, mode, T, top_k, ngram, has_seg, has_att, has_imask, P, has_prefix, N; float temperature, top_p;
+    int B, Lt, Lv, K, mode, T, top_k, ngram, has_seg, has_att, has_imask, P, has_prefix, N, G; float temperature, top_p, penalty;
     bool operator<(const RoundKey& o) const { return std::memcmp(this, &o, sizeof(RoundKey)) < 0; }
   };
   std::map<RoundKey, GraphEntry> round_graphs;
@@ -668,9 +670,9 @@ const int64_t* stage_prefix(gstvd_ctx* c, int B, const int64_t* prefix, int P, c
 }
 
 // Selection state of a decode call: beams / sample rows start from the last token of the prefix (the [CLS] when it is null).
-void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* prefix, cudaStream_t s) {
+void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, int G, const int64_t* prefix, cudaStream_t s) {
   const int P = g.P0 + 1, T = gp.max_new_tokens;
-  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, T, 101, prefix, P, s);
+  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, G, T, 101, prefix, P, s);
   else c->launches += launch_sample_init(g.B * g.K, g.K, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, P + T, (int*)c->d_step.p,
                                          prefix, P, s);
 }
@@ -678,9 +680,9 @@ void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
 // One decode step for all M = B*K rows: embeddings -> 12 x [self-attn over cache, cross-attn, FFN] -> LM head -> selection.
 // step_host = index of this step when the caller knows it (it always does: eager loops and the captured graph both unroll the
 // steps), so kernels that only need it to bound their loads take it as a launch parameter instead of reading *d_step first.
-// prefix: int64 [B, P] decoder prefix (P = g.P0 + 1), null for the [CLS] start.
-void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* prefix, const int64_t* hist_ids,
-                 const int64_t* hist_seg, int Lh, cudaStream_t s, int step_host) {
+// prefix: int64 [B, P] decoder prefix (P = g.P0 + 1), null for the [CLS] start.  G / penalty: beam groups and diversity penalty.
+void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, int G, float penalty, const int64_t* prefix,
+                 const int64_t* hist_ids, const int64_t* hist_seg, int Lh, cudaStream_t s, int step_host) {
   Exec X{c, s};
   PdlScope pdl_scope(!(c->cfg.flags & GSTVD_FLAG_NO_PDL));
   const int H = c->H, M = g.B * g.K;
@@ -756,9 +758,13 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
                                            step_host, n, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }
+    // beam groups: row_select also writes each row's logZ, from which the beam step re-scores the candidates a diversity penalty
+    // lowers (the candidate lists stay ranked by the unpenalised score; launch_beam_step explains why nsel = 2K suffices)
+    float* lz = G > 1 ? (float*)c->logz.p : nullptr;
     c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, (c->dtype == kBF16 && !exact_lse) ? 2 : 0,
-                                     (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, nullptr, s);
-    c->launches += launch_beam_step(bb, g.B, g.K, Tn, c->V, nsel, sv, si, 102, P, nullptr, nullptr, nullptr, s);
+                                     (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, lz, s);
+    c->launches += launch_beam_step(bb, g.B, g.K, G, Tn, c->V, nsel, sv, si, G > 1 ? (const float*)c->logits.p : nullptr, c->Vpad, lz,
+                                    penalty, 102, P, nullptr, nullptr, nullptr, s);
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
   } else {
@@ -790,8 +796,8 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
 
 // Argument checks of a generate call returning N sequences per image; returns the decode rows per image (beam mode: the beams;
 // sample mode: the N candidates).
-int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, int N, const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_seg,
-                   int Lh, const int64_t* out_ids) {
+int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, int N, int G, float penalty, const int64_t* prefix, int P, const int64_t* hist_ids,
+                   const int64_t* hist_seg, int Lh, const int64_t* out_ids) {
   check_ready(c);
   if (c->dec_layers == 0) throw StateError("generate: encoder-only context");
   const int T = gp.max_new_tokens;
@@ -803,11 +809,15 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, int N, const int64_
   if (P - 1 + T > c->cfg.max_position_embeddings)
     throw InvalidArg(fmt("generate: prefix length %d + %d new tokens exceed max_position_embeddings (%d)", P, T, c->cfg.max_position_embeddings));
   if (!out_ids) throw InvalidArg("generate: out_ids is NULL");
+  if (!(penalty >= 0.f) || !std::isfinite(penalty)) throw InvalidArg(fmt("generate: diversity_penalty %g must be finite and >= 0", (double)penalty));
+  if (G < 1) throw InvalidArg(fmt("generate: %d beam groups", G));
+  if (G > 1 && gp.mode != GSTVD_SELECT_BEAM) throw InvalidArg("generate: beam groups need beam search");
   int K = 1;
   if (gp.mode == GSTVD_SELECT_BEAM) {
     K = gp.num_beams;
     if (K < 1 || K > c->K_max || 2 * K > kSelMax) throw InvalidArg("generate: num_beams out of range");
     if (N < 1 || N > K) throw InvalidArg(fmt("generate: %d return sequences outside 1..num_beams (%d)", N, K));
+    if (K % G != 0) throw InvalidArg(fmt("generate: %d beam groups do not divide %d beams", G, K));
   } else if (gp.mode == GSTVD_SELECT_SAMPLE) {
     if (N < 1 || N > c->K_max || N > 8) throw InvalidArg(fmt("generate: %d sampled candidates outside 1..min(8, max_beams = %d)", N, c->K_max));
     K = N;
@@ -828,26 +838,26 @@ void generate_finalize(gstvd_ctx* c, int B, int K, int P, int N, const gstvd_gen
   else c->launches += launch_sample_finalize(B * K, T, 102, (const int32_t*)c->seq.p, out_ids, s);
 }
 
-void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, int N, const int64_t* prefix, int P, const int64_t* hist_ids,
-                 const int64_t* hist_seg, int Lh, int64_t* out_ids, float* out_scores, cudaStream_t s) {
-  const int K = check_generate(c, gp, N, prefix, P, hist_ids, hist_seg, Lh, out_ids);
+void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, int N, int G, float penalty, const int64_t* prefix, int P,
+                 const int64_t* hist_ids, const int64_t* hist_seg, int Lh, int64_t* out_ids, float* out_scores, cudaStream_t s) {
+  const int K = check_generate(c, gp, N, G, penalty, prefix, P, hist_ids, hist_seg, Lh, out_ids);
   if (c->cross_B != B) throw StateError(fmt("generate: cross K/V prefilled for %d images, asked for %d", c->cross_B, B));
   const int T = gp.max_new_tokens;
   const DecodeGeom g = make_geom(c, B, K, T, P);
   const int64_t* pre = stage_prefix(c, B, prefix, P, s);
   // the sampling seed lives in device memory so that a captured graph can be replayed with a new seed
   c->launches += launch_set_u64((uint64_t*)c->d_seed.p, gp.seed, (uint64_t)gp.row_offset, s);
-  decode_init(c, g, gp, pre, s);
+  decode_init(c, g, gp, G, pre, s);
 
   const bool use_graph = !(c->cfg.flags & GSTVD_FLAG_NO_CUDA_GRAPH);
   if (!use_graph) {
     prefix_prefill(c, g, s);
-    for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, hist_ids, hist_seg, Lh, s, t);
+    for (int t = 0; t < T; ++t) decode_step(c, g, gp, G, penalty, pre, hist_ids, hist_seg, Lh, s, t);
   } else {
     GraphKey key;
     std::memset(&key, 0, sizeof key);
     key.B = B; key.K = K; key.mode = gp.mode; key.T = T; key.top_k = gp.top_k; key.ngram = gp.ngram_blocking_size; key.Lh = Lh;
-    key.P = P; key.has_prefix = pre != nullptr; key.N = N;
+    key.P = P; key.has_prefix = pre != nullptr; key.N = N; key.G = G; key.penalty = penalty;
     key.temperature = gp.temperature; key.top_p = gp.top_p;
     key.Le = c->cross_Le;                    // the cross cache geometry is part of the captured launch parameters
     const int64_t* g_ids = hist_ids; const int64_t* g_seg = hist_seg;
@@ -871,7 +881,7 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, int N, const i
       CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
       try {
         prefix_prefill(c, g, s);
-        for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, g_ids, g_seg, Lh, s, t);   // all T steps in ONE graph: no host round trip between steps
+        for (int t = 0; t < T; ++t) decode_step(c, g, gp, G, penalty, pre, g_ids, g_seg, Lh, s, t);   // all T steps in ONE graph: no host round trip between steps
       } catch (...) {
         cudaGraph_t dead; cudaStreamEndCapture(s, &dead);
         throw;
@@ -896,9 +906,9 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, int N, const i
 // order, same results as gstvd_encode + gstvd_prefill_cross + gstvd_generate (asserted by the tests); eager when graphs are
 // disabled or while the GEMM profiler is on (events cannot be recorded inside a graph).
 void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int64_t* seg, const float* att, const float* feat,
-              const float* loc, const float* imask, const gstvd_gen_params& gp, int N, const int64_t* prefix, int P, int64_t* out_ids,
-              float* out_scores, cudaStream_t s) {
-  const int K = check_generate(c, gp, N, prefix, P, ids, seg ? seg : ids, Lt, out_ids);
+              const float* loc, const float* imask, const gstvd_gen_params& gp, int N, int G, float penalty, const int64_t* prefix, int P,
+              int64_t* out_ids, float* out_scores, cudaStream_t s) {
+  const int K = check_generate(c, gp, N, G, penalty, prefix, P, ids, seg ? seg : ids, Lt, out_ids);
   if (B < 1 || B > c->B_max || Lt < 1 || Lt > c->Lt_max || Lv < 1 || Lv > c->Lv_max) throw InvalidArg("round: shape exceeds capacity");
   if (!ids || !feat || !loc) throw InvalidArg("round: input_ids / image_feat / image_loc must not be NULL");
   if (gp.ngram_blocking_size > 0 && !seg) throw InvalidArg("round: n-gram blocking needs token_type_ids");
@@ -915,9 +925,9 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
               imask ? (const float*)c->r_imask.p : nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, s);
     do_prefill(c, B, Lv + Lt, nullptr, nullptr, s);
     const DecodeGeom g = make_geom(c, B, K, T, P);
-    decode_init(c, g, gp, pre, s);
+    decode_init(c, g, gp, G, pre, s);
     prefix_prefill(c, g, s);
-    for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, g_ids, g_seg, Lt, s, t);
+    for (int t = 0; t < T; ++t) decode_step(c, g, gp, G, penalty, pre, g_ids, g_seg, Lt, s, t);
     generate_finalize(c, B, K, P, N, gp, (int64_t*)c->r_out_ids.p, out_scores ? (float*)c->r_out_scores.p : nullptr, s);
   };
   const bool use_graph = !(c->cfg.flags & GSTVD_FLAG_NO_CUDA_GRAPH) && !c->profiling;
@@ -929,7 +939,7 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
     key.B = B; key.Lt = Lt; key.Lv = Lv; key.K = K; key.mode = gp.mode; key.T = T; key.top_k = gp.top_k; key.ngram = gp.ngram_blocking_size;
     key.has_seg = seg != nullptr; key.has_att = att != nullptr; key.has_imask = imask != nullptr;
     key.temperature = gp.temperature; key.top_p = gp.top_p;
-    key.P = P; key.has_prefix = pre != nullptr; key.N = N;
+    key.P = P; key.has_prefix = pre != nullptr; key.N = N; key.G = G; key.penalty = penalty;
     if (out_scores) key.has_imask |= 2;
     auto it = c->round_graphs.find(key);
     if (it == c->round_graphs.end()) {
@@ -1180,12 +1190,19 @@ int gstvd_generate_prefixed(gstvd_ctx* c, int B, const gstvd_gen_params* params,
 int gstvd_generate_candidates(gstvd_ctx* c, int B, const gstvd_gen_params* params, int N, const int64_t* prefix, int P,
                               const int64_t* hist_ids, const int64_t* hist_segments, int Lh, int64_t* out_ids, float* out_scores,
                               void* stream) {
+  return gstvd_generate_groups(c, B, params, 1, 0.f, N, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores, stream);
+}
+
+int gstvd_generate_groups(gstvd_ctx* c, int B, const gstvd_gen_params* params, int num_beam_groups, float diversity_penalty, int N,
+                          const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_segments, int Lh, int64_t* out_ids,
+                          float* out_scores, void* stream) {
   if (!c || !params) { g_last_error = "gstvd_generate: NULL argument"; return GSTVD_ERR_INVALID; }
   return guarded(c, [&] {
     cudaStream_t user = (cudaStream_t)stream;
     CUDA_CHECK(cudaEventRecord(c->ev_in, user));
     CUDA_CHECK(cudaStreamWaitEvent(c->own_stream, c->ev_in, 0));
-    do_generate(c, B, *params, N, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores, c->own_stream);
+    do_generate(c, B, *params, N, num_beam_groups, diversity_penalty, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores,
+                c->own_stream);
     CUDA_CHECK(cudaEventRecord(c->ev_out, c->own_stream));
     CUDA_CHECK(cudaStreamWaitEvent(user, c->ev_out, 0));
   });
@@ -1209,13 +1226,21 @@ int gstvd_round_candidates(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* i
                            const float* attention_mask, const float* image_feat, const float* image_loc, const float* image_mask,
                            const gstvd_gen_params* params, int N, const int64_t* prefix, int P, int64_t* out_ids, float* out_scores,
                            void* stream) {
+  return gstvd_round_groups(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, params, 1, 0.f, N,
+                            prefix, P, out_ids, out_scores, stream);
+}
+
+int gstvd_round_groups(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, const int64_t* token_type_ids,
+                       const float* attention_mask, const float* image_feat, const float* image_loc, const float* image_mask,
+                       const gstvd_gen_params* params, int num_beam_groups, float diversity_penalty, int N, const int64_t* prefix, int P,
+                       int64_t* out_ids, float* out_scores, void* stream) {
   if (!c || !params) { g_last_error = "gstvd_round: NULL argument"; return GSTVD_ERR_INVALID; }
   return guarded(c, [&] {
     cudaStream_t user = (cudaStream_t)stream;
     CUDA_CHECK(cudaEventRecord(c->ev_in, user));
     CUDA_CHECK(cudaStreamWaitEvent(c->own_stream, c->ev_in, 0));
-    do_round(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, *params, N, prefix, P, out_ids,
-             out_scores, c->own_stream);
+    do_round(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, *params, N, num_beam_groups,
+             diversity_penalty, prefix, P, out_ids, out_scores, c->own_stream);
     CUDA_CHECK(cudaEventRecord(c->ev_out, c->own_stream));
     CUDA_CHECK(cudaStreamWaitEvent(user, c->ev_out, 0));
   });
@@ -1466,7 +1491,7 @@ int gstvd_op_beam_begin(gstvd_ctx* c, int B, int K, int max_new, void* stream) {
     if (c->dec_layers == 0) throw StateError("beam ops need a decoder context");
     if (B < 1 || B > c->B_max || K < 1 || K > c->K_max || max_new < 1 || max_new > c->T_max) throw InvalidArg("beam_begin: shape out of range");
     c->op_B = B; c->op_K = K; c->op_T = max_new;
-    c->launches += launch_beam_init(beam_buffers(c), B, K, max_new, 101, nullptr, 1, (cudaStream_t)stream);
+    c->launches += launch_beam_init(beam_buffers(c), B, K, 1, max_new, 101, nullptr, 1, (cudaStream_t)stream);
   });
 }
 
@@ -1479,8 +1504,8 @@ int gstvd_op_beam_step(gstvd_ctx* c, const float* logits, int64_t ldl, int32_t* 
     const int B = c->op_B, K = c->op_K, T = c->op_T, nsel = 2 * K;
     c->launches += launch_row_select(B * K, c->V, logits, ldl, 0, (const float*)c->beam_scores.p, 1.f, nullptr, nullptr, 0, nsel,
                                      (float*)c->sel_val.p, (int32_t*)c->sel_idx.p, nullptr, s);
-    c->launches += launch_beam_step(beam_buffers(c), B, K, T, c->V, nsel, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, 102,
-                                    1, beam_idx, next_tokens, next_scores, s);
+    c->launches += launch_beam_step(beam_buffers(c), B, K, 1, T, c->V, nsel, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, nullptr,
+                                    0, nullptr, 0.f, 102, 1, beam_idx, next_tokens, next_scores, s);
     c->launches += launch_step_advance((int*)c->d_step.p, s);
   });
 }

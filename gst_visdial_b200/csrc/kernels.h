@@ -183,11 +183,15 @@ struct BeamBuffers {
   double* hyp_worst;       // [B]
   int* d_step;             // device step counter
 };
-// prefix: int64 [B, P] decoder prefix (null: start_token, P = 1); len0 = P, the prefix length counted in every hypothesis length
-int launch_beam_init(const BeamBuffers& bb, int B, int K, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream);
-int launch_beam_step(const BeamBuffers& bb, int B, int K, int T, int V, int nsel, const float* sel_val,
-                     const int32_t* sel_idx, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
-                     cudaStream_t stream);
+// prefix: int64 [B, P] decoder prefix (null: start_token, P = 1); len0 = P, the prefix length counted in every hypothesis length.
+// G beam groups of K / G beams (G | K; G = 1: plain beam search): the first beam of every group starts with score 0.
+int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream);
+// G > 1: diverse beam search with the Hamming penalty `penalty` (oracle/beam_groups.py).  A candidate whose token earlier groups took
+// at this step is re-scored from logits [B*K, ldl] fp32 and logz [B*K] (row_select's outputs for this step); needs nsel >= K + K / G.
+// G = 1 reads neither.
+int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
+                     const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, int eos, int len0,
+                     int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores, cudaStream_t stream);
 // out_ids [B*N, T] / out_scores [B*N]: the N <= K best finished hypotheses of every image, image-major, in the pop order of HF
 // BeamSearchScorer.finalize (score descending, the later-inserted first among equal scores); N = 1 is the single best
 int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores,

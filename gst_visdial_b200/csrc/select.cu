@@ -416,13 +416,14 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
 }
 
 // ------------------------------------------------------------------------------------------------------------
-// prefix != null: int64 [B, P] decoder prefix shared by the K beams of an image; the first step's input is its last token
-__global__ void beam_init_kernel(BeamBuffers bb, int B, int K, int T, int start_token, const int64_t* __restrict__ prefix, int P) {
+// prefix != null: int64 [B, P] decoder prefix shared by the K beams of an image; the first step's input is its last token.
+// gs = beams per group: the first beam of every group starts at 0, the others at -1e9 (gs = K: one group)
+__global__ void beam_init_kernel(BeamBuffers bb, int B, int K, int gs, int T, int start_token, const int64_t* __restrict__ prefix, int P) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0) *bb.d_step = 0;
   if (i < B) { bb.done[i] = 0; bb.hyp_count[i] = 0; bb.hyp_worst[i] = 1e9; }
   if (i < B * K) {
-    bb.beam_scores[i] = (i % K == 0) ? 0.f : -1e9f;
+    bb.beam_scores[i] = ((i % K) % gs == 0) ? 0.f : -1e9f;
     bb.cur_tokens[i] = prefix ? (int32_t)prefix[(int64_t)(i / K) * P + P - 1] : start_token;
     bb.beam_idx[i] = i % K;
   }
@@ -460,13 +461,25 @@ __device__ void hyp_add(const BeamBuffers& bb, int b, int K, int T, const int32_
   }
 }
 
-// One warp per image.  The K x nsel per-row candidates are loaded in parallel, ranked in parallel by
-// (score desc, beam * V + token asc) - all pairs are distinct, so the rank is a permutation - and lane 0 then walks the
-// best 2K in order exactly like BeamSearchScorer.process; the token histories are gathered by all lanes.
+// One warp per image.  The K beams form G groups of gs = K / G consecutive beams (diverse beam search: HF 4.16.2
+// group_beam_search with HammingDiversityLogitsProcessor, contract in oracle/beam_groups.py; G = 1 is plain beam search, contract
+// in oracle/beam.py).  The groups run in order.  For group g the gs x nsel per-row candidates are loaded in parallel; a candidate
+// whose token c new beams of groups 0..g-1 took at this step gets the value fp32(fp32(fp32(x - logZ) - fp32(lambda c)) +
+// beam_score), recomputed from the logits and logZ of its row (-inf stays: banned tokens and fillers).  They are ranked in
+// parallel by (score desc, beam * V + token asc) - all pairs are distinct, so the rank is a permutation - and lane 0 walks the
+// best 2 gs exactly like BeamSearchScorer.process with group_size = gs, on the image's one hypothesis heap; `done` is tested before
+// and updated after every group.  The token histories are gathered by all lanes at the end.
+//
+// Why the per-row lists suffice (nsel >= K + gs; the engine keeps nsel = 2K): row_select ranks each row's candidates by the
+// UNPENALISED score.  The penalty only lowers a score and fp32(a + b) is monotone in a, so an element outside a row's list is
+// preceded, in the contract's order, by every unpenalised element of that list.  The earlier groups took at most K - gs distinct
+// tokens, so at least nsel - (K - gs) >= 2 gs listed elements of the row keep their value, and a group takes at most 2 gs
+// candidates from one row: the group's exact top 2 gs lies inside the lists.
 constexpr int kBeamWarps = 4;
 __global__ void __launch_bounds__(kBeamWarps * 32)
-beam_step_kernel(BeamBuffers bb, int B, int K, int T, int V, int nsel, const float* __restrict__ sel_val,
-                 const int32_t* __restrict__ sel_idx, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
+beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, const float* __restrict__ sel_val,
+                 const int32_t* __restrict__ sel_idx, const float* __restrict__ logits, int64_t ldl, const float* __restrict__ logz,
+                 float penalty, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
   __shared__ float s_val[kBeamWarps][128];
   __shared__ int s_flat[kBeamWarps][128];
   __shared__ int s_order[kBeamWarps][16];
@@ -481,14 +494,29 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int T, int V, int nsel, const flo
   const int cur_len = t + len0;                // HF input_ids.shape[-1]: decoder prefix (len0 tokens) + t generated
   const int32_t* src = bb.tokens + (int64_t)(t & 1) * B * K * T + (int64_t)b * K * T;
   int32_t* dst = bb.tokens + (int64_t)((t + 1) & 1) * B * K * T + (int64_t)b * K * T;
-  const int n = K * nsel;                      // <= 8 * 16 = 128
-  if (lane < 8) { nb_s[warp][lane] = 0.f; nb_tok[warp][lane] = 0; nb_par[warp][lane] = 0; }
-  const bool active = !bb.done[b];
-  if (active) {
+  const int gs = K / G;
+  const int n = gs * nsel;                     // candidates of one group, <= 8 * 16 = 128
+  // padded beams (image done): score 0, token PAD, parent = the first beam of their group
+  if (lane < 8) { nb_s[warp][lane] = 0.f; nb_tok[warp][lane] = 0; nb_par[warp][lane] = (lane / gs) * gs; }
+  __syncwarp();
+  bool done = bb.done[b];
+  for (int g = 0; g < G && !done; ++g) {
+    const int lo = g * gs;
+    const int64_t c0 = ((int64_t)b * K + lo) * nsel;
     for (int c = lane; c < n; c += 32) {
-      const int beam = c / nsel;
-      s_val[warp][c] = sel_val[(int64_t)b * n + c];
-      s_flat[warp][c] = beam * V + sel_idx[(int64_t)b * n + c];
+      const int beam = lo + c / nsel;
+      float v = sel_val[c0 + c];
+      const int w = sel_idx[c0 + c];
+      if (g > 0 && v > -INFINITY) {
+        int cnt = 0;
+        for (int j = 0; j < lo; ++j) cnt += nb_tok[warp][j] == w ? 1 : 0;
+        if (cnt > 0) {
+          const int64_t row = (int64_t)b * K + beam;
+          v = __fadd_rn(__fsub_rn(__fsub_rn(logits[row * ldl + w], logz[row]), __fmul_rn(penalty, (float)cnt)), bb.beam_scores[row]);
+        }
+      }
+      s_val[warp][c] = v;
+      s_flat[warp][c] = beam * V + w;
     }
     __syncwarp();
     for (int c = lane; c < n; c += 32) {
@@ -498,33 +526,34 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int T, int V, int nsel, const flo
         const float ov = s_val[warp][o]; const int of = s_flat[warp][o];
         rank += (ov > v || (ov == v && of < f)) ? 1 : 0;
       }
-      if (rank < 2 * K) s_order[warp][rank] = c;
+      if (rank < 2 * gs) s_order[warp][rank] = c;
     }
     __syncwarp();
+    int fin = 0;
     if (lane == 0) {
       int cnt = 0;
       const float best_sum = s_val[warp][s_order[warp][0]];
-      for (int rank = 0; rank < 2 * K; ++rank) {
+      for (int rank = 0; rank < 2 * gs; ++rank) {
         const int c = s_order[warp][rank];
         const float v = s_val[warp][c];
         const int f = s_flat[warp][c];
         const int bk = f / V, bt = f - bk * V;
         if (bt == eos) {
-          if (rank >= K) continue;
+          if (rank >= gs) continue;
           hyp_add(bb, b, K, T, src + (int64_t)bk * T, t, v, cur_len);
         } else {
-          nb_s[warp][cnt] = v; nb_tok[warp][cnt] = bt; nb_par[warp][cnt] = bk; ++cnt;
+          nb_s[warp][lo + cnt] = v; nb_tok[warp][lo + cnt] = bt; nb_par[warp][lo + cnt] = bk; ++cnt;
         }
-        if (cnt == K) break;
+        if (cnt == gs) break;
       }
       if (bb.hyp_count[b] >= K) {
         const double cur = (double)best_sum / (double)cur_len;
-        if (bb.hyp_worst[b] >= cur) bb.done[b] = 1;
+        if (bb.hyp_worst[b] >= cur) { bb.done[b] = 1; fin = 1; }
       }
     }
     __syncwarp();
+    done = __shfl_sync(0xffffffffu, fin, 0) != 0;
   }
-  __syncwarp();
   for (int i = lane; i < K * T; i += 32) {
     const int k = i / T, j = i - k * T;
     dst[i] = (j == t) ? nb_tok[warp][k] : src[nb_par[warp][k] * T + j];
@@ -968,16 +997,21 @@ int launch_row_select(int rows, int V, const float* logits, int64_t ldl, int mod
   return 1;
 }
 
-int launch_beam_init(const BeamBuffers& bb, int B, int K, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream) {
+int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream) {
+  if (G < 1 || K % G != 0) throw std::runtime_error("beam_init: the beam groups must divide the beams");
   const int n = B * K;
-  beam_init_kernel<<<(n + 255) / 256, 256, 0, stream>>>(bb, B, K, T, start_token, prefix, P);
+  beam_init_kernel<<<(n + 255) / 256, 256, 0, stream>>>(bb, B, K, K / G, T, start_token, prefix, P);
   return 1;
 }
-int launch_beam_step(const BeamBuffers& bb, int B, int K, int T, int V, int nsel, const float* sel_val,
-                     const int32_t* sel_idx, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
-                     cudaStream_t stream) {
+int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
+                     const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, int eos, int len0,
+                     int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores, cudaStream_t stream) {
   if (K > 8 || T > kHypMaxT) throw std::runtime_error("beam_step: K <= 8 and T <= 32");
-  launch_k(beam_step_kernel, dim3((B + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, B, K, T, V, nsel, sel_val, sel_idx, eos, len0, out_beam_idx, out_tokens, out_scores);
+  if (G < 1 || K % G != 0) throw std::runtime_error("beam_step: the beam groups must divide the beams");
+  if (G > 1 && (!logits || !logz || nsel < K + K / G))
+    throw std::runtime_error("beam_step: beam groups need the logits, logZ and nsel >= K + K / G per-row candidates");
+  launch_k(beam_step_kernel, dim3((B + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, B, K, G, T, V, nsel, sel_val, sel_idx,
+           logits, ldl, logz, penalty, eos, len0, out_beam_idx, out_tokens, out_scores);
   return 1;
 }
 int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores,

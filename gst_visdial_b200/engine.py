@@ -174,12 +174,14 @@ class Engine:
 
     def generate(self, B, num_beams=1, temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0,
                  max_new_tokens=None, hist_ids=None, hist_segments=None, want_scores=False, row_offset=0, prefix=None,
-                 num_return_sequences=1):
+                 num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0):
         """``row_offset``: global index of row 0; the sampler is keyed by (seed, row_offset + row, step), so an image draws the
         same tokens whichever batch or rank it lands in.  ``prefix``: int64 [B, P] decoder input to continue from (the reference's
         dec_input_ids; include/gstvd.h gstvd_generate_prefixed), None = one [CLS] per row; the result holds the new tokens only.
         ``num_return_sequences`` = N: [B*N, T] image-major - the N best beams, or N sampled candidates per image of which
-        candidate n draws like an N = 1 call with seed ``candidate_seed(seed, n)`` (include/gstvd.h gstvd_generate_candidates)."""
+        candidate n draws like an N = 1 call with seed ``candidate_seed(seed, n)`` (include/gstvd.h gstvd_generate_candidates).
+        ``num_beam_groups`` = G > 1 with ``diversity_penalty``: diverse beam search, the K beams in G groups of K / G with a Hamming
+        penalty between groups (include/gstvd.h gstvd_generate_groups, contract in oracle/beam_groups.py)."""
         gp = GstvdGenParams()
         gp.mode = GSTVD_SELECT_BEAM if num_beams > 1 else GSTVD_SELECT_SAMPLE
         gp.num_beams = int(num_beams)
@@ -194,16 +196,16 @@ class Engine:
         N = int(num_return_sequences)
         out = torch.empty(B * max(N, 1), gp.max_new_tokens, device=self.device, dtype=torch.int64)
         scores = torch.empty(B * max(N, 1), device=self.device, dtype=torch.float32) if want_scores else None
-        check(self.ctx, self.lib.gstvd_generate_candidates(self.ctx, B, ctypes.byref(gp), N, _ptr(pre), P, _ptr(hid), _ptr(hseg), Lh,
-                                                           _ptr(out), _ptr(scores), self._stream()))
+        check(self.ctx, self.lib.gstvd_generate_groups(self.ctx, B, ctypes.byref(gp), int(num_beam_groups), float(diversity_penalty), N,
+                                                       _ptr(pre), P, _ptr(hid), _ptr(hseg), Lh, _ptr(out), _ptr(scores), self._stream()))
         return (out, scores) if want_scores else out
 
     def round(self, input_ids, image_feat, image_loc, token_type_ids=None, attention_mask=None, image_mask=None, num_beams=1,
               temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0, max_new_tokens=None, want_scores=False, row_offset=0,
-              prefix=None, num_return_sequences=1):
+              prefix=None, num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0):
         """encode + prefill_cross + generate of one forward call as ONE graph replay (gstvd_round); the n-gram blocking history is
         ``input_ids`` / ``token_type_ids``.  Leaves the encoder / cross-K/V state resident like the three separate calls.
-        ``prefix`` / ``num_return_sequences``: as in ``generate``."""
+        ``prefix`` / ``num_return_sequences`` / ``num_beam_groups`` / ``diversity_penalty``: as in ``generate``."""
         ids = self._dev(input_ids, torch.int64)
         B, Lt = ids.shape
         feat = self._dev(image_feat, torch.float32)
@@ -223,8 +225,9 @@ class Engine:
         N = int(num_return_sequences)
         out = torch.empty(B * max(N, 1), gp.max_new_tokens, device=self.device, dtype=torch.int64)
         scores = torch.empty(B * max(N, 1), device=self.device, dtype=torch.float32) if want_scores else None
-        check(self.ctx, self.lib.gstvd_round_candidates(self.ctx, B, Lt, Lv, _ptr(ids), _ptr(seg), _ptr(att), _ptr(feat), _ptr(loc), _ptr(imask),
-                                                        ctypes.byref(gp), N, _ptr(pre), P, _ptr(out), _ptr(scores), self._stream()))
+        check(self.ctx, self.lib.gstvd_round_groups(self.ctx, B, Lt, Lv, _ptr(ids), _ptr(seg), _ptr(att), _ptr(feat), _ptr(loc), _ptr(imask),
+                                                    ctypes.byref(gp), int(num_beam_groups), float(diversity_penalty), N, _ptr(pre), P,
+                                                    _ptr(out), _ptr(scores), self._stream()))
         return (out, scores) if want_scores else out
 
     def score(self, dec_ids, dec_mask=None, labels=None, want_logits=False, want_loss=True, options_per_image=1):

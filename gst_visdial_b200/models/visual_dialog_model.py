@@ -52,6 +52,8 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
       num_beams=1        >1 switches the token selection to beam search (contract: oracle/beam.py)
       num_return_sequences=1  N sequences per image, image-major [B*N, 18]: the N best beams (oracle/beam_nbest.py), or N sampled
                          candidates, candidate n drawing like a single-sample call with seed candidate_seed(seed, n)
+      num_beam_groups=1, diversity_penalty=0.0   diverse beam search (HF names): the num_beams beams in num_beam_groups groups with a
+                         Hamming penalty between groups (contract: oracle/beam_groups.py); groups need num_beams > 1
       seed=None          sampling seed (a per-call counter when None)
       enc_valid_len=None   upper bound (python int) on the number of leading history positions that hold a token in ANY row.
                          The encoder, the cross-K/V prefill and the cross-attention then run on ceil32(bound) text positions
@@ -165,6 +167,12 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
         n_ret = int(decoding_kwargs.get("num_return_sequences", 1))
         if n_ret != 1:
             gen_kw["num_return_sequences"] = n_ret
+        groups = int(decoding_kwargs.get("num_beam_groups", 1))
+        penalty = float(decoding_kwargs.get("diversity_penalty", 0.0))
+        if groups != 1 or penalty != 0.0:
+            if groups > 1 and gen_kw["num_beams"] <= 1:
+                raise ValueError(f"num_beam_groups = {groups} needs beam search (num_beams > 1)")
+            gen_kw.update(num_beam_groups=groups, diversity_penalty=penalty)
         gen_kw["prefix"] = self._decoder_prefix(dec_input_ids, B, gen_kw["num_beams"], gen_kw["ngram_blocking_size"])
         if whole_round:
             # the n-gram blocking history is the (trimmed) encoder input itself: positions past the bound hold no token

@@ -36,6 +36,14 @@ def read_command_line(argv=None):
     p.add_argument('-num_beams', default=1, type=int, help='>1: beam search for the answers instead of top-k sampling')
     p.add_argument('-q_num_beams', default=1, type=int,
                    help='>1: beam search for the questions instead of top-k sampling (keeps the 4-gram blocking against the question history)')
+    p.add_argument('-num_beam_groups', default=1, type=int,
+                   help='>1: diverse beam search for the answers: the -num_beams beams in this many groups (must divide -num_beams)')
+    p.add_argument('-diversity_penalty', default=0.0, type=float,
+                   help='Hamming diversity penalty between the answer beam groups (with -num_beam_groups > 1)')
+    p.add_argument('-q_num_beam_groups', default=1, type=int,
+                   help='>1: diverse beam search for the questions: the -q_num_beams beams in this many groups (must divide -q_num_beams)')
+    p.add_argument('-q_diversity_penalty', default=0.0, type=float,
+                   help='Hamming diversity penalty between the question beam groups (with -q_num_beam_groups > 1)')
     p.add_argument('-answer_candidates', default=1, type=int,
                    help='>1: the teacher draws this many answers per round (samples, or the best of its -num_beams beams) and the one with '
                         'the lowest perplexity goes into the dialog')
@@ -48,6 +56,12 @@ def read_command_line(argv=None):
     p.add_argument('-seed', default=0, type=int)
     args = p.parse_args(argv)
     params = vars(args)
+    for who, beams, groups, penalty in (('', 'num_beams', 'num_beam_groups', 'diversity_penalty'),
+                                        ('q_', 'q_num_beams', 'q_num_beam_groups', 'q_diversity_penalty')):
+        if params[groups] < 1 or params[groups] > 1 and (params[beams] <= 1 or params[beams] % params[groups] != 0):
+            p.error(f"-{groups} {params[groups]} must be 1 or divide -{beams} {params[beams]} > 1")
+        if not (0.0 <= params[penalty] < float('inf')):
+            p.error(f"-{penalty} must be finite and >= 0")
     params['device'] = f"cuda:{params['gpu_ids'][0]}"
     params['engine_max_batch'] = params['batch_size']
     params['engine_max_beams'] = max(1, params['num_beams'], params['q_num_beams'], params['answer_candidates'])

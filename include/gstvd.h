@@ -176,6 +176,25 @@ int gstvd_generate_candidates(gstvd_ctx* ctx, int B, const gstvd_gen_params* par
                               const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
                               int64_t* out_ids, float* out_scores, void* stream);
 
+/* gstvd_generate_candidates with diverse beam search (HF num_beam_groups / diversity_penalty; transformers 4.16.2 group_beam_search with
+ * HammingDiversityLogitsProcessor; Vijayakumar et al., "Diverse Beam Search").  gstvd_generate_candidates is this call with
+ * num_beam_groups = 1, diversity_penalty = 0.  Contract (CPU oracle: oracle/beam_groups.py):
+ *   The K beams form G = num_beam_groups groups of gs = K / G consecutive beams; beam k of an image starts with score 0 if
+ *   k % gs == 0, else -1e9.  Every step runs one decoder pass over all K rows; logZ is per row.  Within a step the groups run in order:
+ *   the candidate (beam k of group g, token w) scores fp32(fp32(fp32(x - logZ) - fp32(diversity_penalty * c_w)) + beam_score_k), with
+ *   c_w = the number of new beams of groups 0..g-1 of the same image that took w at this step (an [SEP] that closed a hypothesis does
+ *   not count).  n-gram-banned tokens are -inf and stay -inf.  Each group takes the top 2*gs of its gs*V candidates by (score desc,
+ *   (k - g*gs)*V + w asc) and runs BeamSearchScorer.process with group_size = gs: [SEP] is added to the hypotheses only at rank < gs,
+ *   the group gets gs new beams whose parents stay inside the group.  All groups share the image's hypothesis heap of capacity K; its
+ *   done flag is tested before every group (a group of a done image is padded) and updated after every group with
+ *   is_done(best of the group's 2*gs candidates, P + t).  Finalisation and the N-best order are those of gstvd_generate_candidates.
+ *   With G = 1 the call is gstvd_generate_candidates, launch for launch.
+ *   Rejected with GSTVD_ERR_INVALID: num_beam_groups < 1, num_beams % num_beam_groups != 0, num_beam_groups > 1 in sample mode,
+ *   diversity_penalty negative or not finite. */
+int gstvd_generate_groups(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, int num_beam_groups, float diversity_penalty, int N,
+                          const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
+                          int64_t* out_ids, float* out_scores, void* stream);
+
 /* One whole forward call of the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:24-120): the same work and
  * results as gstvd_encode (no exported outputs) + gstvd_prefill_cross(resident states) + gstvd_generate, replayed from ONE CUDA graph
  * per shape - the host enqueues a few device-to-device copies of the inputs and one graph launch.  The n-gram blocking history is the
@@ -200,6 +219,14 @@ int gstvd_round_candidates(gstvd_ctx* ctx, int B, int Lt, int Lv,
                            const float* image_feat, const float* image_loc, const float* image_mask,
                            const gstvd_gen_params* params, int N, const int64_t* prefix, int P,
                            int64_t* out_ids, float* out_scores, void* stream);
+
+/* gstvd_round_candidates with beam groups and a diversity penalty: the contract of gstvd_generate_groups; gstvd_round_candidates is this
+ * call with num_beam_groups = 1, diversity_penalty = 0. */
+int gstvd_round_groups(gstvd_ctx* ctx, int B, int Lt, int Lv,
+                       const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
+                       const float* image_feat, const float* image_loc, const float* image_mask,
+                       const gstvd_gen_params* params, int num_beam_groups, float diversity_penalty, int N,
+                       const int64_t* prefix, int P, int64_t* out_ids, float* out_scores, void* stream);
 
 /* Replaces VisualDialogDecoder.forward in loss mode (models/visual_dialog_decoder.py:33-86) as driven by
  * generate.py:183-209 and evaluate_gen.py:94-106: teacher-forced pass over dec_ids [B, L].
