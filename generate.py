@@ -82,10 +82,14 @@ def main(argv=None):
     a_kwargs = dict(temperature=0.7, top_k=7, top_p=0.0, ngram_blocking_size=0)
     if params['num_beams'] > 1:
         a_kwargs.update(num_beams=params['num_beams'], num_beam_groups=params['num_beam_groups'], diversity_penalty=params['diversity_penalty'])
+        if params['beam_sample']:
+            a_kwargs.update(do_sample=True)
     q_kwargs = dict(temperature=0.7, top_k=7, top_p=0.0, ngram_blocking_size=4)
     if params['q_num_beams'] > 1:
         q_kwargs.update(num_beams=params['q_num_beams'], num_beam_groups=params['q_num_beam_groups'],
                         diversity_penalty=params['q_diversity_penalty'])
+        if params['q_beam_sample']:
+            q_kwargs.update(do_sample=True)
     decode = None
     if params['vocab_file']:
         from transformers import BertTokenizer

@@ -15,7 +15,7 @@ LIB_PATH = os.path.join(HERE, "lib", "libgstvd.so")
 GSTVD_ABI_VERSION = 2
 GSTVD_MAX_CONNECTIONS = 16
 GSTVD_F32, GSTVD_BF16 = 0, 1
-GSTVD_SELECT_SAMPLE, GSTVD_SELECT_BEAM = 0, 1
+GSTVD_SELECT_SAMPLE, GSTVD_SELECT_BEAM, GSTVD_SELECT_BEAM_SAMPLE = 0, 1, 2
 GSTVD_FLAG_NO_CUDA_GRAPH = 1
 GSTVD_FLAG_DEBUG_SIMT_GEMM = 2
 GSTVD_FLAG_GENERIC_ATTENTION = 4

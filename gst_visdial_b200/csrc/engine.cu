@@ -346,9 +346,12 @@ void alloc_workspace(gstvd_ctx* c) {
     c->prefix.alloc(B * K * (T + c->Ldec_max) * 4); c->seq.alloc(B * K * T * 4);
     c->dec_prefix_own.alloc(B * c->Ldec_max * 8); c->dec_prefix_head.alloc(B * c->Ldec_max * 8);
     c->beam_scores.alloc(B * K * 4); c->beam_tokens.alloc(2 * B * K * T * 4); c->cur_tokens.alloc(R * 4);
-    c->beam_idx.alloc(B * K * 4); c->beam_done.alloc(B); c->hyp_score.alloc(B * (K + 1) * 8);
-    c->hyp_len.alloc(B * (K + 1) * 4); c->hyp_tokens.alloc(B * (K + 1) * T * 4); c->hyp_count.alloc(B * 4);
-    c->hyp_worst.alloc(B * 8);
+    // hypothesis heaps: one per search of K beams with K + 1 slots.  Beam search: B searches of K <= K_max beams; beam sampling: B * N
+    // searches of K >= 2 beams with N * K <= K_max, i.e. at most B * K_max / 2 searches and B * (K_max + K_max / 2) slots.
+    const size_t S = B * std::max<size_t>(1, K / 2), HS = B * (K + std::max<size_t>(1, K / 2));
+    c->beam_idx.alloc(B * K * 4); c->beam_done.alloc(S); c->hyp_score.alloc(HS * 8);
+    c->hyp_len.alloc(HS * 4); c->hyp_tokens.alloc(HS * T * 4); c->hyp_count.alloc(S * 4);
+    c->hyp_worst.alloc(S * 8);
     c->anc.alloc(B * K * 64);
     CUDA_CHECK(cudaMemset(c->anc.p, 0, B * K * 64));
     c->stats_ld = (int64_t)((R + 15) & ~size_t(15));
@@ -672,8 +675,11 @@ const int64_t* stage_prefix(gstvd_ctx* c, int B, const int64_t* prefix, int P, c
 // Selection state of a decode call: beams / sample rows start from the last token of the prefix (the [CLS] when it is null).
 void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, int G, const int64_t* prefix, cudaStream_t s) {
   const int P = g.P0 + 1, T = gp.max_new_tokens;
-  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, G, T, 101, prefix, P, s);
-  else c->launches += launch_sample_init(g.B * g.K, g.K, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, P + T, (int*)c->d_step.p,
+  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, G, 1, T, 101, prefix, P, s);
+  else if (gp.mode == GSTVD_SELECT_BEAM_SAMPLE) {
+    const int K = gp.num_beams, N = g.K / K;      // N searches of K beams per image, all beams at score 0
+    c->launches += launch_beam_init(beam_buffers(c), g.B * N, K, K, N, T, 101, prefix, P, s);
+  } else c->launches += launch_sample_init(g.B * g.K, g.K, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, P + T, (int*)c->d_step.p,
                                          prefix, P, s);
 }
 
@@ -691,7 +697,8 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   // Beam mode with the lean self-attention kernel: the cache is never gathered, the kernel reads each history position from the
   // slot recorded in the ancestry table (token ids identical to the gather, +3 % dialogs/s; env GSTVD_SELF_ANC=0 restores the gather)
   const char* anc_env = getenv("GSTVD_SELF_ANC");
-  const bool use_anc = gp.mode == GSTVD_SELECT_BEAM && (anc_env == nullptr || atoi(anc_env) != 0) &&
+  const bool beams = gp.mode == GSTVD_SELECT_BEAM || gp.mode == GSTVD_SELECT_BEAM_SAMPLE;
+  const bool use_anc = beams && (anc_env == nullptr || atoi(anc_env) != 0) &&
                        dec_self_attn_v2_active(c->dtype, g, c->dqkv.p, c->self_cache.p, c->dctx.p);
   const uint8_t* anc = use_anc ? (const uint8_t*)c->anc.p : nullptr;
   c->launches += launch_embed_step(c->dtype, M, H, (const int32_t*)c->cur_tokens.p, g.P0, d_step, c->word, c->pos, c->type,
@@ -744,8 +751,10 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   }
   X.gemm(c->dh.p, H, c->lm_head, c->logits.p, c->Vpad, M, 0, true);
   float* sv = (float*)c->sel_val.p; int32_t* si = (int32_t*)c->sel_idx.p;
-  if (gp.mode == GSTVD_SELECT_BEAM) {
-    const int nsel = 2 * g.K;
+  if (beams) {
+    // beam sampling: g.K = N * K rows per image (N searches of K beams), each row's 16 best for the warpers and the draw
+    const bool sampled = gp.mode == GSTVD_SELECT_BEAM_SAMPLE;
+    const int nsel = sampled ? kSelMax : 2 * g.K;
     // bf16: log-sum-exp terms in fp32 (mode 2); the fp32 parity path keeps the fp64 terms of the bit-exact contract (mode 0)
     static const bool exact_lse = getenv("GSTVD_EXACT_LSE") != nullptr;
     BeamBuffers bb = beam_buffers(c);
@@ -763,8 +772,14 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     float* lz = G > 1 ? (float*)c->logz.p : nullptr;
     c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, (c->dtype == kBF16 && !exact_lse) ? 2 : 0,
                                      (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, lz, s);
-    c->launches += launch_beam_step(bb, g.B, g.K, G, Tn, c->V, nsel, sv, si, G > 1 ? (const float*)c->logits.p : nullptr, c->Vpad, lz,
-                                    penalty, 102, P, nullptr, nullptr, nullptr, s);
+    if (sampled) {
+      const int K = gp.num_beams;
+      c->launches += launch_beam_sample_step(bb, M / K, g.K / K, K, Tn, c->V, sv, si, gp.top_k, gp.temperature, gp.top_p,
+                                             (const uint64_t*)c->d_seed.p, 102, P, s);
+    } else {
+      c->launches += launch_beam_step(bb, g.B, g.K, G, Tn, c->V, nsel, sv, si, G > 1 ? (const float*)c->logits.p : nullptr, c->Vpad, lz,
+                                      penalty, 102, P, nullptr, nullptr, nullptr, s);
+    }
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
   } else {
@@ -795,7 +810,7 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
 }
 
 // Argument checks of a generate call returning N sequences per image; returns the decode rows per image (beam mode: the beams;
-// sample mode: the N candidates).
+// sample mode: the N candidates; beam sampling: N searches of num_beams beams).
 int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, int N, int G, float penalty, const int64_t* prefix, int P, const int64_t* hist_ids,
                    const int64_t* hist_seg, int Lh, const int64_t* out_ids) {
   check_ready(c);
@@ -818,6 +833,15 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, int N, int G, float
     if (K < 1 || K > c->K_max || 2 * K > kSelMax) throw InvalidArg("generate: num_beams out of range");
     if (N < 1 || N > K) throw InvalidArg(fmt("generate: %d return sequences outside 1..num_beams (%d)", N, K));
     if (K % G != 0) throw InvalidArg(fmt("generate: %d beam groups do not divide %d beams", G, K));
+  } else if (gp.mode == GSTVD_SELECT_BEAM_SAMPLE) {
+    K = gp.num_beams;
+    if (K < 2 || 2 * K > kSelMax) throw InvalidArg(fmt("generate: beam sampling needs 2 <= num_beams <= %d, got %d", kSelMax / 2, K));
+    if (N < 1 || N * K > c->K_max)
+      throw InvalidArg(fmt("generate: %d beam-sampled searches of %d beams exceed max_beams (%d) rows per image", N, K, c->K_max));
+    if (!(gp.temperature > 0.f) || !std::isfinite(gp.temperature)) throw InvalidArg("generate: temperature must be finite and > 0");
+    if (!(gp.top_p >= 0.f && gp.top_p <= 1.f)) throw InvalidArg("generate: top_p must be in [0, 1]");
+    if (gp.top_k < 1 || gp.top_k > GSTVD_MAX_TOP_K) throw Unsupported("generate: beam sampling needs top_k in 1..16");
+    K *= N;
   } else if (gp.mode == GSTVD_SELECT_SAMPLE) {
     if (N < 1 || N > c->K_max || N > 8) throw InvalidArg(fmt("generate: %d sampled candidates outside 1..min(8, max_beams = %d)", N, c->K_max));
     K = N;
@@ -835,6 +859,8 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, int N, int G, float
 void generate_finalize(gstvd_ctx* c, int B, int K, int P, int N, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
   const int T = gp.max_new_tokens;
   if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, P, N, out_ids, out_scores, s);
+  else if (gp.mode == GSTVD_SELECT_BEAM_SAMPLE)   // search n of image b is search b * N + n: its best hypothesis is output row b * N + n
+    c->launches += launch_beam_finalize(beam_buffers(c), B * N, gp.num_beams, T, 102, P, 1, out_ids, out_scores, s);
   else c->launches += launch_sample_finalize(B * K, T, 102, (const int32_t*)c->seq.p, out_ids, s);
 }
 
@@ -1491,7 +1517,7 @@ int gstvd_op_beam_begin(gstvd_ctx* c, int B, int K, int max_new, void* stream) {
     if (c->dec_layers == 0) throw StateError("beam ops need a decoder context");
     if (B < 1 || B > c->B_max || K < 1 || K > c->K_max || max_new < 1 || max_new > c->T_max) throw InvalidArg("beam_begin: shape out of range");
     c->op_B = B; c->op_K = K; c->op_T = max_new;
-    c->launches += launch_beam_init(beam_buffers(c), B, K, 1, max_new, 101, nullptr, 1, (cudaStream_t)stream);
+    c->launches += launch_beam_init(beam_buffers(c), B, K, 1, 1, max_new, 101, nullptr, 1, (cudaStream_t)stream);
   });
 }
 

@@ -184,8 +184,14 @@ struct BeamBuffers {
   int* d_step;             // device step counter
 };
 // prefix: int64 [B, P] decoder prefix (null: start_token, P = 1); len0 = P, the prefix length counted in every hypothesis length.
-// G beam groups of K / G beams (G | K; G = 1: plain beam search): the first beam of every group starts with score 0.
-int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream);
+// G beam groups of K / G beams (G | K; G = 1: plain beam search): the first beam of every group starts with score 0 (G = K: all beams).
+// B = searches of K beams, N consecutive searches per image (beam sampling; 1 otherwise): search s reads prefix row s / N.
+int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int N, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream);
+// Beam sampling (oracle/beam_sample.py): S = B * N searches of K beams, rows search-major; sel_val / sel_idx = row_select mode 0 / 2
+// output with nsel = kSelMax and the beam scores as row bias.  d_seed = {seed, row_offset} (device).  Parents are written image-local
+// (n * K + parent, n = s % N), so the cache reorder runs with N * K rows per image.
+int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, int V, const float* sel_val, const int32_t* sel_idx, int top_k,
+                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, cudaStream_t stream);
 // G > 1: diverse beam search with the Hamming penalty `penalty` (oracle/beam_groups.py).  A candidate whose token earlier groups took
 // at this step is re-scored from logits [B*K, ldl] fp32 and logz [B*K] (row_select's outputs for this step); needs nsel >= K + K / G.
 // G = 1 reads neither.

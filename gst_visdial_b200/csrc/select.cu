@@ -417,14 +417,15 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
 
 // ------------------------------------------------------------------------------------------------------------
 // prefix != null: int64 [B, P] decoder prefix shared by the K beams of an image; the first step's input is its last token.
-// gs = beams per group: the first beam of every group starts at 0, the others at -1e9 (gs = K: one group)
-__global__ void beam_init_kernel(BeamBuffers bb, int B, int K, int gs, int T, int start_token, const int64_t* __restrict__ prefix, int P) {
+// gs = beams per group: the first beam of every group starts at 0, the others at -1e9 (gs = K: one group; gs = 1: all at 0, beam
+// sampling).  B = searches of K beams; N searches per image (beam sampling) share the image's prefix row b / N.
+__global__ void beam_init_kernel(BeamBuffers bb, int B, int K, int gs, int N, int T, int start_token, const int64_t* __restrict__ prefix, int P) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0) *bb.d_step = 0;
   if (i < B) { bb.done[i] = 0; bb.hyp_count[i] = 0; bb.hyp_worst[i] = 1e9; }
   if (i < B * K) {
     bb.beam_scores[i] = ((i % K) % gs == 0) ? 0.f : -1e9f;
-    bb.cur_tokens[i] = prefix ? (int32_t)prefix[(int64_t)(i / K) * P + P - 1] : start_token;
+    bb.cur_tokens[i] = prefix ? (int32_t)prefix[(int64_t)(i / K / N) * P + P - 1] : start_token;
     bb.beam_idx[i] = i % K;
   }
   for (int j = i; j < 2 * B * K * T; j += gridDim.x * blockDim.x) bb.tokens[j] = 0;
@@ -461,6 +462,35 @@ __device__ void hyp_add(const BeamBuffers& bb, int b, int K, int T, const int32_
   }
 }
 
+// BeamSearchScorer.process of one group of gs beams (lane 0): walks the group's 2 gs candidates in rank order (order[rank] = index into
+// val / flat, flat = beam * V + token with the beam counted from the image's / search's first beam): [SEP] at rank < gs closes a
+// hypothesis of beam flat / V (history src + beam * T, t tokens), any other token becomes new beam lo + cnt, until gs beams are filled.
+// Then is_done(val[order[0]], cur_len) on the heap b of capacity K; returns whether it set done[b].
+__device__ __forceinline__ bool beam_process(const BeamBuffers& bb, int b, int K, int T, int V, int eos, const int32_t* src, int t,
+                                             int cur_len, int lo, int gs, const float* val, const int* flat, const int* order,
+                                             float* nb_s, int* nb_tok, int* nb_par) {
+  int cnt = 0;
+  const float best_sum = val[order[0]];
+  for (int rank = 0; rank < 2 * gs; ++rank) {
+    const int c = order[rank];
+    const float v = val[c];
+    const int f = flat[c];
+    const int bk = f / V, bt = f - bk * V;
+    if (bt == eos) {
+      if (rank >= gs) continue;
+      hyp_add(bb, b, K, T, src + (int64_t)bk * T, t, v, cur_len);
+    } else {
+      nb_s[lo + cnt] = v; nb_tok[lo + cnt] = bt; nb_par[lo + cnt] = bk; ++cnt;
+    }
+    if (cnt == gs) break;
+  }
+  if (bb.hyp_count[b] >= K) {
+    const double cur = (double)best_sum / (double)cur_len;
+    if (bb.hyp_worst[b] >= cur) { bb.done[b] = 1; return true; }
+  }
+  return false;
+}
+
 // One warp per image.  The K beams form G groups of gs = K / G consecutive beams (diverse beam search: HF 4.16.2
 // group_beam_search with HammingDiversityLogitsProcessor, contract in oracle/beam_groups.py; G = 1 is plain beam search, contract
 // in oracle/beam.py).  The groups run in order.  For group g the gs x nsel per-row candidates are loaded in parallel; a candidate
@@ -476,7 +506,12 @@ __device__ void hyp_add(const BeamBuffers& bb, int b, int K, int T, const int32_
 // tokens, so at least nsel - (K - gs) >= 2 gs listed elements of the row keep their value, and a group takes at most 2 gs
 // candidates from one row: the group's exact top 2 gs lies inside the lists.
 constexpr int kBeamWarps = 4;
-__global__ void __launch_bounds__(kBeamWarps * 32)
+// Register budget of the two beam-step kernels: 65536 / (7 * 128 threads) = 72 registers per thread.  Left to its default, ptxas
+// keeps them near 48 - 64 registers and spills the values that stay live across the calls into the fp64 / fp32 division subroutines
+// of the hypothesis walk (20 bytes in each kernel); with this budget neither spills (-Xptxas -v: beam_step_kernel 64 registers,
+// beam_sample_step_kernel 70).  The budget still lets 7 blocks share an SM; the grids have B / 4 and B * N / 4 blocks.
+constexpr int kBeamMinBlocks = 7;
+__global__ void __launch_bounds__(kBeamWarps * 32, kBeamMinBlocks)
 beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, const float* __restrict__ sel_val,
                  const int32_t* __restrict__ sel_idx, const float* __restrict__ logits, int64_t ldl, const float* __restrict__ logz,
                  float penalty, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
@@ -530,27 +565,9 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, co
     }
     __syncwarp();
     int fin = 0;
-    if (lane == 0) {
-      int cnt = 0;
-      const float best_sum = s_val[warp][s_order[warp][0]];
-      for (int rank = 0; rank < 2 * gs; ++rank) {
-        const int c = s_order[warp][rank];
-        const float v = s_val[warp][c];
-        const int f = s_flat[warp][c];
-        const int bk = f / V, bt = f - bk * V;
-        if (bt == eos) {
-          if (rank >= gs) continue;
-          hyp_add(bb, b, K, T, src + (int64_t)bk * T, t, v, cur_len);
-        } else {
-          nb_s[warp][lo + cnt] = v; nb_tok[warp][lo + cnt] = bt; nb_par[warp][lo + cnt] = bk; ++cnt;
-        }
-        if (cnt == gs) break;
-      }
-      if (bb.hyp_count[b] >= K) {
-        const double cur = (double)best_sum / (double)cur_len;
-        if (bb.hyp_worst[b] >= cur) { bb.done[b] = 1; fin = 1; }
-      }
-    }
+    if (lane == 0)
+      fin = beam_process(bb, b, K, T, V, eos, src, t, cur_len, lo, gs, s_val[warp], s_flat[warp], s_order[warp], nb_s[warp], nb_tok[warp],
+                         nb_par[warp]) ? 1 : 0;
     __syncwarp();
     done = __shfl_sync(0xffffffffu, fin, 0) != 0;
   }
@@ -687,6 +704,113 @@ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
 // candidate_seed(seed, n) draws, and candidate 0 is that call itself.  Mirrored by models/visual_dialog_model.candidate_seed.
 __device__ __forceinline__ uint64_t candidate_seed(uint64_t seed, int n) {
   return n == 0 ? seed : splitmix64(seed ^ splitmix64((uint64_t)n * 0xD1B54A32D192ED03ull));
+}
+
+// Beam sampling (HF 4.16.2 beam_sample + BeamSearchScorer; contract in oracle/beam_sample.py).  One warp per search s of K beams; N
+// searches per image (search n of image b is s = b N + n, its beams are decode rows s K + k).  Each row's list (row_select mode 0 / 2
+// with the beam scores as row bias, nsel = 16, bans applied) holds s = fp32(fp32(x - logZ) + beam_score) by (s desc, token asc).  Per row:
+//   w = fp32(s / temperature); top-k keeps w >= the k'-th listed w, k' = max(top_k, 2) (a prefix of the list: w is monotone in s);
+//   top-p (> 0) inside it drops rank r >= 2 when the probability mass before r exceeds top_p (sample_step_kernel's rule).
+// The survivors of the K rows (<= 128) get the Gumbel key fp64(w) - log(-log u), u from the counter-based RNG keyed by
+// (candidate_seed(seed, n), row_offset + b, t, k * V + token); the 2K largest keys are a draw of 2K entries without replacement from
+// softmax(w) over the search's K V warped scores (Gumbel-top-k).  The drawn entries are ordered by (w desc, k V + token asc) and
+// walked by beam_process, exactly as in beam_step_kernel.  Parents are written image-local (n K + parent) for the cache reorder.
+__device__ __forceinline__ double gumbel_u(uint64_t sd, uint64_t grow, int t, int flat) {
+  const uint64_t h = splitmix64(splitmix64(sd ^ splitmix64((grow << 20) ^ (uint64_t)t)) ^ (uint64_t)flat);
+  return ((double)(h >> 11) + 0.5) * 0x1p-53;
+}
+
+__global__ void __launch_bounds__(kBeamWarps * 32, kBeamMinBlocks)
+beam_sample_step_kernel(BeamBuffers bb, int S, int N, int K, int T, int V, const float* __restrict__ sel_val, const int32_t* __restrict__ sel_idx,
+                        int top_k, float temperature, float top_p, const uint64_t* __restrict__ d_seed, int eos, int len0) {
+  constexpr int nsel = kSelMax;
+  __shared__ double s_key[kBeamWarps][8 * nsel];
+  __shared__ float s_val[kBeamWarps][8 * nsel];
+  __shared__ int s_flat[kBeamWarps][8 * nsel];
+  __shared__ int s_kept[kBeamWarps][8];
+  __shared__ int s_draw[kBeamWarps][2 * 8], s_order[kBeamWarps][2 * 8];
+  __shared__ float nb_s[kBeamWarps][8];
+  __shared__ int nb_tok[kBeamWarps][8], nb_par[kBeamWarps][8];
+  pdl_wait();
+  pdl_launch_dependents();
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int s = blockIdx.x * kBeamWarps + warp;
+  if (s >= S) return;
+  const int t = *bb.d_step;
+  const int cur_len = t + len0;
+  const int32_t* src = bb.tokens + (int64_t)(t & 1) * S * K * T + (int64_t)s * K * T;
+  int32_t* dst = bb.tokens + (int64_t)((t + 1) & 1) * S * K * T + (int64_t)s * K * T;
+  const int n = K * nsel;
+  if (lane < 8) { nb_s[warp][lane] = 0.f; nb_tok[warp][lane] = 0; nb_par[warp][lane] = 0; }
+  if (!bb.done[s]) {
+    const int64_t c0 = (int64_t)s * K * nsel;
+    for (int c = lane; c < n; c += 32) {
+      s_val[warp][c] = __fdiv_rn(sel_val[c0 + c], temperature);
+      s_flat[warp][c] = (c / nsel) * V + sel_idx[c0 + c];
+    }
+    __syncwarp();
+    if (lane < K) {
+      const float* w = s_val[warp] + lane * nsel;
+      const float thr = w[(top_k > 2 ? top_k : 2) - 1];
+      int kept = 0;
+      while (kept < nsel && w[kept] >= thr && w[kept] > -INFINITY) ++kept;
+      if (top_p > 0.f && kept > 2) {
+        float sum = 0.f;
+        for (int r = 0; r < kept; ++r) sum += expf(w[r] - w[0]);
+        float cum = 0.f;
+        for (int r = 0; r < kept; ++r) {
+          if (r >= 2 && cum > top_p) { kept = r; break; }
+          cum += expf(w[r] - w[0]) / sum;
+        }
+      }
+      s_kept[warp][lane] = kept;
+    }
+    __syncwarp();
+    const uint64_t sd = candidate_seed(d_seed[0], s % N);
+    const uint64_t grow = (uint64_t)(s / N) + d_seed[1];
+    for (int c = lane; c < n; c += 32) {
+      double key = -INFINITY;
+      if (c % nsel < s_kept[warp][c / nsel]) key = (double)s_val[warp][c] - log(-log(gumbel_u(sd, grow, t, s_flat[warp][c])));
+      s_key[warp][c] = key;
+    }
+    __syncwarp();
+    // the 2K largest keys (ties: list position asc), then those 2K by (w desc, flat asc, list position asc)
+    for (int c = lane; c < n; c += 32) {
+      const double kv = s_key[warp][c];
+      int rank = 0;
+      for (int o = 0; o < n; ++o) {
+        const double ok = s_key[warp][o];
+        rank += (ok > kv || (ok == kv && o < c)) ? 1 : 0;
+      }
+      if (rank < 2 * K) s_draw[warp][rank] = c;
+    }
+    __syncwarp();
+    if (lane < 2 * K) {
+      const int c = s_draw[warp][lane];
+      const float v = s_val[warp][c]; const int f = s_flat[warp][c];
+      int rank = 0;
+      for (int o = 0; o < 2 * K; ++o) {
+        const int oc = s_draw[warp][o];
+        const float ov = s_val[warp][oc]; const int of = s_flat[warp][oc];
+        rank += (ov > v || (ov == v && (of < f || (of == f && oc < c)))) ? 1 : 0;
+      }
+      s_order[warp][rank] = c;
+    }
+    __syncwarp();
+    if (lane == 0)
+      beam_process(bb, s, K, T, V, eos, src, t, cur_len, 0, K, s_val[warp], s_flat[warp], s_order[warp], nb_s[warp], nb_tok[warp], nb_par[warp]);
+  }
+  __syncwarp();
+  for (int i = lane; i < K * T; i += 32) {
+    const int k = i / T, j = i - k * T;
+    dst[i] = (j == t) ? nb_tok[warp][k] : src[nb_par[warp][k] * T + j];
+  }
+  if (lane < K) {
+    const int64_t r = (int64_t)s * K + lane;
+    bb.beam_scores[r] = nb_s[warp][lane];
+    bb.cur_tokens[r] = nb_tok[warp][lane];
+    bb.beam_idx[r] = (s % N) * K + nb_par[warp][lane];
+  }
 }
 
 // dec_prefix != null: int64 [rows / N, P] decoder prefix of the row's image; `prefix` (the n-gram key buffer) starts with it, [SEP]
@@ -997,10 +1121,20 @@ int launch_row_select(int rows, int V, const float* logits, int64_t ldl, int mod
   return 1;
 }
 
-int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream) {
+int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int N, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream) {
   if (G < 1 || K % G != 0) throw std::runtime_error("beam_init: the beam groups must divide the beams");
+  if (N < 1 || B % N != 0) throw std::runtime_error("beam_init: the searches must be a multiple of N >= 1");
   const int n = B * K;
-  beam_init_kernel<<<(n + 255) / 256, 256, 0, stream>>>(bb, B, K, K / G, T, start_token, prefix, P);
+  beam_init_kernel<<<(n + 255) / 256, 256, 0, stream>>>(bb, B, K, K / G, N, T, start_token, prefix, P);
+  return 1;
+}
+int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, int V, const float* sel_val, const int32_t* sel_idx, int top_k,
+                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, cudaStream_t stream) {
+  if (K < 2 || 2 * K > kSelMax || T > kHypMaxT) throw std::runtime_error("beam_sample_step: 2 <= K <= 8 and T <= 32");
+  if (N < 1 || S % N != 0) throw std::runtime_error("beam_sample_step: the searches must be a multiple of N >= 1");
+  if (top_k < 1 || top_k > kSelMax) throw std::runtime_error("beam_sample_step: top_k out of range");
+  launch_k(beam_sample_step_kernel, dim3((S + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, S, N, K, T, V, sel_val,
+           sel_idx, top_k, temperature, top_p, d_seed, eos, len0);
   return 1;
 }
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,

@@ -11,10 +11,18 @@ from typing import Mapping, Optional
 import torch
 
 from . import _lib
-from ._lib import (GSTVD_BF16, GSTVD_F32, GSTVD_SELECT_BEAM, GSTVD_SELECT_SAMPLE, GstvdConfig, GstvdError, GstvdGenParams, check)
+from ._lib import (GSTVD_BF16, GSTVD_F32, GSTVD_SELECT_BEAM, GSTVD_SELECT_BEAM_SAMPLE, GSTVD_SELECT_SAMPLE, GstvdConfig, GstvdError,
+                   GstvdGenParams, check)
 
 DTYPES = {"fp32": GSTVD_F32, "float32": GSTVD_F32, "f32": GSTVD_F32, torch.float32: GSTVD_F32,
           "bf16": GSTVD_BF16, "bfloat16": GSTVD_BF16, torch.bfloat16: GSTVD_BF16}
+
+
+def _select_mode(num_beams, do_sample):
+    """HF generate()'s choice: beams with do_sample = beam sampling, beams without = beam search, one beam = the sampler."""
+    if num_beams > 1:
+        return GSTVD_SELECT_BEAM_SAMPLE if do_sample else GSTVD_SELECT_BEAM
+    return GSTVD_SELECT_SAMPLE
 
 
 def _ptr(t: Optional[torch.Tensor]):
@@ -174,16 +182,20 @@ class Engine:
 
     def generate(self, B, num_beams=1, temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0,
                  max_new_tokens=None, hist_ids=None, hist_segments=None, want_scores=False, row_offset=0, prefix=None,
-                 num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0):
+                 num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0, do_sample=False):
         """``row_offset``: global index of row 0; the sampler is keyed by (seed, row_offset + row, step), so an image draws the
         same tokens whichever batch or rank it lands in.  ``prefix``: int64 [B, P] decoder input to continue from (the reference's
         dec_input_ids; include/gstvd.h gstvd_generate_prefixed), None = one [CLS] per row; the result holds the new tokens only.
         ``num_return_sequences`` = N: [B*N, T] image-major - the N best beams, or N sampled candidates per image of which
         candidate n draws like an N = 1 call with seed ``candidate_seed(seed, n)`` (include/gstvd.h gstvd_generate_candidates).
         ``num_beam_groups`` = G > 1 with ``diversity_penalty``: diverse beam search, the K beams in G groups of K / G with a Hamming
-        penalty between groups (include/gstvd.h gstvd_generate_groups, contract in oracle/beam_groups.py)."""
+        penalty between groups (include/gstvd.h gstvd_generate_groups, contract in oracle/beam_groups.py).
+        ``do_sample`` with ``num_beams`` > 1: beam sampling (HF beam_sample) with ``temperature`` / ``top_k`` / ``top_p`` / ``seed``;
+        ``num_return_sequences`` = N then runs N independent searches per image, search n seeded ``candidate_seed(seed, n)``, and
+        returns the best hypothesis of each (include/gstvd.h GSTVD_SELECT_BEAM_SAMPLE, contract in oracle/beam_sample.py).  With
+        ``num_beams`` = 1 the sampler runs whatever ``do_sample`` says."""
         gp = GstvdGenParams()
-        gp.mode = GSTVD_SELECT_BEAM if num_beams > 1 else GSTVD_SELECT_SAMPLE
+        gp.mode = _select_mode(num_beams, do_sample)
         gp.num_beams = int(num_beams)
         gp.max_new_tokens = int(max_new_tokens or self.max_new_tokens)
         gp.top_k, gp.temperature, gp.top_p = int(top_k), float(temperature), float(top_p)
@@ -202,10 +214,10 @@ class Engine:
 
     def round(self, input_ids, image_feat, image_loc, token_type_ids=None, attention_mask=None, image_mask=None, num_beams=1,
               temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0, max_new_tokens=None, want_scores=False, row_offset=0,
-              prefix=None, num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0):
+              prefix=None, num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0, do_sample=False):
         """encode + prefill_cross + generate of one forward call as ONE graph replay (gstvd_round); the n-gram blocking history is
         ``input_ids`` / ``token_type_ids``.  Leaves the encoder / cross-K/V state resident like the three separate calls.
-        ``prefix`` / ``num_return_sequences`` / ``num_beam_groups`` / ``diversity_penalty``: as in ``generate``."""
+        ``prefix`` / ``num_return_sequences`` / ``num_beam_groups`` / ``diversity_penalty`` / ``do_sample``: as in ``generate``."""
         ids = self._dev(input_ids, torch.int64)
         B, Lt = ids.shape
         feat = self._dev(image_feat, torch.float32)
@@ -215,7 +227,7 @@ class Engine:
         att = self._dev(attention_mask, torch.float32)
         imask = self._dev(image_mask, torch.float32)
         gp = GstvdGenParams()
-        gp.mode = GSTVD_SELECT_BEAM if num_beams > 1 else GSTVD_SELECT_SAMPLE
+        gp.mode = _select_mode(num_beams, do_sample)
         gp.num_beams = int(num_beams)
         gp.max_new_tokens = int(max_new_tokens or self.max_new_tokens)
         gp.top_k, gp.temperature, gp.top_p = int(top_k), float(temperature), float(top_p)

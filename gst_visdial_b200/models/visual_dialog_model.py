@@ -54,6 +54,9 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
                          candidates, candidate n drawing like a single-sample call with seed candidate_seed(seed, n)
       num_beam_groups=1, diversity_penalty=0.0   diverse beam search (HF names): the num_beams beams in num_beam_groups groups with a
                          Hamming penalty between groups (contract: oracle/beam_groups.py); groups need num_beams > 1
+      do_sample=False    with num_beams > 1: beam sampling (HF beam_sample; contract: oracle/beam_sample.py) with temperature / top_k /
+                         top_p; num_return_sequences = N runs N independent searches per image, search n seeded candidate_seed(seed, n).
+                         Beam groups cannot be combined with it (HF rejects that too).  With num_beams = 1 the sampler runs either way
       seed=None          sampling seed (a per-call counter when None)
       enc_valid_len=None   upper bound (python int) on the number of leading history positions that hold a token in ANY row.
                          The encoder, the cross-K/V prefill and the cross-attention then run on ceil32(bound) text positions
@@ -173,6 +176,10 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
             if groups > 1 and gen_kw["num_beams"] <= 1:
                 raise ValueError(f"num_beam_groups = {groups} needs beam search (num_beams > 1)")
             gen_kw.update(num_beam_groups=groups, diversity_penalty=penalty)
+        if decoding_kwargs.get("do_sample", False):
+            if groups > 1:
+                raise ValueError(f"num_beam_groups = {groups} cannot be combined with do_sample (beam sampling)")
+            gen_kw["do_sample"] = True
         gen_kw["prefix"] = self._decoder_prefix(dec_input_ids, B, gen_kw["num_beams"], gen_kw["ngram_blocking_size"])
         if whole_round:
             # the n-gram blocking history is the (trimmed) encoder input itself: positions past the bound hold no token

@@ -44,6 +44,11 @@ def read_command_line(argv=None):
                    help='>1: diverse beam search for the questions: the -q_num_beams beams in this many groups (must divide -q_num_beams)')
     p.add_argument('-q_diversity_penalty', default=0.0, type=float,
                    help='Hamming diversity penalty between the question beam groups (with -q_num_beam_groups > 1)')
+    p.add_argument('-beam_sample', action='store_true',
+                   help='beam sampling for the answers (HF do_sample with beams): -num_beams > 1 beams drawn with the answer sampler\'s '
+                        'temperature 0.7 and top-k 7; with -answer_candidates N, N independent searches per image')
+    p.add_argument('-q_beam_sample', action='store_true',
+                   help='beam sampling for the questions: -q_num_beams > 1 beams drawn with temperature 0.7 and top-k 7')
     p.add_argument('-answer_candidates', default=1, type=int,
                    help='>1: the teacher draws this many answers per round (samples, or the best of its -num_beams beams) and the one with '
                         'the lowest perplexity goes into the dialog')
@@ -62,9 +67,15 @@ def read_command_line(argv=None):
             p.error(f"-{groups} {params[groups]} must be 1 or divide -{beams} {params[beams]} > 1")
         if not (0.0 <= params[penalty] < float('inf')):
             p.error(f"-{penalty} must be finite and >= 0")
+    for flag, beams, groups in (('beam_sample', 'num_beams', 'num_beam_groups'), ('q_beam_sample', 'q_num_beams', 'q_num_beam_groups')):
+        if params[flag] and (params[beams] <= 1 or params[groups] > 1):
+            p.error(f"-{flag} needs -{beams} > 1 and no beam groups")
+    if params['beam_sample'] and params['num_beams'] * params['answer_candidates'] > 8:
+        p.error("-beam_sample runs -answer_candidates searches of -num_beams beams per image: their product must be at most 8")
     params['device'] = f"cuda:{params['gpu_ids'][0]}"
     params['engine_max_batch'] = params['batch_size']
-    params['engine_max_beams'] = max(1, params['num_beams'], params['q_num_beams'], params['answer_candidates'])
+    params['engine_max_beams'] = max(1, params['num_beams'], params['q_num_beams'], params['answer_candidates'],
+                                     params['num_beams'] * params['answer_candidates'] if params['beam_sample'] else 1)
     if params['save_name'] == '':
         params['save_name'] = 'generated_dialogs.json'
     os.makedirs(params['save_path'], exist_ok=True)

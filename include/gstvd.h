@@ -44,7 +44,9 @@ typedef enum { GSTVD_F32 = 0, GSTVD_BF16 = 1 } gstvd_dtype;
 typedef enum {
   GSTVD_SELECT_SAMPLE = 0, /* temperature / top-k / top-p filtering + multinomial; top_k == 1 is greedy
                               (models/visual_dialog_model.py:86-110, utils/decoding_utils.py:4-35) */
-  GSTVD_SELECT_BEAM = 1    /* beam search, contract in oracle/beam.py (new behaviour, north_star) */
+  GSTVD_SELECT_BEAM = 1,   /* beam search, contract in oracle/beam.py (new behaviour, north_star) */
+  GSTVD_SELECT_BEAM_SAMPLE = 2 /* beam sampling (HF num_beams > 1 with do_sample): num_beams, top_k, top_p, temperature and seed all
+                                  apply; contract at gstvd_generate_groups and in oracle/beam_sample.py */
 } gstvd_select_mode;
 
 /* Model geometry: the fields of config/bert_base_6layer_6conect_{enc,dec}.json that the path reads
@@ -190,7 +192,27 @@ int gstvd_generate_candidates(gstvd_ctx* ctx, int B, const gstvd_gen_params* par
  *   is_done(best of the group's 2*gs candidates, P + t).  Finalisation and the N-best order are those of gstvd_generate_candidates.
  *   With G = 1 the call is gstvd_generate_candidates, launch for launch.
  *   Rejected with GSTVD_ERR_INVALID: num_beam_groups < 1, num_beams % num_beam_groups != 0, num_beam_groups > 1 in sample mode,
- *   diversity_penalty negative or not finite. */
+ *   diversity_penalty negative or not finite.
+ *
+ * Beam sampling, mode GSTVD_SELECT_BEAM_SAMPLE (transformers 4.16.2 beam_sample + BeamSearchScorer, length_penalty 1, early_stopping
+ * off; CPU oracle: oracle/beam_sample.py).  Per image the call runs N independent stochastic beam searches of K = num_beams beams and
+ * returns the best hypothesis of search n as output row b*N + n (out_scores: its score).  Search n of image b is what an N = 1 call
+ * with seed candidate_seed(seed, n) runs for that image.  Decode rows are search-major, row (b*N + n)*K + k; the N*K <= max_beams rows
+ * of an image share its cross K/V, decoder prefix and n-gram history.  Per search and step t (P = prefix length):
+ *   1. all K beams start at score 0 (unlike beam search, which starts beams 1..K-1 at -1e9; only the draw separates them);
+ *   2. s = fp32(fp32(x - logZ) + beam_score) per (beam k, token w), logZ as in beam search; n-gram-banned tokens are -inf;
+ *   3. the warpers act on s, i.e. AFTER the beam score is added, as in 4.16.2: w = fp32(s / temperature), so the temperature compounds
+ *      through the beam scores (a beam's score is the sum of its warped steps, each divided by the temperature again at the next
+ *      step); top-k keeps w >= the k'-th largest w of the row, k' = max(top_k, 2), ties as far as the row's 16 best reach; top-p
+ *      (0 = off) inside that set keeps ranks 0 and 1 and drops rank r >= 2 once the probability mass before r exceeds top_p;
+ *   4. 2K entries are drawn without replacement from softmax(w) over the search's K*V entries (HF torch.multinomial(probs, 2K)) by
+ *      Gumbel-top-2K: the 2K largest of fp64(w) - log(-log u), u = ((h >> 11) + 0.5) * 2^-53 with
+ *      h = splitmix64(splitmix64(sd ^ splitmix64(((row_offset + b) << 20) ^ t)) ^ (k*V + w)), sd = candidate_seed(seed, n);
+ *      the draws of an image do not depend on how images are split across calls (row_offset);
+ *   5. the drawn entries, ordered by (w desc, k*V + w asc), go through BeamSearchScorer.process as in beam search: [SEP] closes a
+ *      hypothesis only at rank < K, a hypothesis scores its warped sum / (P + t), is_done uses the best drawn w.
+ *   Rejected with GSTVD_ERR_INVALID: num_beams < 2 or > 8, N < 1, N*num_beams > max_beams, num_beam_groups > 1, a temperature that is
+ *   not finite and > 0, top_p outside [0, 1].  Rejected with GSTVD_ERR_UNSUPPORTED: top_k = 0 or top_k > 16. */
 int gstvd_generate_groups(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, int num_beam_groups, float diversity_penalty, int N,
                           const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
                           int64_t* out_ids, float* out_scores, void* stream);
