@@ -12,7 +12,7 @@ from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int6
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "lib", "libgstvd.so")
 
-GSTVD_ABI_VERSION = 2
+GSTVD_ABI_VERSION = 3
 GSTVD_MAX_CONNECTIONS = 16
 GSTVD_F32, GSTVD_BF16 = 0, 1
 GSTVD_SELECT_SAMPLE, GSTVD_SELECT_BEAM, GSTVD_SELECT_BEAM_SAMPLE = 0, 1, 2
@@ -45,7 +45,7 @@ class GstvdGenParams(Structure):
     _fields_ = [
         ("mode", c_int32), ("num_beams", c_int32), ("max_new_tokens", c_int32), ("top_k", c_int32),
         ("temperature", c_float), ("top_p", c_float), ("ngram_blocking_size", c_int32), ("seed", c_uint64),
-        ("row_offset", c_int64),
+        ("row_offset", c_int64), ("num_return_sequences", c_int32), ("num_beam_groups", c_int32), ("diversity_penalty", c_float),
     ]
 
 
@@ -67,15 +67,8 @@ SYMBOLS = [
     ("gstvd_missing_weights", c_int, [_P]),
     ("gstvd_encode", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
     ("gstvd_prefill_cross", c_int, [_P, c_int, c_int, _P, _P, _P]),
-    ("gstvd_generate", c_int, [_P, c_int, POINTER(GstvdGenParams), _P, _P, c_int, _P, _P, _P]),
-    ("gstvd_generate_prefixed", c_int, [_P, c_int, POINTER(GstvdGenParams), _P, c_int, _P, _P, c_int, _P, _P, _P]),
-    ("gstvd_generate_candidates", c_int, [_P, c_int, POINTER(GstvdGenParams), c_int, _P, c_int, _P, _P, c_int, _P, _P, _P]),
-    ("gstvd_generate_groups", c_int, [_P, c_int, POINTER(GstvdGenParams), c_int, c_float, c_int, _P, c_int, _P, _P, c_int, _P, _P, _P]),
-    ("gstvd_round", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(GstvdGenParams), _P, _P, _P]),
-    ("gstvd_round_prefixed", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(GstvdGenParams), _P, c_int, _P, _P, _P]),
-    ("gstvd_round_candidates", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(GstvdGenParams), c_int, _P, c_int, _P, _P, _P]),
-    ("gstvd_round_groups", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(GstvdGenParams), c_int, c_float, c_int, _P, c_int,
-                                   _P, _P, _P]),
+    ("gstvd_generate", c_int, [_P, c_int, POINTER(GstvdGenParams), _P, c_int, _P, _P, c_int, _P, _P, _P]),
+    ("gstvd_round", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, POINTER(GstvdGenParams), _P, c_int, _P, _P, _P]),
     ("gstvd_score", c_int, [_P, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     ("gstvd_score_options", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     ("gstvd_reorder_cache", c_int, [_P, c_int, c_int, c_int, _P, _P]),

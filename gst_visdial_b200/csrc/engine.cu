@@ -67,15 +67,20 @@ struct DevBuf {
   void release() { if (p) cudaFree(p); p = nullptr; bytes = 0; }
 };
 
-// Shapes and selection parameters only: the n-gram blocking history and the decoder prefix are copied into context-owned buffers
-// before a replay, so the caller's tensor addresses are not part of the key (a caching allocator hands out a new address per batch).
-// P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start; N = sequences returned per image; G / penalty = beam groups
-// and diversity penalty.
+// Key of a captured decode graph (gstvd_generate) or round graph (gstvd_round): shapes and selection parameters only, built by
+// graph_key.  The n-gram blocking history, the decoder prefix and the round's inputs are copied into context-owned buffers before a
+// replay, so the caller's tensor addresses are not part of the key (a caching allocator hands out a new address per batch).  seed and
+// row_offset are not either: the graph reads them from device memory, so a replay can use a new seed.  Fields that do not apply to
+// a kind of call are 0: Lh / Le for a generate graph; Lt / Lv and the has_* flags (optional inputs, out_scores) for a round graph.
+// K = decode rows per image; P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start.
 struct GraphKey {
-  int B, K, mode, T, top_k, ngram, Lh, Le, P, has_prefix, N, G; float temperature, top_p, penalty;
+  int B, K, mode, T, top_k, ngram, P, has_prefix, N, G, Lh, Le, Lt, Lv, has_seg, has_att, has_imask, has_scores;
+  float temperature, top_p, penalty;
   bool operator<(const GraphKey& o) const { return std::memcmp(this, &o, sizeof(GraphKey)) < 0; }
 };
 constexpr size_t kMaxGraphs = 24;      // least-recently-used graphs beyond this are destroyed (an 18-step graph holds ~2k kernel nodes)
+struct GraphEntry { cudaGraphExec_t exec; int64_t kernels; uint64_t last_use; };   // kernels per replay, counted during capture
+using GraphPool = std::map<GraphKey, GraphEntry>;
 
 }  // namespace
 
@@ -127,15 +132,9 @@ struct gstvd_ctx {
   // beam op-test state
   int op_B = 0, op_K = 0, op_T = 0;
 
-  struct GraphEntry { cudaGraphExec_t exec; int64_t kernels; uint64_t last_use; };   // kernels per replay, counted during capture
-  std::map<GraphKey, GraphEntry> graphs;
+  GraphPool graphs;                   // decode graphs (gstvd_generate): every decode step of one call
+  GraphPool round_graphs;             // whole-round graphs (gstvd_round): encoder + cross-K/V prefill + every decode step of one call
   uint64_t graph_clock = 0;
-  // whole-round graphs (gstvd_round): encoder + cross-K/V prefill + every decode step of one forward call in ONE graph, keyed by shapes
-  struct RoundKey {
-    int B, Lt, Lv, K, mode, T, top_k, ngram, has_seg, has_att, has_imask, P, has_prefix, N, G; float temperature, top_p, penalty;
-    bool operator<(const RoundKey& o) const { return std::memcmp(this, &o, sizeof(RoundKey)) < 0; }
-  };
-  std::map<RoundKey, GraphEntry> round_graphs;
   DevBuf r_ids, r_seg, r_att, r_feat, r_loc, r_imask, r_out_ids, r_out_scores;   // context-owned copies of a round's inputs / outputs
   DevBuf hist_ids_own, hist_seg_own;                  // int64 [B_max, Lt_max]: n-gram blocking history read by captured graphs
   // optional event profiling of the tcgen05 GEMM launches (bench.py roofline): one event pair per launch
@@ -673,9 +672,10 @@ const int64_t* stage_prefix(gstvd_ctx* c, int B, const int64_t* prefix, int P, c
 }
 
 // Selection state of a decode call: beams / sample rows start from the last token of the prefix (the [CLS] when it is null).
-void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, int G, const int64_t* prefix, cudaStream_t s) {
+void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* prefix, cudaStream_t s) {
   const int P = g.P0 + 1, T = gp.max_new_tokens;
-  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, G, 1, T, 101, prefix, P, s);
+  if (gp.mode == GSTVD_SELECT_BEAM)
+    c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, gp.num_beam_groups, 1, T, 101, prefix, P, s);
   else if (gp.mode == GSTVD_SELECT_BEAM_SAMPLE) {
     const int K = gp.num_beams, N = g.K / K;      // N searches of K beams per image, all beams at score 0
     c->launches += launch_beam_init(beam_buffers(c), g.B * N, K, K, N, T, 101, prefix, P, s);
@@ -686,9 +686,9 @@ void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
 // One decode step for all M = B*K rows: embeddings -> 12 x [self-attn over cache, cross-attn, FFN] -> LM head -> selection.
 // step_host = index of this step when the caller knows it (it always does: eager loops and the captured graph both unroll the
 // steps), so kernels that only need it to bound their loads take it as a launch parameter instead of reading *d_step first.
-// prefix: int64 [B, P] decoder prefix (P = g.P0 + 1), null for the [CLS] start.  G / penalty: beam groups and diversity penalty.
-void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, int G, float penalty, const int64_t* prefix,
-                 const int64_t* hist_ids, const int64_t* hist_seg, int Lh, cudaStream_t s, int step_host) {
+// prefix: int64 [B, P] decoder prefix (P = g.P0 + 1), null for the [CLS] start.
+void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* prefix, const int64_t* hist_ids,
+                 const int64_t* hist_seg, int Lh, cudaStream_t s, int step_host) {
   Exec X{c, s};
   PdlScope pdl_scope(!(c->cfg.flags & GSTVD_FLAG_NO_PDL));
   const int H = c->H, M = g.B * g.K;
@@ -769,6 +769,7 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     }
     // beam groups: row_select also writes each row's logZ, from which the beam step re-scores the candidates a diversity penalty
     // lowers (the candidate lists stay ranked by the unpenalised score; launch_beam_step explains why nsel = 2K suffices)
+    const int G = gp.num_beam_groups;
     float* lz = G > 1 ? (float*)c->logz.p : nullptr;
     c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, (c->dtype == kBF16 && !exact_lse) ? 2 : 0,
                                      (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, lz, s);
@@ -778,12 +779,12 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
                                              (const uint64_t*)c->d_seed.p, 102, P, s);
     } else {
       c->launches += launch_beam_step(bb, g.B, g.K, G, Tn, c->V, nsel, sv, si, G > 1 ? (const float*)c->logits.p : nullptr, c->Vpad, lz,
-                                      penalty, 102, P, nullptr, nullptr, nullptr, s);
+                                      gp.diversity_penalty, 102, P, nullptr, nullptr, nullptr, s);
     }
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
   } else {
-    // g.K rows per image: the sampled candidates of gstvd_generate_candidates, each with its own n-gram key and RNG stream
+    // g.K rows per image: the num_return_sequences sampled candidates, each with its own n-gram key and RNG stream
     const int nsel = kSelMax;
     const int32_t* bt = nullptr; const int32_t* bc = nullptr;
     // key buffer c->prefix [M, P + Tn]: the decoder prefix, then the generated tokens; the samplers append token t at P + t
@@ -809,13 +810,14 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   c->launches += launch_step_advance((int*)c->d_step.p, s);
 }
 
-// Argument checks of a generate call returning N sequences per image; returns the decode rows per image (beam mode: the beams;
-// sample mode: the N candidates; beam sampling: N searches of num_beams beams).
-int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, int N, int G, float penalty, const int64_t* prefix, int P, const int64_t* hist_ids,
-                   const int64_t* hist_seg, int Lh, const int64_t* out_ids) {
+// Argument checks of a generate call returning N = gp.num_return_sequences sequences per image; returns the decode rows per image
+// (beam mode: the beams; sample mode: the N candidates; beam sampling: N searches of num_beams beams).
+int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_seg,
+                   int Lh, const int64_t* out_ids) {
   check_ready(c);
   if (c->dec_layers == 0) throw StateError("generate: encoder-only context");
-  const int T = gp.max_new_tokens;
+  const int T = gp.max_new_tokens, N = gp.num_return_sequences, G = gp.num_beam_groups;
+  const float penalty = gp.diversity_penalty;
   if (T < 1 || T > c->T_max) throw InvalidArg("generate: max_new_tokens out of range");
   if (P < 1 || P > c->Ldec_max) throw InvalidArg(fmt("generate: decoder prefix length %d outside 1..max_dec_len (%d)", P, c->Ldec_max));
   if (!prefix && P > 1) throw InvalidArg("generate: the decoder prefix is NULL but its length is above 1");
@@ -856,74 +858,87 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, int N, int G, float
 }
 
 // out_ids [B*N, T] image-major (sample mode: N == K, one row per candidate)
-void generate_finalize(gstvd_ctx* c, int B, int K, int P, int N, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
-  const int T = gp.max_new_tokens;
+void generate_finalize(gstvd_ctx* c, int B, int K, int P, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
+  const int T = gp.max_new_tokens, N = gp.num_return_sequences;
   if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, P, N, out_ids, out_scores, s);
   else if (gp.mode == GSTVD_SELECT_BEAM_SAMPLE)   // search n of image b is search b * N + n: its best hypothesis is output row b * N + n
     c->launches += launch_beam_finalize(beam_buffers(c), B * N, gp.num_beams, T, 102, P, 1, out_ids, out_scores, s);
   else c->launches += launch_sample_finalize(B * K, T, 102, (const int32_t*)c->seq.p, out_ids, s);
 }
 
-void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, int N, int G, float penalty, const int64_t* prefix, int P,
-                 const int64_t* hist_ids, const int64_t* hist_seg, int Lh, int64_t* out_ids, float* out_scores, cudaStream_t s) {
-  const int K = check_generate(c, gp, N, G, penalty, prefix, P, hist_ids, hist_seg, Lh, out_ids);
+// The key of a generate graph (Lh, Le set) or a round graph (Lt, Lv and the has_* flags set), from the request and the shapes.
+GraphKey graph_key(const gstvd_gen_params& gp, int B, int K, int P, bool has_prefix, int Lh, int Le, int Lt, int Lv, bool has_seg,
+                   bool has_att, bool has_imask, bool has_scores) {
+  GraphKey k;
+  std::memset(&k, 0, sizeof k);
+  k.B = B; k.K = K; k.mode = gp.mode; k.T = gp.max_new_tokens; k.top_k = gp.top_k; k.ngram = gp.ngram_blocking_size;
+  k.P = P; k.has_prefix = has_prefix; k.N = gp.num_return_sequences; k.G = gp.num_beam_groups;
+  k.Lh = Lh; k.Le = Le; k.Lt = Lt; k.Lv = Lv; k.has_seg = has_seg; k.has_att = has_att; k.has_imask = has_imask; k.has_scores = has_scores;
+  k.temperature = gp.temperature; k.top_p = gp.top_p; k.penalty = gp.diversity_penalty;
+  return k;
+}
+
+// Launches the graph of `key` from `pool`.  On a miss it first captures `body` into a new graph, destroying the least recently used
+// graph of a full pool.  The launch counter advances by the kernels the capture counted, as if `body` had run eagerly.
+template <class Body>
+void replay_graph(gstvd_ctx* c, GraphPool& pool, const GraphKey& key, cudaStream_t s, Body&& body) {
+  auto it = pool.find(key);
+  if (it == pool.end()) {
+    if (pool.size() >= kMaxGraphs) {
+      auto victim = pool.begin();
+      for (auto j = pool.begin(); j != pool.end(); ++j) if (j->second.last_use < victim->second.last_use) victim = j;
+      CUDA_CHECK(cudaStreamSynchronize(s));             // it may still be executing on this stream
+      cudaGraphExecDestroy(victim->second.exec);
+      pool.erase(victim);
+    }
+    const int64_t before = c->launches;
+    cudaGraph_t graph;
+    CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+    try {
+      body();
+    } catch (...) {
+      cudaGraph_t dead; cudaStreamEndCapture(s, &dead);
+      throw;
+    }
+    CUDA_CHECK(cudaStreamEndCapture(s, &graph));
+    cudaGraphExec_t exec;
+    CUDA_CHECK(cudaGraphInstantiate(&exec, graph, 0));
+    CUDA_CHECK(cudaGraphDestroy(graph));
+    it = pool.emplace(key, GraphEntry{exec, c->launches - before, 0}).first;
+    c->launches = before;                           // capture itself launches nothing
+  }
+  it->second.last_use = ++c->graph_clock;
+  CUDA_CHECK(cudaGraphLaunch(it->second.exec, s));
+  c->launches += it->second.kernels;
+}
+
+void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t* prefix, int P, const int64_t* hist_ids,
+                 const int64_t* hist_seg, int Lh, int64_t* out_ids, float* out_scores, cudaStream_t s) {
+  const int K = check_generate(c, gp, prefix, P, hist_ids, hist_seg, Lh, out_ids);
   if (c->cross_B != B) throw StateError(fmt("generate: cross K/V prefilled for %d images, asked for %d", c->cross_B, B));
   const int T = gp.max_new_tokens;
   const DecodeGeom g = make_geom(c, B, K, T, P);
   const int64_t* pre = stage_prefix(c, B, prefix, P, s);
   // the sampling seed lives in device memory so that a captured graph can be replayed with a new seed
   c->launches += launch_set_u64((uint64_t*)c->d_seed.p, gp.seed, (uint64_t)gp.row_offset, s);
-  decode_init(c, g, gp, G, pre, s);
+  decode_init(c, g, gp, pre, s);
 
   const bool use_graph = !(c->cfg.flags & GSTVD_FLAG_NO_CUDA_GRAPH);
-  if (!use_graph) {
-    prefix_prefill(c, g, s);
-    for (int t = 0; t < T; ++t) decode_step(c, g, gp, G, penalty, pre, hist_ids, hist_seg, Lh, s, t);
-  } else {
-    GraphKey key;
-    std::memset(&key, 0, sizeof key);
-    key.B = B; key.K = K; key.mode = gp.mode; key.T = T; key.top_k = gp.top_k; key.ngram = gp.ngram_blocking_size; key.Lh = Lh;
-    key.P = P; key.has_prefix = pre != nullptr; key.N = N; key.G = G; key.penalty = penalty;
-    key.temperature = gp.temperature; key.top_p = gp.top_p;
-    key.Le = c->cross_Le;                    // the cross cache geometry is part of the captured launch parameters
-    const int64_t* g_ids = hist_ids; const int64_t* g_seg = hist_seg;
-    if (gp.ngram_blocking_size > 0) {
-      // the graph reads the history from the context's own buffers: refresh them (device-to-device, ordered on this stream)
-      CUDA_CHECK(cudaMemcpyAsync(c->hist_ids_own.p, hist_ids, (size_t)B * Lh * 8, cudaMemcpyDeviceToDevice, s));
-      CUDA_CHECK(cudaMemcpyAsync(c->hist_seg_own.p, hist_seg, (size_t)B * Lh * 8, cudaMemcpyDeviceToDevice, s));
-      g_ids = (const int64_t*)c->hist_ids_own.p; g_seg = (const int64_t*)c->hist_seg_own.p;
-    }
-    auto it = c->graphs.find(key);
-    if (it == c->graphs.end()) {
-      if (c->graphs.size() >= kMaxGraphs) {  // evict the least recently used graph
-        auto victim = c->graphs.begin();
-        for (auto j = c->graphs.begin(); j != c->graphs.end(); ++j) if (j->second.last_use < victim->second.last_use) victim = j;
-        CUDA_CHECK(cudaStreamSynchronize(s));             // it may still be executing on this stream
-        cudaGraphExecDestroy(victim->second.exec);
-        c->graphs.erase(victim);
-      }
-      const int64_t before = c->launches;
-      cudaGraph_t graph;
-      CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-      try {
-        prefix_prefill(c, g, s);
-        for (int t = 0; t < T; ++t) decode_step(c, g, gp, G, penalty, pre, g_ids, g_seg, Lh, s, t);   // all T steps in ONE graph: no host round trip between steps
-      } catch (...) {
-        cudaGraph_t dead; cudaStreamEndCapture(s, &dead);
-        throw;
-      }
-      CUDA_CHECK(cudaStreamEndCapture(s, &graph));
-      cudaGraphExec_t exec;
-      CUDA_CHECK(cudaGraphInstantiate(&exec, graph, 0));
-      CUDA_CHECK(cudaGraphDestroy(graph));
-      it = c->graphs.emplace(key, gstvd_ctx::GraphEntry{exec, c->launches - before, 0}).first;
-      c->launches = before;                           // capture itself launches nothing
-    }
-    it->second.last_use = ++c->graph_clock;
-    CUDA_CHECK(cudaGraphLaunch(it->second.exec, s));
-    c->launches += it->second.kernels;
+  const int64_t* g_ids = hist_ids; const int64_t* g_seg = hist_seg;
+  if (use_graph && gp.ngram_blocking_size > 0) {
+    // the graph reads the history from the context's own buffers: refresh them (device-to-device, ordered on this stream)
+    CUDA_CHECK(cudaMemcpyAsync(c->hist_ids_own.p, hist_ids, (size_t)B * Lh * 8, cudaMemcpyDeviceToDevice, s));
+    CUDA_CHECK(cudaMemcpyAsync(c->hist_seg_own.p, hist_seg, (size_t)B * Lh * 8, cudaMemcpyDeviceToDevice, s));
+    g_ids = (const int64_t*)c->hist_ids_own.p; g_seg = (const int64_t*)c->hist_seg_own.p;
   }
-  generate_finalize(c, B, K, P, N, gp, out_ids, out_scores, s);
+  auto body = [&] {
+    prefix_prefill(c, g, s);
+    for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, g_ids, g_seg, Lh, s, t);   // all T steps in ONE graph: no host round trip between steps
+  };
+  // the cross cache geometry (Le) is part of the captured launch parameters
+  if (!use_graph) body();
+  else replay_graph(c, c->graphs, graph_key(gp, B, K, P, pre, Lh, c->cross_Le, 0, 0, false, false, false, false), s, body);
+  generate_finalize(c, B, K, P, gp, out_ids, out_scores, s);
 }
 
 // One forward call of the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:24-120) - encoder, fusion,
@@ -932,13 +947,13 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, int N, int G, 
 // order, same results as gstvd_encode + gstvd_prefill_cross + gstvd_generate (asserted by the tests); eager when graphs are
 // disabled or while the GEMM profiler is on (events cannot be recorded inside a graph).
 void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int64_t* seg, const float* att, const float* feat,
-              const float* loc, const float* imask, const gstvd_gen_params& gp, int N, int G, float penalty, const int64_t* prefix, int P,
-              int64_t* out_ids, float* out_scores, cudaStream_t s) {
-  const int K = check_generate(c, gp, N, G, penalty, prefix, P, ids, seg ? seg : ids, Lt, out_ids);
+              const float* loc, const float* imask, const gstvd_gen_params& gp, const int64_t* prefix, int P, int64_t* out_ids,
+              float* out_scores, cudaStream_t s) {
+  const int K = check_generate(c, gp, prefix, P, ids, seg ? seg : ids, Lt, out_ids);
   if (B < 1 || B > c->B_max || Lt < 1 || Lt > c->Lt_max || Lv < 1 || Lv > c->Lv_max) throw InvalidArg("round: shape exceeds capacity");
   if (!ids || !feat || !loc) throw InvalidArg("round: input_ids / image_feat / image_loc must not be NULL");
   if (gp.ngram_blocking_size > 0 && !seg) throw InvalidArg("round: n-gram blocking needs token_type_ids");
-  const int T = gp.max_new_tokens, F = c->cfg.v_feature_size;
+  const int T = gp.max_new_tokens, N = gp.num_return_sequences, F = c->cfg.v_feature_size;
   auto d2d = [&](void* dst, const void* src, size_t bytes) { if (src) CUDA_CHECK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s)); };
   d2d(c->r_ids.p, ids, (size_t)B * Lt * 8); d2d(c->r_seg.p, seg, (size_t)B * Lt * 8); d2d(c->r_att.p, att, (size_t)B * Lt * 4);
   d2d(c->r_feat.p, feat, (size_t)B * Lv * F * 4); d2d(c->r_loc.p, loc, (size_t)B * Lv * 5 * 4); d2d(c->r_imask.p, imask, (size_t)B * Lv * 4);
@@ -951,50 +966,16 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
               imask ? (const float*)c->r_imask.p : nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, s);
     do_prefill(c, B, Lv + Lt, nullptr, nullptr, s);
     const DecodeGeom g = make_geom(c, B, K, T, P);
-    decode_init(c, g, gp, G, pre, s);
+    decode_init(c, g, gp, pre, s);
     prefix_prefill(c, g, s);
-    for (int t = 0; t < T; ++t) decode_step(c, g, gp, G, penalty, pre, g_ids, g_seg, Lt, s, t);
-    generate_finalize(c, B, K, P, N, gp, (int64_t*)c->r_out_ids.p, out_scores ? (float*)c->r_out_scores.p : nullptr, s);
+    for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, g_ids, g_seg, Lt, s, t);
+    generate_finalize(c, B, K, P, gp, (int64_t*)c->r_out_ids.p, out_scores ? (float*)c->r_out_scores.p : nullptr, s);
   };
   const bool use_graph = !(c->cfg.flags & GSTVD_FLAG_NO_CUDA_GRAPH) && !c->profiling;
   if (!use_graph) {
     body();
   } else {
-    gstvd_ctx::RoundKey key;
-    std::memset(&key, 0, sizeof key);
-    key.B = B; key.Lt = Lt; key.Lv = Lv; key.K = K; key.mode = gp.mode; key.T = T; key.top_k = gp.top_k; key.ngram = gp.ngram_blocking_size;
-    key.has_seg = seg != nullptr; key.has_att = att != nullptr; key.has_imask = imask != nullptr;
-    key.temperature = gp.temperature; key.top_p = gp.top_p;
-    key.P = P; key.has_prefix = pre != nullptr; key.N = N; key.G = G; key.penalty = penalty;
-    if (out_scores) key.has_imask |= 2;
-    auto it = c->round_graphs.find(key);
-    if (it == c->round_graphs.end()) {
-      if (c->round_graphs.size() >= kMaxGraphs) {
-        auto victim = c->round_graphs.begin();
-        for (auto j = c->round_graphs.begin(); j != c->round_graphs.end(); ++j) if (j->second.last_use < victim->second.last_use) victim = j;
-        CUDA_CHECK(cudaStreamSynchronize(s));
-        cudaGraphExecDestroy(victim->second.exec);
-        c->round_graphs.erase(victim);
-      }
-      const int64_t before = c->launches;
-      cudaGraph_t graph;
-      CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
-      try {
-        body();
-      } catch (...) {
-        cudaGraph_t dead; cudaStreamEndCapture(s, &dead);
-        throw;
-      }
-      CUDA_CHECK(cudaStreamEndCapture(s, &graph));
-      cudaGraphExec_t exec;
-      CUDA_CHECK(cudaGraphInstantiate(&exec, graph, 0));
-      CUDA_CHECK(cudaGraphDestroy(graph));
-      it = c->round_graphs.emplace(key, gstvd_ctx::GraphEntry{exec, c->launches - before, 0}).first;
-      c->launches = before;
-    }
-    it->second.last_use = ++c->graph_clock;
-    CUDA_CHECK(cudaGraphLaunch(it->second.exec, s));
-    c->launches += it->second.kernels;
+    replay_graph(c, c->round_graphs, graph_key(gp, B, K, P, pre, 0, 0, Lt, Lv, seg, att, imask, out_scores), s, body);
     // host-side state the captured calls set (a replay does not run them again)
     c->enc_B = B; c->enc_Le = Lv + Lt; c->cross_B = B; c->cross_Le = Lv + Lt;
   }
@@ -1203,70 +1184,29 @@ int gstvd_prefill_cross(gstvd_ctx* c, int B, int Le, const float* enc_hidden, co
   return guarded(c, [&] { do_prefill(c, B, Le, enc_hidden, enc_mask, (cudaStream_t)stream); });
 }
 
-int gstvd_generate(gstvd_ctx* c, int B, const gstvd_gen_params* params, const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
-                   int64_t* out_ids, float* out_scores, void* stream) {
-  return gstvd_generate_prefixed(c, B, params, nullptr, 1, hist_ids, hist_segments, Lh, out_ids, out_scores, stream);
-}
-
-int gstvd_generate_prefixed(gstvd_ctx* c, int B, const gstvd_gen_params* params, const int64_t* prefix, int P, const int64_t* hist_ids,
-                            const int64_t* hist_segments, int Lh, int64_t* out_ids, float* out_scores, void* stream) {
-  return gstvd_generate_candidates(c, B, params, 1, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores, stream);
-}
-
-int gstvd_generate_candidates(gstvd_ctx* c, int B, const gstvd_gen_params* params, int N, const int64_t* prefix, int P,
-                              const int64_t* hist_ids, const int64_t* hist_segments, int Lh, int64_t* out_ids, float* out_scores,
-                              void* stream) {
-  return gstvd_generate_groups(c, B, params, 1, 0.f, N, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores, stream);
-}
-
-int gstvd_generate_groups(gstvd_ctx* c, int B, const gstvd_gen_params* params, int num_beam_groups, float diversity_penalty, int N,
-                          const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_segments, int Lh, int64_t* out_ids,
-                          float* out_scores, void* stream) {
+int gstvd_generate(gstvd_ctx* c, int B, const gstvd_gen_params* params, const int64_t* prefix, int P, const int64_t* hist_ids,
+                   const int64_t* hist_segments, int Lh, int64_t* out_ids, float* out_scores, void* stream) {
   if (!c || !params) { g_last_error = "gstvd_generate: NULL argument"; return GSTVD_ERR_INVALID; }
   return guarded(c, [&] {
     cudaStream_t user = (cudaStream_t)stream;
     CUDA_CHECK(cudaEventRecord(c->ev_in, user));
     CUDA_CHECK(cudaStreamWaitEvent(c->own_stream, c->ev_in, 0));
-    do_generate(c, B, *params, N, num_beam_groups, diversity_penalty, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores,
-                c->own_stream);
+    do_generate(c, B, *params, prefix, P, hist_ids, hist_segments, Lh, out_ids, out_scores, c->own_stream);
     CUDA_CHECK(cudaEventRecord(c->ev_out, c->own_stream));
     CUDA_CHECK(cudaStreamWaitEvent(user, c->ev_out, 0));
   });
 }
 
 int gstvd_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
-                const float* image_feat, const float* image_loc, const float* image_mask, const gstvd_gen_params* params, int64_t* out_ids,
-                float* out_scores, void* stream) {
-  return gstvd_round_prefixed(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, params, nullptr, 1,
-                              out_ids, out_scores, stream);
-}
-
-int gstvd_round_prefixed(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, const int64_t* token_type_ids,
-                         const float* attention_mask, const float* image_feat, const float* image_loc, const float* image_mask,
-                         const gstvd_gen_params* params, const int64_t* prefix, int P, int64_t* out_ids, float* out_scores, void* stream) {
-  return gstvd_round_candidates(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, params, 1, prefix,
-                                P, out_ids, out_scores, stream);
-}
-
-int gstvd_round_candidates(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, const int64_t* token_type_ids,
-                           const float* attention_mask, const float* image_feat, const float* image_loc, const float* image_mask,
-                           const gstvd_gen_params* params, int N, const int64_t* prefix, int P, int64_t* out_ids, float* out_scores,
-                           void* stream) {
-  return gstvd_round_groups(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, params, 1, 0.f, N,
-                            prefix, P, out_ids, out_scores, stream);
-}
-
-int gstvd_round_groups(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* input_ids, const int64_t* token_type_ids,
-                       const float* attention_mask, const float* image_feat, const float* image_loc, const float* image_mask,
-                       const gstvd_gen_params* params, int num_beam_groups, float diversity_penalty, int N, const int64_t* prefix, int P,
-                       int64_t* out_ids, float* out_scores, void* stream) {
+                const float* image_feat, const float* image_loc, const float* image_mask, const gstvd_gen_params* params,
+                const int64_t* prefix, int P, int64_t* out_ids, float* out_scores, void* stream) {
   if (!c || !params) { g_last_error = "gstvd_round: NULL argument"; return GSTVD_ERR_INVALID; }
   return guarded(c, [&] {
     cudaStream_t user = (cudaStream_t)stream;
     CUDA_CHECK(cudaEventRecord(c->ev_in, user));
     CUDA_CHECK(cudaStreamWaitEvent(c->own_stream, c->ev_in, 0));
-    do_round(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, *params, N, num_beam_groups,
-             diversity_penalty, prefix, P, out_ids, out_scores, c->own_stream);
+    do_round(c, B, Lt, Lv, input_ids, token_type_ids, attention_mask, image_feat, image_loc, image_mask, *params, prefix, P, out_ids,
+             out_scores, c->own_stream);
     CUDA_CHECK(cudaEventRecord(c->ev_out, c->own_stream));
     CUDA_CHECK(cudaStreamWaitEvent(user, c->ev_out, 0));
   });

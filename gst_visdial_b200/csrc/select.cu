@@ -700,7 +700,7 @@ __device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
   return x ^ (x >> 31);
 }
 
-// Sampling seed of candidate n of an image (gstvd_generate_candidates): candidate n draws what a single-sample call seeded
+// Sampling seed of candidate n of an image (gstvd_gen_params.num_return_sequences): candidate n draws what a single-sample call seeded
 // candidate_seed(seed, n) draws, and candidate 0 is that call itself.  Mirrored by models/visual_dialog_model.candidate_seed.
 __device__ __forceinline__ uint64_t candidate_seed(uint64_t seed, int n) {
   return n == 0 ? seed : splitmix64(seed ^ splitmix64((uint64_t)n * 0xD1B54A32D192ED03ull));

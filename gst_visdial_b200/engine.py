@@ -180,20 +180,9 @@ class Engine:
             raise ValueError(f"prefix must be [B={B}, P], got {tuple(pre.shape)}")
         return pre, pre.shape[1]
 
-    def generate(self, B, num_beams=1, temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0,
-                 max_new_tokens=None, hist_ids=None, hist_segments=None, want_scores=False, row_offset=0, prefix=None,
-                 num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0, do_sample=False):
-        """``row_offset``: global index of row 0; the sampler is keyed by (seed, row_offset + row, step), so an image draws the
-        same tokens whichever batch or rank it lands in.  ``prefix``: int64 [B, P] decoder input to continue from (the reference's
-        dec_input_ids; include/gstvd.h gstvd_generate_prefixed), None = one [CLS] per row; the result holds the new tokens only.
-        ``num_return_sequences`` = N: [B*N, T] image-major - the N best beams, or N sampled candidates per image of which
-        candidate n draws like an N = 1 call with seed ``candidate_seed(seed, n)`` (include/gstvd.h gstvd_generate_candidates).
-        ``num_beam_groups`` = G > 1 with ``diversity_penalty``: diverse beam search, the K beams in G groups of K / G with a Hamming
-        penalty between groups (include/gstvd.h gstvd_generate_groups, contract in oracle/beam_groups.py).
-        ``do_sample`` with ``num_beams`` > 1: beam sampling (HF beam_sample) with ``temperature`` / ``top_k`` / ``top_p`` / ``seed``;
-        ``num_return_sequences`` = N then runs N independent searches per image, search n seeded ``candidate_seed(seed, n)``, and
-        returns the best hypothesis of each (include/gstvd.h GSTVD_SELECT_BEAM_SAMPLE, contract in oracle/beam_sample.py).  With
-        ``num_beams`` = 1 the sampler runs whatever ``do_sample`` says."""
+    def _gen_params(self, num_beams=1, temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0, max_new_tokens=None,
+                    row_offset=0, num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0, do_sample=False):
+        """The gstvd_gen_params of one decode request (include/gstvd.h gstvd_generate)."""
         gp = GstvdGenParams()
         gp.mode = _select_mode(num_beams, do_sample)
         gp.num_beams = int(num_beams)
@@ -201,15 +190,35 @@ class Engine:
         gp.top_k, gp.temperature, gp.top_p = int(top_k), float(temperature), float(top_p)
         gp.ngram_blocking_size, gp.seed = int(ngram_blocking_size), int(seed) & (2**64 - 1)
         gp.row_offset = int(row_offset)
+        gp.num_return_sequences, gp.num_beam_groups = int(num_return_sequences), int(num_beam_groups)
+        gp.diversity_penalty = float(diversity_penalty)
+        return gp
+
+    def generate(self, B, num_beams=1, temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0,
+                 max_new_tokens=None, hist_ids=None, hist_segments=None, want_scores=False, row_offset=0, prefix=None,
+                 num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0, do_sample=False):
+        """``row_offset``: global index of row 0; the sampler is keyed by (seed, row_offset + row, step), so an image draws the
+        same tokens whichever batch or rank it lands in.  ``prefix``: int64 [B, P] decoder input to continue from (the reference's
+        dec_input_ids), None = one [CLS] per row; the result holds the new tokens only.
+        ``num_return_sequences`` = N: [B*N, T] image-major - the N best beams, or N sampled candidates per image of which
+        candidate n draws like an N = 1 call with seed ``candidate_seed(seed, n)``.
+        ``num_beam_groups`` = G > 1 with ``diversity_penalty``: diverse beam search, the K beams in G groups of K / G with a Hamming
+        penalty between groups (contract in oracle/beam_groups.py).
+        ``do_sample`` with ``num_beams`` > 1: beam sampling (HF beam_sample) with ``temperature`` / ``top_k`` / ``top_p`` / ``seed``;
+        ``num_return_sequences`` = N then runs N independent searches per image, search n seeded ``candidate_seed(seed, n)``, and
+        returns the best hypothesis of each (GSTVD_SELECT_BEAM_SAMPLE, contract in oracle/beam_sample.py).  With ``num_beams`` = 1
+        the sampler runs whatever ``do_sample`` says.  The whole contract is at gstvd_generate in include/gstvd.h."""
+        gp = self._gen_params(num_beams, temperature, top_k, top_p, ngram_blocking_size, seed, max_new_tokens, row_offset,
+                              num_return_sequences, num_beam_groups, diversity_penalty, do_sample)
         hid = self._dev(hist_ids, torch.int64) if ngram_blocking_size > 0 else None
         hseg = self._dev(hist_segments, torch.int64) if ngram_blocking_size > 0 else None
         Lh = hid.shape[1] if hid is not None else 0
         pre, P = self._prefix(prefix, B)
-        N = int(num_return_sequences)
+        N = gp.num_return_sequences
         out = torch.empty(B * max(N, 1), gp.max_new_tokens, device=self.device, dtype=torch.int64)
         scores = torch.empty(B * max(N, 1), device=self.device, dtype=torch.float32) if want_scores else None
-        check(self.ctx, self.lib.gstvd_generate_groups(self.ctx, B, ctypes.byref(gp), int(num_beam_groups), float(diversity_penalty), N,
-                                                       _ptr(pre), P, _ptr(hid), _ptr(hseg), Lh, _ptr(out), _ptr(scores), self._stream()))
+        check(self.ctx, self.lib.gstvd_generate(self.ctx, B, ctypes.byref(gp), _ptr(pre), P, _ptr(hid), _ptr(hseg), Lh, _ptr(out),
+                                                _ptr(scores), self._stream()))
         return (out, scores) if want_scores else out
 
     def round(self, input_ids, image_feat, image_loc, token_type_ids=None, attention_mask=None, image_mask=None, num_beams=1,
@@ -226,20 +235,14 @@ class Engine:
         seg = self._dev(token_type_ids, torch.int64)
         att = self._dev(attention_mask, torch.float32)
         imask = self._dev(image_mask, torch.float32)
-        gp = GstvdGenParams()
-        gp.mode = _select_mode(num_beams, do_sample)
-        gp.num_beams = int(num_beams)
-        gp.max_new_tokens = int(max_new_tokens or self.max_new_tokens)
-        gp.top_k, gp.temperature, gp.top_p = int(top_k), float(temperature), float(top_p)
-        gp.ngram_blocking_size, gp.seed = int(ngram_blocking_size), int(seed) & (2**64 - 1)
-        gp.row_offset = int(row_offset)
+        gp = self._gen_params(num_beams, temperature, top_k, top_p, ngram_blocking_size, seed, max_new_tokens, row_offset,
+                              num_return_sequences, num_beam_groups, diversity_penalty, do_sample)
         pre, P = self._prefix(prefix, B)
-        N = int(num_return_sequences)
+        N = gp.num_return_sequences
         out = torch.empty(B * max(N, 1), gp.max_new_tokens, device=self.device, dtype=torch.int64)
         scores = torch.empty(B * max(N, 1), device=self.device, dtype=torch.float32) if want_scores else None
-        check(self.ctx, self.lib.gstvd_round_groups(self.ctx, B, Lt, Lv, _ptr(ids), _ptr(seg), _ptr(att), _ptr(feat), _ptr(loc), _ptr(imask),
-                                                    ctypes.byref(gp), int(num_beam_groups), float(diversity_penalty), N, _ptr(pre), P,
-                                                    _ptr(out), _ptr(scores), self._stream()))
+        check(self.ctx, self.lib.gstvd_round(self.ctx, B, Lt, Lv, _ptr(ids), _ptr(seg), _ptr(att), _ptr(feat), _ptr(loc), _ptr(imask),
+                                             ctypes.byref(gp), _ptr(pre), P, _ptr(out), _ptr(scores), self._stream()))
         return (out, scores) if want_scores else out
 
     def score(self, dec_ids, dec_mask=None, labels=None, want_logits=False, want_loss=True, options_per_image=1):
@@ -357,10 +360,8 @@ class Engine:
     def op_sample(self, logits, step, temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0, hist_ids=None,
                   hist_segments=None, prefix=None, row_offset=0):
         lg = self._dev(logits, torch.float32)
-        gp = GstvdGenParams()
-        gp.mode, gp.num_beams, gp.max_new_tokens = GSTVD_SELECT_SAMPLE, 1, self.max_new_tokens
-        gp.top_k, gp.temperature, gp.top_p = int(top_k), float(temperature), float(top_p)
-        gp.ngram_blocking_size, gp.seed, gp.row_offset = int(ngram_blocking_size), int(seed) & (2**64 - 1), int(row_offset)
+        gp = self._gen_params(temperature=temperature, top_k=top_k, top_p=top_p, ngram_blocking_size=ngram_blocking_size, seed=seed,
+                              row_offset=row_offset)
         hid, hseg, pre = self._dev(hist_ids, torch.int64), self._dev(hist_segments, torch.int64), self._dev(prefix, torch.int64)
         rows = lg.shape[0]
         out = torch.empty(rows, device=self.device, dtype=torch.int32)

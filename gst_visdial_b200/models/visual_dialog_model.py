@@ -188,7 +188,7 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
 
     def _check_decoder_start(self, dec_input_ids):
         """The reference continues from whatever prefix the caller passes (models/visual_dialog_model.py:86-110), and so does the
-        engine (include/gstvd.h gstvd_generate_prefixed); its token bookkeeping needs the BERT bos / eos ids."""
+        engine (include/gstvd.h gstvd_generate, its prefix argument); its token bookkeeping needs the BERT bos / eos ids."""
         if dec_input_ids is None:
             return
         bos = int(getattr(self.decoder.config, "bos_token_id", 101) or 101)

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define GSTVD_ABI_VERSION 2
+#define GSTVD_ABI_VERSION 3
 #define GSTVD_MAX_CONNECTIONS 16
 
 typedef enum {
@@ -46,7 +46,7 @@ typedef enum {
                               (models/visual_dialog_model.py:86-110, utils/decoding_utils.py:4-35) */
   GSTVD_SELECT_BEAM = 1,   /* beam search, contract in oracle/beam.py (new behaviour, north_star) */
   GSTVD_SELECT_BEAM_SAMPLE = 2 /* beam sampling (HF num_beams > 1 with do_sample): num_beams, top_k, top_p, temperature and seed all
-                                  apply; contract at gstvd_generate_groups and in oracle/beam_sample.py */
+                                  apply; contract at gstvd_generate and in oracle/beam_sample.py */
 } gstvd_select_mode;
 
 /* Model geometry: the fields of config/bert_base_6layer_6conect_{enc,dec}.json that the path reads
@@ -83,7 +83,7 @@ typedef struct {
 
 typedef struct {
   int32_t mode;               /* gstvd_select_mode */
-  int32_t num_beams;          /* beam mode: K (<= max_beams); sample mode: ignored (N rows per image, gstvd_generate_candidates) */
+  int32_t num_beams;          /* beam mode: K (<= max_beams); sample mode: ignored (num_return_sequences rows per image) */
   int32_t max_new_tokens;     /* <= config.max_new_tokens */
   int32_t top_k;              /* sample mode; 1 = greedy; 2..GSTVD_MAX_TOP_K = top-k set (ties kept); 0 = no top-k cut: multinomial over the
                                  whole - optionally nucleus-filtered - vocabulary (utils/decoding_utils.py:17 skips the cut) */
@@ -94,6 +94,9 @@ typedef struct {
   uint64_t seed;              /* sample mode RNG seed (counter-based; reproducible per (seed, row_offset + row, step)) */
   int64_t row_offset;         /* global index of row 0 (e.g. the image index of the first sample of this batch / shard): the
                                  draws of an image do not depend on how the images were split into batches or ranks */
+  int32_t num_return_sequences; /* N >= 1 sequences per image (HF num_return_sequences); contract at gstvd_generate */
+  int32_t num_beam_groups;    /* G >= 1 (HF num_beam_groups): beam mode splits the K beams into G groups; 1 = plain beam search */
+  float diversity_penalty;    /* Hamming penalty between beam groups (HF diversity_penalty), finite and >= 0 */
 } gstvd_gen_params;
 
 #define GSTVD_MAX_TOP_K 16
@@ -142,30 +145,22 @@ int gstvd_encode(gstvd_ctx* ctx, int B, int Lt, int Lv,
 int gstvd_prefill_cross(gstvd_ctx* ctx, int B, int Le, const float* enc_hidden, const float* enc_mask, void* stream);
 
 /* Replaces the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:74-120) including
- * batch_ngram_blocking / batch_top_k_top_p_sampling (utils/decoding_utils.py:4-78), with a persistent KV cache.
+ * batch_ngram_blocking / batch_top_k_top_p_sampling (utils/decoding_utils.py:4-78), with a persistent KV cache.  The tensors are
+ * positional; params holds the whole selection policy, including N = num_return_sequences, G = num_beam_groups and
+ * diversity_penalty.
+ *   prefix : int64 [B, P], 1 <= P <= max_dec_len: the decoder input to continue from, the reference's dec_input_ids
+ *            (models/visual_dialog_model.py:86-110 continues from whatever the caller passes), shared by the rows of an image; NULL
+ *            means one [CLS] per row (P must be 1).  At every step the decoder sees prefix + the tokens generated so far at positions
+ *            0 .. P-1+t, without a padding mask; a [SEP] in the prefix is read as [PAD] (models/visual_dialog_decoder.py:57).  n-gram
+ *            keys may reach into the prefix.  Beam hypotheses count the prefix in their length (HF beam_search input_ids.shape[-1]).
+ *            The caller's tensor is not modified.  P - 1 + max_new_tokens must not exceed 64 (cached positions of the decode
+ *            kernels) nor max_position_embeddings.
  *   hist_ids, hist_segments : int64 [B, Lh] encoder input ids / segments (only read when ngram_blocking_size > 0, in sample and
  *                             beam mode; the question history is ids * (segments == 0), visual_dialog_model.py:98-99)
- *   out_ids    : int64 [B, max_new_tokens] - sampled / best-beam tokens, PAD(0) after the first [SEP]
- *   out_scores : fp32 [B] (may be NULL)    - beam mode: best hypothesis score (sum log-prob / length) */
-int gstvd_generate(gstvd_ctx* ctx, int B, const gstvd_gen_params* params,
-                   const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
-                   int64_t* out_ids, float* out_scores, void* stream);
-
-/* gstvd_generate continuing from a caller-supplied decoder prefix, the reference's dec_input_ids (models/visual_dialog_model.py:86-110
- * continues from whatever the caller passes).  gstvd_generate is this call with prefix = NULL, P = 1.
- *   prefix : int64 [B, P], 1 <= P <= max_dec_len, shared by the beams of an image; NULL means one [CLS] per row (P must be 1).  At every
- *            step the decoder sees prefix + the tokens generated so far at positions 0 .. P-1+t, without a padding mask; a [SEP] in the
- *            prefix is read as [PAD] (models/visual_dialog_decoder.py:57).  n-gram keys may reach into the prefix.  Beam hypotheses
- *            count the prefix in their length (HF beam_search input_ids.shape[-1]).  The caller's tensor is not modified.
- *   P - 1 + max_new_tokens must not exceed 64 (cached positions of the decode kernels) nor max_position_embeddings.
- *   out_ids holds the new tokens only, as in gstvd_generate. */
-int gstvd_generate_prefixed(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, const int64_t* prefix, int P,
-                            const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
-                            int64_t* out_ids, float* out_scores, void* stream);
-
-/* gstvd_generate_prefixed returning N sequences per image (HF num_return_sequences); gstvd_generate_prefixed is this call with N = 1.
- *   out_ids    : int64 [B*N, max_new_tokens], image-major (row b*N + n), PAD(0) after the first [SEP]
- *   out_scores : fp32 [B*N] (may be NULL; beam mode only)
+ *   out_ids    : int64 [B*N, max_new_tokens], image-major (row b*N + n): the new tokens only, PAD(0) after the first [SEP]
+ *   out_scores : fp32 [B*N] (may be NULL; beam modes only) - hypothesis score (sum log-prob / length)
+ *
+ * Return sequences (HF num_return_sequences):
  *   beam mode, 1 <= N <= num_beams: the N best finished hypotheses of BeamSearchScorer.finalize (transformers 4.16.2) in its pop order -
  *     score descending, the later-inserted hypothesis first among equal scores; contract in oracle/beam_nbest.py.  Decoding is the same
  *     as with N = 1; only the finalisation differs.
@@ -173,25 +168,22 @@ int gstvd_generate_prefixed(gstvd_ctx* ctx, int B, const gstvd_gen_params* param
  *     K/V, decoder prefix and n-gram history.  Candidate n of image b draws exactly what an N = 1 call with seed
  *     candidate_seed(seed, n) draws for image b (the RNG row stays row_offset + b); candidate_seed(seed, 0) = seed and, for n >= 1,
  *     splitmix64(seed ^ splitmix64(n * 0xD1B54A32D192ED03)) (splitmix64 as in the sampler).  No scores are written.
- *   Other N are rejected with GSTVD_ERR_INVALID. */
-int gstvd_generate_candidates(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, int N, const int64_t* prefix, int P,
-                              const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
-                              int64_t* out_ids, float* out_scores, void* stream);
-
-/* gstvd_generate_candidates with diverse beam search (HF num_beam_groups / diversity_penalty; transformers 4.16.2 group_beam_search with
- * HammingDiversityLogitsProcessor; Vijayakumar et al., "Diverse Beam Search").  gstvd_generate_candidates is this call with
- * num_beam_groups = 1, diversity_penalty = 0.  Contract (CPU oracle: oracle/beam_groups.py):
- *   The K beams form G = num_beam_groups groups of gs = K / G consecutive beams; beam k of an image starts with score 0 if
- *   k % gs == 0, else -1e9.  Every step runs one decoder pass over all K rows; logZ is per row.  Within a step the groups run in order:
- *   the candidate (beam k of group g, token w) scores fp32(fp32(fp32(x - logZ) - fp32(diversity_penalty * c_w)) + beam_score_k), with
- *   c_w = the number of new beams of groups 0..g-1 of the same image that took w at this step (an [SEP] that closed a hypothesis does
- *   not count).  n-gram-banned tokens are -inf and stay -inf.  Each group takes the top 2*gs of its gs*V candidates by (score desc,
+ *   Other N are rejected with GSTVD_ERR_INVALID.
+ *
+ * Beam groups, diverse beam search (HF num_beam_groups / diversity_penalty; transformers 4.16.2 group_beam_search with
+ * HammingDiversityLogitsProcessor; Vijayakumar et al., "Diverse Beam Search"; CPU oracle: oracle/beam_groups.py):
+ *   The K beams form G groups of gs = K / G consecutive beams; beam k of an image starts with score 0 if k % gs == 0, else -1e9.
+ *   Every step runs one decoder pass over all K rows; logZ is per row.  Within a step the groups run in order: the candidate (beam k
+ *   of group g, token w) scores fp32(fp32(fp32(x - logZ) - fp32(diversity_penalty * c_w)) + beam_score_k), with c_w = the number of
+ *   new beams of groups 0..g-1 of the same image that took w at this step (an [SEP] that closed a hypothesis does not count).
+ *   n-gram-banned tokens are -inf and stay -inf.  Each group takes the top 2*gs of its gs*V candidates by (score desc,
  *   (k - g*gs)*V + w asc) and runs BeamSearchScorer.process with group_size = gs: [SEP] is added to the hypotheses only at rank < gs,
  *   the group gets gs new beams whose parents stay inside the group.  All groups share the image's hypothesis heap of capacity K; its
  *   done flag is tested before every group (a group of a done image is padded) and updated after every group with
- *   is_done(best of the group's 2*gs candidates, P + t).  Finalisation and the N-best order are those of gstvd_generate_candidates.
- *   With G = 1 the call is gstvd_generate_candidates, launch for launch.
- *   Rejected with GSTVD_ERR_INVALID: num_beam_groups < 1, num_beams % num_beam_groups != 0, num_beam_groups > 1 in sample mode,
+ *   is_done(best of the group's 2*gs candidates, P + t).  Finalisation and the N-best order are those of beam mode above.
+ *   With G = 1 the call is plain beam search, launch for launch, whatever diversity_penalty holds: the penalty only acts on groups
+ *   after the first.
+ *   Rejected with GSTVD_ERR_INVALID: num_beam_groups < 1, num_beams % num_beam_groups != 0, num_beam_groups > 1 outside beam mode,
  *   diversity_penalty negative or not finite.
  *
  * Beam sampling, mode GSTVD_SELECT_BEAM_SAMPLE (transformers 4.16.2 beam_sample + BeamSearchScorer, length_penalty 1, early_stopping
@@ -213,42 +205,21 @@ int gstvd_generate_candidates(gstvd_ctx* ctx, int B, const gstvd_gen_params* par
  *      hypothesis only at rank < K, a hypothesis scores its warped sum / (P + t), is_done uses the best drawn w.
  *   Rejected with GSTVD_ERR_INVALID: num_beams < 2 or > 8, N < 1, N*num_beams > max_beams, num_beam_groups > 1, a temperature that is
  *   not finite and > 0, top_p outside [0, 1].  Rejected with GSTVD_ERR_UNSUPPORTED: top_k = 0 or top_k > 16. */
-int gstvd_generate_groups(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, int num_beam_groups, float diversity_penalty, int N,
-                          const int64_t* prefix, int P, const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
-                          int64_t* out_ids, float* out_scores, void* stream);
+int gstvd_generate(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, const int64_t* prefix, int P,
+                   const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
+                   int64_t* out_ids, float* out_scores, void* stream);
 
 /* One whole forward call of the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:24-120): the same work and
- * results as gstvd_encode (no exported outputs) + gstvd_prefill_cross(resident states) + gstvd_generate, replayed from ONE CUDA graph
- * per shape - the host enqueues a few device-to-device copies of the inputs and one graph launch.  The n-gram blocking history is the
- * call's own input_ids / token_type_ids.  Afterwards the encoder / cross-K/V state is resident exactly as after the three calls (e.g.
- * for the perplexity pass, gstvd_score). */
+ * results as gstvd_encode (no exported outputs) + gstvd_prefill_cross(resident states) + gstvd_generate with the same params and
+ * prefix, replayed from ONE CUDA graph per shape - the host enqueues a few device-to-device copies of the inputs and one graph launch.
+ * params, prefix, P, out_ids and out_scores follow the contract of gstvd_generate.  The n-gram blocking history is the call's own
+ * input_ids / token_type_ids.  Afterwards the encoder / cross-K/V state is resident exactly as after the three calls (e.g. for the
+ * perplexity pass, gstvd_score). */
 int gstvd_round(gstvd_ctx* ctx, int B, int Lt, int Lv,
                 const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
                 const float* image_feat, const float* image_loc, const float* image_mask,
-                const gstvd_gen_params* params, int64_t* out_ids, float* out_scores, void* stream);
-
-/* gstvd_round continuing from a decoder prefix [B, P] (NULL, P = 1: the [CLS] start); the prefix contract of gstvd_generate_prefixed. */
-int gstvd_round_prefixed(gstvd_ctx* ctx, int B, int Lt, int Lv,
-                         const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
-                         const float* image_feat, const float* image_loc, const float* image_mask,
-                         const gstvd_gen_params* params, const int64_t* prefix, int P,
-                         int64_t* out_ids, float* out_scores, void* stream);
-
-/* gstvd_round_prefixed returning N sequences per image: the contract of gstvd_generate_candidates (out_ids [B*N, max_new_tokens],
- * out_scores [B*N]); gstvd_round_prefixed is this call with N = 1. */
-int gstvd_round_candidates(gstvd_ctx* ctx, int B, int Lt, int Lv,
-                           const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
-                           const float* image_feat, const float* image_loc, const float* image_mask,
-                           const gstvd_gen_params* params, int N, const int64_t* prefix, int P,
-                           int64_t* out_ids, float* out_scores, void* stream);
-
-/* gstvd_round_candidates with beam groups and a diversity penalty: the contract of gstvd_generate_groups; gstvd_round_candidates is this
- * call with num_beam_groups = 1, diversity_penalty = 0. */
-int gstvd_round_groups(gstvd_ctx* ctx, int B, int Lt, int Lv,
-                       const int64_t* input_ids, const int64_t* token_type_ids, const float* attention_mask,
-                       const float* image_feat, const float* image_loc, const float* image_mask,
-                       const gstvd_gen_params* params, int num_beam_groups, float diversity_penalty, int N,
-                       const int64_t* prefix, int P, int64_t* out_ids, float* out_scores, void* stream);
+                const gstvd_gen_params* params, const int64_t* prefix, int P,
+                int64_t* out_ids, float* out_scores, void* stream);
 
 /* Replaces VisualDialogDecoder.forward in loss mode (models/visual_dialog_decoder.py:33-86) as driven by
  * generate.py:183-209 and evaluate_gen.py:94-106: teacher-forced pass over dec_ids [B, L].

@@ -32,13 +32,16 @@ def test_header_symbols_exported():
 def test_config_struct_matches_header_field_order():
     L = _lib()
     header = open(os.path.join(ROOT, "include", "gstvd.h")).read()
-    body = header[header.index("typedef struct {", header.index("Model geometry")):header.index("} gstvd_config;")]
-    body = re.sub(r"/\*.*?\*/", "", body, flags=re.S)
-    names = []
-    for decl in re.findall(r"int32_t\s+([^;]+);", body):
-        for part in decl.split(","):
-            names.append(re.sub(r"\[.*\]", "", part).strip())
-    assert names == [f[0] for f in L.GstvdConfig._fields_]
+    c_types = {"int32_t": ctypes.c_int32, "uint64_t": ctypes.c_uint64, "int64_t": ctypes.c_int64, "float": ctypes.c_float}
+    for name, struct in (("gstvd_config", L.GstvdConfig), ("gstvd_gen_params", L.GstvdGenParams)):
+        end = header.index("} %s;" % name)
+        body = re.sub(r"/\*.*?\*/", "", header[header.rindex("typedef struct {", 0, end):end], flags=re.S)
+        fields = []
+        for c_type, decl in re.findall(r"\b(u?int(?:32|64)_t|float)\s+([^;]+);", body):
+            for part in decl.split(","):
+                fields.append((re.sub(r"\[.*\]", "", part).strip(), c_types[c_type]))
+        bound = [(f, t._type_ if issubclass(t, ctypes.Array) else t) for f, t in struct._fields_]
+        assert fields == bound, name
 
 
 def test_create_fails_loudly_without_gpu():

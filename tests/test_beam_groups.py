@@ -1,16 +1,15 @@
-"""Diverse beam search: beam groups with a Hamming diversity penalty (num_beam_groups / diversity_penalty; include/gstvd.h
-gstvd_generate_groups, contract in oracle/beam_groups.py).
+"""Diverse beam search: beam groups with a Hamming diversity penalty (include/gstvd.h gstvd_generate, params.num_beam_groups /
+params.diversity_penalty; contract in oracle/beam_groups.py).
 
 CPU: the group oracle with one group is the plain / blocked / prefixed beam oracle for any penalty; with G = K and no penalty every
 group is greedy; with a large penalty and groups of one beam the groups take pairwise distinct tokens; an image that group 0 finishes
 mid-step adds nothing from the later groups; the four CLI flags.
 GPU: ids identical to the oracle (scores within 1e-4) in fp32 on every call path, with and without blocking and a decoder prefix, at
 tiny and full size; G = K without penalty returns K copies of the greedy sample; the bf16 product path agrees across call paths, G = 1
-through the groups entry point is the candidates call launch for launch, and the penalty separates the beams of every image; the
+gives the same ids, scores and launch count with and without a penalty, and the penalty separates the beams of every image; the
 dialog loop and generate.py run with groups; every rejected argument raises.
 """
 import copy
-import ctypes
 import os
 
 import pytest
@@ -284,7 +283,6 @@ def test_fp32_groups_without_penalty_are_greedy(tiny_cfgs, tiny_sd):
 @pytest.mark.gpu
 def test_full_bf16_group_beams(full_cfgs, full_sd):
     from gst_visdial_b200 import _lib, weights as W
-    from gst_visdial_b200._lib import GstvdGenParams
     from test_gpu_model import _build_model, _call
     enc_cfg, dec_cfg = full_cfgs
     B, K = 64, 6
@@ -305,23 +303,13 @@ def test_full_bf16_group_beams(full_cfgs, full_sd):
 
     e = _engine(enc_cfg, dec_cfg, full_sd, "bf16", b)
     try:
-        # G = 1 through the groups entry point is the candidates call, launch for launch and bit for bit
-        gp = GstvdGenParams()
-        gp.mode, gp.num_beams, gp.max_new_tokens, gp.top_k, gp.temperature = _lib.GSTVD_SELECT_BEAM, K, 18, 1, 1.0
-        gp.ngram_blocking_size = 4
-        hid, hseg = b["enc_input_ids"].cuda(), b["enc_segments"].cuda()
+        # one group pays nothing for the groups machinery: the penalty only acts on groups after the first, so with G = 1 it
+        # changes no id, no score and no launch
         res = []
-        for call in ("candidates", "groups"):
-            out = torch.empty(B * K, 18, dtype=torch.int64, device="cuda:0")
-            sc = torch.empty(B * K, dtype=torch.float32, device="cuda:0")
-            args = (ctypes.c_void_p(hid.data_ptr()), ctypes.c_void_p(hseg.data_ptr()), hid.shape[1], ctypes.c_void_p(out.data_ptr()),
-                    ctypes.c_void_p(sc.data_ptr()), e._stream())
+        for penalty in (0.0, 0.7):
             l0 = e.launch_count
-            if call == "candidates":
-                rc = e.lib.gstvd_generate_candidates(e.ctx, B, ctypes.byref(gp), K, None, 1, *args)
-            else:
-                rc = e.lib.gstvd_generate_groups(e.ctx, B, ctypes.byref(gp), 1, 0.0, K, None, 1, *args)
-            _lib.check(e.ctx, rc)
+            out, sc = e.generate(B, num_beams=K, num_beam_groups=1, diversity_penalty=penalty, num_return_sequences=K, ngram_blocking_size=4,
+                                 want_scores=True, **_hist(b))
             res.append((out.cpu(), sc.cpu(), e.launch_count - l0))
         assert torch.equal(res[0][0], res[1][0]) and torch.equal(res[0][1], res[1][1]) and res[0][2] == res[1][2], (res[0][2], res[1][2])
         grouped = e.generate(B, num_beams=K, num_beam_groups=3, diversity_penalty=0.5, num_return_sequences=K, ngram_blocking_size=4,

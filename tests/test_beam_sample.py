@@ -454,17 +454,18 @@ def test_beam_sample_rejections(tiny_cfgs, tiny_sd):
         # num_beams < 2 in beam-sampling mode: Engine maps num_beams = 1 to the sampler, so call the C ABI with mode 2 directly
         gp = _lib.GstvdGenParams()
         gp.mode, gp.num_beams, gp.max_new_tokens, gp.top_k, gp.temperature = _lib.GSTVD_SELECT_BEAM_SAMPLE, 1, 18, 7, 0.7
+        gp.num_return_sequences = gp.num_beam_groups = 1
         out = torch.empty(B, 18, dtype=torch.int64, device="cuda:0")
         for call in ("generate", "round"):
             if call == "generate":
-                rc = e.lib.gstvd_generate_groups(e.ctx, B, ctypes.byref(gp), 1, 0.0, 1, None, 1, None, None, 0,
-                                                 ctypes.c_void_p(out.data_ptr()), None, e._stream())
+                rc = e.lib.gstvd_generate(e.ctx, B, ctypes.byref(gp), None, 1, None, None, 0, ctypes.c_void_p(out.data_ptr()), None,
+                                          e._stream())
             else:
                 ids, seg = (t.cuda().long().contiguous() for t in (rnd[0], rnd[3]))
                 feat, loc, att, imask = (t.cuda().float().contiguous() for t in (rnd[1], rnd[2], rnd[4], rnd[5]))
-                rc = e.lib.gstvd_round_groups(e.ctx, B, ids.shape[1], feat.shape[1], *[ctypes.c_void_p(t.data_ptr()) for t in
-                                              (ids, seg, att, feat, loc, imask)], ctypes.byref(gp), 1, 0.0, 1, None, 1,
-                                              ctypes.c_void_p(out.data_ptr()), None, e._stream())
+                rc = e.lib.gstvd_round(e.ctx, B, ids.shape[1], feat.shape[1], *[ctypes.c_void_p(t.data_ptr()) for t in
+                                       (ids, seg, att, feat, loc, imask)], ctypes.byref(gp), None, 1,
+                                       ctypes.c_void_p(out.data_ptr()), None, e._stream())
             assert rc == INVALID, (call, rc)
         assert e.generate(B, num_return_sequences=2, **dict(ok, num_beams=4)).shape == (B * 2, 18)
         assert e.generate(B, num_beams=2, do_sample=True, **dict(_WARP, top_k=1, top_p=1.0)).shape == (B, 18)

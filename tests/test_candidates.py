@@ -1,4 +1,4 @@
-"""Several sequences per image from one encoder pass (num_return_sequences; include/gstvd.h gstvd_generate_candidates).
+"""Several sequences per image from one encoder pass (include/gstvd.h gstvd_generate, params.num_return_sequences).
 
 CPU: the N-best oracle (oracle/beam_nbest.py) is the plain finalize at N = 1 for all three beam states and returns equal-score
 hypotheses in HF pop order; candidate_seed; the -answer_candidates flag.

@@ -1,12 +1,12 @@
-"""Decoding from a caller-supplied decoder prefix (dec_input_ids [B, P]; include/gstvd.h gstvd_generate_prefixed).
+"""Decoding from a caller-supplied decoder prefix (dec_input_ids [B, P]; include/gstvd.h gstvd_generate, its prefix / P arguments).
 
 The beam contract with a prefix is defined here (``PrefixBeamState``, ``prefix_beam_search``) on top of oracle/beam.py and
 oracle/beam_ngram.py, which define it for the [CLS] start.
 CPU: that oracle reduces to oracle/beam.py / oracle/beam_ngram.py for the [CLS] start, never selects a banned (beam, token) pair when
 the n-gram key reaches into the prefix, and the restatement continues its own greedy output from a prefix of it.
 GPU: greedy ids identical to the restatement in fp32 (tiny and full size, P up to 25 = 42 cached positions), beam ids and scores
-identical to the prefix oracle in fp32 on every call path, the bf16 product path agrees across call paths and with P = 1 through
-the old entry point, and every rejected argument raises.
+identical to the prefix oracle in fp32 on every call path, the bf16 product path agrees across call paths and an explicit [CLS]
+prefix (P = 1) matches the implicit [CLS] start, and every rejected argument raises.
 """
 import copy
 import ctypes
@@ -384,7 +384,7 @@ def test_full_bf16_prefix_paths_agree(full_cfgs, full_sd):
             new = e.generate(B, prefix=cls, **kw)
             l2 = e.launch_count
             old, new = (old, new) if isinstance(old, tuple) else ((old,), (new,))
-            assert all(torch.equal(x, y) for x, y in zip(old, new)), "P = 1 through the prefixed entry point differs"
+            assert all(torch.equal(x, y) for x, y in zip(old, new)), "an explicit [CLS] prefix differs from the implicit [CLS] start"
             assert l1 - l0 == l2 - l1
         g = e.generate(B, num_beams=1, **_GREEDY).cpu()
         j = 8
@@ -416,9 +416,9 @@ def test_prefix_rejections(tiny_cfgs, tiny_sd):
         e.generate(B, prefix=torch.full((B, 47), R.CLS))                              # 64: accepted
         gp = _lib.GstvdGenParams()
         gp.mode, gp.num_beams, gp.max_new_tokens, gp.top_k, gp.temperature = _lib.GSTVD_SELECT_SAMPLE, 1, 18, 1, 1.0
+        gp.num_return_sequences = gp.num_beam_groups = 1
         out = torch.empty(B, 18, dtype=torch.int64, device="cuda:0")
-        rc = e.lib.gstvd_generate_prefixed(e.ctx, B, ctypes.byref(gp), None, 3, None, None, 0, ctypes.c_void_p(out.data_ptr()), None,
-                                           e._stream())
+        rc = e.lib.gstvd_generate(e.ctx, B, ctypes.byref(gp), None, 3, None, None, 0, ctypes.c_void_p(out.data_ptr()), None, e._stream())
         with pytest.raises(GstvdError):
             _lib.check(e.ctx, rc)                                                     # NULL prefix with P > 1
         with pytest.raises(GstvdError):
