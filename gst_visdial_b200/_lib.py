@@ -77,6 +77,9 @@ SYMBOLS = [
     ("gstvd_op_add_layernorm", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     ("gstvd_op_attention", c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, c_float, c_int, _P, _P]),
     ("gstvd_op_deferred_ln_chain", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
+    ("gstvd_op_dec_self_attn", c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
+    ("gstvd_op_dec_cross_attn", c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, _P, _P, _P]),
+    ("gstvd_op_anc_update", c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P]),
     ("gstvd_debug_self_cache", c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     ("gstvd_op_beam_begin", c_int, [_P, c_int, c_int, c_int, _P]),
     ("gstvd_op_beam_step", c_int, [_P, _P, c_int64, _P, _P, _P, _P]),

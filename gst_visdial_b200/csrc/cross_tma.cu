@@ -476,17 +476,23 @@ void dec_cross_print_times() {
   }
 }
 
+bool dec_cross_tma_fits(int dtype, const DecodeGeom& g) {
+  return dtype == kBF16 && g.D == 64 && g.K <= 8 && g.Le <= kXtLeP && g.H == g.heads * 64;
+}
+
 bool dec_cross_tma_supported(int dtype, const DecodeGeom& g) {
   static const bool off = getenv("GSTVD_CROSS_NO_TMA") != nullptr;
-  return !off && dtype == kBF16 && g.D == 64 && g.K <= 8 && g.Le <= kXtLeP && g.H == g.heads * 64;
+  return !off && dec_cross_tma_fits(dtype, g);
 }
 
 int launch_dec_cross_tma(const DecodeGeom& g, int layer, const void* q, const void* cross_cache, const float* enc_mask,
-                         const int* cross_len, void* out, int num_sms, cudaStream_t stream) {
+                         const int* cross_len, void* out, int num_sms, cudaStream_t stream, int force) {
+  if (force != kDecDefault && force != kCrossWarpTma && force != kCrossCtaTma) throw std::runtime_error("dec_cross_tma: not a TMA kernel");
+  if (!dec_cross_tma_fits(kBF16, g)) throw std::runtime_error("dec_cross_tma: needs head_dim 64, at most 8 beams and 304 keys");
   // GSTVD_CROSS_TMA=2: the CTA-per-item kernel; anything else / unset: one warp per item.  Read at every launch (a captured graph keeps
-  // what it was captured with), so that a test can compare the two in one process.
+  // what it was captured with), so that a test can compare the two in one process.  A forced kernel ignores the variable.
   const char* venv = getenv("GSTVD_CROSS_TMA");
-  const int variant = (venv && atoi(venv) == 2) ? 2 : 4;
+  const int variant = force == kCrossCtaTma ? 2 : force == kCrossWarpTma ? 4 : (venv && atoi(venv) == 2) ? 2 : 4;
   using Cfg2 = X2Cfg<8, 1, 3>;
   static bool configured = false;
   if (!configured) {

@@ -695,12 +695,36 @@ static void launch_self_generic(int dtype, const DecodeGeom& g, dim3 grid, int l
   }
 }
 
+static bool self_v2_fits(int dtype, const DecodeGeom& g, const void* qkv, const void* self_cache, const void* out) {
+  return dtype == kBF16 && g.D == 64 && g.H % 8 == 0 && g.T <= kMaxPos && g.K <= kMaxBeams &&
+         (reinterpret_cast<uintptr_t>(qkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(self_cache) & 15) == 0 &&
+         (reinterpret_cast<uintptr_t>(out) & 15) == 0;
+}
+
 bool dec_self_attn_v2_active(int dtype, const DecodeGeom& g, const void* qkv, const void* self_cache, const void* out) {
   const char* v2_env = getenv("GSTVD_SELF_V2");            // read per call (captured graphs keep what was set at capture time)
   const bool v2 = v2_env == nullptr || atoi(v2_env) != 0;  // default on; GSTVD_SELF_V2=0 selects the first kernel
-  return v2 && dtype == kBF16 && g.D == 64 && g.H % 8 == 0 && g.T <= kMaxPos && g.K <= kMaxBeams &&
-         (reinterpret_cast<uintptr_t>(qkv) & 15) == 0 && (reinterpret_cast<uintptr_t>(self_cache) & 15) == 0 &&
-         (reinterpret_cast<uintptr_t>(out) & 15) == 0;
+  return v2 && self_v2_fits(dtype, g, qkv, self_cache, out);
+}
+
+bool dec_self_attn_supports(int kernel, int dtype, const DecodeGeom& g, const void* qkv, const void* self_cache, const void* out,
+                            const uint8_t* anc) {
+  if (g.T > kMaxPos || g.H != g.heads * g.D) return false;
+  if (kernel == kSelfV2) return self_v2_fits(dtype, g, qkv, self_cache, out);
+  if (kernel == kSelfFirst) return anc == nullptr && (g.D == 64 || g.D == 128);
+  return false;
+}
+
+bool dec_cross_supports(int kernel, int dtype, const DecodeGeom& g) {
+  if (g.H != g.heads * g.D) return false;
+  switch (kernel) {
+    case kCrossWarpTma: case kCrossCtaTma: return dec_cross_tma_fits(dtype, g);
+    case kCrossMma: return dtype == kBF16 && g.D == 64 && g.K <= 8 && g.Le <= 4 * kXMaxTiles * 8;
+    // 512 = the encoder length limit of a context: the shared score tile of 8 rows x 1024 keys would not fit 48 KB
+    case kCrossSimt: return g.D == 64 && g.K <= 8 && g.Le <= 512;
+    case kCrossGeneric: return g.D <= 128 && g.D % 8 == 0 && g.Le <= 512;
+    default: return false;
+  }
 }
 
 int launch_anc_update(const DecodeGeom& g, const int32_t* beam_idx, const int* d_step, uint8_t* anc, cudaStream_t stream) {
@@ -721,12 +745,14 @@ int launch_prefix_kv_store(int dtype, const DecodeGeom& g, int layer, const void
 }
 
 int launch_dec_self_attn(int dtype, const DecodeGeom& g, int layer, const void* qkv, void* self_cache, const int* d_step, int step_host,
-                         const uint8_t* anc, void* out, cudaStream_t stream) {
+                         const uint8_t* anc, void* out, cudaStream_t stream, int force) {
   if (g.D != 64 && g.D != 128) throw std::runtime_error("dec_self_attn: head_dim must be 64 or 128");
   if (g.T > kMaxPos) throw std::runtime_error("dec_self_attn: at most 64 cached positions");
+  if (force != kDecDefault && !dec_self_attn_supports(force, dtype, g, qkv, self_cache, out, anc))
+    throw std::runtime_error("dec_self_attn: the forced kernel does not support these arguments");
   dim3 grid(g.B * g.K, (g.heads + 3) / 4);
   // lean variant: bf16, 64-dim heads, 16-byte aligned rows
-  if (dec_self_attn_v2_active(dtype, g, qkv, self_cache, out)) {
+  if (force == kDecDefault ? dec_self_attn_v2_active(dtype, g, qkv, self_cache, out) : force == kSelfV2) {
     if (g.T <= 20) launch_k(dec_self_attn_v2_kernel<5>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, step_host, anc, (bf16*)out);
     else if (g.T <= kMaxSteps) launch_k(dec_self_attn_v2_kernel<8>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, step_host, anc, (bf16*)out);
     else launch_k(dec_self_attn_v2_kernel<16>, grid, dim3(128), 0, stream, g, layer, (const bf16*)qkv, (bf16*)self_cache, d_step, step_host, anc, (bf16*)out);
@@ -739,17 +765,22 @@ int launch_dec_self_attn(int dtype, const DecodeGeom& g, int layer, const void* 
 }
 
 int launch_dec_cross_attn(int dtype, const DecodeGeom& g, int layer, const void* q, const void* cross_cache,
-                          const float* enc_mask, void* out, cudaStream_t stream) {
+                          const float* enc_mask, void* out, cudaStream_t stream, int force) {
+  if (force != kDecDefault && (force < kCrossMma || !dec_cross_supports(force, dtype, g)))
+    throw std::runtime_error("dec_cross_attn: the forced kernel does not support this geometry");
   const int64_t esz = dtype == kF32 ? 4 : 2;
   const int64_t per_image = (int64_t)2 * g.heads * g.Le * g.D;
   const char* kbase = (const char*)cross_cache + ((int64_t)layer * g.B) * per_image * esz;
-  if (dtype == kBF16 && g.D == 64 && g.K <= 8 && g.Le <= 4 * kXMaxTiles * 8 && getenv("GSTVD_CROSS_SIMT") == nullptr) {
+  const bool mma = force == kDecDefault
+                       ? dtype == kBF16 && g.D == 64 && g.K <= 8 && g.Le <= 4 * kXMaxTiles * 8 && getenv("GSTVD_CROSS_SIMT") == nullptr
+                       : force == kCrossMma;
+  if (mma) {
     const int LeP = (g.Le + 15) & ~15;
     const size_t smem = (size_t)(8 * LeP + LeP + 4 * 8 * 64) * sizeof(float) + (size_t)8 * LeP * sizeof(bf16);
     launch_k(dec_cross_mma_kernel, dim3(g.heads, g.B), dim3(128), smem, stream, g, (const bf16*)q, (const bf16*)kbase, enc_mask, (bf16*)out);
     return 1;
   }
-  if (g.D == 64 && g.K <= 8 && g.Le <= 1024) {
+  if (force == kDecDefault ? g.D == 64 && g.K <= 8 && g.Le <= 1024 : force == kCrossSimt) {
     if (dtype == kF32) launch_cross_t<float>(g, q, kbase, enc_mask, out, stream);
     else launch_cross_t<bf16>(g, q, kbase, enc_mask, out, stream);
     return 1;

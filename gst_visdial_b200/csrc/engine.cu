@@ -717,15 +717,15 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
       // q|k|v from LN_out(x3 of the layer below) (layer 0: from the embedding output, already normalised)
       if (l == 0) X.gemm(c->dh.p, H, L.qkv, c->dqkv.p, 3 * H, M);
       else X.gemm_ln(x3, H, L.qkv, &L.qkv_f, st3, c->dqkv.p, M, 0, nullptr, nullptr, nullptr, nullptr);
-      c->launches += launch_dec_self_attn(c->dtype, g, l, c->dqkv.p, c->self_cache.p, d_step, step_host, anc, c->dctx.p, s);
+      c->launches += launch_dec_self_attn(c->dtype, g, l, c->dqkv.p, c->self_cache.p, d_step, step_host, anc, c->dctx.p, s, kDecDefault);
       // x1 = o(ctx) + input
       X.gemm_ln(c->dctx.p, H, L.o, nullptr, nullptr, x1, M, 0, l == 0 ? c->dh.p : x3, ln_below, st3, st1);
       X.gemm_ln(x1, H, L.cq, &L.cq_f, st1, c->dqc.p, M, 0, nullptr, nullptr, nullptr, nullptr);
       if (dec_cross_tma_supported(c->dtype, g))
         c->launches += launch_dec_cross_tma(g, l, c->dqc.p, c->cross_cache.p, (const float*)c->fused_mask.p, (const int*)c->cross_len.p, c->dctx.p,
-                                            c->num_sms, s);
+                                            c->num_sms, s, kDecDefault);
       else
-        c->launches += launch_dec_cross_attn(c->dtype, g, l, c->dqc.p, c->cross_cache.p, (const float*)c->fused_mask.p, c->dctx.p, s);
+        c->launches += launch_dec_cross_attn(c->dtype, g, l, c->dqc.p, c->cross_cache.p, (const float*)c->fused_mask.p, c->dctx.p, s, kDecDefault);
       // x2 = co(ctx) + LN_att(x1);  ffn = gelu(f1(LN_cross(x2)));  x3 = f2(ffn) + LN_cross(x2)
       X.gemm_ln(c->dctx.p, H, L.co, nullptr, nullptr, x2, M, 0, x1, &L.ln_att, st1, st2);
       X.gemm_ln(x2, H, L.f1, &L.f1_f, st2, c->dffn.p, M, 1, nullptr, nullptr, nullptr, nullptr);
@@ -737,14 +737,14 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   for (int l = 0; l < c->dec_layers; ++l) {
     const DecLayer& L = c->d_layers[l];
     X.gemm(c->dh.p, H, L.qkv, c->dqkv.p, 3 * H, M);
-    c->launches += launch_dec_self_attn(c->dtype, g, l, c->dqkv.p, c->self_cache.p, d_step, step_host, anc, c->dctx.p, s);
+    c->launches += launch_dec_self_attn(c->dtype, g, l, c->dqkv.p, c->self_cache.p, d_step, step_host, anc, c->dctx.p, s, kDecDefault);
     X.gemm_add_ln(c->dctx.p, H, L.o, c->dh.p, L.ln_att, c->dtmp.p, c->da.p, M);
     X.gemm(c->da.p, H, L.cq, c->dqc.p, H, M);
     if (dec_cross_tma_supported(c->dtype, g))
       c->launches += launch_dec_cross_tma(g, l, c->dqc.p, c->cross_cache.p, (const float*)c->fused_mask.p, (const int*)c->cross_len.p, c->dctx.p,
-                                          c->num_sms, s);
+                                          c->num_sms, s, kDecDefault);
     else
-      c->launches += launch_dec_cross_attn(c->dtype, g, l, c->dqc.p, c->cross_cache.p, (const float*)c->fused_mask.p, c->dctx.p, s);
+      c->launches += launch_dec_cross_attn(c->dtype, g, l, c->dqc.p, c->cross_cache.p, (const float*)c->fused_mask.p, c->dctx.p, s, kDecDefault);
     X.gemm_add_ln(c->dctx.p, H, L.co, c->da.p, L.ln_cross, c->dtmp.p, c->db.p, M);
     X.gemm(c->db.p, H, L.f1, c->dffn.p, c->dec_F, M, 1);
     X.gemm_add_ln(c->dffn.p, c->dec_F, L.f2, c->db.p, L.ln_out, c->dtmp.p, c->dh.p, M);
@@ -1448,6 +1448,102 @@ int gstvd_op_attention(gstvd_ctx* c, int dtype, int B, int H, int Lq, int Lk, in
       c->launches += launch_cast_to_f32(kBF16, o16, out, nq, s);
       CUDA_CHECK(cudaStreamSynchronize(s));
     }
+  });
+}
+
+// ---- decode-step attention kernels, one at a time (parity tests): own DecodeGeom with one layer, independent of the context's caches ----
+int gstvd_op_dec_self_attn(gstvd_ctx* c, int dtype, int kernel, int B, int K, int heads, int D, int T, int P0, int step, int step_known,
+                           const float* qkv, const float* prefix_qkv, float* cache, const uint8_t* anc, float* out, void* stream) {
+  if (!c) return GSTVD_ERR_INVALID;
+  return guarded(c, [&] {
+    if (dtype != kF32 && dtype != kBF16) throw InvalidArg("op_dec_self_attn: dtype");
+    if (kernel != kDecDefault && kernel != kSelfFirst && kernel != kSelfV2) throw InvalidArg("op_dec_self_attn: kernel must be -1, 0 or 1");
+    if (B < 1 || K < 1 || K > 8 || heads < 1 || (D != 64 && D != 128) || T < 1 || T > 64 || P0 < 0 || step < 0 || P0 + step >= T)
+      throw InvalidArg("op_dec_self_attn: shape out of range (K <= 8, D 64 or 128, T <= 64, P0 + step < T)");
+    if (!qkv || !cache || !out) throw InvalidArg("op_dec_self_attn: NULL buffer");
+    if (prefix_qkv && P0 < 1) throw InvalidArg("op_dec_self_attn: prefix_qkv needs P0 >= 1");
+    cudaStream_t s = (cudaStream_t)stream;
+    DecodeGeom g;
+    g.B = B; g.K = K; g.H = heads * D; g.heads = heads; g.D = D; g.layers = 1; g.T = T; g.Le = 0; g.P0 = P0;
+    const int64_t M = (int64_t)B * K, n_qkv = M * 3 * g.H, n_pre = (int64_t)B * P0 * 3 * g.H, n_cache = (int64_t)2 * B * T * K * g.H;
+    Scratch sc;
+    int* d_step = (int*)sc.get(4);
+    const void* q_c = qkv; const void* pre_c = prefix_qkv; void* cache_c = cache; void* out_c = out;
+    if (dtype == kBF16) {
+      q_c = sc.get(n_qkv * 2); cache_c = sc.get(n_cache * 2); out_c = sc.get(M * g.H * 2);
+      pre_c = prefix_qkv ? sc.get(n_pre * 2) : nullptr;
+    }
+    const bool fits = kernel == kDecDefault ? (anc == nullptr || dec_self_attn_v2_active(dtype, g, q_c, cache_c, out_c))
+                                            : dec_self_attn_supports(kernel, dtype, g, q_c, cache_c, out_c, anc);
+    if (!fits)
+      throw Unsupported(fmt("op_dec_self_attn: kernel %d does not run dtype %d, D = %d, T = %d, K = %d%s", kernel, dtype, D, T, K,
+                            anc ? " with an ancestry table" : ""));
+    if (dtype == kBF16) {
+      c->launches += launch_cast_f32_to(kBF16, qkv, (void*)q_c, n_qkv, s);
+      c->launches += launch_cast_f32_to(kBF16, cache, cache_c, n_cache, s);
+      if (prefix_qkv) c->launches += launch_cast_f32_to(kBF16, prefix_qkv, (void*)pre_c, n_pre, s);
+    }
+    CUDA_CHECK(cudaMemcpyAsync(d_step, &step, 4, cudaMemcpyHostToDevice, s));
+    if (prefix_qkv) c->launches += launch_prefix_kv_store(dtype, g, 0, pre_c, cache_c, s);
+    c->launches += launch_dec_self_attn(dtype, g, 0, q_c, cache_c, d_step, step_known ? step : -1, anc, out_c, s, kernel);
+    if (dtype == kBF16) {
+      c->launches += launch_cast_to_f32(kBF16, cache_c, cache, n_cache, s);
+      c->launches += launch_cast_to_f32(kBF16, out_c, out, M * g.H, s);
+    }
+    CUDA_CHECK(cudaStreamSynchronize(s));
+  });
+}
+
+int gstvd_op_dec_cross_attn(gstvd_ctx* c, int dtype, int kernel, int B, int K, int heads, int D, int Le, const float* q,
+                            const float* cross_kv, const float* mask, int use_cross_len, int32_t* out_cross_len, float* out, void* stream) {
+  if (!c) return GSTVD_ERR_INVALID;
+  return guarded(c, [&] {
+    if (dtype != kF32 && dtype != kBF16) throw InvalidArg("op_dec_cross_attn: dtype");
+    if (kernel < kDecDefault || kernel > kCrossGeneric) throw InvalidArg("op_dec_cross_attn: kernel must be -1 .. 4");
+    if (B < 1 || K < 1 || K > 8 || heads < 1 || D < 8 || D > 128 || D % 8 || Le < 1 || Le > 512)
+      throw InvalidArg("op_dec_cross_attn: shape out of range (K <= 8, D % 8 == 0 and <= 128, Le <= 512)");
+    if (!q || !cross_kv || !out) throw InvalidArg("op_dec_cross_attn: NULL buffer");
+    if (use_cross_len && !mask) throw InvalidArg("op_dec_cross_attn: cross_len is computed from the mask");
+    cudaStream_t s = (cudaStream_t)stream;
+    DecodeGeom g;
+    g.B = B; g.K = K; g.H = heads * D; g.heads = heads; g.D = D; g.layers = 1; g.T = 1; g.Le = Le; g.P0 = 0;
+    const bool tma = kernel == kDecDefault ? dec_cross_tma_supported(dtype, g) : (kernel == kCrossWarpTma || kernel == kCrossCtaTma);
+    if (kernel != kDecDefault && !dec_cross_supports(kernel, dtype, g))
+      throw Unsupported(fmt("op_dec_cross_attn: kernel %d does not run dtype %d, D = %d, K = %d, Le = %d", kernel, dtype, D, K, Le));
+    const int64_t nq = (int64_t)B * K * g.H, nkv = (int64_t)B * 2 * heads * Le * D;
+    Scratch sc;
+    int* cross_len = use_cross_len ? (int*)sc.get((size_t)B * 4) : nullptr;
+    const void* q_c = q; const void* kv_c = cross_kv; void* out_c = out;
+    if (dtype == kBF16) {
+      q_c = sc.get(nq * 2); kv_c = sc.get(nkv * 2); out_c = sc.get(nq * 2);
+      c->launches += launch_cast_f32_to(kBF16, q, (void*)q_c, nq, s);
+      c->launches += launch_cast_f32_to(kBF16, cross_kv, (void*)kv_c, nkv, s);
+    }
+    if (cross_len) {
+      c->launches += launch_cross_len(B, Le, mask, cross_len, s);
+      if (out_cross_len) CUDA_CHECK(cudaMemcpyAsync(out_cross_len, cross_len, (size_t)B * 4, cudaMemcpyDeviceToDevice, s));
+    }
+    if (tma) c->launches += launch_dec_cross_tma(g, 0, q_c, kv_c, mask, cross_len, out_c, c->num_sms, s, kernel);
+    else c->launches += launch_dec_cross_attn(dtype, g, 0, q_c, kv_c, mask, out_c, s, kernel);
+    if (dtype == kBF16) c->launches += launch_cast_to_f32(kBF16, out_c, out, nq, s);
+    CUDA_CHECK(cudaStreamSynchronize(s));
+  });
+}
+
+int gstvd_op_anc_update(gstvd_ctx* c, int B, int K, int T, int P0, int step, const int32_t* beam_idx, uint8_t* anc, void* stream) {
+  if (!c) return GSTVD_ERR_INVALID;
+  return guarded(c, [&] {
+    if (B < 1 || K < 1 || K > 8 || T < 1 || T > 64 || P0 < 0 || step < 0 || P0 + step >= T)
+      throw InvalidArg("op_anc_update: shape out of range (K <= 8, T <= 64, P0 + step < T)");
+    if (!beam_idx || !anc) throw InvalidArg("op_anc_update: NULL buffer");
+    cudaStream_t s = (cudaStream_t)stream;
+    DecodeGeom g;
+    g.B = B; g.K = K; g.H = 0; g.heads = 0; g.D = 0; g.layers = 1; g.T = T; g.Le = 0; g.P0 = P0;
+    Scratch sc;
+    int* d_step = (int*)sc.get(4);
+    CUDA_CHECK(cudaMemcpyAsync(d_step, &step, 4, cudaMemcpyHostToDevice, s));
+    c->launches += launch_anc_update(g, beam_idx, d_step, anc, s);
+    CUDA_CHECK(cudaStreamSynchronize(s));
   });
 }
 

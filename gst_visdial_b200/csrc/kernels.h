@@ -131,13 +131,23 @@ struct DecodeGeom {
   int Le;                             // encoder length (cross keys)
   int P0 = 0;                         // decoder prefix length - 1: cache positions 0..P0-1 hold the prefix (launch_prefix_kv_store)
 };
+// Forced kernel choices of the decode attention launchers (`force` argument; kDecDefault keeps the launcher's own choice,
+// environment switches included).  The single-kernel test entries use them; the decode step always passes kDecDefault.
+constexpr int kDecDefault = -1;
+enum SelfAttnKernel { kSelfFirst = 0, kSelfV2 = 1 };
+enum CrossAttnKernel { kCrossWarpTma = 0, kCrossCtaTma = 1, kCrossMma = 2, kCrossSimt = 3, kCrossGeneric = 4 };
+
 // self-attention for one new position per row: appends k/v at position P0 + *d_step and attends over 0..P0 + *d_step
 // qkv [M, 3H]; cache layout [layer][kv][b][t][k][H]
 // step_host >= 0: the caller knows the step index (must equal *d_step); the lean kernel then only loads positions <= step
+// force: kDecDefault, kSelfFirst or kSelfV2 (dec_self_attn_supports must hold)
 int launch_dec_self_attn(int dtype, const DecodeGeom& g, int layer, const void* qkv, void* self_cache, const int* d_step, int step_host,
-                         const uint8_t* anc, void* out, cudaStream_t stream);
+                         const uint8_t* anc, void* out, cudaStream_t stream, int force);
 // the lean bf16 / 64-dim kernel will run for these arguments (default on; env GSTVD_SELF_V2=0 disables it)
 bool dec_self_attn_v2_active(int dtype, const DecodeGeom& g, const void* qkv, const void* self_cache, const void* out);
+// kernel (kSelfFirst / kSelfV2) can run these arguments (anc != null: only the lean kernel reads an ancestry table)
+bool dec_self_attn_supports(int kernel, int dtype, const DecodeGeom& g, const void* qkv, const void* self_cache, const void* out,
+                            const uint8_t* anc);
 // anc: uint8 [B*K][32] (rows of 64 when g.T > 32) ancestry table (slot that holds position t of beam k's history), permuted instead of gathering the cache;
 // only the lean kernel reads it - pass null to the self-attention and call launch_reorder_cache otherwise
 int launch_anc_update(const DecodeGeom& g, const int32_t* beam_idx, const int* d_step, uint8_t* anc, cudaStream_t stream);
@@ -145,12 +155,17 @@ int launch_anc_update(const DecodeGeom& g, const int32_t* beam_idx, const int* d
 // positions) into every beam slot of cache positions 0..P0-1; launches nothing when P0 = 0
 int launch_prefix_kv_store(int dtype, const DecodeGeom& g, int layer, const void* qkv, void* self_cache, cudaStream_t stream);
 // cross-attention of every beam row over its image's cross K/V. cross layout [layer][b][kv*heads+h][Le][D]
+// force: kDecDefault, kCrossMma, kCrossSimt or kCrossGeneric (dec_cross_supports must hold)
 int launch_dec_cross_attn(int dtype, const DecodeGeom& g, int layer, const void* q, const void* cross_cache,
-                          const float* enc_mask, void* out, cudaStream_t stream);
+                          const float* enc_mask, void* out, cudaStream_t stream, int force);
 // TMA-streamed bf16 variant (cross_tma.cu); cross_len [B] = keys to fetch per image (launch_cross_len), may be null
+// dec_cross_tma_supported: the decode step's choice (honours env GSTVD_CROSS_NO_TMA); force: kDecDefault, kCrossWarpTma or kCrossCtaTma
 bool dec_cross_tma_supported(int dtype, const DecodeGeom& g);
+bool dec_cross_tma_fits(int dtype, const DecodeGeom& g);   // the same without the environment switch
 int launch_dec_cross_tma(const DecodeGeom& g, int layer, const void* q, const void* cross_cache, const float* enc_mask,
-                         const int* cross_len, void* out, int num_sms, cudaStream_t stream);
+                         const int* cross_len, void* out, int num_sms, cudaStream_t stream, int force);
+// kernel (a CrossAttnKernel) can run this geometry, whatever the environment says
+bool dec_cross_supports(int kernel, int dtype, const DecodeGeom& g);
 int launch_cross_len(int B, int Le, const float* mask, int* out, cudaStream_t stream);
 void dec_cross_print_times();   // measurement aid (env GSTVD_CROSS_TIMES=1): per-CTA phase stamps of the last cross-attention launch
 // cached CUtensorMap (returned as an opaque pointer) over [groups][L][D] bf16 rows, box = D x box_rows (gemm_tc.cu)

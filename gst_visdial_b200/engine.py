@@ -337,6 +337,43 @@ class Engine:
                                                     self._stream()))
         return out
 
+    SELF_KERNELS = {"default": -1, "first": 0, "v2": 1}
+    CROSS_KERNELS = {"default": -1, "warp_tma": 0, "cta_tma": 1, "mma": 2, "simt": 3, "generic": 4}
+
+    def op_dec_self_attn(self, qkv, cache, heads, P0=0, step=0, step_known=True, prefix_qkv=None, anc=None, kernel="default", dtype=None):
+        """One decode-step self-attention launch (include/gstvd.h gstvd_op_dec_self_attn) on fp32 ``qkv`` [B*K, 3H] and ``cache``
+        [2, B, T, K, H]; ``anc`` uint8 [B*K, 32 or 64].  Returns (out [B*K, H], the cache after the call); ``cache`` is not modified."""
+        q = self._dev(qkv, torch.float32)
+        c = self._dev(cache, torch.float32).clone()
+        _, B, T, K, H = c.shape
+        pre = self._dev(prefix_qkv, torch.float32)
+        a = self._dev(anc, torch.uint8)
+        out = torch.empty(B * K, H, device=self.device, dtype=torch.float32)
+        check(self.ctx, self.lib.gstvd_op_dec_self_attn(self.ctx, self.dtype if dtype is None else DTYPES[dtype], self.SELF_KERNELS[kernel], B, K,
+                                                        int(heads), H // heads, T, int(P0), int(step), int(bool(step_known)), _ptr(q), _ptr(pre),
+                                                        _ptr(c), _ptr(a), _ptr(out), self._stream()))
+        return out, c
+
+    def op_dec_cross_attn(self, q, cross_kv, K, mask=None, use_cross_len=True, kernel="default", dtype=None):
+        """One decode-step cross-attention launch (gstvd_op_dec_cross_attn): fp32 ``q`` [B*K, H], ``cross_kv`` [B, 2*heads, Le, D],
+        ``mask`` [B, Le].  Returns (out [B*K, H], cross_len int32 [B] or None)."""
+        qd, kv, m = self._dev(q, torch.float32), self._dev(cross_kv, torch.float32), self._dev(mask, torch.float32)
+        B, two_heads, Le, D = kv.shape
+        cl = torch.empty(B, device=self.device, dtype=torch.int32) if use_cross_len else None
+        out = torch.empty(qd.shape[0], qd.shape[1], device=self.device, dtype=torch.float32)
+        check(self.ctx, self.lib.gstvd_op_dec_cross_attn(self.ctx, self.dtype if dtype is None else DTYPES[dtype], self.CROSS_KERNELS[kernel], B,
+                                                         int(K), two_heads // 2, D, Le, _ptr(qd), _ptr(kv), _ptr(m), int(bool(use_cross_len)),
+                                                         _ptr(cl), _ptr(out), self._stream()))
+        return out, cl
+
+    def op_anc_update(self, anc, beam_idx, T, P0, step):
+        """One ancestry-table update (gstvd_op_anc_update): returns the updated copy of uint8 ``anc`` [B*K, 32 or 64]."""
+        bi = self._dev(beam_idx, torch.int32)
+        B, K = bi.shape
+        a = self._dev(anc, torch.uint8).clone()
+        check(self.ctx, self.lib.gstvd_op_anc_update(self.ctx, B, K, int(T), int(P0), int(step), _ptr(bi), _ptr(a), self._stream()))
+        return a
+
     def op_beam_begin(self, B, K, max_new):
         check(self.ctx, self.lib.gstvd_op_beam_begin(self.ctx, B, K, max_new, self._stream()))
         self._beam_shape = (B, K)

@@ -287,6 +287,32 @@ int gstvd_op_deferred_ln_chain(gstvd_ctx* ctx, int M, int N, int K1, const float
                                const float* res0, const float* gamma1, const float* beta1, const float* w2, const float* b2,
                                const float* gamma2, const float* beta2, float* out, float* out_x1, void* stream);
 
+/* The decode step's attention kernels one at a time, on caller-supplied data (parity tests).  All float buffers are fp32 on the
+ * device; dtype GSTVD_BF16 rounds them to bf16 inside and converts the results back.  Each call uses its own one-layer geometry,
+ * not the context's caches.  `kernel` forces one kernel (-1: the decode step's own choice, environment switches included); a
+ * forced kernel that cannot run the arguments is refused with GSTVD_ERR_UNSUPPORTED before anything is launched.
+ *
+ * Self-attention of one new position per (image, beam) row; kernel 0 = the first kernel (fp32 / bf16, D 64 or 128), 1 = the lean
+ * bf16 / D = 64 kernel (the only reader of an ancestry table).
+ *   qkv [B*K, 3*heads*D]; cache [2 (k, v)][B][T][K][heads*D] in/out: the new k / v are written at position P0 + step of the row's
+ *   own beam slot; prefix_qkv [B*P0, 3*heads*D] or NULL: its k / v are first stored at positions 0..P0-1 of every slot;
+ *   anc uint8 [B*K][T <= 32 ? 32 : 64] or NULL: position t of row (b, k) is read from slot anc[b*K + k][t];
+ *   step_known != 0 hands the step to the launch (loads bounded by it), else only through device memory (every row loaded, masked);
+ *   out [B*K, heads*D].  K <= 8, T <= 64, P0 + step < T. */
+int gstvd_op_dec_self_attn(gstvd_ctx* ctx, int dtype, int kernel, int B, int K, int heads, int D, int T, int P0, int step,
+                           int step_known, const float* qkv, const float* prefix_qkv, float* cache, const uint8_t* anc,
+                           float* out, void* stream);
+/* Cross-attention of B*K rows (K per image) over cross_kv [B][2*heads (k heads, then v heads)][Le][D] with mask [B, Le] (NULL:
+ * all ones; additive (1 - m) * -1e9).  kernel 0 = warp-per-item TMA, 1 = CTA-per-item TMA, 2 = mma.sync, 3 = SIMT, 4 = generic.
+ * use_cross_len != 0 (needs the mask): the TMA kernels fetch keys up to cross_len[b] = last non-zero mask entry + 1 (Le for an
+ * all-zero row), as in the decode step; out_cross_len int32 [B] (may be NULL) receives it.  q / out [B*K, heads*D]; K <= 8, Le <= 512. */
+int gstvd_op_dec_cross_attn(gstvd_ctx* ctx, int dtype, int kernel, int B, int K, int heads, int D, int Le, const float* q,
+                            const float* cross_kv, const float* mask, int use_cross_len, int32_t* out_cross_len, float* out,
+                            void* stream);
+/* One beam-ancestry update of a caller-supplied table anc uint8 [B*K][T <= 32 ? 32 : 64] (in place): beam_idx int32 [B, K] holds each
+ * new beam's parent; row (b, k) becomes the parent's row over positions < P0 + step and holds the parent at P0 + step. */
+int gstvd_op_anc_update(gstvd_ctx* ctx, int B, int K, int T, int P0, int step, const int32_t* beam_idx, uint8_t* anc, void* stream);
+
 /* Test access to the self-attention KV cache in the layout a generate call with (B, K) uses: buf fp32 [B, max_new_tokens, K,
  * hidden] on the device for one (layer, kv in {0: key, 1: value}); write != 0 stores buf into the cache (rounded to the
  * compute dtype), else reads it back.  Lets the tests check gstvd_reorder_cache against index_select(0, beam_idx) directly. */
