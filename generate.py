@@ -90,6 +90,9 @@ def main(argv=None):
                         diversity_penalty=params['q_diversity_penalty'])
         if params['q_beam_sample']:
             q_kwargs.update(do_sample=True)
+    for kw, who in ((a_kwargs, ''), (q_kwargs, 'q_')):
+        kw.update(repetition_penalty=params[f'{who}repetition_penalty'], no_repeat_ngram_size=params[f'{who}no_repeat_ngram_size'],
+                  min_length=params[f'{who}min_length'])
     decode = None
     if params['vocab_file']:
         from transformers import BertTokenizer

@@ -12,7 +12,7 @@ from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int6
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "lib", "libgstvd.so")
 
-GSTVD_ABI_VERSION = 3
+GSTVD_ABI_VERSION = 4
 GSTVD_MAX_CONNECTIONS = 16
 GSTVD_F32, GSTVD_BF16 = 0, 1
 GSTVD_SELECT_SAMPLE, GSTVD_SELECT_BEAM, GSTVD_SELECT_BEAM_SAMPLE = 0, 1, 2
@@ -46,6 +46,7 @@ class GstvdGenParams(Structure):
         ("mode", c_int32), ("num_beams", c_int32), ("max_new_tokens", c_int32), ("top_k", c_int32),
         ("temperature", c_float), ("top_p", c_float), ("ngram_blocking_size", c_int32), ("seed", c_uint64),
         ("row_offset", c_int64), ("num_return_sequences", c_int32), ("num_beam_groups", c_int32), ("diversity_penalty", c_float),
+        ("repetition_penalty", c_float), ("no_repeat_ngram_size", c_int32), ("min_length", c_int32),
     ]
 
 

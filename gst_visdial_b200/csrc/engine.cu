@@ -74,8 +74,8 @@ struct DevBuf {
 // a kind of call are 0: Lh / Le for a generate graph; Lt / Lv and the has_* flags (optional inputs, out_scores) for a round graph.
 // K = decode rows per image; P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start.
 struct GraphKey {
-  int B, K, mode, T, top_k, ngram, P, has_prefix, N, G, Lh, Le, Lt, Lv, has_seg, has_att, has_imask, has_scores;
-  float temperature, top_p, penalty;
+  int B, K, mode, T, top_k, ngram, P, has_prefix, N, G, Lh, Le, Lt, Lv, has_seg, has_att, has_imask, has_scores, no_repeat_ngram, min_length;
+  float temperature, top_p, penalty, repetition_penalty;
   bool operator<(const GraphKey& o) const { return std::memcmp(this, &o, sizeof(GraphKey)) < 0; }
 };
 constexpr size_t kMaxGraphs = 24;      // least-recently-used graphs beyond this are destroyed (an 18-step graph holds ~2k kernel nodes)
@@ -683,6 +683,13 @@ void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
                                          prefix, P, s);
 }
 
+// The request's logits processors; the caller fills in where the rows' decoder input lives.
+LogitsProcs logits_procs(const gstvd_gen_params& gp) {
+  LogitsProcs p;
+  p.repetition_penalty = gp.repetition_penalty; p.no_repeat_ngram = gp.no_repeat_ngram_size; p.min_length = gp.min_length;
+  return p;
+}
+
 // One decode step for all M = B*K rows: embeddings -> 12 x [self-attn over cache, cross-attn, FFN] -> LM head -> selection.
 // step_host = index of this step when the caller knows it (it always does: eager loops and the captured graph both unroll the
 // steps), so kernels that only need it to bound their loads take it as a launch parameter instead of reading *d_step first.
@@ -751,6 +758,9 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   }
   X.gemm(c->dh.p, H, c->lm_head, c->logits.p, c->Vpad, M, 0, true);
   float* sv = (float*)c->sel_val.p; int32_t* si = (int32_t*)c->sel_idx.p;
+  // the logits processors act inside the selection kernels; each reads its rows' decoder input (cur_len = P + step <= 64)
+  LogitsProcs procs = logits_procs(gp);
+  procs.P = P; procs.step = step_host; procs.d_step = d_step;
   if (beams) {
     // beam sampling: g.K = N * K rows per image (N searches of K beams), each row's 16 best for the warpers and the draw
     const bool sampled = gp.mode == GSTVD_SELECT_BEAM_SAMPLE;
@@ -771,15 +781,17 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     // lowers (the candidate lists stay ranked by the unpenalised score; launch_beam_step explains why nsel = 2K suffices)
     const int G = gp.num_beam_groups;
     float* lz = G > 1 ? (float*)c->logz.p : nullptr;
+    // a beam row's decoder input: the image's prefix, then the beam's tokens in the token buffer of this step's parity
+    procs.prefix = prefix; procs.tokens = bb.tokens + (int64_t)(step_host & 1) * M * Tn; procs.tok_stride = Tn; procs.rows_per_image = g.K;
     c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, (c->dtype == kBF16 && !exact_lse) ? 2 : 0,
-                                     (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, lz, s);
+                                     (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, lz, procs, s);
     if (sampled) {
       const int K = gp.num_beams;
       c->launches += launch_beam_sample_step(bb, M / K, g.K / K, K, Tn, c->V, sv, si, gp.top_k, gp.temperature, gp.top_p,
                                              (const uint64_t*)c->d_seed.p, 102, P, s);
     } else {
       c->launches += launch_beam_step(bb, g.B, g.K, G, Tn, c->V, nsel, sv, si, G > 1 ? (const float*)c->logits.p : nullptr, c->Vpad, lz,
-                                      gp.diversity_penalty, 102, P, nullptr, nullptr, nullptr, s);
+                                      gp.diversity_penalty, gp.repetition_penalty, prefix, 102, P, nullptr, nullptr, nullptr, s);
     }
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
@@ -795,14 +807,15 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
                                       (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }
+    procs.keys = (const int32_t*)c->prefix.p; procs.key_stride = kst;      // a sample row's decoder input is its n-gram key
     if (gp.top_k == 0) {
       // no top-k cut (utils/decoding_utils.py:17 skips it): multinomial over the whole, optionally nucleus-filtered, vocabulary
       c->launches += launch_full_vocab_sample(M, g.K, c->V, (const float*)c->logits.p, c->Vpad, gp.temperature, gp.top_p, bt, bc, Lh, Tn, 0, 0,
                                               (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p,
-                                              key_next, kst, nullptr, s);
+                                              key_next, kst, nullptr, procs, s);
     } else {
       c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, 1, nullptr, gp.temperature, bt, bc, Lh, nsel, sv, si,
-                                       nullptr, s);
+                                       nullptr, procs, s);
       c->launches += launch_sample_step(M, g.K, Tn, nsel, sv, si, gp.top_k, gp.top_p, 0, 0, (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p,
                                         (int32_t*)c->cur_tokens.p, key_next, kst, nullptr, s);
     }
@@ -827,6 +840,10 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* pref
     throw InvalidArg(fmt("generate: prefix length %d + %d new tokens exceed max_position_embeddings (%d)", P, T, c->cfg.max_position_embeddings));
   if (!out_ids) throw InvalidArg("generate: out_ids is NULL");
   if (!(penalty >= 0.f) || !std::isfinite(penalty)) throw InvalidArg(fmt("generate: diversity_penalty %g must be finite and >= 0", (double)penalty));
+  if (!(gp.repetition_penalty > 0.f) || !std::isfinite(gp.repetition_penalty))
+    throw InvalidArg(fmt("generate: repetition_penalty %g must be finite and > 0 (1 = off)", (double)gp.repetition_penalty));
+  if (gp.no_repeat_ngram_size < 0) throw InvalidArg(fmt("generate: no_repeat_ngram_size %d must be >= 0", gp.no_repeat_ngram_size));
+  if (gp.min_length < 0) throw InvalidArg(fmt("generate: min_length %d must be >= 0", gp.min_length));
   if (G < 1) throw InvalidArg(fmt("generate: %d beam groups", G));
   if (G > 1 && gp.mode != GSTVD_SELECT_BEAM) throw InvalidArg("generate: beam groups need beam search");
   int K = 1;
@@ -875,6 +892,7 @@ GraphKey graph_key(const gstvd_gen_params& gp, int B, int K, int P, bool has_pre
   k.P = P; k.has_prefix = has_prefix; k.N = gp.num_return_sequences; k.G = gp.num_beam_groups;
   k.Lh = Lh; k.Le = Le; k.Lt = Lt; k.Lv = Lv; k.has_seg = has_seg; k.has_att = has_att; k.has_imask = has_imask; k.has_scores = has_scores;
   k.temperature = gp.temperature; k.top_p = gp.top_p; k.penalty = gp.diversity_penalty;
+  k.repetition_penalty = gp.repetition_penalty; k.no_repeat_ngram = gp.no_repeat_ngram_size; k.min_length = gp.min_length;
   return k;
 }
 
@@ -1565,9 +1583,9 @@ int gstvd_op_beam_step(gstvd_ctx* c, const float* logits, int64_t ldl, int32_t* 
     cudaStream_t s = (cudaStream_t)stream;
     const int B = c->op_B, K = c->op_K, T = c->op_T, nsel = 2 * K;
     c->launches += launch_row_select(B * K, c->V, logits, ldl, 0, (const float*)c->beam_scores.p, 1.f, nullptr, nullptr, 0, nsel,
-                                     (float*)c->sel_val.p, (int32_t*)c->sel_idx.p, nullptr, s);
+                                     (float*)c->sel_val.p, (int32_t*)c->sel_idx.p, nullptr, LogitsProcs(), s);
     c->launches += launch_beam_step(beam_buffers(c), B, K, 1, T, c->V, nsel, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, nullptr,
-                                    0, nullptr, 0.f, 102, 1, beam_idx, next_tokens, next_scores, s);
+                                    0, nullptr, 0.f, 1.f, nullptr, 102, 1, beam_idx, next_tokens, next_scores, s);
     c->launches += launch_step_advance((int*)c->d_step.p, s);
   });
 }
@@ -1589,28 +1607,38 @@ int gstvd_op_sample(gstvd_ctx* c, int rows, const float* logits, int64_t ldl, co
     if (rows < 1 || rows > c->B_max) throw InvalidArg("op_sample: rows out of range");
     if (gp->top_k < 0 || gp->top_k > GSTVD_MAX_TOP_K) throw Unsupported("op_sample: top_k must be 0 (no top-k cut) or in 1..16");
     if (gp->top_k == 0 && c->V > 32768) throw Unsupported("op_sample: top_k = 0 needs a vocabulary of at most 32768 entries");
+    if (!(gp->repetition_penalty > 0.f) || !std::isfinite(gp->repetition_penalty) || gp->no_repeat_ngram_size < 0 || gp->min_length < 0)
+      throw InvalidArg("op_sample: repetition_penalty must be finite and > 0, no_repeat_ngram_size and min_length >= 0");
+    LogitsProcs procs = logits_procs(*gp);
     cudaStream_t s = (cudaStream_t)stream;
     const int T = c->T_max;
+    const bool need_prefix = gp->ngram_blocking_size > 0 || procs.active();
+    if (need_prefix && (!prefix || prefix_len != step + 1 || prefix_len > std::min(T + 1, kProcMaxLen)))
+      throw InvalidArg("op_sample: n-gram blocking and the logits processors need a prefix of step+1 <= min(max_new_tokens + 1, 64) tokens");
+    if (gp->ngram_blocking_size > 0 && (!hist_ids || !hist_segments)) throw InvalidArg("op_sample: n-gram blocking needs the history");
     CUDA_CHECK(cudaMemcpyAsync(c->d_step.p, &step, 4, cudaMemcpyHostToDevice, s));
     CUDA_CHECK(cudaMemcpyAsync(c->d_seed.p, &gp->seed, 8, cudaMemcpyHostToDevice, s));
     CUDA_CHECK(cudaStreamSynchronize(s));
     const int32_t* bt = nullptr; const int32_t* bc = nullptr;
-    if (gp->ngram_blocking_size > 0) {
-      if (!hist_ids || !hist_segments || !prefix || prefix_len != step + 1) throw InvalidArg("op_sample: n-gram blocking needs history and a prefix of step+1 tokens");
+    if (need_prefix) {
       CUDA_CHECK(cudaMemsetAsync(c->prefix.p, 0, c->prefix.bytes, s));
       c->launches += launch_build_prefix_from_ids(rows, prefix_len, prefix, (int32_t*)c->prefix.p, T + 1, 102, s);
+    }
+    if (gp->ngram_blocking_size > 0) {
       c->launches += launch_ngram_ban(rows, 1, Lh, hist_ids, hist_segments, (const int32_t*)c->prefix.p, T + 1, (const int*)c->d_step.p, 1,
                                       gp->ngram_blocking_size, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }
+    // the row's decoder input is the caller's prefix ([SEP] read as [PAD]); the step comes from the device counter
+    procs.keys = (const int32_t*)c->prefix.p; procs.key_stride = T + 1; procs.P = 1; procs.step = -1; procs.d_step = (const int*)c->d_step.p;
     if (gp->top_k == 0) {
       c->launches += launch_full_vocab_sample(rows, 1, c->V, logits, ldl, gp->temperature, gp->top_p, bt, bc, Lh, T, gp->seed, (uint64_t)gp->row_offset, nullptr,
                                               (const int*)c->d_step.p, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, T + 1,
-                                              out_tokens, s);
+                                              out_tokens, procs, s);
       return;
     }
     c->launches += launch_row_select(rows, c->V, logits, ldl, 1, nullptr, gp->temperature, bt, bc, Lh, kSelMax, (float*)c->sel_val.p,
-                                     (int32_t*)c->sel_idx.p, nullptr, s);
+                                     (int32_t*)c->sel_idx.p, nullptr, procs, s);
     c->launches += launch_sample_step(rows, 1, T, kSelMax, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, gp->top_k, gp->top_p, gp->seed, (uint64_t)gp->row_offset, nullptr,
                                       (const int*)c->d_step.p, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, T + 1,
                                       out_tokens, s);

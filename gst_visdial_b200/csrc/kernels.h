@@ -176,14 +176,36 @@ int launch_reorder_cache(int dtype, const DecodeGeom& g, void* self_cache, const
 
 // ---- token selection -------------------------------------------------------------------------------------
 constexpr int kSelMax = 16;   // per-row candidates kept (>= 2*max_beams, >= max top_k)
+constexpr int kProcMaxLen = 64;   // longest decoder input the logits processors read (= the cached positions of the decode kernels)
+
+// HF logits processors on a row's score s (include/gstvd.h gstvd_generate; CPU oracle: oracle/processors.py), applied where the
+// selection kernels apply their ban lists.  d = the row's decoder input of cur_len = P + t ids: the image's decoder prefix ([SEP] read
+// as [PAD]; [CLS] when null), then the row's t generated tokens.
+//   repetition_penalty p (1 = off): every distinct id of d gets s < 0 ? fp32(s * p) : fp32(s / p)
+//   no_repeat_ngram n (0 = off): the id that follows an earlier occurrence of the last n-1 ids of d gets -inf
+//   min_length m (0 = off): [SEP] gets -inf while cur_len < m
+// d is read either from an int32 key buffer (sampling: keys [rows, key_stride], [SEP] already [PAD]) or from the int64 decoder prefix
+// [rows / rows_per_image, P] (null: [CLS], P = 1) followed by the beam token buffer tokens [rows, tok_stride] of this step's parity.
+// t = step, or *d_step when step < 0.
+struct LogitsProcs {
+  float repetition_penalty = 1.f;
+  int no_repeat_ngram = 0, min_length = 0;
+  const int32_t* keys = nullptr; int key_stride = 0;
+  const int64_t* prefix = nullptr; const int32_t* tokens = nullptr; int tok_stride = 0; int rows_per_image = 1;
+  int P = 1, step = -1;
+  const int* d_step = nullptr;
+  __host__ __device__ bool active() const { return repetition_penalty != 1.f || no_repeat_ngram > 0 || min_length > 0; }
+};
+
 // Per row: logZ (fp64 accumulate) and the top `nsel` entries of  score_j by (score desc, index asc), where
-//   mode 0 (beam):   score_j = fp32(fp32(x_j - logZ) + row_bias[row])   (mode 2: the same with the exp terms of logZ in fp32)
-//   mode 1 (sample): score_j = x_j / temperature
-//   banned tokens (every mode) = -inf, applied after the transform: logZ is over the full row
+//   mode 0 (beam):   score_j = fp32(proc(fp32(x_j - logZ)) + row_bias[row])   (mode 2: the same with the exp terms of logZ in fp32)
+//   mode 1 (sample): score_j = proc(fp32(x_j / temperature))
+//   proc = the logits processors of `procs` (identity when inactive); banned tokens (every mode) = -inf, applied after the transform:
+//   logZ is over the full, unprocessed row
 // logits [rows, ldl] fp32.  ban_tokens [rows, ban_stride] / ban_count [rows] may be null.
 int launch_row_select(int rows, int V, const float* logits, int64_t ldl, int mode, const float* row_bias, float temperature,
                       const int32_t* ban_tokens, const int32_t* ban_count, int ban_stride, int nsel,
-                      float* sel_val, int32_t* sel_idx, float* logz, cudaStream_t stream);
+                      float* sel_val, int32_t* sel_idx, float* logz, const LogitsProcs& procs, cudaStream_t stream);
 
 struct BeamBuffers {
   float* beam_scores;      // [B,K]
@@ -209,10 +231,12 @@ int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, i
                             float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, cudaStream_t stream);
 // G > 1: diverse beam search with the Hamming penalty `penalty` (oracle/beam_groups.py).  A candidate whose token earlier groups took
 // at this step is re-scored from logits [B*K, ldl] fp32 and logz [B*K] (row_select's outputs for this step); needs nsel >= K + K / G.
-// G = 1 reads neither.
+// The re-score applies the repetition penalty rep_penalty after the Hamming term when the token occurs in the beam's decoder input
+// (prefix: int64 [B, len0] decoder prefix, null: [CLS]; then the beam's tokens).  G = 1 reads none of these.
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
-                     const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, int eos, int len0,
-                     int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores, cudaStream_t stream);
+                     const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, float rep_penalty,
+                     const int64_t* prefix, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
+                     cudaStream_t stream);
 // out_ids [B*N, T] / out_scores [B*N]: the N <= K best finished hypotheses of every image, image-major, in the pop order of HF
 // BeamSearchScorer.finalize (score descending, the later-inserted first among equal scores); N = 1 is the single best
 int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores,
@@ -231,10 +255,11 @@ int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, 
 // sample-mode selection from row_select output; writes seq[row, step] and cur_tokens[row], prefix[row, step+1]
 // top_k == 0: multinomial over the whole (optionally nucleus-filtered) vocabulary; writes the same state as launch_sample_step
 // N rows per image (sampled candidates): row r draws as row r / N of a single-sample call seeded candidate_seed(seed, r % N)
+// procs: the logits processors, applied after the temperature (their step is *d_step)
 int launch_full_vocab_sample(int rows, int N, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,
                              const int32_t* ban_count, int ban_stride, int T, uint64_t seed, uint64_t row_offset, const uint64_t* d_seed,
                              const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens,
-                             cudaStream_t stream);
+                             const LogitsProcs& procs, cudaStream_t stream);
 int launch_sample_step(int rows, int N, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
                        uint64_t seed, uint64_t row_offset, const uint64_t* d_seed, const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
                        int prefix_stride, int32_t* out_tokens, cudaStream_t stream);

@@ -12,6 +12,7 @@
 //   splice         : generate.py:145-160 and :214-228
 #include <cooperative_groups.h>
 
+#include <cmath>
 #include <cstdlib>
 #include <stdexcept>
 
@@ -29,14 +30,63 @@ constexpr int kHypMaxT = 32;
 struct Cand { float v; int i; };
 __device__ __forceinline__ bool better(float av, int ai, float bv, int bi) { return av > bv || (av == bv && ai < bi); }
 
+// ---- logits processors (LogitsProcs, kernels.h) ----------------------------------------------------------------------
+// The CTA of `row` reads the row's decoder input d (cur_len = P + t <= 64 ids) into shared memory once, marks the positions whose id
+// the n-gram rule bans, and every thread then folds d into two masks over its own slots: `pen` = slots whose id occurs in d (a bit
+// mask, so an id that repeats is penalised once), `ban` = slots set to -inf (n-gram rule; [SEP] while cur_len < min_length).
+// owner(w) = the calling thread's slot of id w, or -1.  Every thread of the CTA must call it (it synchronises).
+template <class Owner>
+__device__ __forceinline__ void procs_masks(const LogitsProcs& pp, int row, int t, int32_t* s_d, uint8_t* s_ban, Owner owner,
+                                            uint32_t& pen, uint32_t& ban) {
+  const int tid = threadIdx.x;
+  const int L = min(pp.P + t, kProcMaxLen);
+  if (tid < L) {
+    int32_t w;
+    if (pp.keys) w = pp.keys[(int64_t)row * pp.key_stride + tid];
+    else if (tid < pp.P) {
+      w = pp.prefix ? (int32_t)pp.prefix[(int64_t)(row / pp.rows_per_image) * pp.P + tid] : 101;
+      if (w == 102) w = 0;                                 // the decoder input holds [PAD] where the prefix has [SEP]
+    } else w = pp.tokens[(int64_t)row * pp.tok_stride + tid - pp.P];
+    s_d[tid] = w;
+  }
+  __syncthreads();
+  const int n = pp.no_repeat_ngram;
+  if (tid < L) {
+    // position tid closes the n-gram d[tid-n+1 .. tid]: its last id is banned when the first n-1 equal the last n-1 ids of d
+    bool b = n > 0 && tid >= n - 1;
+    for (int q = 0; q < n - 1 && b; ++q) b = s_d[tid - n + 1 + q] == s_d[L - n + 1 + q];
+    s_ban[tid] = b ? 1 : 0;
+  }
+  __syncthreads();
+  pen = 0u; ban = 0u;
+  for (int j = 0; j < L; ++j) {
+    const int s = owner(s_d[j]);
+    if (s >= 0) { pen |= 1u << s; if (s_ban[j]) ban |= 1u << s; }
+  }
+  if (L < pp.min_length) { const int s = owner(102); if (s >= 0) ban |= 1u << s; }
+}
+
+template <int NS>
+__device__ __forceinline__ void procs_apply(float (&v)[NS], float p, uint32_t pen, uint32_t ban) {
+#pragma unroll
+  for (int s = 0; s < NS; ++s) {
+    if (p != 1.f && ((pen >> s) & 1u)) v[s] = v[s] < 0.f ? __fmul_rn(v[s], p) : __fdiv_rn(v[s], p);
+    if ((ban >> s) & 1u) v[s] = -INFINITY;
+  }
+}
+
+template <bool kProcs>  // kProcs: the logits processors are on (a separate instance keeps the off path as it was)
 __global__ void __launch_bounds__(kSelThreads)
 row_select_kernel(int V, const float* __restrict__ logits, int64_t ldl, int mode, const float* __restrict__ row_bias,
                   float temperature, const int32_t* __restrict__ ban_tokens, const int32_t* __restrict__ ban_count,
-                  int ban_stride, int nsel, float* __restrict__ sel_val, int32_t* __restrict__ sel_idx, float* __restrict__ logz) {
+                  int ban_stride, int nsel, float* __restrict__ sel_val, int32_t* __restrict__ sel_idx, float* __restrict__ logz,
+                  const LogitsProcs procs) {
   __shared__ float s_f[32];
   __shared__ double s_d[32];
   __shared__ int s_i[32];
   __shared__ int s_bcast_i;
+  __shared__ int32_t s_in[kProcMaxLen];
+  __shared__ uint8_t s_ban[kProcMaxLen];
   pdl_wait();
   pdl_launch_dependents();
   const int row = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -75,11 +125,23 @@ row_select_kernel(int V, const float* __restrict__ logits, int64_t ldl, int mode
     const float bias = row_bias ? row_bias[row] : 0.f;
 #pragma unroll
     for (int s = 0; s < kSlots; ++s)
-      if (tid + s * kSelThreads < V) v[s] = __fadd_rn(__fsub_rn(v[s], lz), bias);
+      if (tid + s * kSelThreads < V) v[s] = kProcs ? __fsub_rn(v[s], lz) : __fadd_rn(__fsub_rn(v[s], lz), bias);   // processors: bias below
   } else {
 #pragma unroll
     for (int s = 0; s < kSlots; ++s)
       if (tid + s * kSelThreads < V) v[s] = __fdiv_rn(v[s], temperature);
+  }
+  if (kProcs) {
+    uint32_t pen, ban;
+    procs_masks(procs, row, procs.step >= 0 ? procs.step : *procs.d_step, s_in, s_ban,
+                [&](int w) { return (w >= 0 && w < kSelThreads * kSlots && (w % kSelThreads) == tid) ? w / kSelThreads : -1; }, pen, ban);
+    procs_apply(v, procs.repetition_penalty, pen, ban);
+    if (mode == 0) {
+      const float bias = row_bias ? row_bias[row] : 0.f;
+#pragma unroll
+      for (int s = 0; s < kSlots; ++s)
+        if (tid + s * kSelThreads < V) v[s] = __fadd_rn(v[s], bias);
+    }
   }
   // banned tokens -> -inf after the transform: in beam mode logZ stays over the full row (log_softmax, then the n-gram
   // processor, then the beam score - the order of HF beam_search, oracle/beam_ngram.py)
@@ -184,10 +246,12 @@ __device__ __forceinline__ double exp_nonpos(double d, const double* __restrict_
   return __hiloint2double(__double2hiint(res) + (k >> 5) * (1 << 20), __double2loint(res));   // * 2^floor(k/32)
 }
 
+template <bool kProcs>  // kProcs: the logits processors are on (a separate instance keeps the off path as it was)
 __global__ void __cluster_dims__(kRsChunks, 1, 1) __launch_bounds__(kRsThreads, 4)
 row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, int mode_in, const float* __restrict__ row_bias,
                           float temperature, const int32_t* __restrict__ ban_tokens, const int32_t* __restrict__ ban_count,
-                          int ban_stride, int nsel, float* __restrict__ sel_val, int32_t* __restrict__ sel_idx, float* __restrict__ logz) {
+                          int ban_stride, int nsel, float* __restrict__ sel_val, int32_t* __restrict__ sel_idx, float* __restrict__ logz,
+                          const LogitsProcs procs) {
   namespace cg = cooperative_groups;
   cg::cluster_group cluster = cg::this_cluster();
   int mode = mode_in;
@@ -206,6 +270,8 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
   __shared__ double s_exp2[32];                      // 2^(j/32)
   __shared__ float s_allv[kRsChunks * kSelMax];      // rank 0: the lists of all four CTAs (written by the peers)
   __shared__ int s_alli[kRsChunks * kSelMax];
+  __shared__ int32_t s_in[kProcMaxLen];              // the row's decoder input (logits processors)
+  __shared__ uint8_t s_ban[kProcMaxLen];
   pdl_wait();
   pdl_launch_dependents();
   const int chunk = (int)cluster.block_rank();
@@ -291,11 +357,25 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
     const float bias = row_bias ? row_bias[row] : 0.f;
 #pragma unroll
     for (int s = 0; s < kRsSlots; ++s)
-      if (base + tid + s * kRsThreads < V) v[s] = __fadd_rn(__fsub_rn(v[s], lz), bias);
+      if (base + tid + s * kRsThreads < V) v[s] = kProcs ? __fsub_rn(v[s], lz) : __fadd_rn(__fsub_rn(v[s], lz), bias);   // processors: bias below
   } else {
 #pragma unroll
     for (int s = 0; s < kRsSlots; ++s)
       if (base + tid + s * kRsThreads < V) v[s] = __fdiv_rn(v[s], temperature);
+  }
+  // logits processors on fp32(x - logZ) (beam modes, before the beam score, as HF beam_search) or fp32(x / temperature) (sampling)
+  if (kProcs) {
+    uint32_t pen, ban;
+    procs_masks(procs, row, procs.step >= 0 ? procs.step : *procs.d_step, s_in, s_ban,
+                [&](int w) { const int o = w - base; return (o >= 0 && o < kRsSpan && (o % kRsThreads) == tid) ? o / kRsThreads : -1; },
+                pen, ban);
+    procs_apply(v, procs.repetition_penalty, pen, ban);
+    if (mode == 0) {
+      const float bias = row_bias ? row_bias[row] : 0.f;
+#pragma unroll
+      for (int s = 0; s < kRsSlots; ++s)
+        if (base + tid + s * kRsThreads < V) v[s] = __fadd_rn(v[s], bias);
+    }
   }
   // banned tokens -> -inf after the transform: in the beam modes logZ stays over the full row (log_softmax, then the n-gram
   // processor, then the beam score - the order of HF beam_search, oracle/beam_ngram.py)
@@ -500,21 +580,27 @@ __device__ __forceinline__ bool beam_process(const BeamBuffers& bb, int b, int K
 // best 2 gs exactly like BeamSearchScorer.process with group_size = gs, on the image's one hypothesis heap; `done` is tested before
 // and updated after every group.  The token histories are gathered by all lanes at the end.
 //
+// With a repetition penalty p the re-scored value is fp32(fp32(rep(fp32(fp32(x - logZ) - fp32(lambda c)))) + beam_score), rep = the
+// penalty when w occurs in the beam's decoder input (HF runs the Hamming processor first, then the repetition penalty); the other
+// processors only produce -inf, which stays.
+//
 // Why the per-row lists suffice (nsel >= K + gs; the engine keeps nsel = 2K): row_select ranks each row's candidates by the
-// UNPENALISED score.  The penalty only lowers a score and fp32(a + b) is monotone in a, so an element outside a row's list is
-// preceded, in the contract's order, by every unpenalised element of that list.  The earlier groups took at most K - gs distinct
+// processed (repetition-penalised) score WITHOUT the Hamming term.  The Hamming term only lowers a score, rep (s < 0 ? s p : s / p,
+// p > 0) is monotone in s and fp32(a + b) is monotone in a, so an element outside a row's list is preceded, in the contract's order,
+// by every element of that list that no earlier group took.  The earlier groups took at most K - gs distinct
 // tokens, so at least nsel - (K - gs) >= 2 gs listed elements of the row keep their value, and a group takes at most 2 gs
 // candidates from one row: the group's exact top 2 gs lies inside the lists.
 constexpr int kBeamWarps = 4;
 // Register budget of the two beam-step kernels: 65536 / (7 * 128 threads) = 72 registers per thread.  Left to its default, ptxas
 // keeps them near 48 - 64 registers and spills the values that stay live across the calls into the fp64 / fp32 division subroutines
-// of the hypothesis walk (20 bytes in each kernel); with this budget neither spills (-Xptxas -v: beam_step_kernel 64 registers,
+// of the hypothesis walk (20 bytes in each kernel); with this budget neither spills (-Xptxas -v: beam_step_kernel 69 registers,
 // beam_sample_step_kernel 70).  The budget still lets 7 blocks share an SM; the grids have B / 4 and B * N / 4 blocks.
 constexpr int kBeamMinBlocks = 7;
 __global__ void __launch_bounds__(kBeamWarps * 32, kBeamMinBlocks)
 beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, const float* __restrict__ sel_val,
                  const int32_t* __restrict__ sel_idx, const float* __restrict__ logits, int64_t ldl, const float* __restrict__ logz,
-                 float penalty, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
+                 float penalty, float rep_penalty, const int64_t* __restrict__ prefix, int eos, int len0, int32_t* out_beam_idx,
+                 int32_t* out_tokens, float* out_scores) {
   __shared__ float s_val[kBeamWarps][128];
   __shared__ int s_flat[kBeamWarps][128];
   __shared__ int s_order[kBeamWarps][16];
@@ -547,7 +633,18 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, co
         for (int j = 0; j < lo; ++j) cnt += nb_tok[warp][j] == w ? 1 : 0;
         if (cnt > 0) {
           const int64_t row = (int64_t)b * K + beam;
-          v = __fadd_rn(__fsub_rn(__fsub_rn(logits[row * ldl + w], logz[row]), __fmul_rn(penalty, (float)cnt)), bb.beam_scores[row]);
+          float s = __fsub_rn(__fsub_rn(logits[row * ldl + w], logz[row]), __fmul_rn(penalty, (float)cnt));
+          if (rep_penalty != 1.f) {
+            // HF order: the Hamming term, then the repetition penalty when w occurs in the beam's decoder input
+            bool seen = false;
+            for (int j = 0; j < len0 && !seen; ++j) {
+              const int32_t pj = prefix ? (int32_t)prefix[(int64_t)b * len0 + j] : 101;
+              seen = (pj == 102 ? 0 : pj) == w;
+            }
+            for (int j = 0; j < t && !seen; ++j) seen = src[beam * T + j] == w;
+            if (seen) s = s < 0.f ? __fmul_rn(s, rep_penalty) : __fdiv_rn(s, rep_penalty);
+          }
+          v = __fadd_rn(s, bb.beam_scores[row]);
         }
       }
       s_val[warp][c] = v;
@@ -882,7 +979,7 @@ __global__ void sample_step_kernel(int rows, int N, int T, int nsel, const float
 // ---- top_k = 0: unrestricted / pure-nucleus multinomial over the whole vocabulary (utils/decoding_utils.py:17-35 with top_k == 0,
 // then softmax + torch.multinomial, models/visual_dialog_model.py:100-105) ---------------------------------------------------------
 // One CTA per row; thread t owns the 32 consecutive tokens [32 t, 32 t + 32) in registers (V <= 32768).
-//   x = logit / temperature, banned tokens -> -inf;  p = exp(x - max);  Z = sum p
+//   x = logit / temperature, then the logits processors, banned tokens -> -inf;  p = exp(x - max);  Z = sum p
 //   nucleus (top_p > 0): the reference sorts descending and removes position r when the cumulative probability of positions 0..r-1
 //     exceeds top_p, i.e. a token survives iff  S(x) = sum of p over tokens with a strictly larger logit  <=  top_p Z.  S is monotone
 //     in x, so the survivors are {x >= x*}; x* is found by a 32-step bit-wise search over the order-preserving integer image of the
@@ -904,15 +1001,19 @@ __device__ __forceinline__ float fv_block_sum(float v, float* s_red) {      // e
   t = warp_sum(t);
   return t;
 }
+template <bool kProcs>  // kProcs: the logits processors are on (a separate instance keeps the off path as it was)
 __global__ void __launch_bounds__(kFvThreads)
 full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t ldl, float temperature, float top_p,
                          const int32_t* __restrict__ ban_tokens, const int32_t* __restrict__ ban_count, int ban_stride,
                          int T, uint64_t seed, uint64_t row_offset, const uint64_t* __restrict__ d_seed, const int* __restrict__ d_step, int eos,
-                         int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens) {
+                         int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens,
+                         const LogitsProcs procs) {
   extern __shared__ float s_p[];                   // [kFvPer][kFvThreads]: p of token 32 t + j at s_p[j * 1024 + t] (conflict free)
   __shared__ float s_red[32];
   __shared__ float s_scan[32];
   __shared__ int s_choice;
+  __shared__ int32_t s_in[kProcMaxLen];
+  __shared__ uint8_t s_ban[kProcMaxLen];
   pdl_wait();
   pdl_launch_dependents();
   const int row = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -922,6 +1023,11 @@ full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t
   float v[kFvPer];
 #pragma unroll
   for (int j = 0; j < kFvPer; ++j) v[j] = (base + j < V) ? __fdiv_rn(x[base + j], temperature) : -INFINITY;
+  if (kProcs) {
+    uint32_t pen, ban;
+    procs_masks(procs, row, step, s_in, s_ban, [&](int w) { return (w >= base && w < base + kFvPer) ? w - base : -1; }, pen, ban);
+    procs_apply(v, procs.repetition_penalty, pen, ban);
+  }
   if (ban_tokens != nullptr) {
     const int nb = ban_count[row];
     for (int i = 0; i < nb; ++i) {
@@ -1103,21 +1209,30 @@ __global__ void build_prefix_kernel(int rows, int len, const int64_t* __restrict
   prefix[(int64_t)r * prefix_stride + j] = (tk == eos) ? 0 : (int32_t)tk;
 }
 
+void check_procs(const LogitsProcs& p, const char* who) {
+  if (!p.active()) return;
+  if (!(p.repetition_penalty > 0.f) || !std::isfinite(p.repetition_penalty) || p.no_repeat_ngram < 0 || p.min_length < 0)
+    throw std::runtime_error(std::string(who) + ": logits processor parameters out of range");
+  if (p.P < 1 || (!p.keys && !p.tokens) || (p.step < 0 && !p.d_step))
+    throw std::runtime_error(std::string(who) + ": the logits processors need the rows' decoder input and step");
+}
+
 }  // namespace
 
 int launch_row_select(int rows, int V, const float* logits, int64_t ldl, int mode, const float* row_bias, float temperature,
                       const int32_t* ban_tokens, const int32_t* ban_count, int ban_stride, int nsel,
-                      float* sel_val, int32_t* sel_idx, float* logz, cudaStream_t stream) {
+                      float* sel_val, int32_t* sel_idx, float* logz, const LogitsProcs& procs, cudaStream_t stream) {
   if (rows <= 0) return 0;
   if (V > kSelThreads * kSlots) throw std::runtime_error("row_select: vocab > 32768");
   if (nsel > kSelMax || nsel < 1) throw std::runtime_error("row_select: nsel out of range");
+  check_procs(procs, "row_select");
   static const bool v1 = getenv("GSTVD_ROW_SELECT_V1") != nullptr;      // A/B aid: the single-CTA-per-row kernel
   if (v1)
-    launch_k(row_select_kernel, dim3(rows), dim3(kSelThreads), 0, stream, V, logits, ldl, mode == 2 ? 0 : mode, row_bias, temperature, ban_tokens, ban_count,
-             ban_stride, nsel, sel_val, sel_idx, logz);
+    launch_k(procs.active() ? row_select_kernel<true> : row_select_kernel<false>, dim3(rows), dim3(kSelThreads), 0, stream, V, logits, ldl, mode == 2 ? 0 : mode, row_bias, temperature, ban_tokens, ban_count,
+             ban_stride, nsel, sel_val, sel_idx, logz, procs);
   else
-    launch_k(row_select_cluster_kernel, dim3(rows * kRsChunks), dim3(kRsThreads), 0, stream, V, logits, ldl, mode, row_bias, temperature,
-             ban_tokens, ban_count, ban_stride, nsel, sel_val, sel_idx, logz);
+    launch_k(procs.active() ? row_select_cluster_kernel<true> : row_select_cluster_kernel<false>, dim3(rows * kRsChunks), dim3(kRsThreads), 0, stream, V, logits, ldl, mode, row_bias, temperature,
+             ban_tokens, ban_count, ban_stride, nsel, sel_val, sel_idx, logz, procs);
   return 1;
 }
 
@@ -1138,14 +1253,17 @@ int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, i
   return 1;
 }
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
-                     const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, int eos, int len0,
-                     int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores, cudaStream_t stream) {
+                     const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, float rep_penalty,
+                     const int64_t* prefix, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
+                     cudaStream_t stream) {
   if (K > 8 || T > kHypMaxT) throw std::runtime_error("beam_step: K <= 8 and T <= 32");
   if (G < 1 || K % G != 0) throw std::runtime_error("beam_step: the beam groups must divide the beams");
   if (G > 1 && (!logits || !logz || nsel < K + K / G))
     throw std::runtime_error("beam_step: beam groups need the logits, logZ and nsel >= K + K / G per-row candidates");
+  if (!(rep_penalty > 0.f) || !std::isfinite(rep_penalty) || (len0 > 1 && !prefix))
+    throw std::runtime_error("beam_step: repetition penalty must be finite and > 0, prefix given when len0 > 1");
   launch_k(beam_step_kernel, dim3((B + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, B, K, G, T, V, nsel, sel_val, sel_idx,
-           logits, ldl, logz, penalty, eos, len0, out_beam_idx, out_tokens, out_scores);
+           logits, ldl, logz, penalty, rep_penalty, prefix, eos, len0, out_beam_idx, out_tokens, out_scores);
   return 1;
 }
 int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores,
@@ -1182,19 +1300,22 @@ int launch_sample_step(int rows, int N, int T, int nsel, const float* sel_val, c
 int launch_full_vocab_sample(int rows, int N, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,
                              const int32_t* ban_count, int ban_stride, int T, uint64_t seed, uint64_t row_offset, const uint64_t* d_seed,
                              const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens,
-                             cudaStream_t stream) {
+                             const LogitsProcs& procs, cudaStream_t stream) {
   if (rows <= 0) return 0;
   if (N < 1 || rows % N != 0) throw std::runtime_error("full_vocab_sample: rows must be a multiple of N >= 1");
   if (V > kFvThreads * kFvPer) throw std::runtime_error("full_vocab_sample: vocab > 32768");
+  check_procs(procs, "full_vocab_sample");
   constexpr size_t smem = (size_t)kFvThreads * kFvPer * sizeof(float);
   static bool attr_set = false;
   if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(full_vocab_sample_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) throw std::runtime_error(std::string("full_vocab_sample: cudaFuncSetAttribute: ") + cudaGetErrorString(e));
+    for (auto k : {full_vocab_sample_kernel<false>, full_vocab_sample_kernel<true>}) {
+      cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+      if (e != cudaSuccess) throw std::runtime_error(std::string("full_vocab_sample: cudaFuncSetAttribute: ") + cudaGetErrorString(e));
+    }
     attr_set = true;
   }
-  launch_k(full_vocab_sample_kernel, dim3(rows), dim3(kFvThreads), smem, stream, N, V, logits, ldl, temperature, top_p, ban_tokens, ban_count, ban_stride,
-           T, seed, row_offset, d_seed, d_step, eos, seq, cur_tokens, prefix, prefix_stride, out_tokens);
+  launch_k(procs.active() ? full_vocab_sample_kernel<true> : full_vocab_sample_kernel<false>, dim3(rows), dim3(kFvThreads), smem, stream, N, V, logits, ldl, temperature, top_p, ban_tokens, ban_count, ban_stride,
+           T, seed, row_offset, d_seed, d_step, eos, seq, cur_tokens, prefix, prefix_stride, out_tokens, procs);
   return 1;
 }
 int launch_sample_init(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,

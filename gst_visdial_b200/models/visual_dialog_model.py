@@ -57,6 +57,9 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
       do_sample=False    with num_beams > 1: beam sampling (HF beam_sample; contract: oracle/beam_sample.py) with temperature / top_k /
                          top_p; num_return_sequences = N runs N independent searches per image, search n seeded candidate_seed(seed, n).
                          Beam groups cannot be combined with it (HF rejects that too).  With num_beams = 1 the sampler runs either way
+      repetition_penalty=1.0, no_repeat_ngram_size=0, min_length=0   HF's logits processors (HF names; 1 / 0 / 0 = off) on each row's
+                         own decoder input, dec_input_ids included; min_length counts the decoder input, not new tokens (contract:
+                         oracle/processors.py and gstvd_generate in include/gstvd.h)
       seed=None          sampling seed (a per-call counter when None)
       enc_valid_len=None   upper bound (python int) on the number of leading history positions that hold a token in ANY row.
                          The encoder, the cross-K/V prefill and the cross-attention then run on ceil32(bound) text positions
@@ -176,6 +179,10 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
             if groups > 1 and gen_kw["num_beams"] <= 1:
                 raise ValueError(f"num_beam_groups = {groups} needs beam search (num_beams > 1)")
             gen_kw.update(num_beam_groups=groups, diversity_penalty=penalty)
+        procs = dict(repetition_penalty=float(decoding_kwargs.get("repetition_penalty", 1.0)),
+                     no_repeat_ngram_size=int(decoding_kwargs.get("no_repeat_ngram_size", 0)), min_length=int(decoding_kwargs.get("min_length", 0)))
+        if procs != dict(repetition_penalty=1.0, no_repeat_ngram_size=0, min_length=0):
+            gen_kw.update(procs)
         if decoding_kwargs.get("do_sample", False):
             if groups > 1:
                 raise ValueError(f"num_beam_groups = {groups} cannot be combined with do_sample (beam sampling)")

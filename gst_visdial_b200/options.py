@@ -49,6 +49,14 @@ def read_command_line(argv=None):
                         'temperature 0.7 and top-k 7; with -answer_candidates N, N independent searches per image')
     p.add_argument('-q_beam_sample', action='store_true',
                    help='beam sampling for the questions: -q_num_beams > 1 beams drawn with temperature 0.7 and top-k 7')
+    for who, what in (('', 'answers'), ('q_', 'questions')):
+        p.add_argument(f'-{who}repetition_penalty', default=1.0, type=float,
+                       help=f'HF repetition penalty for the {what}: scores of ids already in the decoder input are divided (or, when '
+                            'negative, multiplied) by it; 1 = off')
+        p.add_argument(f'-{who}no_repeat_ngram_size', default=0, type=int,
+                       help=f'HF no_repeat_ngram_size for the {what}: no n-gram occurs twice in the decoder input; 0 = off')
+        p.add_argument(f'-{who}min_length', default=0, type=int,
+                       help=f'HF min_length for the {what}: [SEP] is banned while the decoder input ([CLS] included) is shorter; 0 = off')
     p.add_argument('-answer_candidates', default=1, type=int,
                    help='>1: the teacher draws this many answers per round (samples, or the best of its -num_beams beams) and the one with '
                         'the lowest perplexity goes into the dialog')
@@ -67,6 +75,13 @@ def read_command_line(argv=None):
             p.error(f"-{groups} {params[groups]} must be 1 or divide -{beams} {params[beams]} > 1")
         if not (0.0 <= params[penalty] < float('inf')):
             p.error(f"-{penalty} must be finite and >= 0")
+    for who in ('', 'q_'):
+        rp = params[f'{who}repetition_penalty']
+        if not (0.0 < rp < float('inf')):
+            p.error(f"-{who}repetition_penalty must be finite and > 0 (1 = off)")
+        for name in ('no_repeat_ngram_size', 'min_length'):
+            if params[who + name] < 0:
+                p.error(f"-{who}{name} must be >= 0 (0 = off)")
     for flag, beams, groups in (('beam_sample', 'num_beams', 'num_beam_groups'), ('q_beam_sample', 'q_num_beams', 'q_num_beam_groups')):
         if params[flag] and (params[beams] <= 1 or params[groups] > 1):
             p.error(f"-{flag} needs -{beams} > 1 and no beam groups")

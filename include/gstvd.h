@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define GSTVD_ABI_VERSION 3
+#define GSTVD_ABI_VERSION 4
 #define GSTVD_MAX_CONNECTIONS 16
 
 typedef enum {
@@ -97,6 +97,9 @@ typedef struct {
   int32_t num_return_sequences; /* N >= 1 sequences per image (HF num_return_sequences); contract at gstvd_generate */
   int32_t num_beam_groups;    /* G >= 1 (HF num_beam_groups): beam mode splits the K beams into G groups; 1 = plain beam search */
   float diversity_penalty;    /* Hamming penalty between beam groups (HF diversity_penalty), finite and >= 0 */
+  float repetition_penalty;   /* HF repetition_penalty, finite and > 0; 1 = off.  Logits processors: contract at gstvd_generate */
+  int32_t no_repeat_ngram_size; /* HF no_repeat_ngram_size (n-grams of the output itself), >= 0; 0 = off */
+  int32_t min_length;         /* HF min_length: [SEP] banned while the decoder input (prefix included) is shorter, >= 0; 0 = off */
 } gstvd_gen_params;
 
 #define GSTVD_MAX_TOP_K 16
@@ -204,7 +207,33 @@ int gstvd_prefill_cross(gstvd_ctx* ctx, int B, int Le, const float* enc_hidden, 
  *   5. the drawn entries, ordered by (w desc, k*V + w asc), go through BeamSearchScorer.process as in beam search: [SEP] closes a
  *      hypothesis only at rank < K, a hypothesis scores its warped sum / (P + t), is_done uses the best drawn w.
  *   Rejected with GSTVD_ERR_INVALID: num_beams < 2 or > 8, N < 1, N*num_beams > max_beams, num_beam_groups > 1, a temperature that is
- *   not finite and > 0, top_p outside [0, 1].  Rejected with GSTVD_ERR_UNSUPPORTED: top_k = 0 or top_k > 16. */
+ *   not finite and > 0, top_p outside [0, 1].  Rejected with GSTVD_ERR_UNSUPPORTED: top_k = 0 or top_k > 16.
+ *
+ * Logits processors, every mode (HF RepetitionPenaltyLogitsProcessor, NoRepeatNGramLogitsProcessor, MinLengthLogitsProcessor;
+ * CPU oracle: oracle/processors.py).  d = a row's decoder input (HF input_ids) at step t: the image's decoder prefix with [SEP] read
+ * as [PAD] ([CLS] when prefix is NULL), then the row's own t generated tokens (a beam row: the tokens of that beam; a sample row's
+ * generated [SEP] is read as [PAD] too) - the key the question-history blocking uses.  cur_len = P + t.  The processors act on each
+ * row's score s at the point where the question-history bans act; -inf stays -inf:
+ *   1. repetition_penalty p (1 = off): each distinct id of d gets s < 0 ? fp32(s * p) : fp32(s / p), once however often it occurs
+ *      (HF's gather / scatter);
+ *   2. no_repeat_ngram_size n (0 = off), only when cur_len + 1 >= n: wherever the last n-1 ids of d occur earlier in d, the id that
+ *      follows them there gets -inf.  No special id is exempt (unlike the question-history rule): n = 1 bans every id of d, [CLS]
+ *      included;
+ *   3. min_length m (0 = off): [SEP] (102) gets -inf while cur_len < m; the unit is the HF 4.16.2 one, decoder-input length with the
+ *      prefix, not a count of new tokens.
+ *   What s is:
+ *   - sampling (top-k and top_k = 0): s = fp32(x / temperature); the processors act before top-k / top-p and the nucleus mass is
+ *     computed on the processed row.  (HF applies them before the temperature; the reference's loop divides first and then runs its
+ *     blocking processor, and this follows the reference.  The two orders differ only in fp32 rounding.)
+ *   - beam search and beam sampling: s = fp32(x - logZ), logZ over the unprocessed row; the processed value is what the beam score
+ *     accumulates, and so what out_scores reports.  Beam sampling's warpers then act on fp32(s + beam_score) as above.
+ *   - beam groups: the Hamming term first, then the repetition penalty (the order of HF _get_logits_processor): a penalised token
+ *     scores fp32(fp32(fp32(fp32(x - logZ) - fp32(lambda * c_w)) * p) + beam_score) (s / p for s >= 0).  The per-row candidate lists
+ *     are ranked by the processed score without the Hamming term; the Hamming term only lowers a score and the penalty is monotone,
+ *     so the lists still hold each group's exact top 2*gs (argument at beam_step_kernel, csrc/select.cu).
+ *   With p = 1, n = 0 and m = 0 a call launches the same kernels and gives the same results, bit for bit, as without the processors.
+ *   Rejected with GSTVD_ERR_INVALID: repetition_penalty not finite or <= 0, no_repeat_ngram_size < 0, min_length < 0 (so a
+ *   zero-filled params struct is rejected: fill every field). */
 int gstvd_generate(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, const int64_t* prefix, int P,
                    const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
                    int64_t* out_ids, float* out_scores, void* stream);
@@ -271,7 +300,8 @@ int gstvd_op_beam_step(gstvd_ctx* ctx, const float* logits, int64_t ldl, int32_t
                        float* next_scores, void* stream);
 int gstvd_op_beam_end(gstvd_ctx* ctx, int64_t* out_ids, float* out_scores, void* stream);
 /* top-k filter + greedy/multinomial on caller-supplied logits fp32 [rows, V]; prefix int64 [rows, prefix_len] holds
- * the decoded tokens so far (for n-gram blocking, may be NULL); out_tokens int32 [rows] */
+ * the decoded tokens so far (for n-gram blocking, may be NULL); out_tokens int32 [rows].  The logits processors of params act
+ * with d = prefix ([SEP] read as [PAD]) and need prefix_len = step + 1 <= 64 */
 int gstvd_op_sample(gstvd_ctx* ctx, int rows, const float* logits, int64_t ldl, const gstvd_gen_params* params,
                     const int64_t* hist_ids, const int64_t* hist_segments, int Lh, const int64_t* prefix, int prefix_len,
                     int step, int32_t* out_tokens, void* stream);
