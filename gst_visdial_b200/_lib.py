@@ -12,7 +12,7 @@ from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int6
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "lib", "libgstvd.so")
 
-GSTVD_ABI_VERSION = 4
+GSTVD_ABI_VERSION = 5
 GSTVD_MAX_CONNECTIONS = 16
 GSTVD_F32, GSTVD_BF16 = 0, 1
 GSTVD_SELECT_SAMPLE, GSTVD_SELECT_BEAM, GSTVD_SELECT_BEAM_SAMPLE = 0, 1, 2
@@ -78,9 +78,9 @@ SYMBOLS = [
     ("gstvd_op_add_layernorm", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     ("gstvd_op_attention", c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, c_float, c_int, _P, _P]),
     ("gstvd_op_deferred_ln_chain", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
-    ("gstvd_op_dec_self_attn", c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
+    ("gstvd_op_dec_self_attn", c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     ("gstvd_op_dec_cross_attn", c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, _P, _P, _P]),
-    ("gstvd_op_anc_update", c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, _P]),
+    ("gstvd_op_anc_update", c_int, [_P, c_int, c_int, c_int, c_int, _P, c_int, _P, _P, _P]),
     ("gstvd_debug_self_cache", c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     ("gstvd_op_beam_begin", c_int, [_P, c_int, c_int, c_int, _P]),
     ("gstvd_op_beam_step", c_int, [_P, _P, c_int64, _P, _P, _P, _P]),

@@ -3,8 +3,8 @@
 // The reference has no KV cache: it re-runs the whole decoder over the whole prefix and re-projects the
 // cross-attention K/V on every step (use_cache=False hard-wired, models/visual_dialog_decoder.py:64; loop at
 // models/visual_dialog_model.py:86-110).  Here each step processes ONE new position per beam row:
-//   dec_self_attn  : appends the new K/V at position g.P0 + *d_step and attends over positions 0..g.P0 + *d_step
-//                    (g.P0 = decoder prefix length - 1; positions below it were stored by prefix_kv_store)
+//   dec_self_attn  : appends the new K/V at position g.p0(b) + *d_step and attends over positions 0..g.p0(b) + *d_step
+//                    (g.p0(b) = image b's decoder prefix length - 1; positions below it were stored by prefix_kv_store)
 //   dec_cross_attn : every beam row of an image attends over that image's cross K/V (stored once per image)
 //   reorder_cache  : in-place beam gather, the semantic of _reorder_cache / index_select(0, beam_idx)
 //                    (models/visual_dialog_decoder.py:29-31,177-181)
@@ -57,7 +57,7 @@ dec_self_attn_kernel(DecodeGeom g, int layer, const T* __restrict__ qkv, T* __re
   const int h = blockIdx.y * 4 + warp;
   if (h >= g.heads) return;
   const int b = row / g.K, kb = row - b * g.K;
-  const int step = g.P0 + *d_step;             // cache position of the new token
+  const int step = g.p0(b) + *d_step;          // cache position of the new token
   const int H = g.H, D = g.D;
   constexpr int nd = ND;                       // dims per lane (2 for D=64, 4 for D=128)
   const T* qrow = qkv + (int64_t)row * 3 * H + h * D;
@@ -191,8 +191,9 @@ dec_self_attn_v2_kernel(DecodeGeom g, int layer, const bf16* __restrict__ qkv, b
   const uint4 vn_raw = *reinterpret_cast<const uint4*>(qrow + 2 * H);
   // step_host >= 0: the launch knows the step (eager loops and the all-steps graph unroll them), so the loads below are bounded by
   // it - on average half of the g.T cache rows - without waiting for *d_step; otherwise every row is requested and masked afterwards
-  const int step = g.P0 + (step_host >= 0 ? step_host : *d_step);   // cache position of the new token
-  const int bound = step_host >= 0 ? step : g.T;                   // cache positions < bound are requested
+  // cache position of the new token; g.P0s is read after the PDL wait (the init kernel that wrote it may precede this launch)
+  const int step = g.p0(b) + (step_host >= 0 ? step_host : *d_step);
+  const int bound = step_host >= 0 ? step : g.T;                     // cache positions < bound are requested (per row)
   // element offset of (kv, position t) for this beam / head / chunk
   const int64_t pos_stride = (int64_t)g.K * H;
   const int64_t k_base = ((((int64_t)layer * 2 + 0) * g.B + b) * g.T) * pos_stride + h * 64 + chunk * 8;   // slot 0 of position 0
@@ -200,7 +201,7 @@ dec_self_attn_v2_kernel(DecodeGeom g, int layer, const bf16* __restrict__ qkv, b
   // Beam search without moving the cache (anc != null): position t of this beam's history lives in the slot of the beam that
   // wrote it, anc[(b*K + kb)*W + t] (anc_update_kernel permutes the W-byte rows after every selection); the new position is
   // always written to the beam's own slot.  Entries at or past the new position are stale but always < 8; they are clamped and
-  // masked.  Prefix positions (below g.P0) hold the same K / V in every slot, so whatever their entries say is correct.
+  // masked.  Prefix positions (below g.p0(b)) hold the same K / V in every slot, so whatever their entries say is correct.
   constexpr int W = AncRow<NIT>::value;
   int slot[NIT];
 #pragma unroll
@@ -608,14 +609,15 @@ void launch_cross_t(const DecodeGeom& g, const void* q, const void* kv_layer, co
 // parent's row and the position just written (t = *d_step) is found in the parent's slot.  One CTA per image; every entry is
 // read before any is written (parents may repeat).  Replaces reorder_cache_kernel (up to 2 x 100 MB of HBM traffic per step at
 // B = 64, K = 5) when the self-attention kernel reads through the table (dec_self_attn_v2_kernel).  W = row width (positions);
-// the position just written is p0 + *d_step.
+// the position just written is p0 + *d_step, p0 = p0s[b] (per-image decoder prefixes) or the uniform p0.
 template <int W>
 __global__ void __launch_bounds__(kMaxBeams * W)
-anc_update_kernel(int B, int K, int p0, const int32_t* __restrict__ beam_idx, const int* __restrict__ d_step, uint8_t* __restrict__ anc) {
+anc_update_kernel(int B, int K, int p0, const int* __restrict__ p0s, const int32_t* __restrict__ beam_idx, const int* __restrict__ d_step,
+                  uint8_t* __restrict__ anc) {
   pdl_wait();
   pdl_launch_dependents();
   const int b = blockIdx.x, k = threadIdx.x / W, t = threadIdx.x % W;
-  const int step = p0 + *d_step;
+  const int step = (p0s ? p0s[b] : p0) + *d_step;
   int val = 0;
   const bool live = k < K && t <= step;
   if (live) {
@@ -657,7 +659,7 @@ reorder_cache_kernel(DecodeGeom g, T* __restrict__ cache, const int32_t* __restr
   pdl_launch_dependents();
   const int b = blockIdx.x, lk = blockIdx.y;
   if (d_skip && d_skip[b]) return;
-  const int len = d_len ? (*d_len + 1) : len_host;   // positions after the prefix rows (identical in every slot, never moved)
+  const int len = d_len ? (*d_len + 1) : len_host;   // positions after the image's prefix rows (identical in every slot, never moved)
   int parent[kMaxBeams];
   bool moved = false;
 #pragma unroll
@@ -667,7 +669,7 @@ reorder_cache_kernel(DecodeGeom g, T* __restrict__ cache, const int32_t* __restr
   }
   if (!moved) return;
   const int chunks = g.H / 8;
-  T* base = cache + (((int64_t)lk * g.B + b) * g.T + g.P0) * g.K * g.H;
+  T* base = cache + (((int64_t)lk * g.B + b) * g.T + g.p0(b)) * g.K * g.H;
   for (int i = threadIdx.x; i < len * chunks; i += blockDim.x) {
     const int t = i / chunks, c = (i - t * chunks) * 8;
     T* p = base + (int64_t)t * g.K * g.H + c;
@@ -729,8 +731,8 @@ bool dec_cross_supports(int kernel, int dtype, const DecodeGeom& g) {
 
 int launch_anc_update(const DecodeGeom& g, const int32_t* beam_idx, const int* d_step, uint8_t* anc, cudaStream_t stream) {
   if (g.K > kMaxBeams || g.T > kMaxPos) throw std::runtime_error("anc_update: at most 8 beams and 64 positions");
-  if (g.T <= kMaxSteps) launch_k(anc_update_kernel<kMaxSteps>, dim3(g.B), dim3(kMaxBeams * kMaxSteps), 0, stream, g.B, g.K, g.P0, beam_idx, d_step, anc);
-  else launch_k(anc_update_kernel<kMaxPos>, dim3(g.B), dim3(kMaxBeams * kMaxPos), 0, stream, g.B, g.K, g.P0, beam_idx, d_step, anc);
+  if (g.T <= kMaxSteps) launch_k(anc_update_kernel<kMaxSteps>, dim3(g.B), dim3(kMaxBeams * kMaxSteps), 0, stream, g.B, g.K, g.P0, g.P0s, beam_idx, d_step, anc);
+  else launch_k(anc_update_kernel<kMaxPos>, dim3(g.B), dim3(kMaxBeams * kMaxPos), 0, stream, g.B, g.K, g.P0, g.P0s, beam_idx, d_step, anc);
   return 1;
 }
 

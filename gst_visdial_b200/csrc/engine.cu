@@ -123,6 +123,7 @@ struct gstvd_ctx {
   DevBuf d_step, d_seed;
   DevBuf anc;                                         // uint8 [B*K][64]: beam ancestry table (launch_anc_update; rows of 32 up to 32 positions)
   DevBuf dec_prefix_own, dec_prefix_head;             // int64 [B_max, max_dec_len]: decoder prefix of a call; [B, P-1]: its prefill ids
+  DevBuf prefix_p0;                                   // int32 [B_max]: each image's decoder prefix length - 1 (DecodeGeom::P0s)
   DevBuf fold16, foldvec;                             // deferred LayerNorm: folded bf16 weights, c / d vectors
   DevBuf st1, st2, st3;                               // float2 [rows][kLnStatStride]: partial row statistics of the raw x1 / x2 / x3
   bool fold_ready = false;
@@ -343,7 +344,7 @@ void alloc_workspace(gstvd_ctx* c) {
     // outputs and sample-mode state hold up to K_max rows per image: N-best beams / N sampled candidates
     c->r_out_ids.alloc(B * K * T * 8); c->r_out_scores.alloc(B * K * 4);
     c->prefix.alloc(B * K * (T + c->Ldec_max) * 4); c->seq.alloc(B * K * T * 4);
-    c->dec_prefix_own.alloc(B * c->Ldec_max * 8); c->dec_prefix_head.alloc(B * c->Ldec_max * 8);
+    c->dec_prefix_own.alloc(B * c->Ldec_max * 8); c->dec_prefix_head.alloc(B * c->Ldec_max * 8); c->prefix_p0.alloc(B * 4);
     c->beam_scores.alloc(B * K * 4); c->beam_tokens.alloc(2 * B * K * T * 4); c->cur_tokens.alloc(R * 4);
     // hypothesis heaps: one per search of K beams with K + 1 slots.  Beam search: B searches of K <= K_max beams; beam sampling: B * N
     // searches of K >= 2 beams with N * K <= K_max, i.e. at most B * K_max / 2 searches and B * (K_max + K_max / 2) slots.
@@ -593,11 +594,14 @@ void do_prefill(gstvd_ctx* c, int B, int Le, const float* enc_hidden, const floa
   c->cross_B = B; c->cross_Le = Le;
 }
 
-// T = new tokens; P = decoder prefix length (its first P - 1 positions are prefilled, the last one is the first step's input)
-DecodeGeom make_geom(gstvd_ctx* c, int B, int K, int T, int P = 1) {
+// T = new tokens; P = decoder prefix length (its first P - 1 positions are prefilled, the last one is the first step's input).
+// ragged: a caller's prefix of P > 1 columns, whose rows may end early at a negative id; the decode kernels then read every image's
+// own length from the context buffer decode_init fills (a P = 1 prefix has one length and keeps the uniform path).
+DecodeGeom make_geom(gstvd_ctx* c, int B, int K, int T, int P = 1, bool ragged = false) {
   DecodeGeom g;
   g.B = B; g.K = K; g.H = c->H; g.heads = c->dec_heads; g.D = c->H / c->dec_heads; g.layers = c->dec_layers; g.T = P - 1 + T; g.Le = c->cross_Le;
   g.P0 = P - 1;
+  if (ragged && P > 1) g.P0s = (const int*)c->prefix_p0.p;
   return g;
 }
 
@@ -650,7 +654,9 @@ void dec_teacher_layers(gstvd_ctx* c, Exec& X, int B, int L, const float* dec_ma
 
 // Decoder prefix prefill: a teacher-forced pass over the first P0 = P - 1 prefix positions of the g.B images (ids in
 // c->dec_prefix_head, [SEP] embedded as [PAD] like the in-place replacement of models/visual_dialog_decoder.py:57) that leaves every
-// layer's K / V of those positions in the self cache.  P = 1 launches nothing.
+// layer's K / V of those positions in the self cache.  P = 1 launches nothing.  A shorter prefix (image b: P_b = g.p0(b) + 1 tokens)
+// runs in the same pass with its negative ids embedded as [PAD]: the pass is causal, so positions below P_b - 1 see only the image's
+// own prefix and are exact; the rest are padding that b's decode steps overwrite before they read them.
 void prefix_prefill(gstvd_ctx* c, const DecodeGeom& g, cudaStream_t s) {
   if (g.P0 == 0) return;
   PdlScope pdl_scope(!(c->cfg.flags & GSTVD_FLAG_NO_PDL));
@@ -671,16 +677,18 @@ const int64_t* stage_prefix(gstvd_ctx* c, int B, const int64_t* prefix, int P, c
   return (const int64_t*)c->dec_prefix_own.p;
 }
 
-// Selection state of a decode call: beams / sample rows start from the last token of the prefix (the [CLS] when it is null).
+// Selection state of a decode call: beams / sample rows start from the last token of the prefix (the [CLS] when it is null).  The same
+// launch writes every image's prefix length - 1 into g.P0s when the geometry has per-image lengths.
 void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* prefix, cudaStream_t s) {
   const int P = g.P0 + 1, T = gp.max_new_tokens;
+  int* p0s = const_cast<int*>(g.P0s);
   if (gp.mode == GSTVD_SELECT_BEAM)
-    c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, gp.num_beam_groups, 1, T, 101, prefix, P, s);
+    c->launches += launch_beam_init(beam_buffers(c), g.B, g.K, gp.num_beam_groups, 1, T, 101, prefix, P, p0s, s);
   else if (gp.mode == GSTVD_SELECT_BEAM_SAMPLE) {
     const int K = gp.num_beams, N = g.K / K;      // N searches of K beams per image, all beams at score 0
-    c->launches += launch_beam_init(beam_buffers(c), g.B * N, K, K, N, T, 101, prefix, P, s);
+    c->launches += launch_beam_init(beam_buffers(c), g.B * N, K, K, N, T, 101, prefix, P, p0s, s);
   } else c->launches += launch_sample_init(g.B * g.K, g.K, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, P + T, (int*)c->d_step.p,
-                                         prefix, P, s);
+                                         prefix, P, p0s, s);
 }
 
 // The request's logits processors; the caller fills in where the rows' decoder input lives.
@@ -693,7 +701,7 @@ LogitsProcs logits_procs(const gstvd_gen_params& gp) {
 // One decode step for all M = B*K rows: embeddings -> 12 x [self-attn over cache, cross-attn, FFN] -> LM head -> selection.
 // step_host = index of this step when the caller knows it (it always does: eager loops and the captured graph both unroll the
 // steps), so kernels that only need it to bound their loads take it as a launch parameter instead of reading *d_step first.
-// prefix: int64 [B, P] decoder prefix (P = g.P0 + 1), null for the [CLS] start.
+// prefix: int64 [B, P] decoder prefix (P = g.P0 + 1), null for the [CLS] start; image b's own length is g.p0(b) + 1.
 void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, const int64_t* prefix, const int64_t* hist_ids,
                  const int64_t* hist_seg, int Lh, cudaStream_t s, int step_host) {
   Exec X{c, s};
@@ -708,7 +716,7 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   const bool use_anc = beams && (anc_env == nullptr || atoi(anc_env) != 0) &&
                        dec_self_attn_v2_active(c->dtype, g, c->dqkv.p, c->self_cache.p, c->dctx.p);
   const uint8_t* anc = use_anc ? (const uint8_t*)c->anc.p : nullptr;
-  c->launches += launch_embed_step(c->dtype, M, H, (const int32_t*)c->cur_tokens.p, g.P0, d_step, c->word, c->pos, c->type,
+  c->launches += launch_embed_step(c->dtype, M, H, (const int32_t*)c->cur_tokens.p, g.P0, g.P0s, g.K, d_step, c->word, c->pos, c->type,
                                    c->emb_ln.g, c->emb_ln.b, c->dh.p, s);
   // Deferred LayerNorm (default for bf16): no LayerNorm kernel inside the layer stack - the three dense -> LN(x + input) pairs of a
   // layer store raw sums + partial row statistics, their consumers normalise on the fly (GemmArgs::fold_* / res_*), and one
@@ -760,7 +768,7 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   float* sv = (float*)c->sel_val.p; int32_t* si = (int32_t*)c->sel_idx.p;
   // the logits processors act inside the selection kernels; each reads its rows' decoder input (cur_len = P + step <= 64)
   LogitsProcs procs = logits_procs(gp);
-  procs.P = P; procs.step = step_host; procs.d_step = d_step;
+  procs.P = P; procs.step = step_host; procs.d_step = d_step; procs.p0s = g.P0s; procs.rows_per_image = g.K;
   if (beams) {
     // beam sampling: g.K = N * K rows per image (N searches of K beams), each row's 16 best for the warpers and the draw
     const bool sampled = gp.mode == GSTVD_SELECT_BEAM_SAMPLE;
@@ -771,9 +779,10 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     const int32_t* bt = nullptr; const int32_t* bc = nullptr;
     // n-gram blocking: nothing to launch while every key is shorter than n-1 tokens (P + t < n-1) or, for the [CLS] start, still
     // holds the [CLS], which no banned n-gram contains (t < n-1).  A caller's prefix may hold anything: no position is known special.
+    // With per-image lengths the condition uses the longest, P; the kernel skips the images whose key is still too short.
     const int n = gp.ngram_blocking_size;
     if (n > 0 && step_host >= (prefix ? n - 1 - P : n - 1)) {
-      c->launches += launch_beam_ngram_ban(g.B, g.K, Tn, Lh, hist_ids, hist_seg, prefix, P, bb.tokens + (int64_t)(step_host & 1) * M * Tn,
+      c->launches += launch_beam_ngram_ban(g.B, g.K, Tn, Lh, hist_ids, hist_seg, prefix, P, g.P0s, bb.tokens + (int64_t)(step_host & 1) * M * Tn,
                                            step_host, n, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }
@@ -782,16 +791,16 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     const int G = gp.num_beam_groups;
     float* lz = G > 1 ? (float*)c->logz.p : nullptr;
     // a beam row's decoder input: the image's prefix, then the beam's tokens in the token buffer of this step's parity
-    procs.prefix = prefix; procs.tokens = bb.tokens + (int64_t)(step_host & 1) * M * Tn; procs.tok_stride = Tn; procs.rows_per_image = g.K;
+    procs.prefix = prefix; procs.tokens = bb.tokens + (int64_t)(step_host & 1) * M * Tn; procs.tok_stride = Tn;
     c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, (c->dtype == kBF16 && !exact_lse) ? 2 : 0,
                                      (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, lz, procs, s);
     if (sampled) {
       const int K = gp.num_beams;
       c->launches += launch_beam_sample_step(bb, M / K, g.K / K, K, Tn, c->V, sv, si, gp.top_k, gp.temperature, gp.top_p,
-                                             (const uint64_t*)c->d_seed.p, 102, P, s);
+                                             (const uint64_t*)c->d_seed.p, 102, P, g.P0s, s);
     } else {
       c->launches += launch_beam_step(bb, g.B, g.K, G, Tn, c->V, nsel, sv, si, G > 1 ? (const float*)c->logits.p : nullptr, c->Vpad, lz,
-                                      gp.diversity_penalty, gp.repetition_penalty, prefix, 102, P, nullptr, nullptr, nullptr, s);
+                                      gp.diversity_penalty, gp.repetition_penalty, prefix, 102, P, g.P0s, nullptr, nullptr, nullptr, s);
     }
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
@@ -799,7 +808,8 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     // g.K rows per image: the num_return_sequences sampled candidates, each with its own n-gram key and RNG stream
     const int nsel = kSelMax;
     const int32_t* bt = nullptr; const int32_t* bc = nullptr;
-    // key buffer c->prefix [M, P + Tn]: the decoder prefix, then the generated tokens; the samplers append token t at P + t
+    // key buffer c->prefix [M, P + Tn]: the decoder prefix (right-aligned when it is shorter than P), then the generated tokens; the
+    // samplers append token t at P + t
     const int kst = P + Tn;
     int32_t* key_next = (int32_t*)c->prefix.p + (P - 1);
     if (gp.ngram_blocking_size > 0) {
@@ -875,11 +885,11 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* pref
 }
 
 // out_ids [B*N, T] image-major (sample mode: N == K, one row per candidate)
-void generate_finalize(gstvd_ctx* c, int B, int K, int P, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
-  const int T = gp.max_new_tokens, N = gp.num_return_sequences;
-  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, P, N, out_ids, out_scores, s);
+void generate_finalize(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
+  const int B = g.B, K = g.K, P = g.P0 + 1, T = gp.max_new_tokens, N = gp.num_return_sequences;
+  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, P, g.P0s, 1, N, out_ids, out_scores, s);
   else if (gp.mode == GSTVD_SELECT_BEAM_SAMPLE)   // search n of image b is search b * N + n: its best hypothesis is output row b * N + n
-    c->launches += launch_beam_finalize(beam_buffers(c), B * N, gp.num_beams, T, 102, P, 1, out_ids, out_scores, s);
+    c->launches += launch_beam_finalize(beam_buffers(c), B * N, gp.num_beams, T, 102, P, g.P0s, N, 1, out_ids, out_scores, s);
   else c->launches += launch_sample_finalize(B * K, T, 102, (const int32_t*)c->seq.p, out_ids, s);
 }
 
@@ -935,8 +945,8 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
   const int K = check_generate(c, gp, prefix, P, hist_ids, hist_seg, Lh, out_ids);
   if (c->cross_B != B) throw StateError(fmt("generate: cross K/V prefilled for %d images, asked for %d", c->cross_B, B));
   const int T = gp.max_new_tokens;
-  const DecodeGeom g = make_geom(c, B, K, T, P);
   const int64_t* pre = stage_prefix(c, B, prefix, P, s);
+  const DecodeGeom g = make_geom(c, B, K, T, P, pre != nullptr);
   // the sampling seed lives in device memory so that a captured graph can be replayed with a new seed
   c->launches += launch_set_u64((uint64_t*)c->d_seed.p, gp.seed, (uint64_t)gp.row_offset, s);
   decode_init(c, g, gp, pre, s);
@@ -956,7 +966,7 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
   // the cross cache geometry (Le) is part of the captured launch parameters
   if (!use_graph) body();
   else replay_graph(c, c->graphs, graph_key(gp, B, K, P, pre, Lh, c->cross_Le, 0, 0, false, false, false, false), s, body);
-  generate_finalize(c, B, K, P, gp, out_ids, out_scores, s);
+  generate_finalize(c, g, gp, out_ids, out_scores, s);
 }
 
 // One forward call of the decode branch of EncoderDecoderModel.forward (models/visual_dialog_model.py:24-120) - encoder, fusion,
@@ -983,11 +993,11 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
     do_encode(c, B, Lt, Lv, g_ids, g_seg, att ? (const float*)c->r_att.p : nullptr, (const float*)c->r_feat.p, (const float*)c->r_loc.p,
               imask ? (const float*)c->r_imask.p : nullptr, nullptr, nullptr, nullptr, nullptr, nullptr, s);
     do_prefill(c, B, Lv + Lt, nullptr, nullptr, s);
-    const DecodeGeom g = make_geom(c, B, K, T, P);
+    const DecodeGeom g = make_geom(c, B, K, T, P, pre != nullptr);
     decode_init(c, g, gp, pre, s);
     prefix_prefill(c, g, s);
     for (int t = 0; t < T; ++t) decode_step(c, g, gp, pre, g_ids, g_seg, Lt, s, t);
-    generate_finalize(c, B, K, P, gp, (int64_t*)c->r_out_ids.p, out_scores ? (float*)c->r_out_scores.p : nullptr, s);
+    generate_finalize(c, g, gp, (int64_t*)c->r_out_ids.p, out_scores ? (float*)c->r_out_scores.p : nullptr, s);
   };
   const bool use_graph = !(c->cfg.flags & GSTVD_FLAG_NO_CUDA_GRAPH) && !c->profiling;
   if (!use_graph) {
@@ -1135,7 +1145,7 @@ void gstvd_destroy(gstvd_ctx* c) {
                     &c->tmp_v, &c->ffn_t, &c->ffn_v, &c->feat_cast, &c->fused, &c->pool, &c->fused_mask, &c->dh, &c->da, &c->db, &c->dqkv,
                     &c->dctx, &c->dtmp, &c->dffn, &c->dqc, &c->logits, &c->cross_cache, &c->self_cache, &c->cross_len, &c->labels, &c->sel_val, &c->sel_idx,
                     &c->logz, &c->ban_tokens, &c->ban_count, &c->prefix, &c->seq, &c->beam_scores, &c->beam_tokens, &c->cur_tokens,
-                    &c->beam_idx, &c->beam_done, &c->hyp_score, &c->hyp_len, &c->hyp_tokens, &c->hyp_count, &c->hyp_worst, &c->d_step, &c->d_seed, &c->anc, &c->dec_prefix_own, &c->dec_prefix_head, &c->fold16, &c->foldvec,
+                    &c->beam_idx, &c->beam_done, &c->hyp_score, &c->hyp_len, &c->hyp_tokens, &c->hyp_count, &c->hyp_worst, &c->d_step, &c->d_seed, &c->anc, &c->dec_prefix_own, &c->dec_prefix_head, &c->prefix_p0, &c->fold16, &c->foldvec,
                     &c->st1, &c->st2, &c->st3, &c->hist_ids_own, &c->hist_seg_own, &c->r_ids, &c->r_seg, &c->r_att,
                     &c->r_feat, &c->r_loc, &c->r_imask, &c->r_out_ids, &c->r_out_scores};
   for (DevBuf* b : bufs) b->release();
@@ -1470,8 +1480,19 @@ int gstvd_op_attention(gstvd_ctx* c, int dtype, int B, int H, int Lq, int Lk, in
 }
 
 // ---- decode-step attention kernels, one at a time (parity tests): own DecodeGeom with one layer, independent of the context's caches ----
-int gstvd_op_dec_self_attn(gstvd_ctx* c, int dtype, int kernel, int B, int K, int heads, int D, int T, int P0, int step, int step_known,
-                           const float* qkv, const float* prefix_qkv, float* cache, const uint8_t* anc, float* out, void* stream) {
+// Per-image P0 values (int32 [B] on the device) are checked against 0 <= p0s[b] <= P0 on the host before any launch.
+static void check_p0s(const int32_t* p0s, int B, int P0, cudaStream_t s, const char* who) {
+  if (!p0s) return;
+  std::vector<int32_t> h(B);
+  CUDA_CHECK(cudaMemcpyAsync(h.data(), p0s, (size_t)B * 4, cudaMemcpyDeviceToHost, s));
+  CUDA_CHECK(cudaStreamSynchronize(s));
+  for (int b = 0; b < B; ++b)
+    if (h[b] < 0 || h[b] > P0) throw InvalidArg(fmt("%s: p0s[%d] = %d outside 0..P0 (%d)", who, b, h[b], P0));
+}
+
+int gstvd_op_dec_self_attn(gstvd_ctx* c, int dtype, int kernel, int B, int K, int heads, int D, int T, int P0, const int32_t* p0s, int step,
+                           int step_known, const float* qkv, const float* prefix_qkv, float* cache, const uint8_t* anc, float* out,
+                           void* stream) {
   if (!c) return GSTVD_ERR_INVALID;
   return guarded(c, [&] {
     if (dtype != kF32 && dtype != kBF16) throw InvalidArg("op_dec_self_attn: dtype");
@@ -1481,8 +1502,9 @@ int gstvd_op_dec_self_attn(gstvd_ctx* c, int dtype, int kernel, int B, int K, in
     if (!qkv || !cache || !out) throw InvalidArg("op_dec_self_attn: NULL buffer");
     if (prefix_qkv && P0 < 1) throw InvalidArg("op_dec_self_attn: prefix_qkv needs P0 >= 1");
     cudaStream_t s = (cudaStream_t)stream;
+    check_p0s(p0s, B, P0, s, "op_dec_self_attn");
     DecodeGeom g;
-    g.B = B; g.K = K; g.H = heads * D; g.heads = heads; g.D = D; g.layers = 1; g.T = T; g.Le = 0; g.P0 = P0;
+    g.B = B; g.K = K; g.H = heads * D; g.heads = heads; g.D = D; g.layers = 1; g.T = T; g.Le = 0; g.P0 = P0; g.P0s = p0s;
     const int64_t M = (int64_t)B * K, n_qkv = M * 3 * g.H, n_pre = (int64_t)B * P0 * 3 * g.H, n_cache = (int64_t)2 * B * T * K * g.H;
     Scratch sc;
     int* d_step = (int*)sc.get(4);
@@ -1548,15 +1570,17 @@ int gstvd_op_dec_cross_attn(gstvd_ctx* c, int dtype, int kernel, int B, int K, i
   });
 }
 
-int gstvd_op_anc_update(gstvd_ctx* c, int B, int K, int T, int P0, int step, const int32_t* beam_idx, uint8_t* anc, void* stream) {
+int gstvd_op_anc_update(gstvd_ctx* c, int B, int K, int T, int P0, const int32_t* p0s, int step, const int32_t* beam_idx, uint8_t* anc,
+                        void* stream) {
   if (!c) return GSTVD_ERR_INVALID;
   return guarded(c, [&] {
     if (B < 1 || K < 1 || K > 8 || T < 1 || T > 64 || P0 < 0 || step < 0 || P0 + step >= T)
       throw InvalidArg("op_anc_update: shape out of range (K <= 8, T <= 64, P0 + step < T)");
     if (!beam_idx || !anc) throw InvalidArg("op_anc_update: NULL buffer");
     cudaStream_t s = (cudaStream_t)stream;
+    check_p0s(p0s, B, P0, s, "op_anc_update");
     DecodeGeom g;
-    g.B = B; g.K = K; g.H = 0; g.heads = 0; g.D = 0; g.layers = 1; g.T = T; g.Le = 0; g.P0 = P0;
+    g.B = B; g.K = K; g.H = 0; g.heads = 0; g.D = 0; g.layers = 1; g.T = T; g.Le = 0; g.P0 = P0; g.P0s = p0s;
     Scratch sc;
     int* d_step = (int*)sc.get(4);
     CUDA_CHECK(cudaMemcpyAsync(d_step, &step, 4, cudaMemcpyHostToDevice, s));
@@ -1571,7 +1595,7 @@ int gstvd_op_beam_begin(gstvd_ctx* c, int B, int K, int max_new, void* stream) {
     if (c->dec_layers == 0) throw StateError("beam ops need a decoder context");
     if (B < 1 || B > c->B_max || K < 1 || K > c->K_max || max_new < 1 || max_new > c->T_max) throw InvalidArg("beam_begin: shape out of range");
     c->op_B = B; c->op_K = K; c->op_T = max_new;
-    c->launches += launch_beam_init(beam_buffers(c), B, K, 1, 1, max_new, 101, nullptr, 1, (cudaStream_t)stream);
+    c->launches += launch_beam_init(beam_buffers(c), B, K, 1, 1, max_new, 101, nullptr, 1, nullptr, (cudaStream_t)stream);
   });
 }
 
@@ -1585,7 +1609,7 @@ int gstvd_op_beam_step(gstvd_ctx* c, const float* logits, int64_t ldl, int32_t* 
     c->launches += launch_row_select(B * K, c->V, logits, ldl, 0, (const float*)c->beam_scores.p, 1.f, nullptr, nullptr, 0, nsel,
                                      (float*)c->sel_val.p, (int32_t*)c->sel_idx.p, nullptr, LogitsProcs(), s);
     c->launches += launch_beam_step(beam_buffers(c), B, K, 1, T, c->V, nsel, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, nullptr,
-                                    0, nullptr, 0.f, 1.f, nullptr, 102, 1, beam_idx, next_tokens, next_scores, s);
+                                    0, nullptr, 0.f, 1.f, nullptr, 102, 1, nullptr, beam_idx, next_tokens, next_scores, s);
     c->launches += launch_step_advance((int*)c->d_step.p, s);
   });
 }
@@ -1594,7 +1618,7 @@ int gstvd_op_beam_end(gstvd_ctx* c, int64_t* out_ids, float* out_scores, void* s
   if (!c || !out_ids) return GSTVD_ERR_INVALID;
   return guarded(c, [&] {
     if (c->op_B == 0) throw StateError("beam_end before beam_begin");
-    c->launches += launch_beam_finalize(beam_buffers(c), c->op_B, c->op_K, c->op_T, 102, 1, 1, out_ids, out_scores, (cudaStream_t)stream);
+    c->launches += launch_beam_finalize(beam_buffers(c), c->op_B, c->op_K, c->op_T, 102, 1, nullptr, 1, 1, out_ids, out_scores, (cudaStream_t)stream);
     c->op_B = 0;
   });
 }

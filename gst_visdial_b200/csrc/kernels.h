@@ -103,12 +103,15 @@ int launch_fold_ln_weights(int N, int K, const float* W, const float* gamma, con
 int launch_ln_apply_stats(int rows, int width, const void* x, const float2* stats, int64_t stats_ld, int parts, const float* gamma,
                           const float* beta, void* y, cudaStream_t stream);
 // text embeddings: y[row] = LN(word[id] + pos[p] + type[seg]);  positions = row % L + pos_offset(*d_pos_offset if non-null)
+// eos_to_pad: [SEP] and negative ids (the end marker of a shorter decoder prefix) are embedded as [PAD]
 int launch_embed_text(int dtype, int rows, int L, int width, const int64_t* ids, const int64_t* seg, const int* d_pos_offset,
                       int eos_to_pad, const float* word, const float* pos, const float* type, const float* type_ext,
                       int type_vocab, const float* gamma, const float* beta, void* y, cudaStream_t stream);
-// decode-step embeddings from int32 current tokens (EOS -> PAD applied), position pos0 + *d_step
-int launch_embed_step(int dtype, int rows, int width, const int32_t* tokens, int pos0, const int* d_step, const float* word,
-                      const float* pos, const float* type, const float* gamma, const float* beta, void* y, cudaStream_t stream);
+// decode-step embeddings from int32 current tokens (EOS -> PAD applied), position P0 + *d_step with P0 = p0s[row / rows_per_image]
+// (per-image decoder prefix lengths - 1) or pos0 when p0s is null
+int launch_embed_step(int dtype, int rows, int width, const int32_t* tokens, int pos0, const int* p0s, int rows_per_image, const int* d_step,
+                      const float* word, const float* pos, const float* type, const float* gamma, const float* beta, void* y,
+                      cudaStream_t stream);
 // image embeddings: y = LN(x(+bias already) + loc * Wloc^T + bloc)
 int launch_image_embed_ln(int dtype, int rows, int width, const void* x, const float* loc, const float* wloc,
                           const float* bloc, const float* gamma, const float* beta, void* y, cudaStream_t stream);
@@ -130,6 +133,11 @@ struct DecodeGeom {
   int B, K, H, heads, D, layers, T;   // T = max positions in the self cache (P0 + new tokens)
   int Le;                             // encoder length (cross keys)
   int P0 = 0;                         // decoder prefix length - 1: cache positions 0..P0-1 hold the prefix (launch_prefix_kv_store)
+  // Per-image decoder prefixes of different lengths: int32 [B], image b's own P0 (<= P0; its prefix holds P0s[b] + 1 tokens), read
+  // by the kernels of the decode step.  Null: every image has P0.  Cache positions P0s[b] .. P0 - 1 of image b hold the prefill's
+  // padding rows until its decode steps overwrite them; a step never reads a position at or past its own.
+  const int* P0s = nullptr;
+  __host__ __device__ int p0(int b) const { return P0s ? P0s[b] : P0; }
 };
 // Forced kernel choices of the decode attention launchers (`force` argument; kDecDefault keeps the launcher's own choice,
 // environment switches included).  The single-kernel test entries use them; the decode step always passes kDecDefault.
@@ -137,7 +145,7 @@ constexpr int kDecDefault = -1;
 enum SelfAttnKernel { kSelfFirst = 0, kSelfV2 = 1 };
 enum CrossAttnKernel { kCrossWarpTma = 0, kCrossCtaTma = 1, kCrossMma = 2, kCrossSimt = 3, kCrossGeneric = 4 };
 
-// self-attention for one new position per row: appends k/v at position P0 + *d_step and attends over 0..P0 + *d_step
+// self-attention for one new position per row: appends k/v at position g.p0(b) + *d_step and attends over 0..g.p0(b) + *d_step
 // qkv [M, 3H]; cache layout [layer][kv][b][t][k][H]
 // step_host >= 0: the caller knows the step index (must equal *d_step); the lean kernel then only loads positions <= step
 // force: kDecDefault, kSelfFirst or kSelfV2 (dec_self_attn_supports must hold)
@@ -152,7 +160,8 @@ bool dec_self_attn_supports(int kernel, int dtype, const DecodeGeom& g, const vo
 // only the lean kernel reads it - pass null to the self-attention and call launch_reorder_cache otherwise
 int launch_anc_update(const DecodeGeom& g, const int32_t* beam_idx, const int* d_step, uint8_t* anc, cudaStream_t stream);
 // decoder prefix prefill: stores layer `layer`'s K / V of the qkv rows [B * P0][3H] (teacher-forced pass over the first P0 prefix
-// positions) into every beam slot of cache positions 0..P0-1; launches nothing when P0 = 0
+// positions) into every beam slot of cache positions 0..P0-1; launches nothing when P0 = 0.  With g.P0s the rows of image b past
+// its own g.p0(b) are padding, stored like the others and never read.
 int launch_prefix_kv_store(int dtype, const DecodeGeom& g, int layer, const void* qkv, void* self_cache, cudaStream_t stream);
 // cross-attention of every beam row over its image's cross K/V. cross layout [layer][b][kv*heads+h][Le][D]
 // force: kDecDefault, kCrossMma, kCrossSimt or kCrossGeneric (dec_cross_supports must hold)
@@ -170,7 +179,8 @@ int launch_cross_len(int B, int Le, const float* mask, int* out, cudaStream_t st
 void dec_cross_print_times();   // measurement aid (env GSTVD_CROSS_TIMES=1): per-CTA phase stamps of the last cross-attention launch
 // cached CUtensorMap (returned as an opaque pointer) over [groups][L][D] bf16 rows, box = D x box_rows (gemm_tc.cu)
 const void* tma_map_rows3(const void* ptr, int D, int L, int64_t groups, int box_rows);
-// in-place beam gather of the self cache over positions [0, len) ; len = *d_len if d_len else len_host
+// in-place beam gather of the self cache over the generated positions g.p0(b) .. g.p0(b) + len - 1 of image b;
+// len = *d_len + 1 if d_len else len_host
 int launch_reorder_cache(int dtype, const DecodeGeom& g, void* self_cache, const int32_t* beam_idx, const int* d_len,
                          int len_host, const uint8_t* d_skip, cudaStream_t stream);
 
@@ -186,7 +196,8 @@ constexpr int kProcMaxLen = 64;   // longest decoder input the logits processors
 //   min_length m (0 = off): [SEP] gets -inf while cur_len < m
 // d is read either from an int32 key buffer (sampling: keys [rows, key_stride], [SEP] already [PAD]) or from the int64 decoder prefix
 // [rows / rows_per_image, P] (null: [CLS], P = 1) followed by the beam token buffer tokens [rows, tok_stride] of this step's parity.
-// t = step, or *d_step when step < 0.
+// t = step, or *d_step when step < 0.  p0s (DecodeGeom::P0s, rows_per_image rows per image): image b's prefix is its first p0s[b] + 1
+// ids (cur_len = p0s[b] + 1 + t); a key row then holds it right-aligned, columns P - 1 - p0s[b] .. P - 1, before the generated tokens.
 struct LogitsProcs {
   float repetition_penalty = 1.f;
   int no_repeat_ngram = 0, min_length = 0;
@@ -194,6 +205,7 @@ struct LogitsProcs {
   const int64_t* prefix = nullptr; const int32_t* tokens = nullptr; int tok_stride = 0; int rows_per_image = 1;
   int P = 1, step = -1;
   const int* d_step = nullptr;
+  const int* p0s = nullptr;
   __host__ __device__ bool active() const { return repetition_penalty != 1.f || no_repeat_ngram > 0 || min_length > 0; }
 };
 
@@ -223,24 +235,29 @@ struct BeamBuffers {
 // prefix: int64 [B, P] decoder prefix (null: start_token, P = 1); len0 = P, the prefix length counted in every hypothesis length.
 // G beam groups of K / G beams (G | K; G = 1: plain beam search): the first beam of every group starts with score 0 (G = K: all beams).
 // B = searches of K beams, N consecutive searches per image (beam sampling; 1 otherwise): search s reads prefix row s / N.
-int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int N, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream);
+// Image b's prefix ends at its first negative id (prefix_len below); the first step's input is its last token.  p0s (may be null):
+// receives every image's prefix length - 1 (DecodeGeom::P0s).  The kernels below that take p0s read the image's own length from it
+// in place of len0 / P (null: len0 / P for every image).
+int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int N, int T, int start_token, const int64_t* prefix, int P, int* p0s,
+                     cudaStream_t stream);
 // Beam sampling (oracle/beam_sample.py): S = B * N searches of K beams, rows search-major; sel_val / sel_idx = row_select mode 0 / 2
 // output with nsel = kSelMax and the beam scores as row bias.  d_seed = {seed, row_offset} (device).  Parents are written image-local
 // (n * K + parent, n = s % N), so the cache reorder runs with N * K rows per image.
 int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, int V, const float* sel_val, const int32_t* sel_idx, int top_k,
-                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, cudaStream_t stream);
+                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, const int* p0s, cudaStream_t stream);
 // G > 1: diverse beam search with the Hamming penalty `penalty` (oracle/beam_groups.py).  A candidate whose token earlier groups took
 // at this step is re-scored from logits [B*K, ldl] fp32 and logz [B*K] (row_select's outputs for this step); needs nsel >= K + K / G.
 // The re-score applies the repetition penalty rep_penalty after the Hamming term when the token occurs in the beam's decoder input
 // (prefix: int64 [B, len0] decoder prefix, null: [CLS]; then the beam's tokens).  G = 1 reads none of these.
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
                      const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, float rep_penalty,
-                     const int64_t* prefix, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
-                     cudaStream_t stream);
+                     const int64_t* prefix, int eos, int len0, const int* p0s, int32_t* out_beam_idx, int32_t* out_tokens,
+                     float* out_scores, cudaStream_t stream);
 // out_ids [B*N, T] / out_scores [B*N]: the N <= K best finished hypotheses of every image, image-major, in the pop order of HF
-// BeamSearchScorer.finalize (score descending, the later-inserted first among equal scores); N = 1 is the single best
-int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores,
-                         cudaStream_t stream);
+// BeamSearchScorer.finalize (score descending, the later-inserted first among equal scores); N = 1 is the single best.
+// Search b belongs to image b / per_image (p0s).
+int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, const int* p0s, int per_image, int N, int64_t* out_ids,
+                         float* out_scores, cudaStream_t stream);
 
 // n-gram blocking (utils/decoding_utils.py:38-78): ban list per row from the question history and the decoded prefix.
 // prefix_tokens int32 [rows, P+T] (decoder prefix of len0 = P tokens, then the generated ones; EOS already replaced by PAD),
@@ -250,8 +267,10 @@ int launch_ngram_ban(int rows, int N, int Lh, const int64_t* hist_ids, const int
                      cudaStream_t stream);
 // the same for the B*K beam rows: key = the last n-1 tokens of prefix_b ([SEP] read as [PAD]; null: [CLS], P = 1) followed by beam
 // row b*K+k of `tokens` [B, K, T] (the beam token buffer of this step's parity); history row = b.  Needs n - 1 <= P + step, step < T.
+// p0s: prefix_b is the first p0s[b] + 1 ids of row b (stride P); an image whose decoder input is shorter than n - 1 bans nothing.
 int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int64_t* prefix, int P,
-                          const int32_t* tokens, int step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream);
+                          const int* p0s, const int32_t* tokens, int step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
+                          cudaStream_t stream);
 // sample-mode selection from row_select output; writes seq[row, step] and cur_tokens[row], prefix[row, step+1]
 // top_k == 0: multinomial over the whole (optionally nucleus-filtered) vocabulary; writes the same state as launch_sample_step
 // N rows per image (sampled candidates): row r draws as row r / N of a single-sample call seeded candidate_seed(seed, r % N)
@@ -264,9 +283,11 @@ int launch_sample_step(int rows, int N, int T, int nsel, const float* sel_val, c
                        uint64_t seed, uint64_t row_offset, const uint64_t* d_seed, const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
                        int prefix_stride, int32_t* out_tokens, cudaStream_t stream);
 // dec_prefix: int64 [rows / N, P] decoder prefix (null: start_token, P = 1), shared by the N rows of an image; the key buffer
-// `prefix` [rows, prefix_stride >= P + T]
+// `prefix` [rows, prefix_stride >= P + T].  An image's prefix ends at its first negative id; it is written right-aligned into
+// columns P - P_b .. P - 1 of the key rows (zeros before it: [PAD], which no history n-gram holds), so the samplers append token t
+// at column P + t for every row.  p0s (may be null): receives every image's P_b - 1 (DecodeGeom::P0s).
 int launch_sample_init(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                       int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, cudaStream_t stream);
+                       int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, int* p0s, cudaStream_t stream);
 int launch_sample_finalize(int rows, int T, int eos, const int32_t* seq, int64_t* out_ids, cudaStream_t stream);
 int launch_step_advance(int* d_step, cudaStream_t stream);
 // device-side scalar set (a pageable-memory cudaMemcpyAsync would synchronise the stream with the host)

@@ -150,7 +150,7 @@ embed_text_kernel(int rows, int L, int width, const int64_t* __restrict__ ids, c
   const int lane = threadIdx.x & 31;
   if (row >= rows) return;
   int64_t id = ids[row];
-  if (eos_to_pad && id == 102) id = 0;
+  if (eos_to_pad && (id == 102 || id < 0)) id = 0;   // negative: past the end of a shorter decoder prefix
   const int p = (row % L) + (d_pos_offset ? *d_pos_offset : 0);
   const int64_t s = seg ? seg[row] : 0;
   // segments >= type_vocab_size index the "extension" table (models/vilbert_dialog.py:335-346)
@@ -173,7 +173,8 @@ embed_text_kernel(int rows, int L, int width, const int64_t* __restrict__ ids, c
 
 template <typename T>
 __global__ void __launch_bounds__(kRowsPerBlock * 32)
-embed_step_kernel(int rows, int width, const int32_t* __restrict__ tokens, int pos0, const int* __restrict__ d_step,
+embed_step_kernel(int rows, int width, const int32_t* __restrict__ tokens, int pos0, const int* __restrict__ p0s, int rows_per_image,
+                  const int* __restrict__ d_step,
                   const float* __restrict__ word, const float* __restrict__ pos, const float* __restrict__ type,
                   const float* __restrict__ gamma, const float* __restrict__ beta, T* __restrict__ y) {
   pdl_wait();
@@ -183,7 +184,7 @@ embed_step_kernel(int rows, int width, const int32_t* __restrict__ tokens, int p
   if (row >= rows) return;
   int id = tokens[row];
   if (id == 102) id = 0;      // the decoder never sees [SEP] as an input (models/visual_dialog_decoder.py:57)
-  const int p = pos0 + *d_step;   // pos0 = decoder prefix length - 1
+  const int p = (p0s ? p0s[row / rows_per_image] : pos0) + *d_step;   // the image's decoder prefix length - 1, plus the step
   float v[kMaxChunks][8];
 #pragma unroll
   for (int c = 0; c < kMaxChunks; ++c) {
@@ -411,14 +412,18 @@ int launch_embed_text(int dtype, int rows, int L, int width, const int64_t* ids,
   return 1;
 }
 
-int launch_embed_step(int dtype, int rows, int width, const int32_t* tokens, int pos0, const int* d_step, const float* word,
-                      const float* pos, const float* type, const float* gamma, const float* beta, void* y, cudaStream_t stream) {
+int launch_embed_step(int dtype, int rows, int width, const int32_t* tokens, int pos0, const int* p0s, int rows_per_image, const int* d_step,
+                      const float* word, const float* pos, const float* type, const float* gamma, const float* beta, void* y,
+                      cudaStream_t stream) {
   if (rows <= 0) return 0;
   check_width(width);
+  if (p0s && rows_per_image < 1) throw std::runtime_error("embed_step: rows_per_image must be >= 1");
   if (dtype == kF32)
-    launch_k(embed_step_kernel<float>, grid_rows(rows), kRowsPerBlock * 32, 0, stream, rows, width, tokens, pos0, d_step, word, pos, type, gamma, beta, (float*)y);
+    launch_k(embed_step_kernel<float>, grid_rows(rows), kRowsPerBlock * 32, 0, stream, rows, width, tokens, pos0, p0s, rows_per_image, d_step, word,
+             pos, type, gamma, beta, (float*)y);
   else
-    launch_k(embed_step_kernel<bf16>, grid_rows(rows), kRowsPerBlock * 32, 0, stream, rows, width, tokens, pos0, d_step, word, pos, type, gamma, beta, (bf16*)y);
+    launch_k(embed_step_kernel<bf16>, grid_rows(rows), kRowsPerBlock * 32, 0, stream, rows, width, tokens, pos0, p0s, rows_per_image, d_step, word,
+             pos, type, gamma, beta, (bf16*)y);
   return 1;
 }
 

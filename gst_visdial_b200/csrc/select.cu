@@ -31,7 +31,8 @@ struct Cand { float v; int i; };
 __device__ __forceinline__ bool better(float av, int ai, float bv, int bi) { return av > bv || (av == bv && ai < bi); }
 
 // ---- logits processors (LogitsProcs, kernels.h) ----------------------------------------------------------------------
-// The CTA of `row` reads the row's decoder input d (cur_len = P + t <= 64 ids) into shared memory once, marks the positions whose id
+// The CTA of `row` reads the row's decoder input d (cur_len = P_b + t <= 64 ids, P_b = the prefix length of the row's image) into
+// shared memory once, marks the positions whose id
 // the n-gram rule bans, and every thread then folds d into two masks over its own slots: `pen` = slots whose id occurs in d (a bit
 // mask, so an id that repeats is penalised once), `ban` = slots set to -inf (n-gram rule; [SEP] while cur_len < min_length).
 // owner(w) = the calling thread's slot of id w, or -1.  Every thread of the CTA must call it (it synchronises).
@@ -39,14 +40,16 @@ template <class Owner>
 __device__ __forceinline__ void procs_masks(const LogitsProcs& pp, int row, int t, int32_t* s_d, uint8_t* s_ban, Owner owner,
                                             uint32_t& pen, uint32_t& ban) {
   const int tid = threadIdx.x;
-  const int L = min(pp.P + t, kProcMaxLen);
+  const int img = row / pp.rows_per_image;
+  const int Pb = pp.p0s ? pp.p0s[img] + 1 : pp.P;
+  const int L = min(Pb + t, kProcMaxLen);
   if (tid < L) {
     int32_t w;
-    if (pp.keys) w = pp.keys[(int64_t)row * pp.key_stride + tid];
-    else if (tid < pp.P) {
-      w = pp.prefix ? (int32_t)pp.prefix[(int64_t)(row / pp.rows_per_image) * pp.P + tid] : 101;
+    if (pp.keys) w = pp.keys[(int64_t)row * pp.key_stride + (pp.P - Pb) + tid];   // the key row holds the prefix right-aligned
+    else if (tid < Pb) {
+      w = pp.prefix ? (int32_t)pp.prefix[(int64_t)img * pp.P + tid] : 101;
       if (w == 102) w = 0;                                 // the decoder input holds [PAD] where the prefix has [SEP]
-    } else w = pp.tokens[(int64_t)row * pp.tok_stride + tid - pp.P];
+    } else w = pp.tokens[(int64_t)row * pp.tok_stride + tid - Pb];
     s_d[tid] = w;
   }
   __syncthreads();
@@ -496,16 +499,29 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
 }
 
 // ------------------------------------------------------------------------------------------------------------
+// Length of a decoder prefix row of stride P: the column of its first negative id, or P.  A row that starts with a negative id is
+// invalid input; it is read as length 1 so that every index stays in range (its output is unspecified).
+__device__ __forceinline__ int prefix_len(const int64_t* __restrict__ row, int P) {
+  for (int j = 1; j < P; ++j)
+    if (row[j] < 0) return j;
+  return P;
+}
+
 // prefix != null: int64 [B, P] decoder prefix shared by the K beams of an image; the first step's input is its last token.
 // gs = beams per group: the first beam of every group starts at 0, the others at -1e9 (gs = K: one group; gs = 1: all at 0, beam
 // sampling).  B = searches of K beams; N searches per image (beam sampling) share the image's prefix row b / N.
-__global__ void beam_init_kernel(BeamBuffers bb, int B, int K, int gs, int N, int T, int start_token, const int64_t* __restrict__ prefix, int P) {
+// p0s != null (needs prefix): receives every image's prefix length - 1.
+__global__ void beam_init_kernel(BeamBuffers bb, int B, int K, int gs, int N, int T, int start_token, const int64_t* __restrict__ prefix, int P,
+                                 int* __restrict__ p0s) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0) *bb.d_step = 0;
   if (i < B) { bb.done[i] = 0; bb.hyp_count[i] = 0; bb.hyp_worst[i] = 1e9; }
+  if (p0s && i < B && i % N == 0) p0s[i / N] = prefix_len(prefix + (int64_t)(i / N) * P, P) - 1;
   if (i < B * K) {
     bb.beam_scores[i] = ((i % K) % gs == 0) ? 0.f : -1e9f;
-    bb.cur_tokens[i] = prefix ? (int32_t)prefix[(int64_t)(i / K / N) * P + P - 1] : start_token;
+    const int64_t* row = prefix ? prefix + (int64_t)(i / K / N) * P : nullptr;
+    const int32_t w = row ? (int32_t)row[prefix_len(row, P) - 1] : start_token;
+    bb.cur_tokens[i] = w < 0 ? 0 : w;                    // an invalid row's negative start is embedded as [PAD]
     bb.beam_idx[i] = i % K;
   }
   for (int j = i; j < 2 * B * K * T; j += gridDim.x * blockDim.x) bb.tokens[j] = 0;
@@ -599,8 +615,8 @@ constexpr int kBeamMinBlocks = 7;
 __global__ void __launch_bounds__(kBeamWarps * 32, kBeamMinBlocks)
 beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, const float* __restrict__ sel_val,
                  const int32_t* __restrict__ sel_idx, const float* __restrict__ logits, int64_t ldl, const float* __restrict__ logz,
-                 float penalty, float rep_penalty, const int64_t* __restrict__ prefix, int eos, int len0, int32_t* out_beam_idx,
-                 int32_t* out_tokens, float* out_scores) {
+                 float penalty, float rep_penalty, const int64_t* __restrict__ prefix, int eos, int len0, const int* __restrict__ p0s,
+                 int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
   __shared__ float s_val[kBeamWarps][128];
   __shared__ int s_flat[kBeamWarps][128];
   __shared__ int s_order[kBeamWarps][16];
@@ -612,7 +628,8 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, co
   const int b = blockIdx.x * kBeamWarps + warp;
   if (b >= B) return;
   const int t = *bb.d_step;
-  const int cur_len = t + len0;                // HF input_ids.shape[-1]: decoder prefix (len0 tokens) + t generated
+  const int len_b = p0s ? p0s[b] + 1 : len0;   // the image's decoder prefix length (len0 = the prefix row stride)
+  const int cur_len = t + len_b;               // HF input_ids.shape[-1]: decoder prefix (len_b tokens) + t generated
   const int32_t* src = bb.tokens + (int64_t)(t & 1) * B * K * T + (int64_t)b * K * T;
   int32_t* dst = bb.tokens + (int64_t)((t + 1) & 1) * B * K * T + (int64_t)b * K * T;
   const int gs = K / G;
@@ -637,7 +654,7 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, co
           if (rep_penalty != 1.f) {
             // HF order: the Hamming term, then the repetition penalty when w occurs in the beam's decoder input
             bool seen = false;
-            for (int j = 0; j < len0 && !seen; ++j) {
+            for (int j = 0; j < len_b && !seen; ++j) {
               const int32_t pj = prefix ? (int32_t)prefix[(int64_t)b * len0 + j] : 101;
               seen = (pj == 102 ? 0 : pj) == w;
             }
@@ -685,14 +702,16 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, co
 
 // BeamSearchScorer.finalize: a stable ascending sort of the image's hypotheses (kept in insertion order by hyp_add), then N pops.
 // Output n of image b is the hypothesis of rank n by (score desc, insertion index desc); N = 1 is the last of the best scores.
-__global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores) {
+__global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eos, int len0, const int* __restrict__ p0s, int per_image, int N,
+                                     int64_t* out_ids, float* out_scores) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const int t = *bb.d_step;                     // steps executed
   const int HK = K + 1;
   if (!bb.done[b]) {
+    const int len_b = p0s ? p0s[b / per_image] + 1 : len0;
     const int32_t* cur = bb.tokens + (int64_t)(t & 1) * B * K * T + (int64_t)b * K * T;
-    for (int k = 0; k < K; ++k) hyp_add(bb, b, K, T, cur + (int64_t)k * T, t, bb.beam_scores[b * K + k], t + len0);
+    for (int k = 0; k < K; ++k) hyp_add(bb, b, K, T, cur + (int64_t)k * T, t, bb.beam_scores[b * K + k], t + len_b);
   }
   const double* hs = bb.hyp_score + (int64_t)b * HK;
   const int cnt = bb.hyp_count[b];
@@ -721,7 +740,9 @@ ngram_ban_kernel(int N, int Lh, const int64_t* __restrict__ hist_ids, const int6
   const int row = blockIdx.x;
   if (threadIdx.x == 0) cnt = 0;
   __syncthreads();
-  const int cur_len = *d_step + len0;                    // decoder prefix (len0 tokens) + generated
+  // decoder prefix (len0 tokens) + generated.  A shorter prefix sits right-aligned in its key row (launch_sample_init) behind zeros:
+  // a key that reaches into them holds [PAD], which no history n-gram holds, and bans nothing, as the shorter key would.
+  const int cur_len = *d_step + len0;
   const int start = cur_len + 1 - n;
   if (start >= 0) {                                      // a shorter key can never equal an (n-1)-gram
     const int64_t* ids = hist_ids + (int64_t)(row / N) * Lh;   // the history of the row's image
@@ -751,17 +772,23 @@ ngram_ban_kernel(int N, int Lh, const int64_t* __restrict__ hist_ids, const int6
 constexpr int kBanMaxK = 8;
 __global__ void __launch_bounds__(256)
 beam_ngram_ban_kernel(int K, int T, int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __restrict__ hist_seg,
-                      const int64_t* __restrict__ prefix, int P, const int32_t* __restrict__ tokens, int step, int n,
-                      int32_t* __restrict__ ban_tokens, int32_t* __restrict__ ban_count, int ban_stride) {
+                      const int64_t* __restrict__ prefix, int P, const int* __restrict__ p0s, const int32_t* __restrict__ tokens, int step,
+                      int n, int32_t* __restrict__ ban_tokens, int32_t* __restrict__ ban_count, int ban_stride) {
   __shared__ int32_t s_key[kBanMaxK][kHypMaxT];
   __shared__ int s_cnt[kBanMaxK];
   pdl_wait();
   pdl_launch_dependents();
-  const int b = blockIdx.x, klen = n - 1, first = P + step - klen;   // first key position in prefix + generated tokens
+  const int b = blockIdx.x, klen = n - 1;
+  const int Pb = p0s ? p0s[b] + 1 : P;                   // the image's prefix length (P = the row stride)
+  const int first = Pb + step - klen;                    // first key position in prefix + generated tokens
+  if (first < 0) {                                       // a decoder input shorter than n - 1 bans nothing
+    if (threadIdx.x < K) ban_count[b * K + threadIdx.x] = 0;
+    return;
+  }
   for (int i = threadIdx.x; i < K * klen; i += blockDim.x) {
     const int k = i / klen, j = i - k * klen, q = first + j;
     int32_t w;
-    if (q >= P) w = tokens[((int64_t)b * K + k) * T + q - P];
+    if (q >= Pb) w = tokens[((int64_t)b * K + k) * T + q - Pb];
     else {
       w = prefix ? (int32_t)prefix[(int64_t)b * P + q] : 101;
       if (w == 102) w = 0;                               // the decoder input holds [PAD] where the prefix has [SEP]
@@ -819,7 +846,8 @@ __device__ __forceinline__ double gumbel_u(uint64_t sd, uint64_t grow, int t, in
 
 __global__ void __launch_bounds__(kBeamWarps * 32, kBeamMinBlocks)
 beam_sample_step_kernel(BeamBuffers bb, int S, int N, int K, int T, int V, const float* __restrict__ sel_val, const int32_t* __restrict__ sel_idx,
-                        int top_k, float temperature, float top_p, const uint64_t* __restrict__ d_seed, int eos, int len0) {
+                        int top_k, float temperature, float top_p, const uint64_t* __restrict__ d_seed, int eos, int len0,
+                        const int* __restrict__ p0s) {
   constexpr int nsel = kSelMax;
   __shared__ double s_key[kBeamWarps][8 * nsel];
   __shared__ float s_val[kBeamWarps][8 * nsel];
@@ -834,7 +862,7 @@ beam_sample_step_kernel(BeamBuffers bb, int S, int N, int K, int T, int V, const
   const int s = blockIdx.x * kBeamWarps + warp;
   if (s >= S) return;
   const int t = *bb.d_step;
-  const int cur_len = t + len0;
+  const int cur_len = t + (p0s ? p0s[s / N] + 1 : len0);   // the image's decoder prefix + t generated
   const int32_t* src = bb.tokens + (int64_t)(t & 1) * S * K * T + (int64_t)s * K * T;
   int32_t* dst = bb.tokens + (int64_t)((t + 1) & 1) * S * K * T + (int64_t)s * K * T;
   const int n = K * nsel;
@@ -910,20 +938,24 @@ beam_sample_step_kernel(BeamBuffers bb, int S, int N, int K, int T, int V, const
   }
 }
 
-// dec_prefix != null: int64 [rows / N, P] decoder prefix of the row's image; `prefix` (the n-gram key buffer) starts with it, [SEP]
-// read as [PAD]
+// dec_prefix != null: int64 [rows / N, P] decoder prefix of the row's image, Pb = prefix_len tokens; the n-gram key buffer `prefix`
+// holds it right-aligned in columns P - Pb .. P - 1 ([SEP] read as [PAD], zeros before it).  p0s != null: receives Pb - 1 per image.
 __global__ void sample_init_kernel(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                                   int prefix_stride, int* d_step, const int64_t* __restrict__ dec_prefix, int P) {
+                                   int prefix_stride, int* d_step, const int64_t* __restrict__ dec_prefix, int P, int* __restrict__ p0s) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0) *d_step = 0;
   if (i < rows) {
     const int64_t img = i / N;
-    cur_tokens[i] = dec_prefix ? (int32_t)dec_prefix[img * P + P - 1] : start_token;
+    const int64_t* row = dec_prefix ? dec_prefix + img * P : nullptr;
+    const int Pb = row ? prefix_len(row, P) : 1;
+    if (p0s && i % N == 0) p0s[img] = Pb - 1;
+    const int32_t w0 = row ? (int32_t)row[Pb - 1] : start_token;
+    cur_tokens[i] = w0 < 0 ? 0 : w0;                     // an invalid row's negative start is embedded as [PAD]
     for (int j = 0; j < T; ++j) seq[(int64_t)i * T + j] = 0;
     for (int j = 0; j < prefix_stride; ++j) prefix[(int64_t)i * prefix_stride + j] = 0;
-    for (int j = 0; j < P; ++j) {
-      const int32_t w = dec_prefix ? (int32_t)dec_prefix[img * P + j] : start_token;
-      prefix[(int64_t)i * prefix_stride + j] = w == 102 ? 0 : w;
+    for (int j = 0; j < Pb; ++j) {
+      const int32_t w = row ? (int32_t)row[j] : start_token;
+      prefix[(int64_t)i * prefix_stride + P - Pb + j] = (w == 102 || w < 0) ? 0 : w;
     }
   }
 }
@@ -1236,26 +1268,28 @@ int launch_row_select(int rows, int V, const float* logits, int64_t ldl, int mod
   return 1;
 }
 
-int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int N, int T, int start_token, const int64_t* prefix, int P, cudaStream_t stream) {
+int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int N, int T, int start_token, const int64_t* prefix, int P, int* p0s,
+                     cudaStream_t stream) {
   if (G < 1 || K % G != 0) throw std::runtime_error("beam_init: the beam groups must divide the beams");
   if (N < 1 || B % N != 0) throw std::runtime_error("beam_init: the searches must be a multiple of N >= 1");
+  if (p0s && !prefix) throw std::runtime_error("beam_init: per-image prefix lengths need a prefix");
   const int n = B * K;
-  beam_init_kernel<<<(n + 255) / 256, 256, 0, stream>>>(bb, B, K, K / G, N, T, start_token, prefix, P);
+  beam_init_kernel<<<(n + 255) / 256, 256, 0, stream>>>(bb, B, K, K / G, N, T, start_token, prefix, P, p0s);
   return 1;
 }
 int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, int V, const float* sel_val, const int32_t* sel_idx, int top_k,
-                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, cudaStream_t stream) {
+                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, const int* p0s, cudaStream_t stream) {
   if (K < 2 || 2 * K > kSelMax || T > kHypMaxT) throw std::runtime_error("beam_sample_step: 2 <= K <= 8 and T <= 32");
   if (N < 1 || S % N != 0) throw std::runtime_error("beam_sample_step: the searches must be a multiple of N >= 1");
   if (top_k < 1 || top_k > kSelMax) throw std::runtime_error("beam_sample_step: top_k out of range");
   launch_k(beam_sample_step_kernel, dim3((S + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, S, N, K, T, V, sel_val,
-           sel_idx, top_k, temperature, top_p, d_seed, eos, len0);
+           sel_idx, top_k, temperature, top_p, d_seed, eos, len0, p0s);
   return 1;
 }
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
                      const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, float rep_penalty,
-                     const int64_t* prefix, int eos, int len0, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
-                     cudaStream_t stream) {
+                     const int64_t* prefix, int eos, int len0, const int* p0s, int32_t* out_beam_idx, int32_t* out_tokens,
+                     float* out_scores, cudaStream_t stream) {
   if (K > 8 || T > kHypMaxT) throw std::runtime_error("beam_step: K <= 8 and T <= 32");
   if (G < 1 || K % G != 0) throw std::runtime_error("beam_step: the beam groups must divide the beams");
   if (G > 1 && (!logits || !logz || nsel < K + K / G))
@@ -1263,13 +1297,14 @@ int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, i
   if (!(rep_penalty > 0.f) || !std::isfinite(rep_penalty) || (len0 > 1 && !prefix))
     throw std::runtime_error("beam_step: repetition penalty must be finite and > 0, prefix given when len0 > 1");
   launch_k(beam_step_kernel, dim3((B + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, B, K, G, T, V, nsel, sel_val, sel_idx,
-           logits, ldl, logz, penalty, rep_penalty, prefix, eos, len0, out_beam_idx, out_tokens, out_scores);
+           logits, ldl, logz, penalty, rep_penalty, prefix, eos, len0, p0s, out_beam_idx, out_tokens, out_scores);
   return 1;
 }
-int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, int N, int64_t* out_ids, float* out_scores,
-                         cudaStream_t stream) {
+int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, const int* p0s, int per_image, int N, int64_t* out_ids,
+                         float* out_scores, cudaStream_t stream) {
   if (N < 1 || N > K) throw std::runtime_error("beam_finalize: 1 <= N <= K");
-  beam_finalize_kernel<<<(B + 31) / 32, 32, 0, stream>>>(bb, B, K, T, eos, len0, N, out_ids, out_scores);
+  if (per_image < 1 || B % per_image != 0) throw std::runtime_error("beam_finalize: the searches must be a multiple of per_image >= 1");
+  beam_finalize_kernel<<<(B + 31) / 32, 32, 0, stream>>>(bb, B, K, T, eos, len0, p0s, per_image, N, out_ids, out_scores);
   return 1;
 }
 int launch_ngram_ban(int rows, int N, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
@@ -1281,11 +1316,13 @@ int launch_ngram_ban(int rows, int N, int Lh, const int64_t* hist_ids, const int
   return 1;
 }
 int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int64_t* prefix, int P,
-                          const int32_t* tokens, int step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream) {
+                          const int* p0s, const int32_t* tokens, int step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
+                          cudaStream_t stream) {
   if (B <= 0) return 0;
   if (K > kBanMaxK || n < 1 || n - 1 > P + step || n - 1 > kHypMaxT || step >= T || T > kHypMaxT || P < 1 || (P > 1 && !prefix))
     throw std::runtime_error("beam_ngram_ban: K <= 8, 1 <= n <= min(P + step, 32) + 1, step < T <= 32, prefix given when P > 1");
-  launch_k(beam_ngram_ban_kernel, dim3(B), dim3(256), 0, stream, K, T, Lh, hist_ids, hist_seg, prefix, P, tokens, step, n, ban_tokens, ban_count, ban_stride);
+  launch_k(beam_ngram_ban_kernel, dim3(B), dim3(256), 0, stream, K, T, Lh, hist_ids, hist_seg, prefix, P, p0s, tokens, step, n, ban_tokens, ban_count,
+           ban_stride);
   return 1;
 }
 int launch_sample_step(int rows, int N, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
@@ -1319,10 +1356,11 @@ int launch_full_vocab_sample(int rows, int N, int V, const float* logits, int64_
   return 1;
 }
 int launch_sample_init(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                       int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, cudaStream_t stream) {
+                       int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, int* p0s, cudaStream_t stream) {
   if (P < 1 || P > prefix_stride || (P > 1 && !dec_prefix)) throw std::runtime_error("sample_init: 1 <= P <= prefix_stride, prefix given when P > 1");
   if (N < 1 || rows % N != 0) throw std::runtime_error("sample_init: rows must be a multiple of N >= 1");
-  sample_init_kernel<<<(rows + 63) / 64, 64, 0, stream>>>(rows, N, T, start_token, seq, cur_tokens, prefix, prefix_stride, d_step, dec_prefix, P);
+  if (p0s && !dec_prefix) throw std::runtime_error("sample_init: per-image prefix lengths need a prefix");
+  sample_init_kernel<<<(rows + 63) / 64, 64, 0, stream>>>(rows, N, T, start_token, seq, cur_tokens, prefix, prefix_stride, d_step, dec_prefix, P, p0s);
   return 1;
 }
 int launch_sample_finalize(int rows, int T, int eos, const int32_t* seq, int64_t* out_ids, cudaStream_t stream) {

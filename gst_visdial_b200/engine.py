@@ -172,9 +172,15 @@ class Engine:
         check(self.ctx, self.lib.gstvd_prefill_cross(self.ctx, B, Le, _ptr(h), _ptr(m), self._stream()))
 
     def _prefix(self, prefix, B):
-        """(device int64 [B, P] tensor or None, P) of a decoder prefix argument; None stands for one [CLS] per row."""
+        """(device int64 [B, P] tensor or None, P) of a decoder prefix argument; None stands for one [CLS] per row.  A negative id
+        ends a row's prefix (rows of different lengths, include/gstvd.h gstvd_generate); a row cannot start with one, which is
+        checked here for a host tensor (a device tensor is not read on the host)."""
         if prefix is None:
             return None, 1
+        if isinstance(prefix, torch.Tensor) and prefix.device.type == "cpu" and prefix.dim() == 2 and prefix.shape[1] > 0:
+            bad = (prefix[:, 0] < 0).nonzero().flatten()
+            if len(bad):
+                raise ValueError(f"prefix row {int(bad[0])} starts with a negative id: every row needs at least one token")
         pre = self._dev(prefix, torch.int64)
         if pre.dim() != 2 or pre.shape[0] != B:
             raise ValueError(f"prefix must be [B={B}, P], got {tuple(pre.shape)}")
@@ -350,18 +356,21 @@ class Engine:
     SELF_KERNELS = {"default": -1, "first": 0, "v2": 1}
     CROSS_KERNELS = {"default": -1, "warp_tma": 0, "cta_tma": 1, "mma": 2, "simt": 3, "generic": 4}
 
-    def op_dec_self_attn(self, qkv, cache, heads, P0=0, step=0, step_known=True, prefix_qkv=None, anc=None, kernel="default", dtype=None):
+    def op_dec_self_attn(self, qkv, cache, heads, P0=0, step=0, step_known=True, prefix_qkv=None, anc=None, kernel="default", dtype=None,
+                         p0s=None):
         """One decode-step self-attention launch (include/gstvd.h gstvd_op_dec_self_attn) on fp32 ``qkv`` [B*K, 3H] and ``cache``
-        [2, B, T, K, H]; ``anc`` uint8 [B*K, 32 or 64].  Returns (out [B*K, H], the cache after the call); ``cache`` is not modified."""
+        [2, B, T, K, H]; ``anc`` uint8 [B*K, 32 or 64]; ``p0s`` int [B]: each image's own P0 (<= ``P0``), None = ``P0`` for all.
+        Returns (out [B*K, H], the cache after the call); ``cache`` is not modified."""
         q = self._dev(qkv, torch.float32)
         c = self._dev(cache, torch.float32).clone()
         _, B, T, K, H = c.shape
         pre = self._dev(prefix_qkv, torch.float32)
         a = self._dev(anc, torch.uint8)
+        p0 = self._dev(p0s, torch.int32)
         out = torch.empty(B * K, H, device=self.device, dtype=torch.float32)
         check(self.ctx, self.lib.gstvd_op_dec_self_attn(self.ctx, self.dtype if dtype is None else DTYPES[dtype], self.SELF_KERNELS[kernel], B, K,
-                                                        int(heads), H // heads, T, int(P0), int(step), int(bool(step_known)), _ptr(q), _ptr(pre),
-                                                        _ptr(c), _ptr(a), _ptr(out), self._stream()))
+                                                        int(heads), H // heads, T, int(P0), _ptr(p0), int(step), int(bool(step_known)), _ptr(q),
+                                                        _ptr(pre), _ptr(c), _ptr(a), _ptr(out), self._stream()))
         return out, c
 
     def op_dec_cross_attn(self, q, cross_kv, K, mask=None, use_cross_len=True, kernel="default", dtype=None):
@@ -376,12 +385,14 @@ class Engine:
                                                          _ptr(cl), _ptr(out), self._stream()))
         return out, cl
 
-    def op_anc_update(self, anc, beam_idx, T, P0, step):
-        """One ancestry-table update (gstvd_op_anc_update): returns the updated copy of uint8 ``anc`` [B*K, 32 or 64]."""
+    def op_anc_update(self, anc, beam_idx, T, P0, step, p0s=None):
+        """One ancestry-table update (gstvd_op_anc_update): returns the updated copy of uint8 ``anc`` [B*K, 32 or 64].  ``p0s`` int [B]:
+        each image's own P0 (<= ``P0``), None = ``P0`` for all."""
         bi = self._dev(beam_idx, torch.int32)
         B, K = bi.shape
         a = self._dev(anc, torch.uint8).clone()
-        check(self.ctx, self.lib.gstvd_op_anc_update(self.ctx, B, K, int(T), int(P0), int(step), _ptr(bi), _ptr(a), self._stream()))
+        p0 = self._dev(p0s, torch.int32)
+        check(self.ctx, self.lib.gstvd_op_anc_update(self.ctx, B, K, int(T), int(P0), _ptr(p0), int(step), _ptr(bi), _ptr(a), self._stream()))
         return a
 
     def op_beam_begin(self, B, K, max_new):

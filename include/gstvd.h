@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define GSTVD_ABI_VERSION 4
+#define GSTVD_ABI_VERSION 5
 #define GSTVD_MAX_CONNECTIONS 16
 
 typedef enum {
@@ -158,6 +158,14 @@ int gstvd_prefill_cross(gstvd_ctx* ctx, int B, int Le, const float* enc_hidden, 
  *            keys may reach into the prefix.  Beam hypotheses count the prefix in their length (HF beam_search input_ids.shape[-1]).
  *            The caller's tensor is not modified.  P - 1 + max_new_tokens must not exceed 64 (cached positions of the decode
  *            kernels) nor max_position_embeddings.
+ *            Prefixes of different lengths in one call: a negative id ends an image's prefix.  Image b continues from
+ *            prefix[b, :P_b], P_b = the column of the first negative id of row b, or P if it has none; the ids after it are not
+ *            read as tokens.  P stays the row stride and the longest length, and the checks above apply to it.  Every output row of
+ *            image b is exactly what a call holding image b alone with prefix[b, :P_b] returns, in every mode below (sampling with the
+ *            same seed and row_offset + b): its cache positions run 0 .. P_b - 1 + t, step t is embedded at position P_b - 1 + t and
+ *            starts from prefix[b, P_b - 1], its decoder input for n-gram keys and the logits processors is prefix[b, :P_b] followed by
+ *            its tokens with cur_len = P_b + t, and hypothesis lengths, scores and is_done use P_b + t.  A row whose first id is
+ *            negative is invalid input: its output is unspecified (the call stays memory-safe; no negative id is ever looked up).
  *   hist_ids, hist_segments : int64 [B, Lh] encoder input ids / segments (only read when ngram_blocking_size > 0, in sample and
  *                             beam mode; the question history is ids * (segments == 0), visual_dialog_model.py:98-99)
  *   out_ids    : int64 [B*N, max_new_tokens], image-major (row b*N + n): the new tokens only, PAD(0) after the first [SEP]
@@ -324,13 +332,15 @@ int gstvd_op_deferred_ln_chain(gstvd_ctx* ctx, int M, int N, int K1, const float
  *
  * Self-attention of one new position per (image, beam) row; kernel 0 = the first kernel (fp32 / bf16, D 64 or 128), 1 = the lean
  * bf16 / D = 64 kernel (the only reader of an ancestry table).
- *   qkv [B*K, 3*heads*D]; cache [2 (k, v)][B][T][K][heads*D] in/out: the new k / v are written at position P0 + step of the row's
- *   own beam slot; prefix_qkv [B*P0, 3*heads*D] or NULL: its k / v are first stored at positions 0..P0-1 of every slot;
+ *   qkv [B*K, 3*heads*D]; cache [2 (k, v)][B][T][K][heads*D] in/out: the new k / v are written at position P0_b + step of the row's
+ *   own beam slot, P0_b = p0s[b] (int32 [B] on the device, 0 <= p0s[b] <= P0; per-image decoder prefix lengths - 1) or P0 when
+ *   p0s is NULL; the row attends over positions 0 .. P0_b + step;
+ *   prefix_qkv [B*P0, 3*heads*D] or NULL: its k / v are first stored at positions 0..P0-1 of every slot;
  *   anc uint8 [B*K][T <= 32 ? 32 : 64] or NULL: position t of row (b, k) is read from slot anc[b*K + k][t];
  *   step_known != 0 hands the step to the launch (loads bounded by it), else only through device memory (every row loaded, masked);
  *   out [B*K, heads*D].  K <= 8, T <= 64, P0 + step < T. */
-int gstvd_op_dec_self_attn(gstvd_ctx* ctx, int dtype, int kernel, int B, int K, int heads, int D, int T, int P0, int step,
-                           int step_known, const float* qkv, const float* prefix_qkv, float* cache, const uint8_t* anc,
+int gstvd_op_dec_self_attn(gstvd_ctx* ctx, int dtype, int kernel, int B, int K, int heads, int D, int T, int P0, const int32_t* p0s,
+                           int step, int step_known, const float* qkv, const float* prefix_qkv, float* cache, const uint8_t* anc,
                            float* out, void* stream);
 /* Cross-attention of B*K rows (K per image) over cross_kv [B][2*heads (k heads, then v heads)][Le][D] with mask [B, Le] (NULL:
  * all ones; additive (1 - m) * -1e9).  kernel 0 = warp-per-item TMA, 1 = CTA-per-item TMA, 2 = mma.sync, 3 = SIMT, 4 = generic.
@@ -340,8 +350,10 @@ int gstvd_op_dec_cross_attn(gstvd_ctx* ctx, int dtype, int kernel, int B, int K,
                             const float* cross_kv, const float* mask, int use_cross_len, int32_t* out_cross_len, float* out,
                             void* stream);
 /* One beam-ancestry update of a caller-supplied table anc uint8 [B*K][T <= 32 ? 32 : 64] (in place): beam_idx int32 [B, K] holds each
- * new beam's parent; row (b, k) becomes the parent's row over positions < P0 + step and holds the parent at P0 + step. */
-int gstvd_op_anc_update(gstvd_ctx* ctx, int B, int K, int T, int P0, int step, const int32_t* beam_idx, uint8_t* anc, void* stream);
+ * new beam's parent; row (b, k) becomes the parent's row over positions < P0_b + step and holds the parent at P0_b + step, with
+ * P0_b = p0s[b] (int32 [B] on the device, 0 <= p0s[b] <= P0) or P0 when p0s is NULL. */
+int gstvd_op_anc_update(gstvd_ctx* ctx, int B, int K, int T, int P0, const int32_t* p0s, int step, const int32_t* beam_idx, uint8_t* anc,
+                        void* stream);
 
 /* Test access to the self-attention KV cache in the layout a generate call with (B, K) uses: buf fp32 [B, max_new_tokens, K,
  * hidden] on the device for one (layer, kv in {0: key, 1: value}); write != 0 stores buf into the cache (rounded to the
