@@ -12,7 +12,7 @@ from ctypes import POINTER, Structure, c_char_p, c_float, c_int, c_int32, c_int6
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(HERE, "lib", "libgstvd.so")
 
-GSTVD_ABI_VERSION = 5
+GSTVD_ABI_VERSION = 6
 GSTVD_MAX_CONNECTIONS = 16
 GSTVD_F32, GSTVD_BF16 = 0, 1
 GSTVD_SELECT_SAMPLE, GSTVD_SELECT_BEAM, GSTVD_SELECT_BEAM_SAMPLE = 0, 1, 2
@@ -21,6 +21,10 @@ GSTVD_FLAG_DEBUG_SIMT_GEMM = 2
 GSTVD_FLAG_GENERIC_ATTENTION = 4
 GSTVD_FLAG_NO_PDL = 8
 GSTVD_MAX_TOP_K = 16
+# gstvd_gemm_kernel / gstvd_gemm_store
+GEMM_KERNELS = {"simt": 0, "tc32": 1, "tc64": 2, "tc128": 3, "tc256": 4, "skinny32": 5, "skinny64": 6, "pair128": 7, "pair256": 8,
+                "ln32": 9, "ln64": 10}
+GEMM_STORES = {"generic": 0, "tma": 1, "direct": 2}
 
 STATUS_NAMES = {0: "OK", -1: "INVALID", -2: "CUDA", -3: "UNSUPPORTED", -4: "STATE"}
 
@@ -74,7 +78,10 @@ SYMBOLS = [
     ("gstvd_score_options", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     ("gstvd_reorder_cache", c_int, [_P, c_int, c_int, c_int, _P, _P]),
     ("gstvd_splice", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, c_int, c_int, _P, _P]),
-    ("gstvd_op_linear", c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, _P, _P]),
+    ("gstvd_op_linear", c_int, [_P, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, _P, c_int64, c_int, POINTER(c_int32), c_int, c_int,
+                                POINTER(c_int32), _P]),
+    ("gstvd_op_linear_ln", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, c_int, _P, _P, c_int, POINTER(c_int32),
+                                   _P]),
     ("gstvd_op_add_layernorm", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P]),
     ("gstvd_op_attention", c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, _P, c_float, c_int, _P, _P]),
     ("gstvd_op_deferred_ln_chain", c_int, [_P, c_int, c_int, c_int, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P]),
@@ -82,6 +89,7 @@ SYMBOLS = [
     ("gstvd_op_dec_cross_attn", c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, _P, c_int, _P, _P, _P]),
     ("gstvd_op_anc_update", c_int, [_P, c_int, c_int, c_int, c_int, _P, c_int, _P, _P, _P]),
     ("gstvd_debug_self_cache", c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
+    ("gstvd_debug_cross_cache", c_int, [_P, c_int, c_int, _P, _P]),
     ("gstvd_op_beam_begin", c_int, [_P, c_int, c_int, c_int, _P]),
     ("gstvd_op_beam_step", c_int, [_P, _P, c_int64, _P, _P, _P, _P]),
     ("gstvd_op_beam_end", c_int, [_P, _P, _P, _P]),

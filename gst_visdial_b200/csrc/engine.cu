@@ -1309,44 +1309,75 @@ int gstvd_profile_read(gstvd_ctx* c, double* flops, double* bytes, double* ms, i
 }
 
 // ---- single operators ------------------------------------------------------------------------------------------
+// Variant the op entries will launch for g (dtype: operand type of the entry), or Unsupported before anything is launched.
+static GemmVariant op_gemm_variant(gstvd_ctx* c, int dtype, const GemmArgs& g) {
+  GemmVariant v;
+  const bool simt = dtype == kF32 || (g.force_kernel < 0 && (c->cfg.flags & GSTVD_FLAG_DEBUG_SIMT_GEMM));
+  if (dtype == kF32 && (g.force_kernel > 0 || !g.out_f32)) throw Unsupported("op_linear: fp32 operands run the SIMT kernel with fp32 output only");
+  if (simt && g.force_kernel < 0) {
+    GemmArgs s = g;
+    s.force_kernel = kGemmSimt;
+    const std::string why = gemm_tc_variant(s, c->num_sms, &v);
+    if (!why.empty()) throw Unsupported("op_linear: " + why);
+    return v;
+  }
+  const std::string why = gemm_tc_variant(g, c->num_sms, &v);
+  if (!why.empty()) throw Unsupported("op_linear: " + why);
+  return v;
+}
+
 int gstvd_op_linear(gstvd_ctx* c, int dtype, int M, int N, int K, const float* a, const float* w, const float* bias, int act, float* out,
-                    void* stream) {
+                    int64_t ldc, int out_dtype, const int32_t* hm, int kernel, int store, int32_t* ran, void* stream) {
   if (!c) return GSTVD_ERR_INVALID;
   return guarded(c, [&] {
     cudaStream_t s = (cudaStream_t)stream;
+    if (dtype != kF32 && dtype != kBF16) throw InvalidArg("op_linear: dtype");
+    if (out_dtype != kF32 && out_dtype != kBF16) throw InvalidArg("op_linear: out_dtype");
+    if (M < 1 || N < 1 || K < 1 || !a || !w || !out) throw InvalidArg("op_linear: empty shape or NULL buffer");
+    if (kernel < -1 || store < -1) throw InvalidArg("op_linear: kernel / store must be -1 or a variant id");
     GemmArgs g;
-    g.M = M; g.N = N; g.K = K; g.lda = K; g.ldw = K; g.ldc = N; g.bias = bias; g.act = act; g.C = out; g.out_f32 = 1;
-    if (dtype == kF32) {
-      g.A = a; g.W = w;
-      c->launches += launch_gemm_simt(g, kF32, s);
-    } else {
-      Scratch sc;
-      void* a16 = sc.get((size_t)M * K * 2); void* w16 = sc.get((size_t)N * K * 2);
+    g.M = M; g.N = N; g.K = K; g.lda = K; g.ldw = K; g.bias = bias; g.act = act; g.out_f32 = out_dtype == kF32 ? 1 : 0;
+    g.force_kernel = kernel; g.force_store = store;
+    g.ldc = ldc == 0 ? N : ldc;
+    int64_t region = (int64_t)M * g.ldc;                    // elements of the caller's output buffer
+    if (hm) {
+      g.hm_D = hm[0]; g.hm_L = hm[1]; g.hm_G = hm[2]; g.hm_B = hm[3];
+      if (g.hm_D < 1 || g.hm_L < 1 || g.hm_G < 1 || g.hm_B < 1 || M != g.hm_B * g.hm_L || N % (g.hm_D * g.hm_G) != 0 || ldc != 0)
+        throw InvalidArg("op_linear: head-major geometry needs D, L, G, B >= 1, M = B * L, N % (D * G) == 0 and ldc = 0");
+      region = (int64_t)M * N;
+    } else if (g.ldc < N) {
+      throw InvalidArg("op_linear: ldc < N");
+    }
+    Scratch sc;
+    void* a16 = nullptr; void* w16 = nullptr; void* c16 = nullptr;
+    if (dtype == kBF16) { a16 = sc.get((size_t)M * K * 2); w16 = sc.get((size_t)N * K * 2); }
+    if (!g.out_f32) c16 = sc.get((size_t)region * 2);
+    g.A = dtype == kBF16 ? a16 : (const void*)a; g.W = dtype == kBF16 ? w16 : (const void*)w;
+    g.C = g.out_f32 ? (void*)out : c16;
+    const GemmVariant v = op_gemm_variant(c, dtype, g);       // refuses before any launch
+    if (dtype == kBF16) {
       c->launches += launch_cast_f32_to(kBF16, a, a16, (int64_t)M * K, s);
       c->launches += launch_cast_f32_to(kBF16, w, w16, (int64_t)N * K, s);
-      g.A = a16; g.W = w16;
-      static const bool bf16_out = getenv("GSTVD_OP_LINEAR_BF16OUT") != nullptr;   // measurement aid: time the bf16-output epilogue
-      void* c16 = nullptr;
-      if (bf16_out) { c16 = sc.get((size_t)M * N * 2); g.C = c16; g.out_f32 = 0; }
+    }
+    if (c16) c->launches += launch_cast_f32_to(kBF16, out, c16, region, s);    // the caller's sentinels survive where nothing is stored
+    if (v.kernel == kGemmSimt) {
+      c->launches += launch_gemm_simt(g, dtype, s);
+    } else {
       gemm_tc_init();
       static const bool want_times = getenv("GSTVD_GEMM_TIMES") != nullptr;   // measurement aid: per-CTA phase timestamps
       unsigned long long* d_times = nullptr;
       if (want_times) { d_times = (unsigned long long*)sc.get(256 * 8 * 8); CUDA_CHECK(cudaMemsetAsync(d_times, 0, 256 * 8 * 8, s)); g.dbg_times = d_times; }
-      if (c->cfg.flags & GSTVD_FLAG_DEBUG_SIMT_GEMM) c->launches += launch_gemm_simt(g, kBF16, s);
-      else {
-        const bool prof = c->profiling && c->prof_used < c->prof_pool.size();
-        if (prof) cudaEventRecord(c->prof_pool[c->prof_used].a, s);
-        c->launches += launch_gemm_tc(g, c->num_sms, s);
-        if (prof) {
-          auto& r = c->prof_pool[c->prof_used++];
-          cudaEventRecord(r.b, s);
-          r.flops = 2.0 * M * (double)N * K;
-          r.bytes = 2.0 * ((double)M * K + (double)N * K) + 4.0 * M * (double)N;
-        }
+      const bool prof = c->profiling && c->prof_used < c->prof_pool.size();
+      if (prof) cudaEventRecord(c->prof_pool[c->prof_used].a, s);
+      c->launches += launch_gemm_tc(g, c->num_sms, s);
+      if (prof) {
+        auto& r = c->prof_pool[c->prof_used++];
+        cudaEventRecord(r.b, s);
+        r.flops = 2.0 * M * (double)N * K;
+        r.bytes = 2.0 * ((double)M * K + (double)N * K) + (g.out_f32 ? 4.0 : 2.0) * M * (double)N;
       }
-      if (c16) c->launches += launch_cast_to_f32(kBF16, c16, out, (int64_t)M * N, s);
-      CUDA_CHECK(cudaStreamSynchronize(s));
       if (d_times) {
+        CUDA_CHECK(cudaStreamSynchronize(s));
         std::vector<unsigned long long> h(256 * 8);
         CUDA_CHECK(cudaMemcpy(h.data(), d_times, h.size() * 8, cudaMemcpyDeviceToHost));
         unsigned long long t0 = ~0ull; int ctas = 0;
@@ -1357,6 +1388,49 @@ int gstvd_op_linear(gstvd_ctx* c, int dtype, int M, int N, int K, const float* a
                 M, N, K, ctas, sum[0] / ctas, mx[0], sum[1] / ctas, mx[1], sum[2] / ctas, mx[2], sum[3] / ctas, mx[3], sum[4] / ctas, mx[4], sum[5] / ctas, mx[5], sum[6] / ctas, mx[6], sum[7] / ctas, mx[7]);
       }
     }
+    if (c16) c->launches += launch_cast_to_f32(kBF16, c16, out, region, s);
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    if (ran) { ran[0] = v.kernel; ran[1] = v.store; }
+  });
+}
+
+int gstvd_op_linear_ln(gstvd_ctx* c, int M, int N, int K, const float* a, const float* a_stats, const float* ln_gamma, const float* ln_beta,
+                       const float* w, const float* bias, const float* res, const float* res_stats, const float* res_gamma,
+                       const float* res_beta, int act, float* out, float* stats_out, int kernel, int32_t* ran, void* stream) {
+  if (!c) return GSTVD_ERR_INVALID;
+  return guarded(c, [&] {
+    cudaStream_t s = (cudaStream_t)stream;
+    if (M < 1 || N < 32 || N % 32 != 0 || K < 8 || K % 8 != 0) throw InvalidArg("op_linear_ln: shape (N % 32 == 0, K % 8 == 0)");
+    if (!a || !w || !out) throw InvalidArg("op_linear_ln: NULL buffer");
+    if (a_stats && (!ln_gamma || !ln_beta || K % 32 != 0 || K / 32 > kLnStatStride))
+      throw InvalidArg("op_linear_ln: a_stats needs ln_gamma / ln_beta and K % 32 == 0, K <= 1024");
+    if (res_stats && (!res || !res_gamma || !res_beta)) throw InvalidArg("op_linear_ln: res_stats needs res, res_gamma and res_beta");
+    if ((res_stats || stats_out) && N / 32 > kLnStatStride) throw InvalidArg("op_linear_ln: statistics of rows wider than 1024");
+    if (kernel < -1) throw InvalidArg("op_linear_ln: kernel must be -1 or a variant id");
+    Scratch sc;
+    void* a16 = sc.get((size_t)M * K * 2); void* w16 = sc.get((size_t)N * K * 2); void* y16 = sc.get((size_t)M * N * 2);
+    void* r16 = res ? sc.get((size_t)M * N * 2) : nullptr;
+    float* cd = a_stats ? (float*)sc.get((size_t)2 * N * 4) : nullptr;
+    GemmArgs g;
+    g.A = a16; g.lda = K; g.W = w16; g.ldw = K; g.C = y16; g.ldc = N; g.M = M; g.N = N; g.K = K; g.act = act;
+    g.bias = a_stats ? cd + N : bias;
+    if (a_stats) { g.fold_stats = (const float2*)a_stats; g.fold_parts = K / 32; g.fold_c = cd; }
+    g.res = r16; g.ldr = N;
+    if (res_stats) { g.res_stats = (const float2*)res_stats; g.res_parts = N / 32; g.res_gamma = res_gamma; g.res_beta = res_beta; }
+    g.stats_out = (float2*)stats_out; g.stats_ld = M;
+    g.force_kernel = kernel;
+    GemmVariant v;
+    const std::string why = gemm_tc_variant(g, c->num_sms, &v);
+    if (!why.empty()) throw Unsupported("op_linear_ln: " + why);
+    c->launches += launch_cast_f32_to(kBF16, a, a16, (int64_t)M * K, s);
+    if (a_stats) c->launches += launch_fold_ln_weights(N, K, w, ln_gamma, ln_beta, bias, w16, cd, cd + N, s);
+    else c->launches += launch_cast_f32_to(kBF16, w, w16, (int64_t)N * K, s);
+    if (res) c->launches += launch_cast_f32_to(kBF16, res, r16, (int64_t)M * N, s);
+    gemm_tc_init();
+    c->launches += launch_gemm_tc(g, c->num_sms, s);
+    c->launches += launch_cast_to_f32(kBF16, y16, out, (int64_t)M * N, s);
+    CUDA_CHECK(cudaStreamSynchronize(s));
+    if (ran) { ran[0] = v.kernel; ran[1] = v.store; }
   });
 }
 
@@ -1447,6 +1521,17 @@ int gstvd_debug_self_cache(gstvd_ctx* c, int write, int B, int K, int layer, int
     char* base = (char*)c->self_cache.p + ((int64_t)layer * 2 + kv) * n * c->esz;
     if (write) c->launches += launch_cast_f32_to(c->dtype, buf, base, n, s);
     else c->launches += launch_cast_to_f32(c->dtype, base, buf, n, s);
+  });
+}
+
+int gstvd_debug_cross_cache(gstvd_ctx* c, int B, int Le, float* buf, void* stream) {
+  if (!c || !buf) return GSTVD_ERR_INVALID;
+  return guarded(c, [&] {
+    if (c->dec_layers == 0) throw StateError("debug_cross_cache: encoder-only context");
+    if (B != c->cross_B || Le != c->cross_Le || B < 1)
+      throw StateError(fmt("debug_cross_cache: the resident cross K/V is [%d, %d], asked for [%d, %d]", c->cross_B, c->cross_Le, B, Le));
+    const int64_t n = (int64_t)c->dec_layers * B * 2 * c->H * Le;      // [layer][image][kv * heads + h][Le][D]
+    c->launches += launch_cast_to_f32(c->dtype, c->cross_cache.p, buf, n, (cudaStream_t)stream);
   });
 }
 

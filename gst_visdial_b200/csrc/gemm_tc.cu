@@ -714,42 +714,29 @@ void launch_cfg(const GemmArgs& a_in, int num_sms, cudaStream_t stream) {
   }
   const bool ln_args = a_in.fold_stats != nullptr || a_in.res != nullptr || a_in.stats_out != nullptr;
   if (ln_args != LN) throw std::runtime_error("gemm_tc: deferred-LayerNorm arguments reached a kernel configuration without that epilogue");
+  // a.tma_store = the store gemm_tc_variant chose and checked: TMA store when the output is expressible as a tensor map, direct row
+  // stores, or the generic register/shared path
   GemmArgs a = a_in;
   const CUtensorMap* ma_ptr = Cfg::kCK > 1 ? &get_map_k3(a.A, a.M, a.K, a.lda, Cfg::kBM, Cfg::kCK) : &get_map(a.A, a.M, a.K, a.lda, Cfg::kBM);
   const CUtensorMap& mb = Cfg::kCK > 1 ? get_map_k3(a.W, a.N, a.K, a.ldw, BN, Cfg::kCK) : get_map(a.W, a.N, a.K, a.ldw, BN);
-  // TMA-store epilogue when the output is expressible as a tensor map; otherwise the generic register/shared path
   const int esz = a.out_f32 ? 4 : 2;
   const int cw = 32;                                  // columns per TMA-store box (bf16: 64-byte rows, fp32: 128-byte rows)
   const CUtensorMap* mc = ma_ptr;
-  a.tma_store = 0;
-  static const bool no_tma_store = getenv("GSTVD_GEMM_NO_TMA_STORE") != nullptr;
-  static const bool no_tma_hm = getenv("GSTVD_GEMM_NO_TMA_HM") != nullptr;
-  if (!no_tma_store && (reinterpret_cast<uintptr_t>(a.C) & 15) == 0) {
+  if (a.tma_store == kStoreTma) {
     if (a.hm_D > 0) {
-      if (!no_tma_hm && Cfg::kCK == 1 && !a.out_f32 && a.hm_D % cw == 0 && a.M == a.hm_B * a.hm_L) {
-        const int64_t LB = (int64_t)(a.N / (a.hm_D * a.hm_G)) * a.hm_B;
-        mc = &get_map_hm3(a.C, a.hm_D, a.hm_L, LB * a.hm_G, cw);
-        a.hm_tpi = (a.hm_L + BM - 1) / BM;
-        ma_ptr = &get_map_a3(a.A, a.K, a.hm_L, a.hm_B, a.lda);
-        a.tma_store = 1;
-      }
-    } else if ((a.ldc * esz) % 16 == 0) {
-      static const bool no_direct = getenv("GSTVD_GEMM_NO_DIRECT") != nullptr;     // A/B aid
-      if (a.M <= 4 * BM && (int64_t)a.M * a.N * esz <= (4 << 20) && !no_direct) {
-        a.tma_store = 2;                                 // skinny (decode) problems: latency matters, the tile is tiny
-      } else {
-        mc = &get_map_c(a.C, a.M, a.N, a.ldc, esz, cw);
-        a.tma_store = 1;
-      }
+      const int64_t LB = (int64_t)(a.N / (a.hm_D * a.hm_G)) * a.hm_B;
+      mc = &get_map_hm3(a.C, a.hm_D, a.hm_L, LB * a.hm_G, cw);
+      a.hm_tpi = (a.hm_L + BM - 1) / BM;
+      ma_ptr = &get_map_a3(a.A, a.K, a.hm_L, a.hm_B, a.lda);
+    } else {
+      a.tma_cols = tma_store_cols(a.N, esz);
+      mc = &get_map_c(a.C, a.M, a.tma_cols, a.ldc, esz, cw);
     }
   }
   const int tiles_m = a.hm_tpi > 0 ? a.hm_B * a.hm_tpi : (a.M + Cfg::kBM - 1) / Cfg::kBM;
   const int tiles = tiles_m * ((a.N + BN - 1) / BN);
-  if (Cfg::kSkinny && a.tma_store != 2) throw std::runtime_error("gemm_tc: the skinny configuration only has the direct-store epilogue");
   if (a.fold_stats != nullptr || a.res != nullptr || a.stats_out != nullptr) {
     auto al16 = [](const void* q) { return (reinterpret_cast<uintptr_t>(q) & 15) == 0; };
-    if (a.tma_store != 2 || a.out_f32 || a.N % 32 != 0 || a.ldc % 8 != 0)
-      throw std::runtime_error("gemm_tc: the deferred-LayerNorm epilogue needs the direct-store path, bf16 output and N % 32 == 0");
     if ((a.bias && !al16(a.bias)) || (a.fold_stats && (!a.fold_c || !al16(a.fold_c) || a.fold_parts < 1 || a.fold_parts > kLnStatStride)) ||
         ((a.fold_stats || a.res_stats || a.stats_out) && a.stats_ld < a.M) ||
         (a.res && (!al16(a.res) || a.ldr % 8 != 0)) ||
@@ -786,24 +773,18 @@ const void* tma_map_rows3(const void* ptr, int D, int L, int64_t groups, int box
   return &cached_map(key, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, gdim, gstride, box, CU_TENSOR_MAP_SWIZZLE_128B);
 }
 
-int launch_gemm_tc(const GemmArgs& a_in, int num_sms, cudaStream_t stream) {
-  if (a_in.M <= 0 || a_in.N <= 0) return 0;
-  static const int dbg_env = [] { const char* e = getenv("GSTVD_GEMM_DBG"); return e ? atoi(e) : 0; }();
+namespace {
+
+// The selection rule (engine call sites: force_kernel = force_store = -1).  Environment switches are A/B aids and act here only.
+int rule_kernel(const GemmArgs& a, int num_sms) {
   static const int bn_env = [] { const char* e = getenv("GSTVD_GEMM_BN"); return e ? atoi(e) : 0; }();
-  GemmArgs a = a_in;
-  a.dbg = dbg_env;
-  if (a.K % 8 != 0) throw std::runtime_error("gemm_tc: K must be a multiple of 8");
-  if (a.hm_D > 0 && (a.hm_D % 32 != 0)) throw std::runtime_error("gemm_tc: head-major scatter needs head_dim % 32 == 0");
-  gemm_tc_init();
   if (a.fold_stats != nullptr || a.res != nullptr || a.stats_out != nullptr) {
     // deferred-LayerNorm epilogue (decode step): the M = 64 two-per-SM configuration with 32-column tiles while they fit the
     // resident slots (the N = H projections, the only ones that write statistics), 64-column tiles of 128 rows for the wide ones
-    if (a.K % BK != 0 || a.M > 4 * BM) throw std::runtime_error("gemm_tc: the deferred-LayerNorm epilogue needs K % 64 == 0 and M <= 512");
-    if (((a.M + 63) / 64) * ((a.N + 31) / 32) <= 2 * num_sms) launch_cfg<32, kEpiWarpsSkinny, true>(a, num_sms, stream);
-    else { if (a.stats_out != nullptr) throw std::runtime_error("gemm_tc: statistics are only written by 32-column tiles"); launch_cfg<64, kEpiWarpsWide, true>(a, num_sms, stream); }
-    return 1;
+    return ((a.M + 63) / 64) * ((a.N + 31) / 32) <= 2 * num_sms ? kGemmLn32 : kGemmLn64;
   }
-  if (launch_gemm_tc2_if_selected(a, num_sms, stream)) return 1;   // CTA-pair tiles (cta_group::2) where they measured faster: large M
+  const int pair_bn = pick_pair_bn(a);   // CTA-pair tiles (cta_group::2) where they measured faster: large M
+  if (pair_bn) return pair_bn == 256 ? kGemmPair256 : kGemmPair128;
   const int tiles_m = (a.M + BM - 1) / BM;
   int bn = 32;
   const int cand[4] = {256, 128, 64, 32};
@@ -841,19 +822,126 @@ int launch_gemm_tc(const GemmArgs& a_in, int num_sms, cudaStream_t stream) {
     if (skinny && direct_ok && a.K % BK == 0 && !bn_env) {
       const int tm64 = (a.M + 63) / 64;
       static const int multi = [] { const char* e = getenv("GSTVD_GEMM_SKINNY_WAVES"); return e ? atoi(e) : 1; }();   // A/B aid
-      if (tm64 * ((a.N + 31) / 32) <= 2 * num_sms * multi) { launch_cfg<32, kEpiWarpsSkinny>(a, num_sms, stream); return 1; }
+      if (tm64 * ((a.N + 31) / 32) <= 2 * num_sms * multi) return kGemmSkinny32;
       // wider outputs (N = 2304 / 3072 at M = 320) measured faster in the 128-row configuration with 16 epilogue warps
       // (5.5 / 5.7 us vs 5.9 / 6.2 us): 64-column tiles make each of the four epilogue warps handle two column blocks
       static const bool wide64 = getenv("GSTVD_GEMM_SKINNY64") != nullptr;
-      if (wide64 && tm64 * ((a.N + 63) / 64) <= 2 * num_sms) { launch_cfg<64, kEpiWarpsSkinny>(a, num_sms, stream); return 1; }
+      if (wide64 && tm64 * ((a.N + 63) / 64) <= 2 * num_sms) return kGemmSkinny64;
     }
   }
   switch (bn) {
-    case 256: launch_cfg<256>(a, num_sms, stream); break;
-    case 128: launch_cfg<128>(a, num_sms, stream); break;
-    case 64: launch_cfg<64>(a, num_sms, stream); break;
-    default: launch_cfg<32>(a, num_sms, stream); break;
+    case 256: return kGemmTc256;
+    case 128: return kGemmTc128;
+    case 64: return kGemmTc64;
+    default: return kGemmTc32;
   }
+}
+
+// The store the rule picks for `kernel`: TMA store when the output is expressible as a tensor map (head-major: 128-row tiles of
+// whole k-blocks only), direct row stores for small outputs, else the generic register/shared path.
+int rule_store(const GemmArgs& a, int kernel) {
+  if (kernel == kGemmSimt) return kStoreGeneric;
+  if (kernel == kGemmPair128 || kernel == kGemmPair256) return kStoreTma;
+  static const bool no_tma_store = getenv("GSTVD_GEMM_NO_TMA_STORE") != nullptr;
+  static const bool no_tma_hm = getenv("GSTVD_GEMM_NO_TMA_HM") != nullptr;
+  static const bool no_direct = getenv("GSTVD_GEMM_NO_DIRECT") != nullptr;     // A/B aid
+  const int esz = a.out_f32 ? 4 : 2;
+  if (no_tma_store || (reinterpret_cast<uintptr_t>(a.C) & 15) != 0) return kStoreGeneric;
+  if (a.hm_D > 0) {
+    const bool whole_kblocks = kernel == kGemmTc128 || kernel == kGemmTc256;
+    return !no_tma_hm && whole_kblocks && !a.out_f32 && a.hm_D % 32 == 0 && a.M == a.hm_B * a.hm_L ? kStoreTma : kStoreGeneric;
+  }
+  if ((a.ldc * esz) % 16 != 0) return kStoreGeneric;
+  // skinny (decode) problems: latency matters, the tile is tiny
+  if (a.M <= 4 * BM && (int64_t)a.M * a.N * esz <= (4 << 20) && !no_direct) return kStoreDirect;
+  return tma_store_cols(a.N, esz) > 0 ? kStoreTma : kStoreGeneric;
+}
+
+const char* const kKernelNames[kGemmKernels] = {"simt", "tc32", "tc64", "tc128", "tc256", "skinny32", "skinny64", "pair128", "pair256", "ln32", "ln64"};
+const char* const kStoreNames[kGemmStores] = {"generic", "TMA", "direct"};
+
+// What (kernel, store) cannot run, or "".  Only kernel limits are checked here, never the rule's preferences.
+std::string variant_unsupported(const GemmArgs& a, int kernel, int store) {
+  if (kernel < 0 || kernel >= kGemmKernels) return "unknown GEMM kernel id " + std::to_string(kernel);
+  if (store < 0 || store >= kGemmStores) return "unknown GEMM store id " + std::to_string(store);
+  const std::string what = std::string(kKernelNames[kernel]) + " with the " + kStoreNames[store] + " store: ";
+  const bool ln_args = a.fold_stats != nullptr || a.res != nullptr || a.stats_out != nullptr;
+  const bool ln = kernel == kGemmLn32 || kernel == kGemmLn64;
+  const bool skinny = kernel == kGemmSkinny32 || kernel == kGemmSkinny64;
+  const bool pair = kernel == kGemmPair128 || kernel == kGemmPair256;
+  const bool chunked = kernel == kGemmTc32 || kernel == kGemmTc64 || skinny || ln;    // 3-D boxes of several 64-element k-chunks
+  const int esz = a.out_f32 ? 4 : 2;
+  const bool c16 = (reinterpret_cast<uintptr_t>(a.C) & 15) == 0;
+  if (kernel == kGemmSimt) {
+    if (store != kStoreGeneric) return what + "the SIMT kernel stores element by element (generic store only)";
+    if (ln_args) return what + "the SIMT kernel has no deferred-LayerNorm epilogue";
+    return "";
+  }
+  if (ln_args != ln) return what + (ln ? "the deferred-LayerNorm kernels need a deferred-LayerNorm argument"
+                                       : "deferred-LayerNorm arguments need the ln32 / ln64 kernels");
+  if (a.K % 8 != 0) return what + "K must be a multiple of 8 (16-byte TMA strides)";
+  if (chunked && a.K % BK != 0) return what + "this configuration loads whole 64-element k-chunks: K % 64 == 0";
+  if (a.hm_D > 0 && a.hm_D % 32 != 0) return what + "the head-major scatter needs head_dim % 32 == 0";
+  if (skinny && store != kStoreDirect) return what + "the 64-row configurations only have the direct-store epilogue";
+  if (ln && store != kStoreDirect) return what + "the deferred-LayerNorm epilogue stores directly";
+  if (ln && (a.out_f32 || a.N % 32 != 0 || (a.ldc * 2) % 16 != 0)) return what + "the deferred-LayerNorm epilogue needs bf16 output, N % 32 == 0, ldc % 8 == 0";
+  if (pair && store != kStoreTma) return what + "the CTA-pair kernel only has the TMA-store epilogue";
+  switch (store) {
+    case kStoreTma:
+      if (!c16) return what + "the output must be 16-byte aligned";
+      if (a.hm_D > 0) {
+        if (!(kernel == kGemmTc128 || kernel == kGemmTc256 || pair)) return what + "head-major TMA tiles need whole 64-element k-blocks per stage (tc128 / tc256 / pairs)";
+        if (a.out_f32) return what + "the head-major TMA store writes bf16";
+        if (a.M != a.hm_B * a.hm_L || a.N % (a.hm_D * a.hm_G) != 0) return what + "the head-major TMA store needs M = B * L and N % (D * G) == 0";
+      } else if ((a.ldc * esz) % 16 != 0 || tma_store_cols(a.N, esz) == 0) {
+        return what + "output rows must be 16-byte aligned (ldc * element size % 16 == 0) and at least 16 bytes long";
+      }
+      break;
+    case kStoreDirect:
+      if (a.hm_D > 0) return what + "direct stores write row-major rows, not the head-major layout";
+      if (!c16 || (a.ldc * esz) % 16 != 0) return what + "direct stores need a 16-byte aligned output and rows (ldc * element size % 16 == 0)";
+      break;
+    default:
+      if (skinny || ln || pair) return what + "no generic epilogue in this configuration";
+      break;
+  }
+  return "";
+}
+
+}  // namespace
+
+std::string gemm_tc_variant(const GemmArgs& a, int num_sms, GemmVariant* v) {
+  const int kernel = a.force_kernel >= 0 ? a.force_kernel : rule_kernel(a, num_sms);
+  const int store = a.force_store >= 0 ? a.force_store : rule_store(a, kernel);
+  std::string why = variant_unsupported(a, kernel, store);
+  if (why.empty() && v) { v->kernel = kernel; v->store = store; }
+  return why;
+}
+
+int launch_gemm_tc(const GemmArgs& a_in, int num_sms, cudaStream_t stream, GemmVariant* ran) {
+  if (a_in.M <= 0 || a_in.N <= 0) return 0;
+  static const int dbg_env = [] { const char* e = getenv("GSTVD_GEMM_DBG"); return e ? atoi(e) : 0; }();
+  GemmArgs a = a_in;
+  a.dbg = dbg_env;
+  GemmVariant v;
+  const std::string why = gemm_tc_variant(a, num_sms, &v);
+  if (!why.empty()) throw std::runtime_error("gemm_tc: " + why);
+  gemm_tc_init();
+  a.tma_store = v.store;
+  switch (v.kernel) {
+    case kGemmTc32: launch_cfg<32>(a, num_sms, stream); break;
+    case kGemmTc64: launch_cfg<64>(a, num_sms, stream); break;
+    case kGemmTc128: launch_cfg<128>(a, num_sms, stream); break;
+    case kGemmTc256: launch_cfg<256>(a, num_sms, stream); break;
+    case kGemmSkinny32: launch_cfg<32, kEpiWarpsSkinny>(a, num_sms, stream); break;
+    case kGemmSkinny64: launch_cfg<64, kEpiWarpsSkinny>(a, num_sms, stream); break;
+    case kGemmPair128: launch_gemm_tc2(a, 128, num_sms, stream); break;
+    case kGemmPair256: launch_gemm_tc2(a, 256, num_sms, stream); break;
+    case kGemmLn32: launch_cfg<32, kEpiWarpsSkinny, true>(a, num_sms, stream); break;
+    case kGemmLn64: launch_cfg<64, kEpiWarpsWide, true>(a, num_sms, stream); break;
+    default: throw std::runtime_error("gemm_tc: the SIMT kernel is launched by launch_gemm_simt");
+  }
+  if (ran) *ran = v;
   return 1;
 }
 

@@ -248,6 +248,24 @@ __device__ __forceinline__ void epilogue_tma_block(const GemmArgs& p, const CUte
       }
     }
   }
+  if (p.hm_D == 0 && col0 + CW > p.tma_cols && p.dbg != 1 && p.dbg != 5) {
+    // the row's last partial 16-byte chunk: past the map's columns (a TMA store would write the whole chunk, beyond N)
+    const int row = tile_row0 + r;
+    if (row < p.M) {
+      OutT* dst = reinterpret_cast<OutT*>(p.C) + (int64_t)row * p.ldc + col0;
+#pragma unroll
+      for (int j = 0; j < CW; ++j) {
+        if (col0 + j >= p.tma_cols && col0 + j < p.N) {
+          if constexpr (sizeof(OutT) == 2) {
+            const __nv_bfloat162 h = *reinterpret_cast<const __nv_bfloat162*>(&packed[j >> 1]);
+            dst[j] = (j & 1) ? h.y : h.x;
+          } else {
+            dst[j] = __uint_as_float(packed[j]);
+          }
+        }
+      }
+    }
+  }
   const int sw = (kRowBytes == 128) ? (r & 7) : ((r >> 1) & 3);
   const uint32_t row_addr = stage_addr + r * kRowBytes;
   if (p.dbg == 5) {                                     // measurement: keep the math alive without touching shared memory
@@ -310,17 +328,21 @@ __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.
 const CUtensorMap& get_map(const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_rows);
 // Operand viewed as [K/64 chunks][rows][64]: one box = 64 elements x box_rows rows x `chunks` consecutive k-chunks.
 const CUtensorMap& get_map_k3(const void* ptr, int64_t rows, int64_t cols, int64_t ld, int box_rows, int chunks);
-// Output map for the TMA-store epilogue: [M, N] row-major with box = box_cols x 128 rows.
+// Output map for the TMA-store epilogue: [M, N] row-major with box = box_cols x 128 rows (N: GemmArgs::tma_cols).
 const CUtensorMap& get_map_c(const void* ptr, int64_t rows, int64_t cols, int64_t ld, int esz, int box_cols);
 
 // Head-major mode (cross-attention K/V prefill, GemmArgs::hm_*): activations viewed as [B][L][K] (box = 64 k x 128 positions of one
 // image, rows past L zero-filled) and the output [layers*B*G][L][D] (box = box_cols x 128 positions of one (layer-image, group)).
 const CUtensorMap& get_map_a3(const void* ptr, int64_t K, int L, int B, int64_t ld);
 const CUtensorMap& get_map_hm3(const void* ptr, int D, int L, int64_t LBG, int box_cols);
+// GemmArgs::tma_cols: N rounded down to whole 16-byte chunks of esz-byte elements.
+inline int tma_store_cols(int N, int esz) { return N - N % (16 / esz); }
 
-// CTA-pair kernel (gemm_tc2.cu): launches it and returns 1 when it is the faster configuration for this problem (large M, see
-// pick_pair_bn; env GSTVD_GEMM_2CTA=0 disables it, =128 / =256 force a pair tile width), else returns 0.
-int launch_gemm_tc2_if_selected(const GemmArgs& a, int num_sms, cudaStream_t stream);
+// CTA-pair kernel (gemm_tc2.cu).  pick_pair_bn: the pair tile width the selection rule picks for this problem, or 0 (large M, see its
+// definition; env GSTVD_GEMM_2CTA=0 disables it, =128 / =256 force a width wherever the kernel applies).  launch_gemm_tc2 launches the
+// bn-column pair kernel with the TMA-store epilogue on arguments gemm_tc_variant has accepted.
+int pick_pair_bn(const GemmArgs& a);
+void launch_gemm_tc2(const GemmArgs& a, int bn, int num_sms, cudaStream_t stream);
 
 }  // namespace tc
 }  // namespace gstvd

@@ -280,10 +280,11 @@ void launch_cfg2(const GemmArgs& a_in, int num_sms, cudaStream_t stream) {
   const bool hm = a.hm_D > 0;                                 // head-major prefill mode (pick_pair_bn has checked its preconditions)
   a.tma_store = 1;
   a.hm_tpi = hm ? (a.hm_L + BM - 1) / BM : 0;
+  a.tma_cols = hm ? a.N : tma_store_cols(a.N, esz);
   const CUtensorMap& ma = hm ? get_map_a3(a.A, a.K, a.hm_L, a.hm_B, a.lda) : get_map(a.A, a.M, a.K, a.lda, BM);
   const CUtensorMap& mb = get_map(a.W, a.N, a.K, a.ldw, Cfg::kBH);
   const CUtensorMap& mc = hm ? get_map_hm3(a.C, a.hm_D, a.hm_L, (int64_t)(a.N / (a.hm_D * a.hm_G)) * a.hm_B * a.hm_G, 32)
-                             : get_map_c(a.C, a.M, a.N, a.ldc, esz, 32);
+                             : get_map_c(a.C, a.M, a.tma_cols, a.ldc, esz, 32);
   const int units = hm ? a.hm_B * a.hm_tpi : (a.M + BM - 1) / BM;
   const int tiles = ((units + 1) / 2) * ((a.N + BN - 1) / BN);
   const int pairs = std::min(tiles, num_sms / 2);
@@ -299,12 +300,17 @@ void launch_cfg2(const GemmArgs& a_in, int num_sms, cudaStream_t stream) {
   if (e != cudaSuccess) throw std::runtime_error(std::string("gemm_tc2: launch failed: ") + cudaGetErrorString(e));
 }
 
-// CTA-pair configuration for this problem, or 0.  Needs the plain [M, N] (or head-major) TMA-store epilogue and enough rows to
-// fill pair tiles.  Selection rule from a same-box sweep over the encoder shapes (profiles/r2_gemm_pair_vs_single.txt): the
+}  // namespace
+
+namespace tc {
+
+// CTA-pair configuration the rule picks for this problem, or 0.  Needs the plain [M, N] (or head-major) TMA-store epilogue and enough
+// rows to fill pair tiles.  Selection rule from a same-box sweep over the encoder shapes (profiles/r2_gemm_pair_vs_single.txt): the
 // 256-column pair tile is 2-8 % faster than the single-CTA 128 x 256 tile from M = 12 288 on (and from M = 8 192 for the wide / deep
-// problems), slower below (fewer, larger tiles quantise worse); the 128-column pair tile never wins.
+// problems), slower below (fewer, larger tiles quantise worse); the 128-column pair tile never wins.  M >= 8 BM and N >= 128 are
+// policy: the kernel itself runs any M and N (a half-empty pair tile's second CTA stores nothing, TMA zero-fills missing rows).
 // env GSTVD_GEMM_2CTA: 0 = never, 128 / 256 = force that pair width wherever the kernel applies (tests), unset / 1 = the rule.
-int pick_pair_bn(const GemmArgs& a, int num_sms) {
+int pick_pair_bn(const GemmArgs& a) {
   const char* env = getenv("GSTVD_GEMM_2CTA");
   const int forced = env ? atoi(env) : 1;
   if (forced == 0) return 0;
@@ -318,23 +324,14 @@ int pick_pair_bn(const GemmArgs& a, int num_sms) {
   } else if ((a.ldc * esz) % 16 != 0) {
     return 0;
   }
-  (void)num_sms;
   if (forced == 128 || forced == 256) return forced;
   if (a.M >= 12288) return 256;
   if (a.M >= 8192 && (a.N >= 2304 || a.K >= 2048)) return 256;
   return 0;
 }
 
-}  // namespace
-
-namespace tc {
-
-int launch_gemm_tc2_if_selected(const GemmArgs& a, int num_sms, cudaStream_t stream) {
-  const int bn2 = pick_pair_bn(a, num_sms);
-  if (bn2 == 0) return 0;
-  gemm_tc_init();
-  if (bn2 == 256) launch_cfg2<256>(a, num_sms, stream); else launch_cfg2<128>(a, num_sms, stream);
-  return 1;
+void launch_gemm_tc2(const GemmArgs& a, int bn, int num_sms, cudaStream_t stream) {
+  if (bn == 256) launch_cfg2<256>(a, num_sms, stream); else launch_cfg2<128>(a, num_sms, stream);
 }
 
 }  // namespace tc

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <string>
 #include <utility>
 
 namespace gstvd {
@@ -48,6 +49,8 @@ struct GemmArgs {
   int hm_D = 0, hm_L = 0, hm_G = 0, hm_B = 0;
   int hm_tpi = 0;      // set by launch_gemm_tc: head-major TMA mode, M tiles per image (tiles never straddle images)
   int tma_store = 0;   // set by launch_gemm_tc: 1 = epilogue stores through a TMA tensor map, 2 = direct 16-byte row stores (skinny problems)
+  int tma_cols = 0;    // set by the launchers with tma_store = 1 (row-major): columns the TMA-store map covers, N rounded down to 16 bytes
+                       // (TMA stores clip at 16-byte granularity); the epilogue stores columns tma_cols .. N-1 directly
   // ---- deferred LayerNorm (decode step, direct-store epilogue only; DESIGN.md section 4) ----
   // The decoder's dense -> LayerNorm(x + input) pairs (HF BertSelfOutput / BertOutput, call site models/visual_dialog_decoder.py:300-311)
   // run without a LayerNorm kernel: the producing GEMM stores the RAW sum x = A W^T + b + residual (bf16) and, per 32-column block,
@@ -65,16 +68,31 @@ struct GemmArgs {
   float2* stats_out = nullptr;          // (mean, M2) of this launch's stored values per 32-column block
   unsigned long long* dbg_times = nullptr;   // measurement aid: per-CTA globaltimer stamps (8 per CTA)
   int dbg = 0;   // measurement aid (env GSTVD_GEMM_DBG): 1 = epilogue without global stores, 2 = epilogue skipped, 3 = no MMA
+  // Forced variant (single-operator tests; host only): a GemmKernel / GemmStore, or -1 = the launcher's rule, environment switches
+  // included.  The engine's call sites leave both at -1.
+  int force_kernel = -1, force_store = -1;
 };
 
 constexpr int kLnStatStride = 32;   // partial statistics per row (rows of at most 1024 columns)
 constexpr float kLnEpsDeferred = 1e-12f;
 
+// GEMM variants: kernel configuration (tile width; skinny = 64-row tiles, two CTAs per SM; pair = CTA-pair tiles of gemm_tc2.cu;
+// ln = the deferred-LayerNorm epilogue) and epilogue store (the values of GemmArgs::tma_store).  Numbered as in include/gstvd.h.
+enum GemmKernel { kGemmSimt = 0, kGemmTc32, kGemmTc64, kGemmTc128, kGemmTc256, kGemmSkinny32, kGemmSkinny64, kGemmPair128, kGemmPair256,
+                  kGemmLn32, kGemmLn64, kGemmKernels };
+enum GemmStore { kStoreGeneric = 0, kStoreTma = 1, kStoreDirect = 2, kGemmStores };
+struct GemmVariant { int kernel = -1, store = -1; };
+
 // SIMT GEMM: dtype kF32 (all fp32) or kBF16 (bf16 operands, fp32 accumulate; debugging aid)
 int launch_gemm_simt(const GemmArgs& a, int dtype, cudaStream_t stream);
+// The (kernel, store) the bf16 launchers run for `a`: the selection rule fills the fields left at -1, then the chosen pair is checked
+// against what the kernels can run (not against what the rule prefers).  Returns "" and sets *v, or the reason it cannot run.
+// kGemmSimt is accepted (store generic) for the single-operator entries, which launch it through launch_gemm_simt.
+std::string gemm_tc_variant(const GemmArgs& a, int num_sms, GemmVariant* v);
 // tcgen05 / TMEM / TMA GEMM, bf16 operands, fp32 accumulate.
 // Skinny (M <= 512) problems use the 6-warp / ~100 KB configuration of which two CTAs fit one SM.
-int launch_gemm_tc(const GemmArgs& a, int num_sms, cudaStream_t stream);
+// Throws when gemm_tc_variant refuses the arguments; `ran` (may be null) receives the variant launched.
+int launch_gemm_tc(const GemmArgs& a, int num_sms, cudaStream_t stream, GemmVariant* ran = nullptr);
 void gemm_tc_init();  // resolves cuTensorMapEncodeTiled, sets kernel attributes
 struct AttnArgs {
   const void* q = nullptr; int64_t q_bs = 0, q_hs = 0, q_rs = 0;   // element strides: batch, head, row

@@ -29,6 +29,15 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
+_KERNEL_NAMES = {v: k for k, v in _lib.GEMM_KERNELS.items()}
+_STORE_NAMES = {v: k for k, v in _lib.GEMM_STORES.items()}
+
+
+def _variant_names(ran):
+    """(kernel, store) names of the int32 pair a GEMM op entry reports."""
+    return _KERNEL_NAMES.get(ran[0]), _STORE_NAMES.get(ran[1])
+
+
 class Engine:
     """Owns a gstvd_ctx.  ``dec_cfg=None`` builds an encoder-only context (enc_only_a / NSP ranking)."""
 
@@ -293,15 +302,59 @@ class Engine:
                                               self._stream()))
 
     # ---- single operators (parity tests) ----------------------------------------------------------------------
-    def op_linear(self, a, w, bias=None, act=0, dtype=None):
+    def op_linear(self, a, w, bias=None, act=0, dtype=None, out_dtype="fp32", ldc=None, hm=None, kernel=None, store=None, out=None,
+                  want_variant=False):
+        """One GEMM launch (gstvd_op_linear): act(a w^T + bias) from fp32 ``a`` [M, K], ``w`` [N, K].  ``out_dtype``: what the kernel
+        stores (returned as fp32).  ``ldc``: row stride of the result (default N).  ``hm`` = (D, L, G, B): the head-major K/V layout of
+        the cross-attention prefill, result [N / (D * G)][B][G][L][D].  ``kernel`` / ``store``: a name of _lib.GEMM_KERNELS /
+        GEMM_STORES to force, None = the engine's choice.  ``out``: fp32 buffer holding the whole output region (M * ldc, or M * N
+        head-major) whose elements the kernel does not store are kept; default NaN.  ``want_variant``: also return the
+        (kernel, store) names that ran."""
         a, w = self._dev(a, torch.float32), self._dev(w, torch.float32)
         b = self._dev(bias, torch.float32)
         M, K = a.shape
         N = w.shape[0]
-        out = torch.empty(M, N, device=self.device, dtype=torch.float32)
+        ld = N if ldc is None else int(ldc)
+        if out is None:
+            shape = (N // (hm[0] * hm[2]), hm[3], hm[2], hm[1], hm[0]) if hm is not None else (M, ld)
+            out = torch.full(shape, float("nan"), device=self.device, dtype=torch.float32)
+        hm_arr = (ctypes.c_int32 * 4)(*[int(x) for x in hm]) if hm is not None else None
+        ran = (ctypes.c_int32 * 2)(-1, -1)
         check(self.ctx, self.lib.gstvd_op_linear(self.ctx, self.dtype if dtype is None else DTYPES[dtype], M, N, K, _ptr(a), _ptr(w),
-                                                 _ptr(b), int(act), _ptr(out), self._stream()))
-        return out
+                                                 _ptr(b), int(act), _ptr(out), 0 if hm is not None else ld, DTYPES[out_dtype], hm_arr,
+                                                 -1 if kernel is None else _lib.GEMM_KERNELS[kernel],
+                                                 -1 if store is None else _lib.GEMM_STORES[store], ran, self._stream()))
+        if hm is None and ldc is None:
+            out = out.view(M, N)
+        return (out, _variant_names(ran)) if want_variant else out
+
+    def op_linear_ln(self, a, w, bias=None, a_stats=None, ln_gamma=None, ln_beta=None, res=None, res_stats=None, res_gamma=None,
+                     res_beta=None, act=0, want_stats=False, kernel=None):
+        """One deferred-LayerNorm GEMM launch (gstvd_op_linear_ln), fp32 tensors in and out: act(LN(a) w^T + bias + R) stored bf16.
+        ``a_stats`` [K/32, M, 2]: per-32-column (mean, M2) of a's rows, with ``ln_gamma`` / ``ln_beta``: a's rows are LayerNormed
+        through folded weights.  ``res`` [M, N]: raw residual, or with ``res_stats`` [N/32, M, 2] / ``res_gamma`` / ``res_beta`` its
+        LayerNorm.  Returns (out [M, N], stats_out [N/32, M, 2] or None, (kernel, store) names)."""
+        f = lambda t: self._dev(t, torch.float32)
+        a, w, bias, a_stats, ln_gamma, ln_beta, res, res_stats, res_gamma, res_beta = map(
+            f, (a, w, bias, a_stats, ln_gamma, ln_beta, res, res_stats, res_gamma, res_beta))
+        M, K = a.shape
+        N = w.shape[0]
+        out = torch.empty(M, N, device=self.device, dtype=torch.float32)
+        st = torch.full((N // 32, M, 2), float("nan"), device=self.device, dtype=torch.float32) if want_stats else None
+        ran = (ctypes.c_int32 * 2)(-1, -1)
+        check(self.ctx, self.lib.gstvd_op_linear_ln(self.ctx, M, N, K, _ptr(a), _ptr(a_stats), _ptr(ln_gamma), _ptr(ln_beta), _ptr(w),
+                                                    _ptr(bias), _ptr(res), _ptr(res_stats), _ptr(res_gamma), _ptr(res_beta), int(act),
+                                                    _ptr(out), _ptr(st), -1 if kernel is None else _lib.GEMM_KERNELS[kernel], ran,
+                                                    self._stream()))
+        return out, st, _variant_names(ran)
+
+    def debug_cross_cache(self, B, Le):
+        """The cross-attention K/V of the last prefill_cross, fp32 [layers, B, 2 * heads, Le, D] (k heads, then v heads)."""
+        d = self.dec_cfg
+        heads = int(d.num_attention_heads)
+        buf = torch.empty(int(d.num_hidden_layers), B, 2 * heads, Le, int(d.hidden_size) // heads, dtype=torch.float32, device=self.device)
+        check(self.ctx, self.lib.gstvd_debug_cross_cache(self.ctx, int(B), int(Le), _ptr(buf), self._stream()))
+        return buf
 
     def op_add_layernorm(self, x, residual, gamma, beta, dtype=None):
         x = self._dev(x, torch.float32)

@@ -27,7 +27,7 @@
 extern "C" {
 #endif
 
-#define GSTVD_ABI_VERSION 5
+#define GSTVD_ABI_VERSION 6
 #define GSTVD_MAX_CONNECTIONS 16
 
 typedef enum {
@@ -290,10 +290,56 @@ int gstvd_splice(gstvd_ctx* ctx, int B, int Lt, int Lu, int64_t* enc_input_ids, 
                  int32_t* abnormal, void* stream);
 
 /* ---- single operators, exported for the parity tests ------------------------------------------------------ */
-/* C[M,N] = act(A[M,K] * W[N,K]^T + bias).  a/w/c are fp32 device buffers; with dtype == GSTVD_BF16 the operands are
- * rounded to bf16 and the tcgen05 kernel runs, with GSTVD_F32 the SIMT fp32 kernel runs. act: 0 none, 1 erf-GELU. */
+/* GEMM variants the single-operator GEMM entries can force (kernel / store arguments; -1 = the engine's own choice, environment
+ * switches included).  Kernels: SIMT fp32-accumulate; tcgen05 128-row tiles of 32 / 64 / 128 / 256 columns; 64-row "skinny" tiles of
+ * 32 / 64 columns (two CTAs per SM); CTA-pair tiles of 256 rows and 128 / 256 columns; the deferred-LayerNorm epilogue in 64-row x
+ * 32-column and 128-row x 64-column tiles.  Stores: generic (transposed through shared memory, any layout), TMA tensor store, direct
+ * 16-byte row stores.  What each kernel can run (anything else is refused with GSTVD_ERR_UNSUPPORTED before any launch, and
+ * gstvd_launch_count does not move):
+ *   tc32 / tc64        generic, TMA, direct; head-major only with the generic store; K % 64 == 0
+ *   tc128 / tc256      generic, TMA, direct; head-major with the generic store, or TMA (bf16 output, M = B * L, N % (D * G) == 0)
+ *   skinny32 / 64      direct only; no head-major; K % 64 == 0
+ *   pair128 / 256      TMA only (head-major as for tc128 / tc256)
+ *   ln32 / ln64        direct only, bf16 output, N % 32 == 0; K % 64 == 0; only gstvd_op_linear_ln (deferred-LayerNorm arguments)
+ *   simt               generic only
+ * Every tcgen05 kernel needs K % 8 == 0 and, head-major, D % 32 == 0; TMA and direct stores need a 16-byte aligned output with
+ * ldc * element size % 16 == 0.  The rest is the engine's selection policy (e.g. pair tiles from M >= 1024, skinny and ln tiles for
+ * M <= 512, statistics from the 32-column tiles), which a forced variant does not have to follow. */
+typedef enum {
+  GSTVD_GEMM_SIMT = 0, GSTVD_GEMM_TC32 = 1, GSTVD_GEMM_TC64 = 2, GSTVD_GEMM_TC128 = 3, GSTVD_GEMM_TC256 = 4, GSTVD_GEMM_SKINNY32 = 5,
+  GSTVD_GEMM_SKINNY64 = 6, GSTVD_GEMM_PAIR128 = 7, GSTVD_GEMM_PAIR256 = 8, GSTVD_GEMM_LN32 = 9, GSTVD_GEMM_LN64 = 10
+} gstvd_gemm_kernel;
+typedef enum { GSTVD_STORE_GENERIC = 0, GSTVD_STORE_TMA = 1, GSTVD_STORE_DIRECT = 2 } gstvd_gemm_store;
+
+/* C = act(A[M,K] * W[N,K]^T + bias).  a/w/c are fp32 device buffers; with dtype == GSTVD_BF16 the operands are rounded to bf16 and
+ * a tcgen05 kernel runs (or the forced SIMT kernel), with GSTVD_F32 the SIMT fp32 kernel runs (fp32 output only). act: 0 none,
+ * 1 erf-GELU (tcgen05: the fast GELU, |error| <= 2.5e-4 |x| and < 2e-4).
+ *   out_dtype : GSTVD_F32 or GSTVD_BF16, the type the kernel stores (bf16 results are returned widened to fp32 in c);
+ *   ldc       : row stride of c in elements (0: N), >= N;
+ *   hm        : NULL, or host int32 {D, L, G, B}: the head-major scatter of the cross-attention K/V prefill, row r = b * L + pos,
+ *               column n = g * D + d with g = layer * G + j, stored at c[(((layer * B + b) * G + j) * L + pos) * D + d]; needs
+ *               M = B * L, N % (D * G) == 0, ldc = 0;
+ *   c         : the whole output region, M * ldc elements (head-major: M * N).  It is copied into the output buffer before the GEMM and
+ *               back after it, so elements the kernel does not store (columns N .. ldc-1) keep what the caller put there;
+ *   kernel / store : a gstvd_gemm_kernel / gstvd_gemm_store to force, or -1;
+ *   ran       : NULL or host int32 [2]: receives the (kernel, store) that ran, also when chosen by the engine. */
 int gstvd_op_linear(gstvd_ctx* ctx, int dtype, int M, int N, int K, const float* a, const float* w, const float* bias,
-                    int act, float* c, void* stream);
+                    int act, float* c, int64_t ldc, int out_dtype, const int32_t* hm, int kernel, int store, int32_t* ran,
+                    void* stream);
+/* One deferred-LayerNorm GEMM launch (the decode step's gemm_ln; DESIGN.md section 4) on caller-supplied operands, bf16 inside:
+ *   y = act(LNa(A) W^T + bias + R),  stored bf16 and returned in out fp32 [M, N];
+ *   LNa(A) = A when a_stats is NULL, else LayerNorm of the raw rows of A [M, K] with affine ln_gamma / ln_beta [K], applied through
+ *            folded weights (W' = bf16(W * gamma), c = sum_k W'_nk, d = sum_k beta_k W_nk + bias_n): y = rstd (A W'^T - mean c) + d;
+ *            a_stats fp32 [K/32][M][2] holds each row's (mean, M2) per 32-column block, merged by the kernel (eps 1e-12);
+ *   R = 0 when res is NULL; res fp32 [M, N] (rounded to bf16), raw, or with res_stats [N/32][M][2] its LayerNorm with res_gamma /
+ *       res_beta [N];
+ *   stats_out : NULL or fp32 [N/32][M][2]: (mean, M2) of the 32 stored bf16 values of every row and 32-column block.
+ * N % 32 == 0; K % 32 == 0 and K <= 1024 with a_stats; N <= 1024 with res_stats or stats_out.  kernel: -1, GSTVD_GEMM_LN32 or
+ * GSTVD_GEMM_LN64 (refusals as for gstvd_op_linear); ran as there.  At least one of a_stats, res, stats_out must be given. */
+int gstvd_op_linear_ln(gstvd_ctx* ctx, int M, int N, int K, const float* a, const float* a_stats, const float* ln_gamma,
+                       const float* ln_beta, const float* w, const float* bias, const float* res, const float* res_stats,
+                       const float* res_gamma, const float* res_beta, int act, float* out, float* stats_out, int kernel,
+                       int32_t* ran, void* stream);
 /* y = LayerNorm(x + residual) with eps 1e-12 inside the sqrt (models/vilbert_dialog.py:283-296). residual may be NULL */
 int gstvd_op_add_layernorm(gstvd_ctx* ctx, int dtype, int rows, int width, const float* x, const float* residual,
                            const float* gamma, const float* beta, float* y, void* stream);
@@ -359,6 +405,10 @@ int gstvd_op_anc_update(gstvd_ctx* ctx, int B, int K, int T, int P0, const int32
  * hidden] on the device for one (layer, kv in {0: key, 1: value}); write != 0 stores buf into the cache (rounded to the
  * compute dtype), else reads it back.  Lets the tests check gstvd_reorder_cache against index_select(0, beam_idx) directly. */
 int gstvd_debug_self_cache(gstvd_ctx* ctx, int write, int B, int K, int layer, int kv, float* buf, void* stream);
+
+/* Test access to the cross-attention K/V that gstvd_prefill_cross wrote: buf fp32 [layers][B][2 * heads][Le][D] on the device (k heads,
+ * then v heads; D = hidden / heads), read only.  B and Le must be those of the last prefill. */
+int gstvd_debug_cross_cache(gstvd_ctx* ctx, int B, int Le, float* buf, void* stream);
 
 /* Measurement aid (bench.py's decode-step roofline): out int32 [B] (device) = keys of each image's resident cross-attention K/V
  * that a decode step fetches (last unmasked key + 1, computed at gstvd_prefill_cross). */

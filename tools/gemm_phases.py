@@ -3,7 +3,6 @@ import os
 import sys
 
 os.environ.setdefault("GSTVD_GEMM_TIMES", "1")
-os.environ.setdefault("GSTVD_OP_LINEAR_BF16OUT", "1")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch  # noqa: E402
@@ -20,5 +19,5 @@ for N, K in ((768, 768), (2304, 768), (3072, 768), (768, 3072), (30522, 768)):
     b = torch.randn(N, device="cuda")
     for rep in range(3):
         sys.stderr.write(f"--- M={M} N={N} K={K} rep {rep}\n"); sys.stderr.flush()
-        eng.op_linear(a, w, b)
+        eng.op_linear(a, w, b, out_dtype="bf16")
 eng.close()

@@ -3,7 +3,6 @@ import os
 import sys
 
 os.environ.setdefault("GSTVD_GEMM_TIMES", "1")
-os.environ.setdefault("GSTVD_OP_LINEAR_BF16OUT", "1")
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch  # noqa: E402
@@ -23,5 +22,5 @@ for K1 in (768, 3072):
         eng.op_deferred_ln_chain(a1, w1, b1, res0, g1, be1, w2, b2, g1, be1)
     for rep in range(3):
         sys.stderr.write(f"--- plain M={M} N={N} K={K1} rep {rep}\n"); sys.stderr.flush()
-        eng.op_linear(a1, w1, b1)
+        eng.op_linear(a1, w1, b1, out_dtype="bf16")
 eng.close()
