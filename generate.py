@@ -92,7 +92,8 @@ def main(argv=None):
             q_kwargs.update(do_sample=True)
     for kw, who in ((a_kwargs, ''), (q_kwargs, 'q_')):
         kw.update(repetition_penalty=params[f'{who}repetition_penalty'], no_repeat_ngram_size=params[f'{who}no_repeat_ngram_size'],
-                  min_length=params[f'{who}min_length'])
+                  min_length=params[f'{who}min_length'], length_penalty=params[f'{who}length_penalty'],
+                  early_stopping=params[f'{who}early_stopping'], bad_words_ids=params[f'{who}bad_words_ids'])
     decode = None
     if params['vocab_file']:
         from transformers import BertTokenizer

@@ -72,10 +72,14 @@ struct DevBuf {
 // replay, so the caller's tensor addresses are not part of the key (a caching allocator hands out a new address per batch).  seed and
 // row_offset are not either: the graph reads them from device memory, so a replay can use a new seed.  Fields that do not apply to
 // a kind of call are 0: Lh / Le for a generate graph; Lt / Lv and the has_* flags (optional inputs, out_scores) for a round graph.
-// K = decode rows per image; P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start.
+// K = decode rows per image; P = decoder prefix length; has_prefix = 0 for the implicit [CLS] start.  length_penalty / early_stopping
+// (beam modes; 1 / 0 in sampling, which ignores them) are baked into the launches; of the bad-word list only its shape is (bw_single:
+// whether it has one-id sequences, bw_count: its longer sequences), its content is re-uploaded into the context's buffer before a replay.
 struct GraphKey {
   int B, K, mode, T, top_k, ngram, P, has_prefix, N, G, Lh, Le, Lt, Lv, has_seg, has_att, has_imask, has_scores, no_repeat_ngram, min_length;
   float temperature, top_p, penalty, repetition_penalty;
+  float length_penalty;
+  int early_stopping, bw_single, bw_count;
   bool operator<(const GraphKey& o) const { return std::memcmp(this, &o, sizeof(GraphKey)) < 0; }
 };
 constexpr size_t kMaxGraphs = 24;      // least-recently-used graphs beyond this are destroyed (an 18-step graph holds ~2k kernel nodes)
@@ -144,6 +148,13 @@ struct gstvd_ctx {
   std::vector<ProfRec> prof_pool; size_t prof_used = 0;
   cudaStream_t own_stream = nullptr;     // decode steps run (and are graph-captured) here: the caller may be on the legacy stream
   cudaEvent_t ev_in = nullptr, ev_out = nullptr;
+  // bad_words_ids of the current call in the kernels' form (stage_bad_words): device copy, pinned staging buffer (a pageable copy would
+  // drain the stream), the event of its last upload and the content the device copy holds
+  DevBuf bw_dev;
+  int32_t* bw_host = nullptr;
+  cudaEvent_t bw_ev = nullptr;
+  std::vector<int32_t> bw_words;
+  int bw_single = 0, bw_count = 0;       // the current list: one-id sequences present, multi-id sequences
 
   size_t act_bytes(size_t elems) const { return elems * esz; }
 };
@@ -691,10 +702,62 @@ void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
                                          prefix, P, p0s, s);
 }
 
-// The request's logits processors; the caller fills in where the rows' decoder input lives.
-LogitsProcs logits_procs(const gstvd_gen_params& gp) {
+// Device form of the bad-word list (LogitsProcs::bw_*): [vocab bitmap of the one-id sequences, (V + 31) / 32 words][bw_count entries
+// {offset, m, last}][the first m ids of every longer sequence].  Words of the bitmap region.
+int bw_bitmap_words(const gstvd_ctx* c) { return (c->V + 31) / 32; }
+
+// Checks the request's bad_words_ids (host memory: sequences of ids each closed by -1) and makes the context's device copy hold it:
+// a list whose content differs from what the copy holds is staged in pinned memory (after the previous upload from there has
+// completed) and copied on `s`.  A lone [SEP] sequence is dropped (HF filters [eos_token_id]).  Sets c->bw_single / c->bw_count.
+void stage_bad_words(gstvd_ctx* c, const gstvd_gen_params& gp, cudaStream_t s) {
+  const int n = gp.bad_words_len;
+  const int32_t* ids = reinterpret_cast<const int32_t*>(static_cast<uintptr_t>(gp.bad_words_ids));
+  if (n < 0) throw InvalidArg(fmt("generate: bad_words_len %d must be >= 0", n));
+  if (n > 0 && !ids) throw InvalidArg("generate: bad_words_len > 0 with a NULL bad_words_ids");
+  c->bw_single = 0; c->bw_count = 0;
+  if (n == 0) return;
+  const int W = bw_bitmap_words(c);
+  std::vector<int32_t> words(W, 0), head, tail;
+  int seqs = 0, total = 0;
+  for (int i = 0; i < n;) {
+    int j = i;
+    while (j < n && ids[j] != -1) {
+      if (ids[j] < 0 || ids[j] >= c->V) throw InvalidArg(fmt("generate: bad word id %d outside [0, vocab = %d)", ids[j], c->V));
+      ++j;
+    }
+    if (j == n) throw InvalidArg("generate: the last bad-word sequence is not closed by -1");
+    const int L = j - i;
+    if (L < 1 || L > kBadWordsMaxLen) throw InvalidArg(fmt("generate: a bad-word sequence of %d ids (1..%d)", L, kBadWordsMaxLen));
+    if (++seqs > kBadWordsMaxSeqs) throw InvalidArg(fmt("generate: more than %d bad-word sequences", kBadWordsMaxSeqs));
+    if ((total += L) > kBadWordsMaxIds) throw InvalidArg(fmt("generate: more than %d bad-word ids", kBadWordsMaxIds));
+    if (L == 1 && ids[i] != 102) {
+      words[ids[i] >> 5] |= (int32_t)(1u << (ids[i] & 31));
+      c->bw_single = 1;
+    } else if (L > 1) {
+      head.push_back((int32_t)tail.size()); head.push_back(L - 1); head.push_back(ids[j - 1]);
+      tail.insert(tail.end(), ids + i, ids + j - 1);
+    }
+    i = j + 1;
+  }
+  c->bw_count = (int)head.size() / 3;
+  for (size_t e = 0; e < head.size(); e += 3) head[e] += (int32_t)head.size();     // offsets from the start of the entries
+  words.insert(words.end(), head.begin(), head.end());
+  words.insert(words.end(), tail.begin(), tail.end());
+  if (words == c->bw_words) return;
+  CUDA_CHECK(cudaEventSynchronize(c->bw_ev));            // the previous upload has read the staging buffer
+  std::memcpy(c->bw_host, words.data(), words.size() * 4);
+  CUDA_CHECK(cudaMemcpyAsync(c->bw_dev.p, c->bw_host, words.size() * 4, cudaMemcpyHostToDevice, s));
+  CUDA_CHECK(cudaEventRecord(c->bw_ev, s));
+  c->bw_words.swap(words);
+}
+
+// The request's logits processors, with the bad-word list stage_bad_words left in the context; the caller fills in where the rows'
+// decoder input lives.
+LogitsProcs logits_procs(const gstvd_ctx* c, const gstvd_gen_params& gp) {
   LogitsProcs p;
   p.repetition_penalty = gp.repetition_penalty; p.no_repeat_ngram = gp.no_repeat_ngram_size; p.min_length = gp.min_length;
+  if (c->bw_single) p.bw_single = (const uint32_t*)c->bw_dev.p;
+  if (c->bw_count) { p.bw_seq = (const int32_t*)c->bw_dev.p + bw_bitmap_words(c); p.bw_count = c->bw_count; }
   return p;
 }
 
@@ -767,7 +830,7 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   X.gemm(c->dh.p, H, c->lm_head, c->logits.p, c->Vpad, M, 0, true);
   float* sv = (float*)c->sel_val.p; int32_t* si = (int32_t*)c->sel_idx.p;
   // the logits processors act inside the selection kernels; each reads its rows' decoder input (cur_len = P + step <= 64)
-  LogitsProcs procs = logits_procs(gp);
+  LogitsProcs procs = logits_procs(c, gp);
   procs.P = P; procs.step = step_host; procs.d_step = d_step; procs.p0s = g.P0s; procs.rows_per_image = g.K;
   if (beams) {
     // beam sampling: g.K = N * K rows per image (N searches of K beams), each row's 16 best for the warpers and the draw
@@ -797,10 +860,11 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     if (sampled) {
       const int K = gp.num_beams;
       c->launches += launch_beam_sample_step(bb, M / K, g.K / K, K, Tn, c->V, sv, si, gp.top_k, gp.temperature, gp.top_p,
-                                             (const uint64_t*)c->d_seed.p, 102, P, g.P0s, s);
+                                             (const uint64_t*)c->d_seed.p, 102, P, g.P0s, len_penalty(gp.length_penalty, gp.early_stopping), s);
     } else {
       c->launches += launch_beam_step(bb, g.B, g.K, G, Tn, c->V, nsel, sv, si, G > 1 ? (const float*)c->logits.p : nullptr, c->Vpad, lz,
-                                      gp.diversity_penalty, gp.repetition_penalty, prefix, 102, P, g.P0s, nullptr, nullptr, nullptr, s);
+                                      gp.diversity_penalty, gp.repetition_penalty, prefix, 102, P, g.P0s,
+                                      len_penalty(gp.length_penalty, gp.early_stopping), nullptr, nullptr, nullptr, s);
     }
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
@@ -854,6 +918,8 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* pref
     throw InvalidArg(fmt("generate: repetition_penalty %g must be finite and > 0 (1 = off)", (double)gp.repetition_penalty));
   if (gp.no_repeat_ngram_size < 0) throw InvalidArg(fmt("generate: no_repeat_ngram_size %d must be >= 0", gp.no_repeat_ngram_size));
   if (gp.min_length < 0) throw InvalidArg(fmt("generate: min_length %d must be >= 0", gp.min_length));
+  if (!std::isfinite(gp.length_penalty)) throw InvalidArg(fmt("generate: length_penalty %g must be finite (1 = HF default)", (double)gp.length_penalty));
+  if (gp.early_stopping != 0 && gp.early_stopping != 1) throw InvalidArg(fmt("generate: early_stopping %d must be 0 or 1", gp.early_stopping));
   if (G < 1) throw InvalidArg(fmt("generate: %d beam groups", G));
   if (G > 1 && gp.mode != GSTVD_SELECT_BEAM) throw InvalidArg("generate: beam groups need beam search");
   int K = 1;
@@ -887,15 +953,16 @@ int check_generate(gstvd_ctx* c, const gstvd_gen_params& gp, const int64_t* pref
 // out_ids [B*N, T] image-major (sample mode: N == K, one row per candidate)
 void generate_finalize(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, int64_t* out_ids, float* out_scores, cudaStream_t s) {
   const int B = g.B, K = g.K, P = g.P0 + 1, T = gp.max_new_tokens, N = gp.num_return_sequences;
-  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, P, g.P0s, 1, N, out_ids, out_scores, s);
+  const LenPenalty lp = len_penalty(gp.length_penalty, gp.early_stopping);
+  if (gp.mode == GSTVD_SELECT_BEAM) c->launches += launch_beam_finalize(beam_buffers(c), B, K, T, 102, P, g.P0s, 1, N, lp, out_ids, out_scores, s);
   else if (gp.mode == GSTVD_SELECT_BEAM_SAMPLE)   // search n of image b is search b * N + n: its best hypothesis is output row b * N + n
-    c->launches += launch_beam_finalize(beam_buffers(c), B * N, gp.num_beams, T, 102, P, g.P0s, N, 1, out_ids, out_scores, s);
+    c->launches += launch_beam_finalize(beam_buffers(c), B * N, gp.num_beams, T, 102, P, g.P0s, N, 1, lp, out_ids, out_scores, s);
   else c->launches += launch_sample_finalize(B * K, T, 102, (const int32_t*)c->seq.p, out_ids, s);
 }
 
 // The key of a generate graph (Lh, Le set) or a round graph (Lt, Lv and the has_* flags set), from the request and the shapes.
-GraphKey graph_key(const gstvd_gen_params& gp, int B, int K, int P, bool has_prefix, int Lh, int Le, int Lt, int Lv, bool has_seg,
-                   bool has_att, bool has_imask, bool has_scores) {
+GraphKey graph_key(const gstvd_ctx* c, const gstvd_gen_params& gp, int B, int K, int P, bool has_prefix, int Lh, int Le, int Lt, int Lv,
+                   bool has_seg, bool has_att, bool has_imask, bool has_scores) {
   GraphKey k;
   std::memset(&k, 0, sizeof k);
   k.B = B; k.K = K; k.mode = gp.mode; k.T = gp.max_new_tokens; k.top_k = gp.top_k; k.ngram = gp.ngram_blocking_size;
@@ -903,6 +970,9 @@ GraphKey graph_key(const gstvd_gen_params& gp, int B, int K, int P, bool has_pre
   k.Lh = Lh; k.Le = Le; k.Lt = Lt; k.Lv = Lv; k.has_seg = has_seg; k.has_att = has_att; k.has_imask = has_imask; k.has_scores = has_scores;
   k.temperature = gp.temperature; k.top_p = gp.top_p; k.penalty = gp.diversity_penalty;
   k.repetition_penalty = gp.repetition_penalty; k.no_repeat_ngram = gp.no_repeat_ngram_size; k.min_length = gp.min_length;
+  const bool beams = gp.mode != GSTVD_SELECT_SAMPLE;
+  k.length_penalty = beams ? gp.length_penalty : 1.f; k.early_stopping = beams ? gp.early_stopping : 0;
+  k.bw_single = c->bw_single; k.bw_count = c->bw_count;
   return k;
 }
 
@@ -944,6 +1014,7 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
                  const int64_t* hist_seg, int Lh, int64_t* out_ids, float* out_scores, cudaStream_t s) {
   const int K = check_generate(c, gp, prefix, P, hist_ids, hist_seg, Lh, out_ids);
   if (c->cross_B != B) throw StateError(fmt("generate: cross K/V prefilled for %d images, asked for %d", c->cross_B, B));
+  stage_bad_words(c, gp, s);
   const int T = gp.max_new_tokens;
   const int64_t* pre = stage_prefix(c, B, prefix, P, s);
   const DecodeGeom g = make_geom(c, B, K, T, P, pre != nullptr);
@@ -965,7 +1036,7 @@ void do_generate(gstvd_ctx* c, int B, const gstvd_gen_params& gp, const int64_t*
   };
   // the cross cache geometry (Le) is part of the captured launch parameters
   if (!use_graph) body();
-  else replay_graph(c, c->graphs, graph_key(gp, B, K, P, pre, Lh, c->cross_Le, 0, 0, false, false, false, false), s, body);
+  else replay_graph(c, c->graphs, graph_key(c, gp, B, K, P, pre, Lh, c->cross_Le, 0, 0, false, false, false, false), s, body);
   generate_finalize(c, g, gp, out_ids, out_scores, s);
 }
 
@@ -981,6 +1052,7 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
   if (B < 1 || B > c->B_max || Lt < 1 || Lt > c->Lt_max || Lv < 1 || Lv > c->Lv_max) throw InvalidArg("round: shape exceeds capacity");
   if (!ids || !feat || !loc) throw InvalidArg("round: input_ids / image_feat / image_loc must not be NULL");
   if (gp.ngram_blocking_size > 0 && !seg) throw InvalidArg("round: n-gram blocking needs token_type_ids");
+  stage_bad_words(c, gp, s);
   const int T = gp.max_new_tokens, N = gp.num_return_sequences, F = c->cfg.v_feature_size;
   auto d2d = [&](void* dst, const void* src, size_t bytes) { if (src) CUDA_CHECK(cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, s)); };
   d2d(c->r_ids.p, ids, (size_t)B * Lt * 8); d2d(c->r_seg.p, seg, (size_t)B * Lt * 8); d2d(c->r_att.p, att, (size_t)B * Lt * 4);
@@ -1003,7 +1075,7 @@ void do_round(gstvd_ctx* c, int B, int Lt, int Lv, const int64_t* ids, const int
   if (!use_graph) {
     body();
   } else {
-    replay_graph(c, c->round_graphs, graph_key(gp, B, K, P, pre, 0, 0, Lt, Lv, seg, att, imask, out_scores), s, body);
+    replay_graph(c, c->round_graphs, graph_key(c, gp, B, K, P, pre, 0, 0, Lt, Lv, seg, att, imask, out_scores), s, body);
     // host-side state the captured calls set (a replay does not run them again)
     c->enc_B = B; c->enc_Le = Lv + Lt; c->cross_B = B; c->cross_Le = Lv + Lt;
   }
@@ -1126,6 +1198,10 @@ int gstvd_create(const gstvd_config* cfg, int device, gstvd_ctx** out) {
     CUDA_CHECK(cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking));
     CUDA_CHECK(cudaEventCreateWithFlags(&c->ev_in, cudaEventDisableTiming));
     CUDA_CHECK(cudaEventCreateWithFlags(&c->ev_out, cudaEventDisableTiming));
+    const size_t bw_bytes = (size_t)(bw_bitmap_words(c) + 3 * kBadWordsMaxSeqs + kBadWordsMaxIds) * 4;
+    c->bw_dev.alloc(bw_bytes);
+    CUDA_CHECK(cudaMallocHost(&c->bw_host, bw_bytes));
+    CUDA_CHECK(cudaEventCreateWithFlags(&c->bw_ev, cudaEventDisableTiming));
     CUDA_CHECK(cudaDeviceSynchronize());
   });
   if (rc != GSTVD_OK) { if (c) gstvd_destroy(c); return rc; }
@@ -1147,11 +1223,13 @@ void gstvd_destroy(gstvd_ctx* c) {
                     &c->logz, &c->ban_tokens, &c->ban_count, &c->prefix, &c->seq, &c->beam_scores, &c->beam_tokens, &c->cur_tokens,
                     &c->beam_idx, &c->beam_done, &c->hyp_score, &c->hyp_len, &c->hyp_tokens, &c->hyp_count, &c->hyp_worst, &c->d_step, &c->d_seed, &c->anc, &c->dec_prefix_own, &c->dec_prefix_head, &c->prefix_p0, &c->fold16, &c->foldvec,
                     &c->st1, &c->st2, &c->st3, &c->hist_ids_own, &c->hist_seg_own, &c->r_ids, &c->r_seg, &c->r_att,
-                    &c->r_feat, &c->r_loc, &c->r_imask, &c->r_out_ids, &c->r_out_scores};
+                    &c->r_feat, &c->r_loc, &c->r_imask, &c->r_out_ids, &c->r_out_scores, &c->bw_dev};
   for (DevBuf* b : bufs) b->release();
   for (auto& r : c->prof_pool) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
   if (c->ev_in) cudaEventDestroy(c->ev_in);
   if (c->ev_out) cudaEventDestroy(c->ev_out);
+  if (c->bw_ev) cudaEventDestroy(c->bw_ev);
+  if (c->bw_host) cudaFreeHost(c->bw_host);
   if (c->own_stream) cudaStreamDestroy(c->own_stream);
   delete c;
   if (prev >= 0) cudaSetDevice(prev);
@@ -1694,7 +1772,7 @@ int gstvd_op_beam_step(gstvd_ctx* c, const float* logits, int64_t ldl, int32_t* 
     c->launches += launch_row_select(B * K, c->V, logits, ldl, 0, (const float*)c->beam_scores.p, 1.f, nullptr, nullptr, 0, nsel,
                                      (float*)c->sel_val.p, (int32_t*)c->sel_idx.p, nullptr, LogitsProcs(), s);
     c->launches += launch_beam_step(beam_buffers(c), B, K, 1, T, c->V, nsel, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, nullptr,
-                                    0, nullptr, 0.f, 1.f, nullptr, 102, 1, nullptr, beam_idx, next_tokens, next_scores, s);
+                                    0, nullptr, 0.f, 1.f, nullptr, 102, 1, nullptr, len_penalty(1.f, 0), beam_idx, next_tokens, next_scores, s);
     c->launches += launch_step_advance((int*)c->d_step.p, s);
   });
 }
@@ -1703,7 +1781,8 @@ int gstvd_op_beam_end(gstvd_ctx* c, int64_t* out_ids, float* out_scores, void* s
   if (!c || !out_ids) return GSTVD_ERR_INVALID;
   return guarded(c, [&] {
     if (c->op_B == 0) throw StateError("beam_end before beam_begin");
-    c->launches += launch_beam_finalize(beam_buffers(c), c->op_B, c->op_K, c->op_T, 102, 1, nullptr, 1, 1, out_ids, out_scores, (cudaStream_t)stream);
+    c->launches += launch_beam_finalize(beam_buffers(c), c->op_B, c->op_K, c->op_T, 102, 1, nullptr, 1, 1, len_penalty(1.f, 0), out_ids, out_scores,
+                                        (cudaStream_t)stream);
     c->op_B = 0;
   });
 }
@@ -1718,8 +1797,9 @@ int gstvd_op_sample(gstvd_ctx* c, int rows, const float* logits, int64_t ldl, co
     if (gp->top_k == 0 && c->V > 32768) throw Unsupported("op_sample: top_k = 0 needs a vocabulary of at most 32768 entries");
     if (!(gp->repetition_penalty > 0.f) || !std::isfinite(gp->repetition_penalty) || gp->no_repeat_ngram_size < 0 || gp->min_length < 0)
       throw InvalidArg("op_sample: repetition_penalty must be finite and > 0, no_repeat_ngram_size and min_length >= 0");
-    LogitsProcs procs = logits_procs(*gp);
     cudaStream_t s = (cudaStream_t)stream;
+    stage_bad_words(c, *gp, s);
+    LogitsProcs procs = logits_procs(c, *gp);
     const int T = c->T_max;
     const bool need_prefix = gp->ngram_blocking_size > 0 || procs.active();
     if (need_prefix && (!prefix || prefix_len != step + 1 || prefix_len > std::min(T + 1, kProcMaxLen)))

@@ -216,6 +216,12 @@ constexpr int kProcMaxLen = 64;   // longest decoder input the logits processors
 // [rows / rows_per_image, P] (null: [CLS], P = 1) followed by the beam token buffer tokens [rows, tok_stride] of this step's parity.
 // t = step, or *d_step when step < 0.  p0s (DecodeGeom::P0s, rows_per_image rows per image): image b's prefix is its first p0s[b] + 1
 // ids (cur_len = p0s[b] + 1 + t); a key row then holds it right-aligned, columns P - 1 - p0s[b] .. P - 1, before the generated tokens.
+//   bad_words_ids (HF NoBadWordsLogitsProcessor, 4.16.2): the ids of one-id sequences are -inf at every step (bw_single: vocab bitmap,
+//   bit w of word w / 32; null when there are none); a sequence w[0..m] of m + 1 >= 2 ids bans w[m] when m <= cur_len and the last m
+//   ids of d are w[0..m-1].  bw_seq holds bw_count entries {offset, m, w[m]} and then the ids, w[0..m-1] of entry j at bw_seq + offset.
+constexpr int kBadWordsMaxSeqs = 1024;   // sequences of one list
+constexpr int kBadWordsMaxLen = 64;      // ids of one sequence
+constexpr int kBadWordsMaxIds = 4096;    // ids of one list
 struct LogitsProcs {
   float repetition_penalty = 1.f;
   int no_repeat_ngram = 0, min_length = 0;
@@ -224,7 +230,11 @@ struct LogitsProcs {
   int P = 1, step = -1;
   const int* d_step = nullptr;
   const int* p0s = nullptr;
-  __host__ __device__ bool active() const { return repetition_penalty != 1.f || no_repeat_ngram > 0 || min_length > 0; }
+  const uint32_t* bw_single = nullptr;
+  const int32_t* bw_seq = nullptr; int bw_count = 0;
+  __host__ __device__ bool active() const {
+    return repetition_penalty != 1.f || no_repeat_ngram > 0 || min_length > 0 || bw_single != nullptr || bw_count > 0;
+  }
 };
 
 // Per row: logZ (fp64 accumulate) and the top `nsel` entries of  score_j by (score desc, index asc), where
@@ -250,6 +260,17 @@ struct BeamBuffers {
   double* hyp_worst;       // [B]
   int* d_step;             // device step counter
 };
+// BeamHypotheses length penalty and early stopping (HF length_penalty / early_stopping, transformers 4.16.2): a hypothesis of length
+// len scores sum_logprobs / denom[len], is_done compares worst_score >= best_sum / denom[cur_len], and early_stopping makes is_done true
+// as soon as the heap holds num_beams hypotheses.  denom[len] = len ** lambda in fp64, computed on the host with the libm pow that
+// Python's float ** float uses (the device pow is not correctly rounded); lambda = 1 gives denom[len] = len exactly.  Passed by value:
+// a captured graph holds it.  len <= kMaxHypLen: a decoder prefix of P ids and T new tokens have P - 1 + T <= 64.
+constexpr int kMaxHypLen = 65;
+struct LenPenalty {
+  double denom[kMaxHypLen + 1];
+  int early_stopping;
+};
+LenPenalty len_penalty(float length_penalty, int early_stopping);
 // prefix: int64 [B, P] decoder prefix (null: start_token, P = 1); len0 = P, the prefix length counted in every hypothesis length.
 // G beam groups of K / G beams (G | K; G = 1: plain beam search): the first beam of every group starts with score 0 (G = K: all beams).
 // B = searches of K beams, N consecutive searches per image (beam sampling; 1 otherwise): search s reads prefix row s / N.
@@ -262,20 +283,21 @@ int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int N, int T, i
 // output with nsel = kSelMax and the beam scores as row bias.  d_seed = {seed, row_offset} (device).  Parents are written image-local
 // (n * K + parent, n = s % N), so the cache reorder runs with N * K rows per image.
 int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, int V, const float* sel_val, const int32_t* sel_idx, int top_k,
-                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, const int* p0s, cudaStream_t stream);
+                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, const int* p0s, const LenPenalty& lp,
+                            cudaStream_t stream);
 // G > 1: diverse beam search with the Hamming penalty `penalty` (oracle/beam_groups.py).  A candidate whose token earlier groups took
 // at this step is re-scored from logits [B*K, ldl] fp32 and logz [B*K] (row_select's outputs for this step); needs nsel >= K + K / G.
 // The re-score applies the repetition penalty rep_penalty after the Hamming term when the token occurs in the beam's decoder input
 // (prefix: int64 [B, len0] decoder prefix, null: [CLS]; then the beam's tokens).  G = 1 reads none of these.
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
                      const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, float rep_penalty,
-                     const int64_t* prefix, int eos, int len0, const int* p0s, int32_t* out_beam_idx, int32_t* out_tokens,
-                     float* out_scores, cudaStream_t stream);
+                     const int64_t* prefix, int eos, int len0, const int* p0s, const LenPenalty& lp, int32_t* out_beam_idx,
+                     int32_t* out_tokens, float* out_scores, cudaStream_t stream);
 // out_ids [B*N, T] / out_scores [B*N]: the N <= K best finished hypotheses of every image, image-major, in the pop order of HF
 // BeamSearchScorer.finalize (score descending, the later-inserted first among equal scores); N = 1 is the single best.
 // Search b belongs to image b / per_image (p0s).
-int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, const int* p0s, int per_image, int N, int64_t* out_ids,
-                         float* out_scores, cudaStream_t stream);
+int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, const int* p0s, int per_image, int N,
+                         const LenPenalty& lp, int64_t* out_ids, float* out_scores, cudaStream_t stream);
 
 // n-gram blocking (utils/decoding_utils.py:38-78): ban list per row from the question history and the decoded prefix.
 // prefix_tokens int32 [rows, P+T] (decoder prefix of len0 = P tokens, then the generated ones; EOS already replaced by PAD),

@@ -35,10 +35,14 @@ __device__ __forceinline__ bool better(float av, int ai, float bv, int bi) { ret
 // shared memory once, marks the positions whose id
 // the n-gram rule bans, and every thread then folds d into two masks over its own slots: `pen` = slots whose id occurs in d (a bit
 // mask, so an id that repeats is penalised once), `ban` = slots set to -inf (n-gram rule; [SEP] while cur_len < min_length).
-// owner(w) = the calling thread's slot of id w, or -1.  Every thread of the CTA must call it (it synchronises).
-template <class Owner>
-__device__ __forceinline__ void procs_masks(const LogitsProcs& pp, int row, int t, int32_t* s_d, uint8_t* s_ban, Owner owner,
-                                            uint32_t& pen, uint32_t& ban) {
+// Bad words: the threads test the multi-id sequences whose banned id lies in [lo, hi) (the CTA's ids) against the tail of d and mark
+// the matches in s_bw (one bit per sequence); every thread then folds the matches and the one-id bitmap into `ban`.
+// owner(w) = the calling thread's slot of id w, or -1; slot_id(s) = the id of the calling thread's slot s, or -1 past the vocabulary.
+// Every thread of the CTA must call it (it synchronises).
+constexpr int kBwWords = kBadWordsMaxSeqs / 32;
+template <class Owner, class SlotId>
+__device__ __forceinline__ void procs_masks(const LogitsProcs& pp, int row, int t, int32_t* s_d, uint8_t* s_ban, uint32_t* s_bw, int lo,
+                                            int hi, Owner owner, SlotId slot_id, uint32_t& pen, uint32_t& ban) {
   const int tid = threadIdx.x;
   const int img = row / pp.rows_per_image;
   const int Pb = pp.p0s ? pp.p0s[img] + 1 : pp.P;
@@ -52,6 +56,7 @@ __device__ __forceinline__ void procs_masks(const LogitsProcs& pp, int row, int 
     } else w = pp.tokens[(int64_t)row * pp.tok_stride + tid - Pb];
     s_d[tid] = w;
   }
+  if (tid < kBwWords) s_bw[tid] = 0u;
   __syncthreads();
   const int n = pp.no_repeat_ngram;
   if (tid < L) {
@@ -60,6 +65,16 @@ __device__ __forceinline__ void procs_masks(const LogitsProcs& pp, int row, int 
     for (int q = 0; q < n - 1 && b; ++q) b = s_d[tid - n + 1 + q] == s_d[L - n + 1 + q];
     s_ban[tid] = b ? 1 : 0;
   }
+  // a sequence of m + 1 ids bans its last id when m <= cur_len and the last m ids of d are its first m (4.16.2 _tokens_match)
+  for (int j = tid; j < pp.bw_count; j += blockDim.x) {
+    const int32_t* e = pp.bw_seq + 3 * j;
+    const int m = e[1], last = e[2];
+    if (last < lo || last >= hi || m > L) continue;
+    const int32_t* w = pp.bw_seq + e[0];
+    bool hit = true;
+    for (int q = 0; q < m && hit; ++q) hit = s_d[L - m + q] == w[q];
+    if (hit) atomicOr(&s_bw[j >> 5], 1u << (j & 31));
+  }
   __syncthreads();
   pen = 0u; ban = 0u;
   for (int j = 0; j < L; ++j) {
@@ -67,6 +82,19 @@ __device__ __forceinline__ void procs_masks(const LogitsProcs& pp, int row, int 
     if (s >= 0) { pen |= 1u << s; if (s_ban[j]) ban |= 1u << s; }
   }
   if (L < pp.min_length) { const int s = owner(102); if (s >= 0) ban |= 1u << s; }
+  for (int i = 0; i * 32 < pp.bw_count; ++i) {
+    for (uint32_t m = s_bw[i]; m != 0u; m &= m - 1u) {
+      const int s = owner(pp.bw_seq[3 * (i * 32 + __ffs(m) - 1) + 2]);
+      if (s >= 0) ban |= 1u << s;
+    }
+  }
+  if (pp.bw_single) {
+#pragma unroll
+    for (int s = 0; s < 32; ++s) {
+      const int w = slot_id(s);
+      if (w >= 0 && ((__ldg(pp.bw_single + (w >> 5)) >> (w & 31)) & 1u)) ban |= 1u << s;
+    }
+  }
 }
 
 template <int NS>
@@ -90,6 +118,7 @@ row_select_kernel(int V, const float* __restrict__ logits, int64_t ldl, int mode
   __shared__ int s_bcast_i;
   __shared__ int32_t s_in[kProcMaxLen];
   __shared__ uint8_t s_ban[kProcMaxLen];
+  __shared__ uint32_t s_bw[kBwWords];
   pdl_wait();
   pdl_launch_dependents();
   const int row = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -136,8 +165,9 @@ row_select_kernel(int V, const float* __restrict__ logits, int64_t ldl, int mode
   }
   if (kProcs) {
     uint32_t pen, ban;
-    procs_masks(procs, row, procs.step >= 0 ? procs.step : *procs.d_step, s_in, s_ban,
-                [&](int w) { return (w >= 0 && w < kSelThreads * kSlots && (w % kSelThreads) == tid) ? w / kSelThreads : -1; }, pen, ban);
+    procs_masks(procs, row, procs.step >= 0 ? procs.step : *procs.d_step, s_in, s_ban, s_bw, 0, V,
+                [&](int w) { return (w >= 0 && w < kSelThreads * kSlots && (w % kSelThreads) == tid) ? w / kSelThreads : -1; },
+                [&](int s) { const int w = tid + s * kSelThreads; return w < V ? w : -1; }, pen, ban);
     procs_apply(v, procs.repetition_penalty, pen, ban);
     if (mode == 0) {
       const float bias = row_bias ? row_bias[row] : 0.f;
@@ -275,6 +305,7 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
   __shared__ int s_alli[kRsChunks * kSelMax];
   __shared__ int32_t s_in[kProcMaxLen];              // the row's decoder input (logits processors)
   __shared__ uint8_t s_ban[kProcMaxLen];
+  __shared__ uint32_t s_bw[kBwWords];                // bad-word sequences that match the row's decoder input
   pdl_wait();
   pdl_launch_dependents();
   const int chunk = (int)cluster.block_rank();
@@ -369,9 +400,9 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
   // logits processors on fp32(x - logZ) (beam modes, before the beam score, as HF beam_search) or fp32(x / temperature) (sampling)
   if (kProcs) {
     uint32_t pen, ban;
-    procs_masks(procs, row, procs.step >= 0 ? procs.step : *procs.d_step, s_in, s_ban,
+    procs_masks(procs, row, procs.step >= 0 ? procs.step : *procs.d_step, s_in, s_ban, s_bw, base, base + kRsSpan,
                 [&](int w) { const int o = w - base; return (o >= 0 && o < kRsSpan && (o % kRsThreads) == tid) ? o / kRsThreads : -1; },
-                pen, ban);
+                [&](int s) { const int w = base + tid + s * kRsThreads; return w < V ? w : -1; }, pen, ban);
     procs_apply(v, procs.repetition_penalty, pen, ban);
     if (mode == 0) {
       const float bias = row_bias ? row_bias[row] : 0.f;
@@ -527,9 +558,10 @@ __global__ void beam_init_kernel(BeamBuffers bb, int B, int K, int gs, int N, in
   for (int j = i; j < 2 * B * K * T; j += gridDim.x * blockDim.x) bb.tokens[j] = 0;
 }
 
-// BeamHypotheses.add (transformers 4.16.2): slots are kept in insertion order, capacity K (+1 transient)
-__device__ void hyp_add(const BeamBuffers& bb, int b, int K, int T, const int32_t* toks, int ntok, float sum_logprobs, int length) {
-  const double score = (double)sum_logprobs / (double)length;
+// BeamHypotheses.add (transformers 4.16.2): slots are kept in insertion order, capacity K (+1 transient).  den = LenPenalty::denom of the
+// hypothesis length.
+__device__ void hyp_add(const BeamBuffers& bb, int b, int K, int T, const int32_t* toks, int ntok, float sum_logprobs, double den) {
+  const double score = (double)sum_logprobs / den;
   const int HK = K + 1;
   double* hs = bb.hyp_score + (int64_t)b * HK;
   int32_t* hl = bb.hyp_len + (int64_t)b * HK;
@@ -561,9 +593,10 @@ __device__ void hyp_add(const BeamBuffers& bb, int b, int K, int T, const int32_
 // BeamSearchScorer.process of one group of gs beams (lane 0): walks the group's 2 gs candidates in rank order (order[rank] = index into
 // val / flat, flat = beam * V + token with the beam counted from the image's / search's first beam): [SEP] at rank < gs closes a
 // hypothesis of beam flat / V (history src + beam * T, t tokens), any other token becomes new beam lo + cnt, until gs beams are filled.
-// Then is_done(val[order[0]], cur_len) on the heap b of capacity K; returns whether it set done[b].
+// Then is_done(val[order[0]], cur_len) on the heap b of capacity K; returns whether it set done[b].  den = LenPenalty::denom[cur_len];
+// early = early_stopping: done as soon as the heap is full.
 __device__ __forceinline__ bool beam_process(const BeamBuffers& bb, int b, int K, int T, int V, int eos, const int32_t* src, int t,
-                                             int cur_len, int lo, int gs, const float* val, const int* flat, const int* order,
+                                             double den, int early, int lo, int gs, const float* val, const int* flat, const int* order,
                                              float* nb_s, int* nb_tok, int* nb_par) {
   int cnt = 0;
   const float best_sum = val[order[0]];
@@ -574,15 +607,15 @@ __device__ __forceinline__ bool beam_process(const BeamBuffers& bb, int b, int K
     const int bk = f / V, bt = f - bk * V;
     if (bt == eos) {
       if (rank >= gs) continue;
-      hyp_add(bb, b, K, T, src + (int64_t)bk * T, t, v, cur_len);
+      hyp_add(bb, b, K, T, src + (int64_t)bk * T, t, v, den);
     } else {
       nb_s[lo + cnt] = v; nb_tok[lo + cnt] = bt; nb_par[lo + cnt] = bk; ++cnt;
     }
     if (cnt == gs) break;
   }
   if (bb.hyp_count[b] >= K) {
-    const double cur = (double)best_sum / (double)cur_len;
-    if (bb.hyp_worst[b] >= cur) { bb.done[b] = 1; return true; }
+    const double cur = (double)best_sum / den;
+    if (early || bb.hyp_worst[b] >= cur) { bb.done[b] = 1; return true; }
   }
   return false;
 }
@@ -598,14 +631,18 @@ __device__ __forceinline__ bool beam_process(const BeamBuffers& bb, int b, int K
 //
 // With a repetition penalty p the re-scored value is fp32(fp32(rep(fp32(fp32(x - logZ) - fp32(lambda c)))) + beam_score), rep = the
 // penalty when w occurs in the beam's decoder input (HF runs the Hamming processor first, then the repetition penalty); the other
-// processors only produce -inf, which stays.
+// processors (n-gram bans, min_length, bad words) only produce -inf, which stays.
 //
 // Why the per-row lists suffice (nsel >= K + gs; the engine keeps nsel = 2K): row_select ranks each row's candidates by the
 // processed (repetition-penalised) score WITHOUT the Hamming term.  The Hamming term only lowers a score, rep (s < 0 ? s p : s / p,
 // p > 0) is monotone in s and fp32(a + b) is monotone in a, so an element outside a row's list is preceded, in the contract's order,
 // by every element of that list that no earlier group took.  The earlier groups took at most K - gs distinct
 // tokens, so at least nsel - (K - gs) >= 2 gs listed elements of the row keep their value, and a group takes at most 2 gs
-// candidates from one row: the group's exact top 2 gs lies inside the lists.
+// candidates from one row: the group's exact top 2 gs lies inside the lists.  The bans (question-history n-grams, no_repeat_ngram_size,
+// min_length, bad_words_ids) only set -inf, before the lists are ranked, and the same element is -inf with or without the Hamming term:
+// they leave the argument as it is.
+//
+// Hypothesis scores and is_done use the LenPenalty denominators (length_penalty, early_stopping).
 constexpr int kBeamWarps = 4;
 // Register budget of the two beam-step kernels: 65536 / (7 * 128 threads) = 72 registers per thread.  Left to its default, ptxas
 // keeps them near 48 - 64 registers and spills the values that stay live across the calls into the fp64 / fp32 division subroutines
@@ -616,7 +653,7 @@ __global__ void __launch_bounds__(kBeamWarps * 32, kBeamMinBlocks)
 beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, const float* __restrict__ sel_val,
                  const int32_t* __restrict__ sel_idx, const float* __restrict__ logits, int64_t ldl, const float* __restrict__ logz,
                  float penalty, float rep_penalty, const int64_t* __restrict__ prefix, int eos, int len0, const int* __restrict__ p0s,
-                 int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
+                 const LenPenalty lp, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
   __shared__ float s_val[kBeamWarps][128];
   __shared__ int s_flat[kBeamWarps][128];
   __shared__ int s_order[kBeamWarps][16];
@@ -680,8 +717,8 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, co
     __syncwarp();
     int fin = 0;
     if (lane == 0)
-      fin = beam_process(bb, b, K, T, V, eos, src, t, cur_len, lo, gs, s_val[warp], s_flat[warp], s_order[warp], nb_s[warp], nb_tok[warp],
-                         nb_par[warp]) ? 1 : 0;
+      fin = beam_process(bb, b, K, T, V, eos, src, t, lp.denom[cur_len], lp.early_stopping, lo, gs, s_val[warp], s_flat[warp], s_order[warp],
+                         nb_s[warp], nb_tok[warp], nb_par[warp]) ? 1 : 0;
     __syncwarp();
     done = __shfl_sync(0xffffffffu, fin, 0) != 0;
   }
@@ -703,7 +740,7 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, co
 // BeamSearchScorer.finalize: a stable ascending sort of the image's hypotheses (kept in insertion order by hyp_add), then N pops.
 // Output n of image b is the hypothesis of rank n by (score desc, insertion index desc); N = 1 is the last of the best scores.
 __global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eos, int len0, const int* __restrict__ p0s, int per_image, int N,
-                                     int64_t* out_ids, float* out_scores) {
+                                     const LenPenalty lp, int64_t* out_ids, float* out_scores) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const int t = *bb.d_step;                     // steps executed
@@ -711,7 +748,8 @@ __global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eo
   if (!bb.done[b]) {
     const int len_b = p0s ? p0s[b / per_image] + 1 : len0;
     const int32_t* cur = bb.tokens + (int64_t)(t & 1) * B * K * T + (int64_t)b * K * T;
-    for (int k = 0; k < K; ++k) hyp_add(bb, b, K, T, cur + (int64_t)k * T, t, bb.beam_scores[b * K + k], t + len_b);
+    const double den = lp.denom[t + len_b];
+    for (int k = 0; k < K; ++k) hyp_add(bb, b, K, T, cur + (int64_t)k * T, t, bb.beam_scores[b * K + k], den);
   }
   const double* hs = bb.hyp_score + (int64_t)b * HK;
   const int cnt = bb.hyp_count[b];
@@ -847,7 +885,7 @@ __device__ __forceinline__ double gumbel_u(uint64_t sd, uint64_t grow, int t, in
 __global__ void __launch_bounds__(kBeamWarps * 32, kBeamMinBlocks)
 beam_sample_step_kernel(BeamBuffers bb, int S, int N, int K, int T, int V, const float* __restrict__ sel_val, const int32_t* __restrict__ sel_idx,
                         int top_k, float temperature, float top_p, const uint64_t* __restrict__ d_seed, int eos, int len0,
-                        const int* __restrict__ p0s) {
+                        const int* __restrict__ p0s, const LenPenalty lp) {
   constexpr int nsel = kSelMax;
   __shared__ double s_key[kBeamWarps][8 * nsel];
   __shared__ float s_val[kBeamWarps][8 * nsel];
@@ -923,7 +961,8 @@ beam_sample_step_kernel(BeamBuffers bb, int S, int N, int K, int T, int V, const
     }
     __syncwarp();
     if (lane == 0)
-      beam_process(bb, s, K, T, V, eos, src, t, cur_len, 0, K, s_val[warp], s_flat[warp], s_order[warp], nb_s[warp], nb_tok[warp], nb_par[warp]);
+      beam_process(bb, s, K, T, V, eos, src, t, lp.denom[cur_len], lp.early_stopping, 0, K, s_val[warp], s_flat[warp], s_order[warp], nb_s[warp],
+                   nb_tok[warp], nb_par[warp]);
   }
   __syncwarp();
   for (int i = lane; i < K * T; i += 32) {
@@ -1046,6 +1085,7 @@ full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t
   __shared__ int s_choice;
   __shared__ int32_t s_in[kProcMaxLen];
   __shared__ uint8_t s_ban[kProcMaxLen];
+  __shared__ uint32_t s_bw[kBwWords];
   pdl_wait();
   pdl_launch_dependents();
   const int row = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
@@ -1057,7 +1097,8 @@ full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t
   for (int j = 0; j < kFvPer; ++j) v[j] = (base + j < V) ? __fdiv_rn(x[base + j], temperature) : -INFINITY;
   if (kProcs) {
     uint32_t pen, ban;
-    procs_masks(procs, row, step, s_in, s_ban, [&](int w) { return (w >= base && w < base + kFvPer) ? w - base : -1; }, pen, ban);
+    procs_masks(procs, row, step, s_in, s_ban, s_bw, 0, V, [&](int w) { return (w >= base && w < base + kFvPer) ? w - base : -1; },
+                [&](int s) { return base + s < V ? base + s : -1; }, pen, ban);
     procs_apply(v, procs.repetition_penalty, pen, ban);
   }
   if (ban_tokens != nullptr) {
@@ -1247,6 +1288,8 @@ void check_procs(const LogitsProcs& p, const char* who) {
     throw std::runtime_error(std::string(who) + ": logits processor parameters out of range");
   if (p.P < 1 || (!p.keys && !p.tokens) || (p.step < 0 && !p.d_step))
     throw std::runtime_error(std::string(who) + ": the logits processors need the rows' decoder input and step");
+  if (p.bw_count < 0 || p.bw_count > kBadWordsMaxSeqs || (p.bw_count > 0 && !p.bw_seq))
+    throw std::runtime_error(std::string(who) + ": bad-word sequences out of range");
 }
 
 }  // namespace
@@ -1277,34 +1320,46 @@ int launch_beam_init(const BeamBuffers& bb, int B, int K, int G, int N, int T, i
   beam_init_kernel<<<(n + 255) / 256, 256, 0, stream>>>(bb, B, K, K / G, N, T, start_token, prefix, P, p0s);
   return 1;
 }
+LenPenalty len_penalty(float length_penalty, int early_stopping) {
+  LenPenalty lp;
+  for (int len = 0; len <= kMaxHypLen; ++len)
+    lp.denom[len] = length_penalty == 1.f ? (double)len : std::pow((double)len, (double)length_penalty);
+  lp.early_stopping = early_stopping ? 1 : 0;
+  return lp;
+}
+
 int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, int V, const float* sel_val, const int32_t* sel_idx, int top_k,
-                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, const int* p0s, cudaStream_t stream) {
+                            float temperature, float top_p, const uint64_t* d_seed, int eos, int len0, const int* p0s, const LenPenalty& lp,
+                            cudaStream_t stream) {
   if (K < 2 || 2 * K > kSelMax || T > kHypMaxT) throw std::runtime_error("beam_sample_step: 2 <= K <= 8 and T <= 32");
+  if (len0 - 1 + T > kMaxHypLen - 1) throw std::runtime_error("beam_sample_step: prefix + new tokens exceed the length table");
   if (N < 1 || S % N != 0) throw std::runtime_error("beam_sample_step: the searches must be a multiple of N >= 1");
   if (top_k < 1 || top_k > kSelMax) throw std::runtime_error("beam_sample_step: top_k out of range");
   launch_k(beam_sample_step_kernel, dim3((S + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, S, N, K, T, V, sel_val,
-           sel_idx, top_k, temperature, top_p, d_seed, eos, len0, p0s);
+           sel_idx, top_k, temperature, top_p, d_seed, eos, len0, p0s, lp);
   return 1;
 }
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
                      const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, float rep_penalty,
-                     const int64_t* prefix, int eos, int len0, const int* p0s, int32_t* out_beam_idx, int32_t* out_tokens,
-                     float* out_scores, cudaStream_t stream) {
+                     const int64_t* prefix, int eos, int len0, const int* p0s, const LenPenalty& lp, int32_t* out_beam_idx,
+                     int32_t* out_tokens, float* out_scores, cudaStream_t stream) {
   if (K > 8 || T > kHypMaxT) throw std::runtime_error("beam_step: K <= 8 and T <= 32");
+  if (len0 - 1 + T > kMaxHypLen - 1) throw std::runtime_error("beam_step: prefix + new tokens exceed the length table");
   if (G < 1 || K % G != 0) throw std::runtime_error("beam_step: the beam groups must divide the beams");
   if (G > 1 && (!logits || !logz || nsel < K + K / G))
     throw std::runtime_error("beam_step: beam groups need the logits, logZ and nsel >= K + K / G per-row candidates");
   if (!(rep_penalty > 0.f) || !std::isfinite(rep_penalty) || (len0 > 1 && !prefix))
     throw std::runtime_error("beam_step: repetition penalty must be finite and > 0, prefix given when len0 > 1");
   launch_k(beam_step_kernel, dim3((B + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, B, K, G, T, V, nsel, sel_val, sel_idx,
-           logits, ldl, logz, penalty, rep_penalty, prefix, eos, len0, p0s, out_beam_idx, out_tokens, out_scores);
+           logits, ldl, logz, penalty, rep_penalty, prefix, eos, len0, p0s, lp, out_beam_idx, out_tokens, out_scores);
   return 1;
 }
-int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, const int* p0s, int per_image, int N, int64_t* out_ids,
-                         float* out_scores, cudaStream_t stream) {
+int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, const int* p0s, int per_image, int N,
+                         const LenPenalty& lp, int64_t* out_ids, float* out_scores, cudaStream_t stream) {
   if (N < 1 || N > K) throw std::runtime_error("beam_finalize: 1 <= N <= K");
+  if (len0 + T > kMaxHypLen) throw std::runtime_error("beam_finalize: prefix + new tokens exceed the length table");
   if (per_image < 1 || B % per_image != 0) throw std::runtime_error("beam_finalize: the searches must be a multiple of per_image >= 1");
-  beam_finalize_kernel<<<(B + 31) / 32, 32, 0, stream>>>(bb, B, K, T, eos, len0, p0s, per_image, N, out_ids, out_scores);
+  beam_finalize_kernel<<<(B + 31) / 32, 32, 0, stream>>>(bb, B, K, T, eos, len0, p0s, per_image, N, lp, out_ids, out_scores);
   return 1;
 }
 int launch_ngram_ban(int rows, int N, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,

@@ -29,6 +29,18 @@ def _ptr(t: Optional[torch.Tensor]):
     return None if t is None else ctypes.c_void_p(t.data_ptr())
 
 
+def bad_words_array(bad_words_ids):
+    """HF-style ``bad_words_ids`` (a list of id lists) as the int32 array gstvd_gen_params.bad_words_ids points to: the sequences
+    concatenated, each closed by -1.  None or [] gives None."""
+    if not bad_words_ids:
+        return None
+    flat = []
+    for seq in bad_words_ids:
+        flat.extend(int(w) for w in seq)
+        flat.append(-1)
+    return (ctypes.c_int32 * len(flat))(*flat)
+
+
 _KERNEL_NAMES = {v: k for k, v in _lib.GEMM_KERNELS.items()}
 _STORE_NAMES = {v: k for k, v in _lib.GEMM_STORES.items()}
 
@@ -197,8 +209,9 @@ class Engine:
 
     def _gen_params(self, num_beams=1, temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0, max_new_tokens=None,
                     row_offset=0, num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0, do_sample=False,
-                    repetition_penalty=1.0, no_repeat_ngram_size=0, min_length=0):
-        """The gstvd_gen_params of one decode request (include/gstvd.h gstvd_generate)."""
+                    repetition_penalty=1.0, no_repeat_ngram_size=0, min_length=0, length_penalty=1.0, early_stopping=False, bad_words_ids=None):
+        """The gstvd_gen_params of one decode request (include/gstvd.h gstvd_generate).  The bad-word array stays referenced by the
+        returned struct (attribute ``_bad_words``) for as long as the struct lives."""
         gp = GstvdGenParams()
         gp.mode = _select_mode(num_beams, do_sample)
         gp.num_beams = int(num_beams)
@@ -209,12 +222,16 @@ class Engine:
         gp.num_return_sequences, gp.num_beam_groups = int(num_return_sequences), int(num_beam_groups)
         gp.diversity_penalty = float(diversity_penalty)
         gp.repetition_penalty, gp.no_repeat_ngram_size, gp.min_length = float(repetition_penalty), int(no_repeat_ngram_size), int(min_length)
+        gp.length_penalty, gp.early_stopping = float(length_penalty), int(early_stopping)
+        gp._bad_words = bad_words_array(bad_words_ids)
+        gp.bad_words_ids = ctypes.addressof(gp._bad_words) if gp._bad_words is not None else 0
+        gp.bad_words_len = len(gp._bad_words) if gp._bad_words is not None else 0
         return gp
 
     def generate(self, B, num_beams=1, temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0,
                  max_new_tokens=None, hist_ids=None, hist_segments=None, want_scores=False, row_offset=0, prefix=None,
                  num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0, do_sample=False, repetition_penalty=1.0,
-                 no_repeat_ngram_size=0, min_length=0):
+                 no_repeat_ngram_size=0, min_length=0, length_penalty=1.0, early_stopping=False, bad_words_ids=None):
         """``row_offset``: global index of row 0; the sampler is keyed by (seed, row_offset + row, step), so an image draws the
         same tokens whichever batch or rank it lands in.  ``prefix``: int64 [B, P] decoder input to continue from (the reference's
         dec_input_ids), None = one [CLS] per row; the result holds the new tokens only.
@@ -227,11 +244,13 @@ class Engine:
         returns the best hypothesis of each (GSTVD_SELECT_BEAM_SAMPLE, contract in oracle/beam_sample.py).  With ``num_beams`` = 1
         the sampler runs whatever ``do_sample`` says.
         ``repetition_penalty`` (1 = off) / ``no_repeat_ngram_size`` (0 = off) / ``min_length`` (0 = off): HF's logits processors on each
-        row's own decoder input, prefix included (contract in oracle/processors.py).  The whole contract is at gstvd_generate in
-        include/gstvd.h."""
+        row's own decoder input, prefix included (contract in oracle/processors.py).
+        ``length_penalty`` (1 = HF default) / ``early_stopping``: the beam modes' hypothesis scores sum / len ** length_penalty and
+        is_done (contract in oracle/decode_args.py).  ``bad_words_ids``: HF-style list of id lists that the output never completes, in
+        every mode.  The whole contract is at gstvd_generate in include/gstvd.h."""
         gp = self._gen_params(num_beams, temperature, top_k, top_p, ngram_blocking_size, seed, max_new_tokens, row_offset,
                               num_return_sequences, num_beam_groups, diversity_penalty, do_sample, repetition_penalty,
-                              no_repeat_ngram_size, min_length)
+                              no_repeat_ngram_size, min_length, length_penalty, early_stopping, bad_words_ids)
         hid = self._dev(hist_ids, torch.int64) if ngram_blocking_size > 0 else None
         hseg = self._dev(hist_segments, torch.int64) if ngram_blocking_size > 0 else None
         Lh = hid.shape[1] if hid is not None else 0
@@ -246,11 +265,11 @@ class Engine:
     def round(self, input_ids, image_feat, image_loc, token_type_ids=None, attention_mask=None, image_mask=None, num_beams=1,
               temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0, max_new_tokens=None, want_scores=False, row_offset=0,
               prefix=None, num_return_sequences=1, num_beam_groups=1, diversity_penalty=0.0, do_sample=False, repetition_penalty=1.0,
-              no_repeat_ngram_size=0, min_length=0):
+              no_repeat_ngram_size=0, min_length=0, length_penalty=1.0, early_stopping=False, bad_words_ids=None):
         """encode + prefill_cross + generate of one forward call as ONE graph replay (gstvd_round); the n-gram blocking history is
         ``input_ids`` / ``token_type_ids``.  Leaves the encoder / cross-K/V state resident like the three separate calls.
         ``prefix`` / ``num_return_sequences`` / ``num_beam_groups`` / ``diversity_penalty`` / ``do_sample`` / ``repetition_penalty`` /
-        ``no_repeat_ngram_size`` / ``min_length``: as in ``generate``."""
+        ``no_repeat_ngram_size`` / ``min_length`` / ``length_penalty`` / ``early_stopping`` / ``bad_words_ids``: as in ``generate``."""
         ids = self._dev(input_ids, torch.int64)
         B, Lt = ids.shape
         feat = self._dev(image_feat, torch.float32)
@@ -261,7 +280,7 @@ class Engine:
         imask = self._dev(image_mask, torch.float32)
         gp = self._gen_params(num_beams, temperature, top_k, top_p, ngram_blocking_size, seed, max_new_tokens, row_offset,
                               num_return_sequences, num_beam_groups, diversity_penalty, do_sample, repetition_penalty,
-                              no_repeat_ngram_size, min_length)
+                              no_repeat_ngram_size, min_length, length_penalty, early_stopping, bad_words_ids)
         pre, P = self._prefix(prefix, B)
         N = gp.num_return_sequences
         out = torch.empty(B * max(N, 1), gp.max_new_tokens, device=self.device, dtype=torch.int64)
@@ -469,13 +488,14 @@ class Engine:
         return out, sc
 
     def op_sample(self, logits, step, temperature=1.0, top_k=1, top_p=0.0, ngram_blocking_size=0, seed=0, hist_ids=None,
-                  hist_segments=None, prefix=None, row_offset=0, repetition_penalty=1.0, no_repeat_ngram_size=0, min_length=0):
+                  hist_segments=None, prefix=None, row_offset=0, repetition_penalty=1.0, no_repeat_ngram_size=0, min_length=0,
+                  bad_words_ids=None):
         """One sampling step on caller logits; ``prefix`` [rows, step + 1] is each row's decoder input so far, which n-gram blocking and
-        the logits processors read."""
+        the logits processors (``bad_words_ids`` included) read."""
         lg = self._dev(logits, torch.float32)
         gp = self._gen_params(temperature=temperature, top_k=top_k, top_p=top_p, ngram_blocking_size=ngram_blocking_size, seed=seed,
                               row_offset=row_offset, repetition_penalty=repetition_penalty, no_repeat_ngram_size=no_repeat_ngram_size,
-                              min_length=min_length)
+                              min_length=min_length, bad_words_ids=bad_words_ids)
         hid, hseg, pre = self._dev(hist_ids, torch.int64), self._dev(hist_segments, torch.int64), self._dev(prefix, torch.int64)
         rows = lg.shape[0]
         out = torch.empty(rows, device=self.device, dtype=torch.int32)

@@ -60,6 +60,9 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
       repetition_penalty=1.0, no_repeat_ngram_size=0, min_length=0   HF's logits processors (HF names; 1 / 0 / 0 = off) on each row's
                          own decoder input, dec_input_ids included; min_length counts the decoder input, not new tokens (contract:
                          oracle/processors.py and gstvd_generate in include/gstvd.h)
+      length_penalty=1.0, early_stopping=False   HF's beam hypothesis scoring (HF names and defaults): score = sum / len ** length_penalty,
+                         is_done as soon as num_beams hypotheses are finished with early_stopping; beam modes only (oracle/decode_args.py)
+      bad_words_ids=None   HF-style list of id lists the output never completes, every mode (oracle/decode_args.py)
       seed=None          sampling seed (a per-call counter when None)
       enc_valid_len=None   upper bound (python int) on the number of leading history positions that hold a token in ANY row.
                          The encoder, the cross-K/V prefill and the cross-attention then run on ceil32(bound) text positions
@@ -183,6 +186,12 @@ class EncoderDecoderModel(_EngineOwner, nn.Module):
                      no_repeat_ngram_size=int(decoding_kwargs.get("no_repeat_ngram_size", 0)), min_length=int(decoding_kwargs.get("min_length", 0)))
         if procs != dict(repetition_penalty=1.0, no_repeat_ngram_size=0, min_length=0):
             gen_kw.update(procs)
+        beam_args = dict(length_penalty=float(decoding_kwargs.get("length_penalty", 1.0)),
+                         early_stopping=bool(decoding_kwargs.get("early_stopping", False)))
+        if beam_args != dict(length_penalty=1.0, early_stopping=False):
+            gen_kw.update(beam_args)
+        if decoding_kwargs.get("bad_words_ids"):
+            gen_kw["bad_words_ids"] = decoding_kwargs["bad_words_ids"]
         if decoding_kwargs.get("do_sample", False):
             if groups > 1:
                 raise ValueError(f"num_beam_groups = {groups} cannot be combined with do_sample (beam sampling)")

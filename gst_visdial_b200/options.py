@@ -3,9 +3,29 @@ generation / scoring path reads, with the same names and defaults, plus a few ad
 from __future__ import annotations
 
 import argparse
+import json
+import math
 import os
 
 from . import weights as W
+
+
+def _bad_words(p, flag, path):
+    """The id lists of a -bad_words_ids FILE (None without a file), within the engine's limits (include/gstvd.h gstvd_generate)."""
+    if not path:
+        return None
+    try:
+        with open(path) as f:
+            words = json.load(f)
+    except (OSError, ValueError) as e:
+        p.error(f"{flag} {path}: {e}")
+    if not isinstance(words, list) or not all(isinstance(s, list) and 1 <= len(s) <= 64 for s in words) or not words:
+        p.error(f"{flag} {path}: expected a non-empty JSON list of lists of 1..64 token ids")
+    if not all(isinstance(w, int) and not isinstance(w, bool) and w >= 0 for s in words for w in s):
+        p.error(f"{flag} {path}: token ids must be non-negative integers")
+    if len(words) > 1024 or sum(map(len, words)) > 4096:
+        p.error(f"{flag} {path}: at most 1024 sequences and 4096 ids")
+    return words
 
 
 def read_command_line(argv=None):
@@ -57,6 +77,13 @@ def read_command_line(argv=None):
                        help=f'HF no_repeat_ngram_size for the {what}: no n-gram occurs twice in the decoder input; 0 = off')
         p.add_argument(f'-{who}min_length', default=0, type=int,
                        help=f'HF min_length for the {what}: [SEP] is banned while the decoder input ([CLS] included) is shorter; 0 = off')
+        p.add_argument(f'-{who}length_penalty', default=1.0, type=float,
+                       help=f'HF length_penalty for the {what} (beam modes): a hypothesis scores sum log-prob / length ** this; '
+                            '> 1 favours longer outputs')
+        p.add_argument(f'-{who}early_stopping', action='store_true',
+                       help=f'HF early_stopping for the {what} (beam modes): an image is done as soon as it has num_beams finished hypotheses')
+        p.add_argument(f'-{who}bad_words_ids', default='', metavar='FILE',
+                       help=f'HF bad_words_ids for the {what}: JSON file holding a list of token-id lists the output never completes')
     p.add_argument('-answer_candidates', default=1, type=int,
                    help='>1: the teacher draws this many answers per round (samples, or the best of its -num_beams beams) and the one with '
                         'the lowest perplexity goes into the dialog')
@@ -82,6 +109,9 @@ def read_command_line(argv=None):
         for name in ('no_repeat_ngram_size', 'min_length'):
             if params[who + name] < 0:
                 p.error(f"-{who}{name} must be >= 0 (0 = off)")
+        if not math.isfinite(params[f'{who}length_penalty']):
+            p.error(f"-{who}length_penalty must be finite")
+        params[f'{who}bad_words_ids'] = _bad_words(p, f'-{who}bad_words_ids', params[f'{who}bad_words_ids'])
     for flag, beams, groups in (('beam_sample', 'num_beams', 'num_beam_groups'), ('q_beam_sample', 'q_num_beams', 'q_num_beam_groups')):
         if params[flag] and (params[beams] <= 1 or params[groups] > 1):
             p.error(f"-{flag} needs -{beams} > 1 and no beam groups")

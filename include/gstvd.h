@@ -12,7 +12,9 @@
  *     gstvd_last_error(ctx) (ctx may be NULL for errors raised before a context exists);
  *   - the caller owns every tensor it passes: raw DEVICE pointers (row-major, contiguous, fp32 / int64 as
  *     stated), explicit sizes, and the cudaStream_t (as void*) the work must be enqueued on.  Only
- *     gstvd_load_weight accepts host or device memory;
+ *     gstvd_load_weight accepts host or device memory, and gstvd_gen_params.bad_words_ids is HOST memory: the list is small, usually
+ *     the same for a whole run, and is validated on the host (the context keeps its own device copy and uploads it again only when
+ *     its content changes);
  *   - the library owns its context: packed weights, workspace, KV caches, CUDA graphs;
  *   - one context per (process, device); calls on one context must be serialised by the caller, different
  *     contexts are independent (one per DataParallel replica / per rank);
@@ -27,7 +29,7 @@
 extern "C" {
 #endif
 
-#define GSTVD_ABI_VERSION 6
+#define GSTVD_ABI_VERSION 7
 #define GSTVD_MAX_CONNECTIONS 16
 
 typedef enum {
@@ -100,6 +102,10 @@ typedef struct {
   float repetition_penalty;   /* HF repetition_penalty, finite and > 0; 1 = off.  Logits processors: contract at gstvd_generate */
   int32_t no_repeat_ngram_size; /* HF no_repeat_ngram_size (n-grams of the output itself), >= 0; 0 = off */
   int32_t min_length;         /* HF min_length: [SEP] banned while the decoder input (prefix included) is shorter, >= 0; 0 = off */
+  float length_penalty;       /* HF length_penalty, beam modes: hypothesis score sum_logprobs / len ** length_penalty; finite; 1 = HF default */
+  int32_t early_stopping;     /* HF early_stopping, beam modes: 0 or 1 */
+  uint64_t bad_words_ids;     /* HF bad_words_ids: address of HOST int32 memory, may be 0: the sequences concatenated, each closed by -1 */
+  int32_t bad_words_len;      /* int32 values at bad_words_ids, terminators included (0 = no list) */
 } gstvd_gen_params;
 
 #define GSTVD_MAX_TOP_K 16
@@ -169,7 +175,8 @@ int gstvd_prefill_cross(gstvd_ctx* ctx, int B, int Le, const float* enc_hidden, 
  *   hist_ids, hist_segments : int64 [B, Lh] encoder input ids / segments (only read when ngram_blocking_size > 0, in sample and
  *                             beam mode; the question history is ids * (segments == 0), visual_dialog_model.py:98-99)
  *   out_ids    : int64 [B*N, max_new_tokens], image-major (row b*N + n): the new tokens only, PAD(0) after the first [SEP]
- *   out_scores : fp32 [B*N] (may be NULL; beam modes only) - hypothesis score (sum log-prob / length)
+ *   out_scores : fp32 [B*N] (may be NULL; beam modes only) - hypothesis score (sum log-prob / length ** length_penalty, HF
+ *                sequences_scores)
  *
  * Return sequences (HF num_return_sequences):
  *   beam mode, 1 <= N <= num_beams: the N best finished hypotheses of BeamSearchScorer.finalize (transformers 4.16.2) in its pop order -
@@ -197,8 +204,8 @@ int gstvd_prefill_cross(gstvd_ctx* ctx, int B, int Le, const float* enc_hidden, 
  *   Rejected with GSTVD_ERR_INVALID: num_beam_groups < 1, num_beams % num_beam_groups != 0, num_beam_groups > 1 outside beam mode,
  *   diversity_penalty negative or not finite.
  *
- * Beam sampling, mode GSTVD_SELECT_BEAM_SAMPLE (transformers 4.16.2 beam_sample + BeamSearchScorer, length_penalty 1, early_stopping
- * off; CPU oracle: oracle/beam_sample.py).  Per image the call runs N independent stochastic beam searches of K = num_beams beams and
+ * Beam sampling, mode GSTVD_SELECT_BEAM_SAMPLE (transformers 4.16.2 beam_sample + BeamSearchScorer with length_penalty and
+ * early_stopping as below; CPU oracle: oracle/beam_sample.py).  Per image the call runs N independent stochastic beam searches of K = num_beams beams and
  * returns the best hypothesis of search n as output row b*N + n (out_scores: its score).  Search n of image b is what an N = 1 call
  * with seed candidate_seed(seed, n) runs for that image.  Decode rows are search-major, row (b*N + n)*K + k; the N*K <= max_beams rows
  * of an image share its cross K/V, decoder prefix and n-gram history.  Per search and step t (P = prefix length):
@@ -213,13 +220,13 @@ int gstvd_prefill_cross(gstvd_ctx* ctx, int B, int Le, const float* enc_hidden, 
  *      h = splitmix64(splitmix64(sd ^ splitmix64(((row_offset + b) << 20) ^ t)) ^ (k*V + w)), sd = candidate_seed(seed, n);
  *      the draws of an image do not depend on how images are split across calls (row_offset);
  *   5. the drawn entries, ordered by (w desc, k*V + w asc), go through BeamSearchScorer.process as in beam search: [SEP] closes a
- *      hypothesis only at rank < K, a hypothesis scores its warped sum / (P + t), is_done uses the best drawn w.
+ *      hypothesis only at rank < K, a hypothesis scores its warped sum / (P + t) ** length_penalty, is_done uses the best drawn w.
  *   Rejected with GSTVD_ERR_INVALID: num_beams < 2 or > 8, N < 1, N*num_beams > max_beams, num_beam_groups > 1, a temperature that is
  *   not finite and > 0, top_p outside [0, 1].  Rejected with GSTVD_ERR_UNSUPPORTED: top_k = 0 or top_k > 16.
  *
- * Logits processors, every mode (HF RepetitionPenaltyLogitsProcessor, NoRepeatNGramLogitsProcessor, MinLengthLogitsProcessor;
- * CPU oracle: oracle/processors.py).  d = a row's decoder input (HF input_ids) at step t: the image's decoder prefix with [SEP] read
- * as [PAD] ([CLS] when prefix is NULL), then the row's own t generated tokens (a beam row: the tokens of that beam; a sample row's
+ * Logits processors, every mode (HF RepetitionPenaltyLogitsProcessor, NoRepeatNGramLogitsProcessor, MinLengthLogitsProcessor,
+ * NoBadWordsLogitsProcessor; CPU oracles: oracle/processors.py, bad words in oracle/decode_args.py).  d = a row's decoder input (HF
+ * input_ids) at step t: the image's decoder prefix with [SEP] read as [PAD] ([CLS] when prefix is NULL), then the row's own t generated tokens (a beam row: the tokens of that beam; a sample row's
  * generated [SEP] is read as [PAD] too) - the key the question-history blocking uses.  cur_len = P + t.  The processors act on each
  * row's score s at the point where the question-history bans act; -inf stays -inf:
  *   1. repetition_penalty p (1 = off): each distinct id of d gets s < 0 ? fp32(s * p) : fp32(s / p), once however often it occurs
@@ -239,9 +246,28 @@ int gstvd_prefill_cross(gstvd_ctx* ctx, int B, int Le, const float* enc_hidden, 
  *     scores fp32(fp32(fp32(fp32(x - logZ) - fp32(lambda * c_w)) * p) + beam_score) (s / p for s >= 0).  The per-row candidate lists
  *     are ranked by the processed score without the Hamming term; the Hamming term only lowers a score and the penalty is monotone,
  *     so the lists still hold each group's exact top 2*gs (argument at beam_step_kernel, csrc/select.cu).
- *   With p = 1, n = 0 and m = 0 a call launches the same kernels and gives the same results, bit for bit, as without the processors.
+ *   4. bad_words_ids (HF NoBadWordsLogitsProcessor, transformers 4.16.2): for every listed sequence w[0..L-1], w[L-1] gets -inf when
+ *      L = 1, or when L > 1, L - 1 <= cur_len and the last L - 1 ids of d are w[0..L-2] (4.16.2 _tokens_match; the prefix of a sequence
+ *      may reach into the decoder prefix and may cover the whole of d).  A sequence that is [SEP] alone is dropped, as HF drops
+ *      [eos_token_id]; min_length is the way to hold back [SEP].  Like 2 and 3 it only writes -inf, so the argument for the beam-group
+ *      candidate lists holds with it.
+ *   With p = 1, n = 0, m = 0 and no bad words a call launches the same kernels and gives the same results, bit for bit, as without the
+ *   processors.
  *   Rejected with GSTVD_ERR_INVALID: repetition_penalty not finite or <= 0, no_repeat_ngram_size < 0, min_length < 0 (so a
- *   zero-filled params struct is rejected: fill every field). */
+ *   zero-filled params struct is rejected: fill every field); bad_words_len < 0, bad_words_len > 0 with bad_words_ids 0, a list
+ *   that does not end with -1, an empty sequence, a sequence of more than 64 ids, more than 1024 sequences or 4096 ids, an id outside
+ *   [0, vocab_size).
+ *
+ * Length penalty and early stopping, beam modes (beam search, beam groups, N-best, beam sampling; HF length_penalty / early_stopping,
+ * transformers 4.16.2 BeamHypotheses; CPU oracle: oracle/decode_args.py).  lambda = length_penalty as stored (fp32), len = the length
+ * of a hypothesis's decoder input: its image's prefix length P_b plus its generated tokens, without the closing [SEP] (P_b + t for a
+ * hypothesis closed at step t, the cur_len above):
+ *   - a hypothesis scores fp64(sum_logprobs) / len ** fp64(lambda), the power in fp64 with the host's libm pow (what Python's
+ *     float ** float computes); lambda = 1 divides by len exactly as before, lambda = 0 does not normalise;
+ *   - is_done at step t: the heap holds num_beams hypotheses and (early_stopping, or worst_score >= best_sum / (P_b + t) ** lambda);
+ *   - finalisation scores the unfinished beams the same way; out_scores reports the penalised score.
+ *   early_stopping changes which hypotheses are kept, not how many steps a call runs.  Sampling ignores both.  Rejected with
+ *   GSTVD_ERR_INVALID (every mode): a length_penalty that is not finite, an early_stopping other than 0 or 1. */
 int gstvd_generate(gstvd_ctx* ctx, int B, const gstvd_gen_params* params, const int64_t* prefix, int P,
                    const int64_t* hist_ids, const int64_t* hist_segments, int Lh,
                    int64_t* out_ids, float* out_scores, void* stream);
@@ -354,8 +380,8 @@ int gstvd_op_beam_step(gstvd_ctx* ctx, const float* logits, int64_t ldl, int32_t
                        float* next_scores, void* stream);
 int gstvd_op_beam_end(gstvd_ctx* ctx, int64_t* out_ids, float* out_scores, void* stream);
 /* top-k filter + greedy/multinomial on caller-supplied logits fp32 [rows, V]; prefix int64 [rows, prefix_len] holds
- * the decoded tokens so far (for n-gram blocking, may be NULL); out_tokens int32 [rows].  The logits processors of params act
- * with d = prefix ([SEP] read as [PAD]) and need prefix_len = step + 1 <= 64 */
+ * the decoded tokens so far (for n-gram blocking, may be NULL); out_tokens int32 [rows].  The logits processors of params, bad_words_ids
+ * included, act with d = prefix ([SEP] read as [PAD]) and need prefix_len = step + 1 <= 64 */
 int gstvd_op_sample(gstvd_ctx* ctx, int rows, const float* logits, int64_t ldl, const gstvd_gen_params* params,
                     const int64_t* hist_ids, const int64_t* hist_segments, int Lh, const int64_t* prefix, int prefix_len,
                     int step, int32_t* out_tokens, void* stream);
