@@ -122,7 +122,7 @@ struct gstvd_ctx {
   DevBuf cross_len;                                   // int32 [B]: keys up to the last unmasked one (launch_cross_len)
   DevBuf labels;                                      // int64 [B*Ldec]
   DevBuf sel_val, sel_idx, logz;                      // [rows, kSelMax]
-  DevBuf ban_tokens, ban_count, prefix, seq;          // sample-mode state, one row per decode row (B*K: sampled candidates)
+  DevBuf ban_tokens, ban_count, seq;                  // sample-mode state, one row per decode row (B*K: sampled candidates)
   DevBuf beam_scores, beam_tokens, cur_tokens, beam_idx, beam_done, hyp_score, hyp_len, hyp_tokens, hyp_count, hyp_worst;
   DevBuf d_step, d_seed;
   DevBuf anc;                                         // uint8 [B*K][64]: beam ancestry table (launch_anc_update; rows of 32 up to 32 positions)
@@ -354,7 +354,7 @@ void alloc_workspace(gstvd_ctx* c) {
     c->r_feat.alloc(B * Lv * (size_t)c->cfg.v_feature_size * 4); c->r_loc.alloc(B * Lv * 5 * 4); c->r_imask.alloc(B * Lv * 4);
     // outputs and sample-mode state hold up to K_max rows per image: N-best beams / N sampled candidates
     c->r_out_ids.alloc(B * K * T * 8); c->r_out_scores.alloc(B * K * 4);
-    c->prefix.alloc(B * K * (T + c->Ldec_max) * 4); c->seq.alloc(B * K * T * 4);
+    c->seq.alloc(B * K * T * 4);
     c->dec_prefix_own.alloc(B * c->Ldec_max * 8); c->dec_prefix_head.alloc(B * c->Ldec_max * 8); c->prefix_p0.alloc(B * 4);
     c->beam_scores.alloc(B * K * 4); c->beam_tokens.alloc(2 * B * K * T * 4); c->cur_tokens.alloc(R * 4);
     // hypothesis heaps: one per search of K beams with K + 1 slots.  Beam search: B searches of K <= K_max beams; beam sampling: B * N
@@ -698,8 +698,8 @@ void decode_init(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   else if (gp.mode == GSTVD_SELECT_BEAM_SAMPLE) {
     const int K = gp.num_beams, N = g.K / K;      // N searches of K beams per image, all beams at score 0
     c->launches += launch_beam_init(beam_buffers(c), g.B * N, K, K, N, T, 101, prefix, P, p0s, s);
-  } else c->launches += launch_sample_init(g.B * g.K, g.K, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, P + T, (int*)c->d_step.p,
-                                         prefix, P, p0s, s);
+  } else c->launches += launch_sample_init(g.B * g.K, g.K, T, 101, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int*)c->d_step.p, prefix, P,
+                                         p0s, s);
 }
 
 // Device form of the bad-word list (LogitsProcs::bw_*): [vocab bitmap of the one-id sequences, (V + 31) / 32 words][bw_count entries
@@ -829,9 +829,24 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
   }
   X.gemm(c->dh.p, H, c->lm_head, c->logits.p, c->Vpad, M, 0, true);
   float* sv = (float*)c->sel_val.p; int32_t* si = (int32_t*)c->sel_idx.p;
-  // the logits processors act inside the selection kernels; each reads its rows' decoder input (cur_len = P + step <= 64)
+  // the logits processors act inside the selection kernels; each reads its rows' decoder input (cur_len = P + step <= 64): the
+  // image's prefix, then the row's tokens (beams: the token buffer of this step's parity; sampling: seq)
   LogitsProcs procs = logits_procs(c, gp);
-  procs.P = P; procs.step = step_host; procs.d_step = d_step; procs.p0s = g.P0s; procs.rows_per_image = g.K;
+  DecInput& d = procs.d;
+  d.prefix = prefix; d.P = P; d.p0s = g.P0s; d.rows_per_image = g.K; d.tok_stride = Tn;
+  d.tokens = beams ? (const int32_t*)c->beam_tokens.p + (int64_t)(step_host & 1) * M * Tn : (const int32_t*)c->seq.p;
+  procs.step = step_host;
+  // n-gram blocking.  Beams: nothing to launch while every key is shorter than n-1 tokens (P + t < n-1) or, for the [CLS] start,
+  // still holds the [CLS], which no banned n-gram contains (t < n-1); a caller's prefix may hold anything: no position is known
+  // special.  With per-image lengths the condition uses the longest, P; the kernel skips the images whose key is still too short.
+  // Sampling launches at every step.
+  const int n = gp.ngram_blocking_size;
+  const int32_t* bt = nullptr; const int32_t* bc = nullptr;
+  if (n > 0 && (!beams || step_host >= (prefix ? n - 1 - P : n - 1))) {
+    c->launches += launch_beam_ngram_ban(g.B, Lh, hist_ids, hist_seg, d, step_host, n, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p,
+                                         Lh, s);
+    bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
+  }
   if (beams) {
     // beam sampling: g.K = N * K rows per image (N searches of K beams), each row's 16 best for the warpers and the draw
     const bool sampled = gp.mode == GSTVD_SELECT_BEAM_SAMPLE;
@@ -839,22 +854,10 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
     // bf16: log-sum-exp terms in fp32 (mode 2); the fp32 parity path keeps the fp64 terms of the bit-exact contract (mode 0)
     static const bool exact_lse = getenv("GSTVD_EXACT_LSE") != nullptr;
     BeamBuffers bb = beam_buffers(c);
-    const int32_t* bt = nullptr; const int32_t* bc = nullptr;
-    // n-gram blocking: nothing to launch while every key is shorter than n-1 tokens (P + t < n-1) or, for the [CLS] start, still
-    // holds the [CLS], which no banned n-gram contains (t < n-1).  A caller's prefix may hold anything: no position is known special.
-    // With per-image lengths the condition uses the longest, P; the kernel skips the images whose key is still too short.
-    const int n = gp.ngram_blocking_size;
-    if (n > 0 && step_host >= (prefix ? n - 1 - P : n - 1)) {
-      c->launches += launch_beam_ngram_ban(g.B, g.K, Tn, Lh, hist_ids, hist_seg, prefix, P, g.P0s, bb.tokens + (int64_t)(step_host & 1) * M * Tn,
-                                           step_host, n, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
-      bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
-    }
     // beam groups: row_select also writes each row's logZ, from which the beam step re-scores the candidates a diversity penalty
     // lowers (the candidate lists stay ranked by the unpenalised score; launch_beam_step explains why nsel = 2K suffices)
     const int G = gp.num_beam_groups;
     float* lz = G > 1 ? (float*)c->logz.p : nullptr;
-    // a beam row's decoder input: the image's prefix, then the beam's tokens in the token buffer of this step's parity
-    procs.prefix = prefix; procs.tokens = bb.tokens + (int64_t)(step_host & 1) * M * Tn; procs.tok_stride = Tn;
     c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, (c->dtype == kBF16 && !exact_lse) ? 2 : 0,
                                      (const float*)c->beam_scores.p, 1.f, bt, bc, Lh, nsel, sv, si, lz, procs, s);
     if (sampled) {
@@ -863,35 +866,24 @@ void decode_step(gstvd_ctx* c, const DecodeGeom& g, const gstvd_gen_params& gp, 
                                              (const uint64_t*)c->d_seed.p, 102, P, g.P0s, len_penalty(gp.length_penalty, gp.early_stopping), s);
     } else {
       c->launches += launch_beam_step(bb, g.B, g.K, G, Tn, c->V, nsel, sv, si, G > 1 ? (const float*)c->logits.p : nullptr, c->Vpad, lz,
-                                      gp.diversity_penalty, gp.repetition_penalty, prefix, 102, P, g.P0s,
-                                      len_penalty(gp.length_penalty, gp.early_stopping), nullptr, nullptr, nullptr, s);
+                                      gp.diversity_penalty, gp.repetition_penalty, d, 102, len_penalty(gp.length_penalty, gp.early_stopping),
+                                      nullptr, nullptr, nullptr, s);
     }
     if (use_anc) c->launches += launch_anc_update(g, bb.beam_idx, d_step, (uint8_t*)c->anc.p, s);
     else c->launches += launch_reorder_cache(c->dtype, g, c->self_cache.p, bb.beam_idx, d_step, 0, nullptr, s);
   } else {
     // g.K rows per image: the num_return_sequences sampled candidates, each with its own n-gram key and RNG stream
     const int nsel = kSelMax;
-    const int32_t* bt = nullptr; const int32_t* bc = nullptr;
-    // key buffer c->prefix [M, P + Tn]: the decoder prefix (right-aligned when it is shorter than P), then the generated tokens; the
-    // samplers append token t at P + t
-    const int kst = P + Tn;
-    int32_t* key_next = (int32_t*)c->prefix.p + (P - 1);
-    if (gp.ngram_blocking_size > 0) {
-      c->launches += launch_ngram_ban(M, g.K, Lh, hist_ids, hist_seg, (const int32_t*)c->prefix.p, kst, d_step, P, gp.ngram_blocking_size,
-                                      (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
-      bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
-    }
-    procs.keys = (const int32_t*)c->prefix.p; procs.key_stride = kst;      // a sample row's decoder input is its n-gram key
     if (gp.top_k == 0) {
       // no top-k cut (utils/decoding_utils.py:17 skips it): multinomial over the whole, optionally nucleus-filtered, vocabulary
       c->launches += launch_full_vocab_sample(M, g.K, c->V, (const float*)c->logits.p, c->Vpad, gp.temperature, gp.top_p, bt, bc, Lh, Tn, 0, 0,
-                                              (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p,
-                                              key_next, kst, nullptr, procs, s);
+                                              (const uint64_t*)c->d_seed.p, d_step, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, nullptr,
+                                              procs, s);
     } else {
       c->launches += launch_row_select(M, c->V, (const float*)c->logits.p, c->Vpad, 1, nullptr, gp.temperature, bt, bc, Lh, nsel, sv, si,
                                        nullptr, procs, s);
-      c->launches += launch_sample_step(M, g.K, Tn, nsel, sv, si, gp.top_k, gp.top_p, 0, 0, (const uint64_t*)c->d_seed.p, d_step, 102, (int32_t*)c->seq.p,
-                                        (int32_t*)c->cur_tokens.p, key_next, kst, nullptr, s);
+      c->launches += launch_sample_step(M, g.K, Tn, nsel, sv, si, gp.top_k, gp.top_p, 0, 0, (const uint64_t*)c->d_seed.p, d_step,
+                                        (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, nullptr, s);
     }
   }
   c->launches += launch_step_advance((int*)c->d_step.p, s);
@@ -1220,7 +1212,7 @@ void gstvd_destroy(gstvd_ctx* c) {
   DevBuf* bufs[] = {&c->mat32, &c->mat16, &c->vec32, &c->xt, &c->yt, &c->xv, &c->yv, &c->qkv_t, &c->qkv_v, &c->ctx_t, &c->ctx_v, &c->tmp_t,
                     &c->tmp_v, &c->ffn_t, &c->ffn_v, &c->feat_cast, &c->fused, &c->pool, &c->fused_mask, &c->dh, &c->da, &c->db, &c->dqkv,
                     &c->dctx, &c->dtmp, &c->dffn, &c->dqc, &c->logits, &c->cross_cache, &c->self_cache, &c->cross_len, &c->labels, &c->sel_val, &c->sel_idx,
-                    &c->logz, &c->ban_tokens, &c->ban_count, &c->prefix, &c->seq, &c->beam_scores, &c->beam_tokens, &c->cur_tokens,
+                    &c->logz, &c->ban_tokens, &c->ban_count, &c->seq, &c->beam_scores, &c->beam_tokens, &c->cur_tokens,
                     &c->beam_idx, &c->beam_done, &c->hyp_score, &c->hyp_len, &c->hyp_tokens, &c->hyp_count, &c->hyp_worst, &c->d_step, &c->d_seed, &c->anc, &c->dec_prefix_own, &c->dec_prefix_head, &c->prefix_p0, &c->fold16, &c->foldvec,
                     &c->st1, &c->st2, &c->st3, &c->hist_ids_own, &c->hist_seg_own, &c->r_ids, &c->r_seg, &c->r_att,
                     &c->r_feat, &c->r_loc, &c->r_imask, &c->r_out_ids, &c->r_out_scores, &c->bw_dev};
@@ -1772,7 +1764,7 @@ int gstvd_op_beam_step(gstvd_ctx* c, const float* logits, int64_t ldl, int32_t* 
     c->launches += launch_row_select(B * K, c->V, logits, ldl, 0, (const float*)c->beam_scores.p, 1.f, nullptr, nullptr, 0, nsel,
                                      (float*)c->sel_val.p, (int32_t*)c->sel_idx.p, nullptr, LogitsProcs(), s);
     c->launches += launch_beam_step(beam_buffers(c), B, K, 1, T, c->V, nsel, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, nullptr,
-                                    0, nullptr, 0.f, 1.f, nullptr, 102, 1, nullptr, len_penalty(1.f, 0), beam_idx, next_tokens, next_scores, s);
+                                    0, nullptr, 0.f, 1.f, DecInput(), 102, len_penalty(1.f, 0), beam_idx, next_tokens, next_scores, s);
     c->launches += launch_step_advance((int*)c->d_step.p, s);
   });
 }
@@ -1809,28 +1801,22 @@ int gstvd_op_sample(gstvd_ctx* c, int rows, const float* logits, int64_t ldl, co
     CUDA_CHECK(cudaMemcpyAsync(c->d_seed.p, &gp->seed, 8, cudaMemcpyHostToDevice, s));
     CUDA_CHECK(cudaStreamSynchronize(s));
     const int32_t* bt = nullptr; const int32_t* bc = nullptr;
-    if (need_prefix) {
-      CUDA_CHECK(cudaMemsetAsync(c->prefix.p, 0, c->prefix.bytes, s));
-      c->launches += launch_build_prefix_from_ids(rows, prefix_len, prefix, (int32_t*)c->prefix.p, T + 1, 102, s);
-    }
+    // the row's decoder input is the caller's prefix ([SEP] read as [PAD]) and no generated tokens; the RNG step comes from d_step
+    procs.d.prefix = prefix; procs.d.P = prefix_len; procs.step = 0;
     if (gp->ngram_blocking_size > 0) {
-      c->launches += launch_ngram_ban(rows, 1, Lh, hist_ids, hist_segments, (const int32_t*)c->prefix.p, T + 1, (const int*)c->d_step.p, 1,
-                                      gp->ngram_blocking_size, (int32_t*)c->ban_tokens.p, (int32_t*)c->ban_count.p, Lh, s);
+      c->launches += launch_beam_ngram_ban(rows, Lh, hist_ids, hist_segments, procs.d, 0, gp->ngram_blocking_size, (int32_t*)c->ban_tokens.p,
+                                           (int32_t*)c->ban_count.p, Lh, s);
       bt = (const int32_t*)c->ban_tokens.p; bc = (const int32_t*)c->ban_count.p;
     }
-    // the row's decoder input is the caller's prefix ([SEP] read as [PAD]); the step comes from the device counter
-    procs.keys = (const int32_t*)c->prefix.p; procs.key_stride = T + 1; procs.P = 1; procs.step = -1; procs.d_step = (const int*)c->d_step.p;
     if (gp->top_k == 0) {
       c->launches += launch_full_vocab_sample(rows, 1, c->V, logits, ldl, gp->temperature, gp->top_p, bt, bc, Lh, T, gp->seed, (uint64_t)gp->row_offset, nullptr,
-                                              (const int*)c->d_step.p, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, T + 1,
-                                              out_tokens, procs, s);
+                                              (const int*)c->d_step.p, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, out_tokens, procs, s);
       return;
     }
     c->launches += launch_row_select(rows, c->V, logits, ldl, 1, nullptr, gp->temperature, bt, bc, Lh, kSelMax, (float*)c->sel_val.p,
                                      (int32_t*)c->sel_idx.p, nullptr, procs, s);
     c->launches += launch_sample_step(rows, 1, T, kSelMax, (const float*)c->sel_val.p, (const int32_t*)c->sel_idx.p, gp->top_k, gp->top_p, gp->seed, (uint64_t)gp->row_offset, nullptr,
-                                      (const int*)c->d_step.p, 102, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, (int32_t*)c->prefix.p, T + 1,
-                                      out_tokens, s);
+                                      (const int*)c->d_step.p, (int32_t*)c->seq.p, (int32_t*)c->cur_tokens.p, out_tokens, s);
   });
 }
 

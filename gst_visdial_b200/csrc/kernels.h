@@ -206,16 +206,33 @@ int launch_reorder_cache(int dtype, const DecodeGeom& g, void* self_cache, const
 constexpr int kSelMax = 16;   // per-row candidates kept (>= 2*max_beams, >= max top_k)
 constexpr int kProcMaxLen = 64;   // longest decoder input the logits processors read (= the cached positions of the decode kernels)
 
+// The decoder input d of a decode row after t generated tokens: its image's decoder prefix ([SEP] read as [PAD]; [CLS] when prefix
+// is null, P = 1), then the row's t generated tokens.  rows_per_image consecutive rows share image row / rows_per_image.
+//   prefix: int64 [images, P]; p0s (DecodeGeom::P0s, may be null): image b's prefix is its first P_b = p0s[b] + 1 ids (null: P_b = P)
+//   tokens: int32 [rows, tok_stride], the row's generated tokens (beams: the token buffer of this step's parity; may be null at t = 0)
+// len(row, t) = P_b + t <= kProcMaxLen ids; at(row, j), j < len: id j of d, with [SEP] read as [PAD] (the generated tokens of a beam
+// never hold [SEP]; those of a sample row hold it where the row ended).
+struct DecInput {
+  const int64_t* prefix = nullptr;
+  int P = 1;
+  const int* p0s = nullptr;
+  int rows_per_image = 1;
+  const int32_t* tokens = nullptr;
+  int tok_stride = 0;
+  __host__ __device__ int len(int row, int t) const { return (p0s ? p0s[row / rows_per_image] + 1 : P) + t; }
+  __host__ __device__ int32_t at(int row, int j) const {
+    const int Pb = len(row, 0);
+    const int32_t w = j >= Pb ? tokens[(int64_t)row * tok_stride + j - Pb]
+                              : prefix ? (int32_t)prefix[(int64_t)(row / rows_per_image) * P + j] : 101;
+    return w == 102 ? 0 : w;
+  }
+};
+
 // HF logits processors on a row's score s (include/gstvd.h gstvd_generate; CPU oracle: oracle/processors.py), applied where the
-// selection kernels apply their ban lists.  d = the row's decoder input of cur_len = P + t ids: the image's decoder prefix ([SEP] read
-// as [PAD]; [CLS] when null), then the row's t generated tokens.
+// selection kernels apply their ban lists, on the row's decoder input d (DecInput) of cur_len = d.len(row, step) ids.
 //   repetition_penalty p (1 = off): every distinct id of d gets s < 0 ? fp32(s * p) : fp32(s / p)
 //   no_repeat_ngram n (0 = off): the id that follows an earlier occurrence of the last n-1 ids of d gets -inf
 //   min_length m (0 = off): [SEP] gets -inf while cur_len < m
-// d is read either from an int32 key buffer (sampling: keys [rows, key_stride], [SEP] already [PAD]) or from the int64 decoder prefix
-// [rows / rows_per_image, P] (null: [CLS], P = 1) followed by the beam token buffer tokens [rows, tok_stride] of this step's parity.
-// t = step, or *d_step when step < 0.  p0s (DecodeGeom::P0s, rows_per_image rows per image): image b's prefix is its first p0s[b] + 1
-// ids (cur_len = p0s[b] + 1 + t); a key row then holds it right-aligned, columns P - 1 - p0s[b] .. P - 1, before the generated tokens.
 //   bad_words_ids (HF NoBadWordsLogitsProcessor, 4.16.2): the ids of one-id sequences are -inf at every step (bw_single: vocab bitmap,
 //   bit w of word w / 32; null when there are none); a sequence w[0..m] of m + 1 >= 2 ids bans w[m] when m <= cur_len and the last m
 //   ids of d are w[0..m-1].  bw_seq holds bw_count entries {offset, m, w[m]} and then the ids, w[0..m-1] of entry j at bw_seq + offset.
@@ -225,11 +242,8 @@ constexpr int kBadWordsMaxIds = 4096;    // ids of one list
 struct LogitsProcs {
   float repetition_penalty = 1.f;
   int no_repeat_ngram = 0, min_length = 0;
-  const int32_t* keys = nullptr; int key_stride = 0;
-  const int64_t* prefix = nullptr; const int32_t* tokens = nullptr; int tok_stride = 0; int rows_per_image = 1;
-  int P = 1, step = -1;
-  const int* d_step = nullptr;
-  const int* p0s = nullptr;
+  DecInput d;
+  int step = -1;
   const uint32_t* bw_single = nullptr;
   const int32_t* bw_seq = nullptr; int bw_count = 0;
   __host__ __device__ bool active() const {
@@ -288,46 +302,39 @@ int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, i
 // G > 1: diverse beam search with the Hamming penalty `penalty` (oracle/beam_groups.py).  A candidate whose token earlier groups took
 // at this step is re-scored from logits [B*K, ldl] fp32 and logz [B*K] (row_select's outputs for this step); needs nsel >= K + K / G.
 // The re-score applies the repetition penalty rep_penalty after the Hamming term when the token occurs in the beam's decoder input
-// (prefix: int64 [B, len0] decoder prefix, null: [CLS]; then the beam's tokens).  G = 1 reads none of these.
+// d (rows_per_image = K; its tokens are bb.tokens of this step's parity).  G = 1 reads none of these.  Hypothesis lengths are
+// d.len(row, t).
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
                      const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, float rep_penalty,
-                     const int64_t* prefix, int eos, int len0, const int* p0s, const LenPenalty& lp, int32_t* out_beam_idx,
-                     int32_t* out_tokens, float* out_scores, cudaStream_t stream);
+                     const DecInput& d, int eos, const LenPenalty& lp, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
+                     cudaStream_t stream);
 // out_ids [B*N, T] / out_scores [B*N]: the N <= K best finished hypotheses of every image, image-major, in the pop order of HF
 // BeamSearchScorer.finalize (score descending, the later-inserted first among equal scores); N = 1 is the single best.
 // Search b belongs to image b / per_image (p0s).
 int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, const int* p0s, int per_image, int N,
                          const LenPenalty& lp, int64_t* out_ids, float* out_scores, cudaStream_t stream);
 
-// n-gram blocking (utils/decoding_utils.py:38-78): ban list per row from the question history and the decoded prefix.
-// prefix_tokens int32 [rows, P+T] (decoder prefix of len0 = P tokens, then the generated ones; EOS already replaced by PAD),
-// prefix_len = *d_step + len0.  N rows per image (sampled candidates): row r reads the history of image r / N
-int launch_ngram_ban(int rows, int N, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
-                     int prefix_stride, const int* d_step, int len0, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
-                     cudaStream_t stream);
-// the same for the B*K beam rows: key = the last n-1 tokens of prefix_b ([SEP] read as [PAD]; null: [CLS], P = 1) followed by beam
-// row b*K+k of `tokens` [B, K, T] (the beam token buffer of this step's parity); history row = b.  Needs n - 1 <= P + step, step < T.
-// p0s: prefix_b is the first p0s[b] + 1 ids of row b (stride P); an image whose decoder input is shorter than n - 1 bans nothing.
-int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int64_t* prefix, int P,
-                          const int* p0s, const int32_t* tokens, int step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
-                          cudaStream_t stream);
-// sample-mode selection from row_select output; writes seq[row, step] and cur_tokens[row], prefix[row, step+1]
+// Question-history n-gram blocking (utils/decoding_utils.py:38-78; beams: oracle/beam_ngram.py), every decode mode: ban list
+// [rows, ban_stride] / ban_count [rows] per row of the B images of d (rows_per_image <= 8 rows each) at step `step`.  A row's key is
+// the last n-1 ids of its decoder input d.len(row, step); image b's question history is row b of hist_ids / hist_seg [B, Lh].  A
+// key longer than the decoder input bans nothing.
+int launch_beam_ngram_ban(int B, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const DecInput& d, int step, int n,
+                          int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream);
+// sample-mode selection from row_select output; writes seq[row, step] and cur_tokens[row]
 // top_k == 0: multinomial over the whole (optionally nucleus-filtered) vocabulary; writes the same state as launch_sample_step
 // N rows per image (sampled candidates): row r draws as row r / N of a single-sample call seeded candidate_seed(seed, r % N)
-// procs: the logits processors, applied after the temperature (their step is *d_step)
+// procs: the logits processors, applied after the temperature
 int launch_full_vocab_sample(int rows, int N, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,
                              const int32_t* ban_count, int ban_stride, int T, uint64_t seed, uint64_t row_offset, const uint64_t* d_seed,
-                             const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens,
-                             const LogitsProcs& procs, cudaStream_t stream);
+                             const int* d_step, int32_t* seq, int32_t* cur_tokens, int32_t* out_tokens, const LogitsProcs& procs,
+                             cudaStream_t stream);
 int launch_sample_step(int rows, int N, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
-                       uint64_t seed, uint64_t row_offset, const uint64_t* d_seed, const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                       int prefix_stride, int32_t* out_tokens, cudaStream_t stream);
-// dec_prefix: int64 [rows / N, P] decoder prefix (null: start_token, P = 1), shared by the N rows of an image; the key buffer
-// `prefix` [rows, prefix_stride >= P + T].  An image's prefix ends at its first negative id; it is written right-aligned into
-// columns P - P_b .. P - 1 of the key rows (zeros before it: [PAD], which no history n-gram holds), so the samplers append token t
-// at column P + t for every row.  p0s (may be null): receives every image's P_b - 1 (DecodeGeom::P0s).
-int launch_sample_init(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                       int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, int* p0s, cudaStream_t stream);
+                       uint64_t seed, uint64_t row_offset, const uint64_t* d_seed, const int* d_step, int32_t* seq, int32_t* cur_tokens,
+                       int32_t* out_tokens, cudaStream_t stream);
+// dec_prefix: int64 [rows / N, P] decoder prefix (null: start_token, P = 1), shared by the N rows of an image.  An image's prefix ends
+// at its first negative id; its last id is the rows' first input.  p0s (may be null): receives every image's P_b - 1 (DecodeGeom::P0s).
+int launch_sample_init(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int* d_step, const int64_t* dec_prefix,
+                       int P, int* p0s, cudaStream_t stream);
 int launch_sample_finalize(int rows, int T, int eos, const int32_t* seq, int64_t* out_ids, cudaStream_t stream);
 int launch_step_advance(int* d_step, cudaStream_t stream);
 // device-side scalar set (a pageable-memory cudaMemcpyAsync would synchronise the stream with the host)
@@ -339,7 +346,5 @@ int launch_ce_loss(int rows, int V, const float* logits, int64_t ldl, const int6
 // history splice (generate.py:145-160, :214-228)
 int launch_splice(int B, int Lt, int Lu, int64_t* ids, int64_t* seg, float* mask, int32_t* enc_len, const int64_t* utt,
                   int segment_value, int strip_sep, int32_t* abnormal, int sep, cudaStream_t stream);
-int launch_build_prefix_from_ids(int rows, int len, const int64_t* prefix_ids, int32_t* prefix, int prefix_stride, int eos,
-                                 cudaStream_t stream);
 
 }  // namespace gstvd

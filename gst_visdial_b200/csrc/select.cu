@@ -5,8 +5,8 @@
 //   row_select     : replaces torch.topk + masked fill (utils/decoding_utils.py:17-21) and, for beams, the
 //                    log_softmax + top-2K of HF beam_search (absent from the reference; contract in oracle/beam.py)
 //   beam_step/...  : BeamSearchScorer.process / finalize + BeamHypotheses (transformers 4.16.2 semantics)
-//   ngram_ban      : batch_ngram_blocking (utils/decoding_utils.py:38-78) without host round trips; beam_ngram_ban: the
-//                    same ban lists for every beam row (contract in oracle/beam_ngram.py)
+//   beam_ngram_ban : batch_ngram_blocking (utils/decoding_utils.py:38-78) without host round trips, for the sample and the beam
+//                    rows (contract in oracle/beam_ngram.py)
 //   sample_step    : softmax + multinomial (models/visual_dialog_model.py:106-107), counter-based RNG
 //   ce_loss        : CrossEntropyLoss(ignore_index=0, reduction='none') (models/visual_dialog_decoder.py:70-77)
 //   splice         : generate.py:145-160 and :214-228
@@ -31,32 +31,27 @@ struct Cand { float v; int i; };
 __device__ __forceinline__ bool better(float av, int ai, float bv, int bi) { return av > bv || (av == bv && ai < bi); }
 
 // ---- logits processors (LogitsProcs, kernels.h) ----------------------------------------------------------------------
-// The CTA of `row` reads the row's decoder input d (cur_len = P_b + t <= 64 ids, P_b = the prefix length of the row's image) into
-// shared memory once, marks the positions whose id
-// the n-gram rule bans, and every thread then folds d into two masks over its own slots: `pen` = slots whose id occurs in d (a bit
-// mask, so an id that repeats is penalised once), `ban` = slots set to -inf (n-gram rule; [SEP] while cur_len < min_length).
+// procs_read: the CTA of `row` reads the row's decoder input d (cur_len = pp.d.len(row, pp.step) <= 64 ids) into shared memory once
+// and clears s_bw.  The kernels call it first, while few registers are live (reading d next to the row's logits makes ptxas spill).
+// procs_masks, later, marks the positions whose id the n-gram rule bans, and every thread then folds d into two masks over its own
+// slots: `pen` = slots whose id occurs in d (a bit mask, so an id that repeats is penalised once), `ban` = slots set to -inf (n-gram
+// rule; [SEP] while cur_len < min_length).
 // Bad words: the threads test the multi-id sequences whose banned id lies in [lo, hi) (the CTA's ids) against the tail of d and mark
 // the matches in s_bw (one bit per sequence); every thread then folds the matches and the one-id bitmap into `ban`.
 // owner(w) = the calling thread's slot of id w, or -1; slot_id(s) = the id of the calling thread's slot s, or -1 past the vocabulary.
-// Every thread of the CTA must call it (it synchronises).
+// Every thread of the CTA must call both (procs_masks synchronises).
 constexpr int kBwWords = kBadWordsMaxSeqs / 32;
+__device__ __forceinline__ void procs_read(const LogitsProcs& pp, int row, int32_t* s_d, uint32_t* s_bw) {
+  const int tid = threadIdx.x;
+  const int L = min(pp.d.len(row, pp.step), kProcMaxLen);
+  if (tid < L) s_d[tid] = pp.d.at(row, tid);
+  if (tid < kBwWords) s_bw[tid] = 0u;
+}
 template <class Owner, class SlotId>
-__device__ __forceinline__ void procs_masks(const LogitsProcs& pp, int row, int t, int32_t* s_d, uint8_t* s_ban, uint32_t* s_bw, int lo,
+__device__ __forceinline__ void procs_masks(const LogitsProcs& pp, int row, int32_t* s_d, uint8_t* s_ban, uint32_t* s_bw, int lo,
                                             int hi, Owner owner, SlotId slot_id, uint32_t& pen, uint32_t& ban) {
   const int tid = threadIdx.x;
-  const int img = row / pp.rows_per_image;
-  const int Pb = pp.p0s ? pp.p0s[img] + 1 : pp.P;
-  const int L = min(Pb + t, kProcMaxLen);
-  if (tid < L) {
-    int32_t w;
-    if (pp.keys) w = pp.keys[(int64_t)row * pp.key_stride + (pp.P - Pb) + tid];   // the key row holds the prefix right-aligned
-    else if (tid < Pb) {
-      w = pp.prefix ? (int32_t)pp.prefix[(int64_t)img * pp.P + tid] : 101;
-      if (w == 102) w = 0;                                 // the decoder input holds [PAD] where the prefix has [SEP]
-    } else w = pp.tokens[(int64_t)row * pp.tok_stride + tid - Pb];
-    s_d[tid] = w;
-  }
-  if (tid < kBwWords) s_bw[tid] = 0u;
+  const int L = min(pp.d.len(row, pp.step), kProcMaxLen);
   __syncthreads();
   const int n = pp.no_repeat_ngram;
   if (tid < L) {
@@ -122,6 +117,7 @@ row_select_kernel(int V, const float* __restrict__ logits, int64_t ldl, int mode
   pdl_wait();
   pdl_launch_dependents();
   const int row = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  if (kProcs) procs_read(procs, row, s_in, s_bw);
   const float* __restrict__ x = logits + (int64_t)row * ldl;
   float v[kSlots];
 #pragma unroll
@@ -165,7 +161,7 @@ row_select_kernel(int V, const float* __restrict__ logits, int64_t ldl, int mode
   }
   if (kProcs) {
     uint32_t pen, ban;
-    procs_masks(procs, row, procs.step >= 0 ? procs.step : *procs.d_step, s_in, s_ban, s_bw, 0, V,
+    procs_masks(procs, row, s_in, s_ban, s_bw, 0, V,
                 [&](int w) { return (w >= 0 && w < kSelThreads * kSlots && (w % kSelThreads) == tid) ? w / kSelThreads : -1; },
                 [&](int s) { const int w = tid + s * kSelThreads; return w < V ? w : -1; }, pen, ban);
     procs_apply(v, procs.repetition_penalty, pen, ban);
@@ -310,6 +306,7 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
   pdl_launch_dependents();
   const int chunk = (int)cluster.block_rank();
   const int row = blockIdx.x / kRsChunks, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  if (kProcs) procs_read(procs, row, s_in, s_bw);
   const int base = chunk * kRsSpan;
   const float* __restrict__ x = logits + (int64_t)row * ldl;
   float v[kRsSlots];
@@ -400,7 +397,7 @@ row_select_cluster_kernel(int V, const float* __restrict__ logits, int64_t ldl, 
   // logits processors on fp32(x - logZ) (beam modes, before the beam score, as HF beam_search) or fp32(x / temperature) (sampling)
   if (kProcs) {
     uint32_t pen, ban;
-    procs_masks(procs, row, procs.step >= 0 ? procs.step : *procs.d_step, s_in, s_ban, s_bw, base, base + kRsSpan,
+    procs_masks(procs, row, s_in, s_ban, s_bw, base, base + kRsSpan,
                 [&](int w) { const int o = w - base; return (o >= 0 && o < kRsSpan && (o % kRsThreads) == tid) ? o / kRsThreads : -1; },
                 [&](int s) { const int w = base + tid + s * kRsThreads; return w < V ? w : -1; }, pen, ban);
     procs_apply(v, procs.repetition_penalty, pen, ban);
@@ -646,14 +643,14 @@ __device__ __forceinline__ bool beam_process(const BeamBuffers& bb, int b, int K
 constexpr int kBeamWarps = 4;
 // Register budget of the two beam-step kernels: 65536 / (7 * 128 threads) = 72 registers per thread.  Left to its default, ptxas
 // keeps them near 48 - 64 registers and spills the values that stay live across the calls into the fp64 / fp32 division subroutines
-// of the hypothesis walk (20 bytes in each kernel); with this budget neither spills (-Xptxas -v: beam_step_kernel 69 registers,
+// of the hypothesis walk (20 bytes in each kernel); with this budget neither spills (-Xptxas -v: beam_step_kernel 68 registers,
 // beam_sample_step_kernel 70).  The budget still lets 7 blocks share an SM; the grids have B / 4 and B * N / 4 blocks.
 constexpr int kBeamMinBlocks = 7;
 __global__ void __launch_bounds__(kBeamWarps * 32, kBeamMinBlocks)
 beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, const float* __restrict__ sel_val,
                  const int32_t* __restrict__ sel_idx, const float* __restrict__ logits, int64_t ldl, const float* __restrict__ logz,
-                 float penalty, float rep_penalty, const int64_t* __restrict__ prefix, int eos, int len0, const int* __restrict__ p0s,
-                 const LenPenalty lp, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores) {
+                 float penalty, float rep_penalty, const DecInput d, int eos, const LenPenalty lp, int32_t* out_beam_idx,
+                 int32_t* out_tokens, float* out_scores) {
   __shared__ float s_val[kBeamWarps][128];
   __shared__ int s_flat[kBeamWarps][128];
   __shared__ int s_order[kBeamWarps][16];
@@ -665,8 +662,7 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, co
   const int b = blockIdx.x * kBeamWarps + warp;
   if (b >= B) return;
   const int t = *bb.d_step;
-  const int len_b = p0s ? p0s[b] + 1 : len0;   // the image's decoder prefix length (len0 = the prefix row stride)
-  const int cur_len = t + len_b;               // HF input_ids.shape[-1]: decoder prefix (len_b tokens) + t generated
+  const int cur_len = d.len(b * K, t);         // HF input_ids.shape[-1]: the image's decoder prefix + t generated
   const int32_t* src = bb.tokens + (int64_t)(t & 1) * B * K * T + (int64_t)b * K * T;
   int32_t* dst = bb.tokens + (int64_t)((t + 1) & 1) * B * K * T + (int64_t)b * K * T;
   const int gs = K / G;
@@ -691,11 +687,7 @@ beam_step_kernel(BeamBuffers bb, int B, int K, int G, int T, int V, int nsel, co
           if (rep_penalty != 1.f) {
             // HF order: the Hamming term, then the repetition penalty when w occurs in the beam's decoder input
             bool seen = false;
-            for (int j = 0; j < len_b && !seen; ++j) {
-              const int32_t pj = prefix ? (int32_t)prefix[(int64_t)b * len0 + j] : 101;
-              seen = (pj == 102 ? 0 : pj) == w;
-            }
-            for (int j = 0; j < t && !seen; ++j) seen = src[beam * T + j] == w;
+            for (int j = 0; j < cur_len && !seen; ++j) seen = d.at((int)row, j) == w;
             if (seen) s = s < 0.f ? __fmul_rn(s, rep_penalty) : __fdiv_rn(s, rep_penalty);
           }
           v = __fadd_rn(s, bb.beam_scores[row]);
@@ -768,70 +760,26 @@ __global__ void beam_finalize_kernel(BeamBuffers bb, int B, int K, int T, int eo
 // ------------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ bool is_special(int64_t t) { return t == 0 || (t >= 100 && t <= 103); }
 
-__global__ void __launch_bounds__(256)
-ngram_ban_kernel(int N, int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __restrict__ hist_seg,
-                 const int32_t* __restrict__ prefix, int prefix_stride, const int* __restrict__ d_step, int len0, int n,
-                 int32_t* __restrict__ ban_tokens, int32_t* __restrict__ ban_count, int ban_stride) {
-  __shared__ int cnt;
-  pdl_wait();
-  pdl_launch_dependents();
-  const int row = blockIdx.x;
-  if (threadIdx.x == 0) cnt = 0;
-  __syncthreads();
-  // decoder prefix (len0 tokens) + generated.  A shorter prefix sits right-aligned in its key row (launch_sample_init) behind zeros:
-  // a key that reaches into them holds [PAD], which no history n-gram holds, and bans nothing, as the shorter key would.
-  const int cur_len = *d_step + len0;
-  const int start = cur_len + 1 - n;
-  if (start >= 0) {                                      // a shorter key can never equal an (n-1)-gram
-    const int64_t* ids = hist_ids + (int64_t)(row / N) * Lh;   // the history of the row's image
-    const int64_t* seg = hist_seg + (int64_t)(row / N) * Lh;
-    const int32_t* key = prefix + (int64_t)row * prefix_stride + start;
-    for (int p = threadIdx.x; p + n <= Lh; p += blockDim.x) {
-      bool ok = true;
-      for (int j = 0; j < n && ok; ++j) {
-        const int64_t tk = (seg[p + j] == 0) ? ids[p + j] : 0;   // question history = ids * (segments == 0)
-        if (is_special(tk)) ok = false;
-        else if (j < n - 1 && tk != (int64_t)key[j]) ok = false;
-      }
-      if (ok) {
-        const int slot = atomicAdd(&cnt, 1);
-        if (slot < ban_stride) ban_tokens[(int64_t)row * ban_stride + slot] = (int32_t)ids[p + n - 1];
-      }
-    }
-  }
-  __syncthreads();
-  if (threadIdx.x == 0) ban_count[row] = cnt < ban_stride ? cnt : ban_stride;
-}
-
-// Beam mode: one CTA per image scans its question history once and tests every n-gram against the K beam keys.  The key of beam
-// k at step t is the last n-1 tokens of prefix_b + tokens[b, k, :t], with prefix_b the image's decoder prefix ([SEP] read as
-// [PAD]; [CLS] when prefix is null, P = 1).  The host launches this only when P + t >= n-1 (a shorter key bans nothing) and, for
-// the [CLS] start, only once the key has left it (n-grams with a special id are never banned).  Ban lists are per beam row b*K + k.
+// One CTA per image scans its question history once and tests every n-gram against the keys of the image's rows: the key of row r
+// at step t is the last n-1 ids of its decoder input d (DecInput).  A key longer than the decoder input bans nothing, as a key that
+// holds a special id does (the [CLS] start): n-grams with a special id are never banned.  Ban lists are per row.
 constexpr int kBanMaxK = 8;
 __global__ void __launch_bounds__(256)
-beam_ngram_ban_kernel(int K, int T, int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __restrict__ hist_seg,
-                      const int64_t* __restrict__ prefix, int P, const int* __restrict__ p0s, const int32_t* __restrict__ tokens, int step,
+beam_ngram_ban_kernel(int Lh, const int64_t* __restrict__ hist_ids, const int64_t* __restrict__ hist_seg, const DecInput d, int step,
                       int n, int32_t* __restrict__ ban_tokens, int32_t* __restrict__ ban_count, int ban_stride) {
-  __shared__ int32_t s_key[kBanMaxK][kHypMaxT];
+  __shared__ int32_t s_key[kBanMaxK][kProcMaxLen];
   __shared__ int s_cnt[kBanMaxK];
   pdl_wait();
   pdl_launch_dependents();
-  const int b = blockIdx.x, klen = n - 1;
-  const int Pb = p0s ? p0s[b] + 1 : P;                   // the image's prefix length (P = the row stride)
-  const int first = Pb + step - klen;                    // first key position in prefix + generated tokens
+  const int b = blockIdx.x, K = d.rows_per_image, klen = n - 1;
+  const int first = d.len(b * K, step) - klen;           // first key position in the decoder input
   if (first < 0) {                                       // a decoder input shorter than n - 1 bans nothing
     if (threadIdx.x < K) ban_count[b * K + threadIdx.x] = 0;
     return;
   }
   for (int i = threadIdx.x; i < K * klen; i += blockDim.x) {
-    const int k = i / klen, j = i - k * klen, q = first + j;
-    int32_t w;
-    if (q >= Pb) w = tokens[((int64_t)b * K + k) * T + q - Pb];
-    else {
-      w = prefix ? (int32_t)prefix[(int64_t)b * P + q] : 101;
-      if (w == 102) w = 0;                               // the decoder input holds [PAD] where the prefix has [SEP]
-    }
-    s_key[k][j] = w;
+    const int k = i / klen, j = i - k * klen;
+    s_key[k][j] = d.at(b * K + k, first + j);
   }
   if (threadIdx.x < K) s_cnt[threadIdx.x] = 0;
   __syncthreads();
@@ -977,10 +925,10 @@ beam_sample_step_kernel(BeamBuffers bb, int S, int N, int K, int T, int V, const
   }
 }
 
-// dec_prefix != null: int64 [rows / N, P] decoder prefix of the row's image, Pb = prefix_len tokens; the n-gram key buffer `prefix`
-// holds it right-aligned in columns P - Pb .. P - 1 ([SEP] read as [PAD], zeros before it).  p0s != null: receives Pb - 1 per image.
-__global__ void sample_init_kernel(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                                   int prefix_stride, int* d_step, const int64_t* __restrict__ dec_prefix, int P, int* __restrict__ p0s) {
+// dec_prefix != null: int64 [rows / N, P] decoder prefix of the row's image, Pb = prefix_len tokens.  p0s != null: receives Pb - 1
+// per image.
+__global__ void sample_init_kernel(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int* d_step,
+                                   const int64_t* __restrict__ dec_prefix, int P, int* __restrict__ p0s) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i == 0) *d_step = 0;
   if (i < rows) {
@@ -991,17 +939,12 @@ __global__ void sample_init_kernel(int rows, int N, int T, int start_token, int3
     const int32_t w0 = row ? (int32_t)row[Pb - 1] : start_token;
     cur_tokens[i] = w0 < 0 ? 0 : w0;                     // an invalid row's negative start is embedded as [PAD]
     for (int j = 0; j < T; ++j) seq[(int64_t)i * T + j] = 0;
-    for (int j = 0; j < prefix_stride; ++j) prefix[(int64_t)i * prefix_stride + j] = 0;
-    for (int j = 0; j < Pb; ++j) {
-      const int32_t w = row ? (int32_t)row[j] : start_token;
-      prefix[(int64_t)i * prefix_stride + P - Pb + j] = (w == 102 || w < 0) ? 0 : w;
-    }
   }
 }
 
 __global__ void sample_step_kernel(int rows, int N, int T, int nsel, const float* __restrict__ sel_val, const int32_t* __restrict__ sel_idx,
                                    int top_k, float top_p, uint64_t seed, uint64_t row_offset, const uint64_t* __restrict__ d_seed,
-                                   const int* __restrict__ d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens) {
+                                   const int* __restrict__ d_step, int32_t* seq, int32_t* cur_tokens, int32_t* out_tokens) {
   pdl_wait();
   pdl_launch_dependents();
   const int row = blockIdx.x * blockDim.x + threadIdx.x;
@@ -1043,7 +986,6 @@ __global__ void sample_step_kernel(int rows, int N, int T, int nsel, const float
   const int tok = ix[choice];
   if (step < T) seq[(int64_t)row * T + step] = tok;
   cur_tokens[row] = tok;
-  if (step + 1 < prefix_stride) prefix[(int64_t)row * prefix_stride + step + 1] = (tok == eos) ? 0 : tok;
   if (out_tokens) out_tokens[row] = tok;
 }
 
@@ -1076,9 +1018,8 @@ template <bool kProcs>  // kProcs: the logits processors are on (a separate inst
 __global__ void __launch_bounds__(kFvThreads)
 full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t ldl, float temperature, float top_p,
                          const int32_t* __restrict__ ban_tokens, const int32_t* __restrict__ ban_count, int ban_stride,
-                         int T, uint64_t seed, uint64_t row_offset, const uint64_t* __restrict__ d_seed, const int* __restrict__ d_step, int eos,
-                         int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens,
-                         const LogitsProcs procs) {
+                         int T, uint64_t seed, uint64_t row_offset, const uint64_t* __restrict__ d_seed, const int* __restrict__ d_step,
+                         int32_t* seq, int32_t* cur_tokens, int32_t* out_tokens, const LogitsProcs procs) {
   extern __shared__ float s_p[];                   // [kFvPer][kFvThreads]: p of token 32 t + j at s_p[j * 1024 + t] (conflict free)
   __shared__ float s_red[32];
   __shared__ float s_scan[32];
@@ -1089,7 +1030,7 @@ full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t
   pdl_wait();
   pdl_launch_dependents();
   const int row = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int step = *d_step;
+  if (kProcs) procs_read(procs, row, s_in, s_bw);
   const float* x = logits + (int64_t)row * ldl;
   const int base = tid * kFvPer;
   float v[kFvPer];
@@ -1097,7 +1038,7 @@ full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t
   for (int j = 0; j < kFvPer; ++j) v[j] = (base + j < V) ? __fdiv_rn(x[base + j], temperature) : -INFINITY;
   if (kProcs) {
     uint32_t pen, ban;
-    procs_masks(procs, row, step, s_in, s_ban, s_bw, 0, V, [&](int w) { return (w >= base && w < base + kFvPer) ? w - base : -1; },
+    procs_masks(procs, row, s_in, s_ban, s_bw, 0, V, [&](int w) { return (w >= base && w < base + kFvPer) ? w - base : -1; },
                 [&](int s) { return base + s < V ? base + s : -1; }, pen, ban);
     procs_apply(v, procs.repetition_penalty, pen, ban);
   }
@@ -1152,6 +1093,7 @@ full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t
     }
   }
   // draw: first token (in index order) whose inclusive prefix sum exceeds u * total
+  const int step = *d_step;
   const uint64_t sd = candidate_seed(d_seed ? d_seed[0] : seed, row % N);
   const uint64_t grow = (uint64_t)(row / N) + (d_seed ? d_seed[1] : row_offset);
   const uint64_t h = splitmix64(sd ^ splitmix64((grow << 20) ^ (uint64_t)step));
@@ -1189,7 +1131,6 @@ full_vocab_sample_kernel(int N, int V, const float* __restrict__ logits, int64_t
     const int tok = s_choice < 0 ? 0 : s_choice;
     if (step < T) seq[(int64_t)row * T + step] = tok;
     cur_tokens[row] = tok;
-    if (step + 1 < prefix_stride) prefix[(int64_t)row * prefix_stride + step + 1] = (tok == eos) ? 0 : tok;
     if (out_tokens) out_tokens[row] = tok;
   }
 }
@@ -1274,20 +1215,17 @@ __global__ void splice_kernel(int B, int Lt, int Lu, int64_t* ids, int64_t* seg,
     for (int j = 0; j < Lt; ++j) mask[(int64_t)b * Lt + j] = row[j] != 0 ? 1.f : 0.f;
 }
 
-__global__ void build_prefix_kernel(int rows, int len, const int64_t* __restrict__ prefix_ids, int32_t* prefix, int prefix_stride, int eos) {
-  const int i = blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= rows * len) return;
-  const int r = i / len, j = i % len;
-  const int64_t tk = prefix_ids[i];
-  prefix[(int64_t)r * prefix_stride + j] = (tk == eos) ? 0 : (int32_t)tk;
+void check_dec_input(const DecInput& d, int step, const char* who) {
+  if (d.P < 1 || (d.P > 1 && !d.prefix) || d.rows_per_image < 1 || step < 0 || d.P + step > kProcMaxLen || (step > 0 && !d.tokens))
+    throw std::runtime_error(std::string(who) + ": the rows' decoder input needs 1 <= P <= P + step <= 64, the prefix when P > 1 and "
+                             "the tokens when step > 0");
 }
 
 void check_procs(const LogitsProcs& p, const char* who) {
   if (!p.active()) return;
   if (!(p.repetition_penalty > 0.f) || !std::isfinite(p.repetition_penalty) || p.no_repeat_ngram < 0 || p.min_length < 0)
     throw std::runtime_error(std::string(who) + ": logits processor parameters out of range");
-  if (p.P < 1 || (!p.keys && !p.tokens) || (p.step < 0 && !p.d_step))
-    throw std::runtime_error(std::string(who) + ": the logits processors need the rows' decoder input and step");
+  check_dec_input(p.d, p.step, who);
   if (p.bw_count < 0 || p.bw_count > kBadWordsMaxSeqs || (p.bw_count > 0 && !p.bw_seq))
     throw std::runtime_error(std::string(who) + ": bad-word sequences out of range");
 }
@@ -1341,17 +1279,17 @@ int launch_beam_sample_step(const BeamBuffers& bb, int S, int N, int K, int T, i
 }
 int launch_beam_step(const BeamBuffers& bb, int B, int K, int G, int T, int V, int nsel, const float* sel_val,
                      const int32_t* sel_idx, const float* logits, int64_t ldl, const float* logz, float penalty, float rep_penalty,
-                     const int64_t* prefix, int eos, int len0, const int* p0s, const LenPenalty& lp, int32_t* out_beam_idx,
-                     int32_t* out_tokens, float* out_scores, cudaStream_t stream) {
+                     const DecInput& d, int eos, const LenPenalty& lp, int32_t* out_beam_idx, int32_t* out_tokens, float* out_scores,
+                     cudaStream_t stream) {
   if (K > 8 || T > kHypMaxT) throw std::runtime_error("beam_step: K <= 8 and T <= 32");
-  if (len0 - 1 + T > kMaxHypLen - 1) throw std::runtime_error("beam_step: prefix + new tokens exceed the length table");
+  if (d.P - 1 + T > kMaxHypLen - 1) throw std::runtime_error("beam_step: prefix + new tokens exceed the length table");
   if (G < 1 || K % G != 0) throw std::runtime_error("beam_step: the beam groups must divide the beams");
   if (G > 1 && (!logits || !logz || nsel < K + K / G))
     throw std::runtime_error("beam_step: beam groups need the logits, logZ and nsel >= K + K / G per-row candidates");
-  if (!(rep_penalty > 0.f) || !std::isfinite(rep_penalty) || (len0 > 1 && !prefix))
-    throw std::runtime_error("beam_step: repetition penalty must be finite and > 0, prefix given when len0 > 1");
+  if (!(rep_penalty > 0.f) || !std::isfinite(rep_penalty) || (d.P > 1 && !d.prefix))
+    throw std::runtime_error("beam_step: repetition penalty must be finite and > 0, prefix given when P > 1");
   launch_k(beam_step_kernel, dim3((B + kBeamWarps - 1) / kBeamWarps), dim3(kBeamWarps * 32), 0, stream, bb, B, K, G, T, V, nsel, sel_val, sel_idx,
-           logits, ldl, logz, penalty, rep_penalty, prefix, eos, len0, p0s, lp, out_beam_idx, out_tokens, out_scores);
+           logits, ldl, logz, penalty, rep_penalty, d, eos, lp, out_beam_idx, out_tokens, out_scores);
   return 1;
 }
 int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, int len0, const int* p0s, int per_image, int N,
@@ -1362,37 +1300,27 @@ int launch_beam_finalize(const BeamBuffers& bb, int B, int K, int T, int eos, in
   beam_finalize_kernel<<<(B + 31) / 32, 32, 0, stream>>>(bb, B, K, T, eos, len0, p0s, per_image, N, lp, out_ids, out_scores);
   return 1;
 }
-int launch_ngram_ban(int rows, int N, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int32_t* prefix,
-                     int prefix_stride, const int* d_step, int len0, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
-                     cudaStream_t stream) {
-  if (rows <= 0) return 0;
-  if (N < 1 || rows % N != 0) throw std::runtime_error("ngram_ban: rows must be a multiple of N >= 1");
-  launch_k(ngram_ban_kernel, dim3(rows), dim3(256), 0, stream, N, Lh, hist_ids, hist_seg, prefix, prefix_stride, d_step, len0, n, ban_tokens, ban_count, ban_stride);
-  return 1;
-}
-int launch_beam_ngram_ban(int B, int K, int T, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const int64_t* prefix, int P,
-                          const int* p0s, const int32_t* tokens, int step, int n, int32_t* ban_tokens, int32_t* ban_count, int ban_stride,
-                          cudaStream_t stream) {
+int launch_beam_ngram_ban(int B, int Lh, const int64_t* hist_ids, const int64_t* hist_seg, const DecInput& d, int step, int n,
+                          int32_t* ban_tokens, int32_t* ban_count, int ban_stride, cudaStream_t stream) {
   if (B <= 0) return 0;
-  if (K > kBanMaxK || n < 1 || n - 1 > P + step || n - 1 > kHypMaxT || step >= T || T > kHypMaxT || P < 1 || (P > 1 && !prefix))
-    throw std::runtime_error("beam_ngram_ban: K <= 8, 1 <= n <= min(P + step, 32) + 1, step < T <= 32, prefix given when P > 1");
-  launch_k(beam_ngram_ban_kernel, dim3(B), dim3(256), 0, stream, K, T, Lh, hist_ids, hist_seg, prefix, P, p0s, tokens, step, n, ban_tokens, ban_count,
-           ban_stride);
+  if (d.rows_per_image > kBanMaxK || n < 1) throw std::runtime_error("beam_ngram_ban: at most 8 rows per image, n >= 1");
+  check_dec_input(d, step, "beam_ngram_ban");
+  launch_k(beam_ngram_ban_kernel, dim3(B), dim3(256), 0, stream, Lh, hist_ids, hist_seg, d, step, n, ban_tokens, ban_count, ban_stride);
   return 1;
 }
 int launch_sample_step(int rows, int N, int T, int nsel, const float* sel_val, const int32_t* sel_idx, int top_k, float top_p,
-                       uint64_t seed, uint64_t row_offset, const uint64_t* d_seed, const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                       int prefix_stride, int32_t* out_tokens, cudaStream_t stream) {
+                       uint64_t seed, uint64_t row_offset, const uint64_t* d_seed, const int* d_step, int32_t* seq, int32_t* cur_tokens,
+                       int32_t* out_tokens, cudaStream_t stream) {
   if (top_k < 1 || top_k > nsel) throw std::runtime_error("sample_step: top_k out of range");
   if (N < 1 || rows % N != 0) throw std::runtime_error("sample_step: rows must be a multiple of N >= 1");
-  launch_k(sample_step_kernel, dim3((rows + 63) / 64), dim3(64), 0, stream, rows, N, T, nsel, sel_val, sel_idx, top_k, top_p, seed, row_offset, d_seed, d_step, eos, seq,
-                                                          cur_tokens, prefix, prefix_stride, out_tokens);
+  launch_k(sample_step_kernel, dim3((rows + 63) / 64), dim3(64), 0, stream, rows, N, T, nsel, sel_val, sel_idx, top_k, top_p, seed, row_offset, d_seed, d_step, seq,
+                                                          cur_tokens, out_tokens);
   return 1;
 }
 int launch_full_vocab_sample(int rows, int N, int V, const float* logits, int64_t ldl, float temperature, float top_p, const int32_t* ban_tokens,
                              const int32_t* ban_count, int ban_stride, int T, uint64_t seed, uint64_t row_offset, const uint64_t* d_seed,
-                             const int* d_step, int eos, int32_t* seq, int32_t* cur_tokens, int32_t* prefix, int prefix_stride, int32_t* out_tokens,
-                             const LogitsProcs& procs, cudaStream_t stream) {
+                             const int* d_step, int32_t* seq, int32_t* cur_tokens, int32_t* out_tokens, const LogitsProcs& procs,
+                             cudaStream_t stream) {
   if (rows <= 0) return 0;
   if (N < 1 || rows % N != 0) throw std::runtime_error("full_vocab_sample: rows must be a multiple of N >= 1");
   if (V > kFvThreads * kFvPer) throw std::runtime_error("full_vocab_sample: vocab > 32768");
@@ -1407,15 +1335,15 @@ int launch_full_vocab_sample(int rows, int N, int V, const float* logits, int64_
     attr_set = true;
   }
   launch_k(procs.active() ? full_vocab_sample_kernel<true> : full_vocab_sample_kernel<false>, dim3(rows), dim3(kFvThreads), smem, stream, N, V, logits, ldl, temperature, top_p, ban_tokens, ban_count, ban_stride,
-           T, seed, row_offset, d_seed, d_step, eos, seq, cur_tokens, prefix, prefix_stride, out_tokens, procs);
+           T, seed, row_offset, d_seed, d_step, seq, cur_tokens, out_tokens, procs);
   return 1;
 }
-int launch_sample_init(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int32_t* prefix,
-                       int prefix_stride, int* d_step, const int64_t* dec_prefix, int P, int* p0s, cudaStream_t stream) {
-  if (P < 1 || P > prefix_stride || (P > 1 && !dec_prefix)) throw std::runtime_error("sample_init: 1 <= P <= prefix_stride, prefix given when P > 1");
+int launch_sample_init(int rows, int N, int T, int start_token, int32_t* seq, int32_t* cur_tokens, int* d_step, const int64_t* dec_prefix,
+                       int P, int* p0s, cudaStream_t stream) {
+  if (P < 1 || (P > 1 && !dec_prefix)) throw std::runtime_error("sample_init: P >= 1, prefix given when P > 1");
   if (N < 1 || rows % N != 0) throw std::runtime_error("sample_init: rows must be a multiple of N >= 1");
   if (p0s && !dec_prefix) throw std::runtime_error("sample_init: per-image prefix lengths need a prefix");
-  sample_init_kernel<<<(rows + 63) / 64, 64, 0, stream>>>(rows, N, T, start_token, seq, cur_tokens, prefix, prefix_stride, d_step, dec_prefix, P, p0s);
+  sample_init_kernel<<<(rows + 63) / 64, 64, 0, stream>>>(rows, N, T, start_token, seq, cur_tokens, d_step, dec_prefix, P, p0s);
   return 1;
 }
 int launch_sample_finalize(int rows, int T, int eos, const int32_t* seq, int64_t* out_ids, cudaStream_t stream) {
@@ -1442,13 +1370,6 @@ int launch_ce_loss(int rows, int V, const float* logits, int64_t ldl, const int6
 int launch_splice(int B, int Lt, int Lu, int64_t* ids, int64_t* seg, float* mask, int32_t* enc_len, const int64_t* utt,
                   int segment_value, int strip_sep, int32_t* abnormal, int sep, cudaStream_t stream) {
   splice_kernel<<<(B + 63) / 64, 64, 0, stream>>>(B, Lt, Lu, ids, seg, mask, enc_len, utt, segment_value, strip_sep, abnormal, sep);
-  return 1;
-}
-int launch_build_prefix_from_ids(int rows, int len, const int64_t* prefix_ids, int32_t* prefix, int prefix_stride, int eos,
-                                 cudaStream_t stream) {
-  const int n = rows * len;
-  if (n <= 0) return 0;
-  build_prefix_kernel<<<(n + 255) / 256, 256, 0, stream>>>(rows, len, prefix_ids, prefix, prefix_stride, eos);
   return 1;
 }
 

@@ -175,6 +175,22 @@ def test_tiny_fp32_ragged_beams_match_per_image_oracles(tiny_cfgs, tiny_engines,
 
 
 @pytest.mark.gpu
+def test_tiny_fp32_ragged_beams_with_a_35_id_key_match_per_image_oracles(tiny_cfgs, tiny_engines):
+    """n = 36: the 35-id key first fits the 25-token prefix's decoder input at step 10 and never fits the shorter ones; the call
+    decodes every step and equals the per-image oracles."""
+    from test_logits_processors import _run
+    enc_cfg, dec_cfg = tiny_cfgs
+    es, b, sd = tiny_engines
+    base, pre = tiny_prefix(enc_cfg)
+    kw = dict(num_beams=3)
+    ids, _ = _run(es["separate_calls"], b, "separate_calls", ngram_blocking_size=36, prefix=pre, **kw)
+    ids = ids.cpu().view(3, 1, -1)
+    for i, Pb in enumerate(TINY_LENS):
+        ref, _ = _oracle_image(sd, enc_cfg, dec_cfg, b, i, base[i:i + 1, :Pb], "beam", kw, 36, None)
+        assert torch.equal(ids[i], ref), f"image {i} (P_b={Pb}): {ids[i].tolist()} vs {ref.tolist()}"
+
+
+@pytest.mark.gpu
 def test_tiny_fp32_invalid_row_leaves_the_others_exact(tiny_cfgs, tiny_engines):
     """A row that starts with a negative id is invalid input with unspecified output; the call still completes and every other
     image decodes exactly as alone."""
